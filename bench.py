@@ -2,6 +2,7 @@
 """bench.py -- depth-evals/s of the statdepth hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload mbd|bd|perm]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload at every N (strong scaling: the total work is BASELINE's configuration, fixed):
@@ -58,7 +59,33 @@ def parse():
     ap.add_argument("--bd-impl", default="auto", choices=["auto", "bits", "gemm", "match"])
     ap.add_argument("--nq", type=int, default=None, help="bd workload: number of query curves (default all)")
     ap.add_argument("--ties", action="store_true", help="tie-stress variant: round the random walks to integers")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy "
+                         "(float64; inputs are seeded, so two builds can be compared output for output)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU arm's outputs; the reference arm times the CPU oracle on a sample")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Write each array as DIR/<name>.npy in float64 (integer counts below 2**53 are exact).  An array larger than its
+    share of DUMP_BYTES is replaced by a fixed, seeded sample of its elements; the sampled positions go to
+    DIR/<name>_index.npy, so that two dumps compare element for element."""
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_BYTES // (2 * len(arrays))  # room for a sample and its index
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64).ravel()
+        if a.nbytes > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share // 8, replace=False))
+            np.save(os.path.join(dirname, name + "_index.npy"), idx.astype(np.float64))
+            a = a[idx]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def workload_shape(args):
@@ -604,6 +631,8 @@ def main():
                    seed=1 if relax else 2)
     clocks = sampler.stop() if rank == 0 else None
     ms, ms_e2e, Tl, nq_local = r["ms"], r["ms_e2e"], r["Tl"], r["nq_local"]
+    # the counts of the device-resident call and the depths of the host-buffer call, all queries on every rank
+    outputs = {"counts": r["last"].cpu().numpy(), "depth": r["depth"]}
     impl_used = {k: v for k, v in eng.timings().items() if k in ("fallback_rows", "bd_impl_used")}
 
     # ---- sanity inside the bench: tie-free checksum of the relaxed numerators ----------------------
@@ -628,10 +657,11 @@ def main():
         if world > 1:
             dist.barrier()
         t0 = time.perf_counter()
-        k_api = 3
+        k_api = args.steps
         for _ in range(k_api):
             d_api = FunctionalDepth([df], relax=True)
         dt = (time.perf_counter() - t0) / k_api
+        outputs["depth_api"] = d_api.values
         t = torch.tensor([dt], dtype=torch.float64, device=c.dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -715,6 +745,8 @@ def main():
         if not args.no_reference_python:
             cb["reference_python"] = reference_python()
         line["cpu_baseline"] = cb
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -761,6 +793,8 @@ def main_perm(c: Ctx, args, n, T, name, config, sampler):
         cb = cpu_baseline(args, n, T)
         cb.pop("seconds_sample", None)
         line["cpu_baseline"] = cb
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"null": res["null"], "observed": [res["observed"]], "p_value": [res["p_value"]]})
     emit(line)
     if c.world > 1:
         dist.destroy_process_group()

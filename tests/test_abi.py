@@ -28,7 +28,10 @@ def test_library_exports_every_declared_symbol():
 def test_built_for_sm100a_only():
     import subprocess
     from statdepth_b200 import build
-    out = subprocess.run(["cuobjdump", "--list-elf", build.build()], capture_output=True, text=True).stdout
+    # the cuobjdump of the toolkit build.py compiles with: its bin directory need not be on PATH
+    bindir = os.path.dirname(build._nvcc())
+    cuobjdump = os.path.join(bindir, "cuobjdump") if bindir else "cuobjdump"
+    out = subprocess.run([cuobjdump, "--list-elf", build.build()], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 
