@@ -208,6 +208,44 @@ int sd_pointcloud_blocks_f64(sd_ctx *ctx, const double *P, int64_t n, int d, con
                              const double *hull_volume, double *out);
 
 /*
+ * Out-of-sample depth: the depth of NEW observations Y against a reference sample S.  The value for new
+ * observation g is what the in-sample entry point returns for g after g alone is appended to S (the reference:
+ * FunctionalDepth([pd.concat([S, g], axis=1)], to_compute=[g]) / PointcloudDepth(pd.concat([S, g]), ...)).
+ * Other new observations never take part in g's depth.  The host forms the depth with the population size
+ * nS + 1, e.g. relaxed band depth = sum_j count_j / T / C(nS + 1, j).
+ *
+ * Band depth, S [T, nS] and Y [T, nY] in SD_LAYOUT_TN (S[t*ldS + c], Y[t*ldY + g]), j = 2 or 3:
+ *   relax != 0 : count_out[g] = sum_t [C(nS,j) - C(b_t,j) - C(a_t,j)], b_t / a_t = #sample curves strictly
+ *                below / above Y[t, g].  O((nS + nY) T): two exact rank passes (pooled [S | Y], and Y alone),
+ *                b_t = below among the pool - below among Y.
+ *   relax == 0 : count_out[g] = #{j-subsets of the nS sample curves whose band contains curve g at all T
+ *                points}.  Always the bit-mask kernels (SD_BD_BITS): the sign-vector matcher and the Gram
+ *                route are not used here, so tie-heavy strict data costs what the bit kernel costs.
+ * SD_ERR_OVERFLOW when T * C(nS, j) exceeds int64.
+ */
+int sd_band_depth_oos_f64(sd_ctx *ctx, const double *S, int64_t T, int64_t nS, int64_t ldS,
+                          const double *Y, int64_t nY, int64_t ldY, int j, int relax,
+                          int64_t *count_out);
+
+/* same with DEVICE pointers (count_out too).  When Y is the continuation of S in one matrix
+ * (dY == dS + nS, ldY == ldS) the data is used in place; otherwise it is first pooled on the device. */
+int sd_band_depth_oos_f64_dev(sd_ctx *ctx, const double *dS, int64_t T, int64_t nS, int64_t ldS,
+                              const double *dY, int64_t nY, int64_t ldY, int j, int relax,
+                              int64_t *d_count_out);
+
+/* Point clouds S[i*d + c] (nS points) and Y[g*d + c] (nY points), d in 1..3:
+ * count_out[g] = #{(d+1)-subsets of S whose closed simplex contains Y[g]} with the tolerance band `tol` of
+ * sd_pointcloud_simplicial_f64 (enumerated, or counted for d = 2 when nS + 1 > 64, as there).
+ * The host divides by C(nS + 1, d + 1). */
+int sd_pointcloud_simplicial_oos_f64(sd_ctx *ctx, const double *S, int64_t nS, int d,
+                                     const double *Y, int64_t nY, double tol, int64_t *count_out);
+
+/* depth_out[g] = 1 - ||sum_{s in S} (s - y)/||s - y|| || / (nS + 1), d in 1..16 (NaN when y equals a
+ * sample point, as in the reference). */
+int sd_pointcloud_l1_oos_f64(sd_ctx *ctx, const double *S, int64_t nS, int d, const double *Y,
+                             int64_t nY, double *depth_out);
+
+/*
  * Batched band depth over sub-populations of one matrix (K-sampled blocks, homogeneity
  * permutations): membership[b*n + c] != 0 selects the curves of batch b; queries[b*nqb + i] is
  * the i-th query curve of batch b (must be a member).  count_out[b*nqb + i] as in

@@ -78,6 +78,14 @@ SIGNATURES = {
                                         C.c_void_p, C.c_int64, C.c_double, C.c_void_p]),
     "sd_pointcloud_blocks_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p,
                                            C.c_void_p, C.c_int64, C.c_int, C.c_double, C.c_void_p, C.c_void_p]),
+    "sd_band_depth_oos_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
+                                        C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
+    "sd_band_depth_oos_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
+                                            C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
+    "sd_pointcloud_simplicial_oos_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p,
+                                                   C.c_int64, C.c_double, C.c_void_p]),
+    "sd_pointcloud_l1_oos_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int64,
+                                           C.c_void_p]),
     "sd_band_depth_batched_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                             C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -262,6 +270,61 @@ class Engine:
         out = np.empty((B, nqb), dtype=np.int64)
         self._check(self.lib.sd_band_depth_batched_f64(self._ctx, _ptr(X), T, n, n, _ptr(mem), B, _ptr(qs), nqb,
                                                        int(j), int(bool(relax)), _ptr(out)))
+        return out
+
+    # -- out-of-sample depth ----------------------------------------------------------------------------
+    @staticmethod
+    def _rows(A):
+        """float64 [rows, cols] with unit column stride (a column slice of a C-order matrix stays a view) and its
+        leading dimension in elements."""
+        A = np.asarray(A, dtype=np.float64)
+        if A.ndim != 2:
+            raise ValueError("expected a 2-D array")
+        if A.shape[1] > 0 and not (A.strides[1] == 8 and A.strides[0] % 8 == 0 and A.strides[0] >= 8 * A.shape[1]):
+            A = np.ascontiguousarray(A)
+        return A, (A.strides[0] // 8 if A.shape[0] > 1 else max(A.shape[1], 1))
+
+    def band_depth_oos_counts(self, S, Y, j=2, relax=False):
+        """Numerators of the new curves Y [T, nY] against the sample S [T, nS] (each new curve alone appended)."""
+        S, ldS = self._rows(S)
+        Y, ldY = self._rows(Y)
+        T, nS = S.shape
+        if Y.shape[0] != T:
+            raise ValueError("S and Y must have the same number of rows (time points)")
+        nY = Y.shape[1]
+        out = np.empty(nY, dtype=np.int64)
+        if nY == 0:
+            return out
+        self._check(self.lib.sd_band_depth_oos_f64(self._ctx, C.c_void_p(S.ctypes.data), T, nS, ldS,
+                                                   C.c_void_p(Y.ctypes.data), nY, ldY, int(j), int(bool(relax)),
+                                                   _ptr(out)))
+        return out
+
+    def band_depth_oos_counts_dev(self, dS_ptr, T, nS, ldS, dY_ptr, nY, ldY, d_out_ptr, j=2, relax=False):
+        """Device-pointer variant: no host copies; int64 counts [nY] stay on the device."""
+        self._check(self.lib.sd_band_depth_oos_f64_dev(self._ctx, C.c_void_p(int(dS_ptr)), int(T), int(nS), int(ldS),
+                                                       C.c_void_p(int(dY_ptr)), int(nY), int(ldY), int(j),
+                                                       int(bool(relax)), C.c_void_p(int(d_out_ptr))))
+
+    def simplicial_oos_counts(self, S, Y, tol=1e-7):
+        S = np.ascontiguousarray(S, dtype=np.float64)
+        Y = np.ascontiguousarray(Y, dtype=np.float64)
+        nS, d = S.shape
+        out = np.empty(Y.shape[0], dtype=np.int64)
+        if Y.shape[0] == 0:
+            return out
+        self._check(self.lib.sd_pointcloud_simplicial_oos_f64(self._ctx, _ptr(S), nS, d, _ptr(Y), Y.shape[0],
+                                                              float(tol), _ptr(out)))
+        return out
+
+    def l1_oos_depth(self, S, Y):
+        S = np.ascontiguousarray(S, dtype=np.float64)
+        Y = np.ascontiguousarray(Y, dtype=np.float64)
+        nS, d = S.shape
+        out = np.empty(Y.shape[0], dtype=np.float64)
+        if Y.shape[0] == 0:
+            return out
+        self._check(self.lib.sd_pointcloud_l1_oos_f64(self._ctx, _ptr(S), nS, d, _ptr(Y), Y.shape[0], _ptr(out)))
         return out
 
     # -- multivariate / point clouds -----------------------------------------------------------------

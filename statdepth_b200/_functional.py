@@ -18,7 +18,7 @@ from . import _dist, settings
 from ._engine import get_engine
 from ._helper import DepthDegeneracy, _check_containment, _handle_depth_errors
 
-__all__ = ['_functionaldepth', '_samplefunctionaldepth']
+__all__ = ['_functionaldepth', '_samplefunctionaldepth', '_functionaldepth_of']
 
 
 def _positions(labels, axis_index: pd.Index, what: str) -> np.ndarray:
@@ -133,6 +133,66 @@ def _functionaldepth(
     queries = np.asarray([int(i) for i in f], dtype=np.int64)
     depths = _multivariate_depths(data, queries, relax)
     return pd.Series(index=f, data=depths)
+
+
+def _univariate_depths_of(S: np.ndarray, Y: np.ndarray, J: int, relax: bool) -> np.ndarray:
+    """Depth of every new curve (column of Y [T, nY]) inside S [T, nS] u {that curve}: the arithmetic of
+    _univariate_depths with n = nS + 1, so the result is bit-identical to the in-sample call on the pooled frame."""
+    eng = get_engine()
+    T, nS = S.shape
+    nY = Y.shape[1]
+    depth = np.zeros(nY, dtype=np.float64)
+    if nY == 0:
+        return depth
+    ys = np.arange(nY, dtype=np.int64)
+    X = None
+    for j in range(2, J + 1):
+        if relax:
+            # additive over time rows: shard the rows of the pooled [S | Y] matrix, split it at nS per block
+            if X is None:
+                X = np.ascontiguousarray(np.concatenate([S, Y], axis=1))
+            cnt = _dist.relaxed_counts(lambda Xr, q, jj: eng.band_depth_oos_counts(Xr[:, :nS], Xr[:, nS:], jj, True)[q],
+                                       X, ys, j)
+        else:
+            if j == 3:  # bd_triple_kernel enumerates the C(nS, 3) sample triples of every new curve
+                settings.check_enumeration(float(nY) * binom(nS, 3),
+                                           'out-of-sample strict band depth with J=3 (n=%d)' % (nS + 1))
+            cnt = _dist.query_sharded(lambda qb: eng.band_depth_oos_counts(S, Y[:, qb], j, False), ys, np.int64)
+        s_nj = cnt.astype(np.float64)
+        if relax:
+            s_nj = s_nj / float(T)
+        depth = depth + s_nj / binom(nS + 1, j)
+    return depth
+
+
+def _functionaldepth_of(
+    data: List[pd.DataFrame],
+    sample: List[pd.DataFrame],
+    J=2,
+    containment='r2',
+    relax=False,
+    deep_check=False,
+    quiet=True,
+) -> pd.Series:
+    """Band depth of every curve of data[0] against the reference sample sample[0], each curve counted as if it
+    alone were appended to the sample.  Indexed by data[0].columns (labels may repeat those of the sample)."""
+    _handle_depth_errors(data=data, J=J, containment=containment, relax=relax, deep_check=deep_check)
+    _handle_depth_errors(data=sample, J=J, containment=containment, relax=relax, deep_check=deep_check)
+    name = _check_containment(containment)
+    if len(data) != 1 or len(sample) != 1:
+        raise NotImplementedError('out-of-sample depth is implemented for univariate data ([DataFrame] with '
+                                  'containment=\'r2\'); multivariate simplex depth is not')
+    if name == 'r2_enum':
+        raise NotImplementedError  # as _functionaldepth (_containment.py:103)
+    df, ref = data[0], sample[0]
+    if df.shape[0] != ref.shape[0]:
+        raise ValueError('data and sample must have the same number of time points.')
+    if deep_check and not (len(df.index) == len(ref.index) and all(df.index == ref.index)):
+        raise ValueError('DataFrames indices must be the same')
+    if J > 3:
+        raise NotImplementedError('out-of-sample band depth is implemented for J <= 3 on the B200 engine')
+    depths = _univariate_depths_of(_values(ref), _values(df), J, relax)
+    return pd.Series(index=df.columns, data=depths)
 
 
 def _sample_blocks(df: pd.DataFrame, cols, K: int):

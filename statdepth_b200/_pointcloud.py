@@ -16,7 +16,7 @@ from ._engine import get_engine
 from ._functional import _positions, _values
 from ._helper import DepthDegeneracy
 
-__all__ = ['_pointwisedepth', '_samplepointwisedepth']
+__all__ = ['_pointwisedepth', '_samplepointwisedepth', '_pointwisedepth_of']
 
 
 def _pointwisedepth(
@@ -76,6 +76,41 @@ def _pointwisedepth(
         return pd.Series(index=to_compute, data=vals)
     else:
         raise ValueError(f'{containment} is not a valid containment measure. ')
+
+
+def _pointwisedepth_of(
+    data: pd.DataFrame,
+    sample: pd.DataFrame,
+    containment='simplex',
+    quiet=True,
+) -> pd.Series:
+    """Depth of every row of data against the reference cloud sample, each point counted as if it alone were
+    appended to the sample (population nS + 1).  Indexed by data.index."""
+    if containment not in ('simplex', 'l1', 'mahalanobis', 'oja'):
+        raise ValueError(f'{containment} is not a valid containment measure. ')
+    if containment in ('mahalanobis', 'oja'):
+        raise NotImplementedError(f'out-of-sample {containment} depth is not implemented; use \'simplex\' or \'l1\'')
+    nY, d = data.shape
+    nS, dS = sample.shape
+    if d != dS:
+        raise ValueError('data and sample must have the same number of dimensions.')
+    S = np.ascontiguousarray(_values(sample))
+    Y = np.ascontiguousarray(_values(data))
+    ys = np.arange(nY, dtype=np.int64)
+    eng = get_engine()
+    if containment == 'simplex':
+        if d > 3:
+            raise NotImplementedError('simplicial depth is implemented for d <= 3 on the B200 engine')
+        tol = settings.get_simplex_tolerance()
+        if d != 2 or nS + 1 <= 64:  # as _pointwisedepth with n = nS + 1: larger 2-D samples are counted
+            settings.check_enumeration(float(nY) * binom(nS, d + 1),
+                                       'out-of-sample simplicial depth (d=%d, n=%d)' % (d, nS + 1))
+        cnt = _dist.query_sharded(lambda qb: eng.simplicial_oos_counts(S, Y[qb], tol), ys, np.int64)
+        return pd.Series(index=data.index, data=cnt.astype(np.float64) / binom(nS + 1, d + 1))
+    if d > 16:
+        raise NotImplementedError('L1 depth is implemented for d <= 16 on the B200 engine')
+    dep = _dist.query_sharded(lambda qb: eng.l1_oos_depth(S, Y[qb]), ys, np.float64)
+    return pd.Series(index=data.index, data=dep)
 
 
 def _mahalanobis_depth(data: pd.DataFrame, to_compute=None) -> pd.Series:

@@ -29,6 +29,7 @@ SOURCES = {
     "bd_bits.cu": [],
     "bd_gemm.cu": [],
     "bd_match.cu": [],
+    "oos.cu": [],
     "pointcloud.cu": ["-fmad=false"],
     "simplicial_count.cu": ["-fmad=false"],
 }

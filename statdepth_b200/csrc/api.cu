@@ -396,6 +396,114 @@ int sd_pointcloud_l1_f64(sd_ctx *ctx, const double *P, int64_t n, int d, const i
     return end_call(ctx, true);
 }
 
+// ---------------------------------------------------------------------------------------------
+// out-of-sample depth: sample and new observations are pooled on the device (sample first), see oos.cu
+// ---------------------------------------------------------------------------------------------
+// [rows, colsA] (ldA) next to [rows, colsB] (ldB) -> dense device [rows, colsA + colsB]
+static int upload_pooled(sd_ctx *ctx, cudaMemcpyKind kind, const double *A, i64 colsA, i64 ldA, const double *B,
+                         i64 colsB, i64 ldB, i64 rows, double **d) {
+    const i64 ld = colsA + colsB;
+    SD_TRY(ctx->buf[BUF_IN].reserve((size_t)(rows * ld > 0 ? rows * ld : 1) * sizeof(double)));
+    *d = ctx->buf[BUF_IN].as<double>();
+    if (rows > 0 && colsA > 0)
+        SD_CUDA(cudaMemcpy2DAsync(*d, (size_t)ld * sizeof(double), A, (size_t)ldA * sizeof(double),
+                                  (size_t)colsA * sizeof(double), (size_t)rows, kind, ctx->stream));
+    if (rows > 0 && colsB > 0)
+        SD_CUDA(cudaMemcpy2DAsync(*d + colsA, (size_t)ld * sizeof(double), B, (size_t)ldB * sizeof(double),
+                                  (size_t)colsB * sizeof(double), (size_t)rows, kind, ctx->stream));
+    return SD_OK;
+}
+
+int sd_band_depth_oos_f64(sd_ctx *ctx, const double *S, int64_t T, int64_t nS, int64_t ldS, const double *Y,
+                          int64_t nY, int64_t ldY, int j, int relax, int64_t *count_out) {
+    SD_TRY(check_common(ctx, S, count_out, "sd_band_depth_oos_f64"));
+    SD_REQUIRE(Y || nY == 0, "sd_band_depth_oos_f64: NULL Y");
+    SD_REQUIRE(T >= 1 && nS >= 1 && nY >= 0 && ldS >= nS && ldY >= nY, "sd_band_depth_oos_f64: bad sizes");
+    SD_TRY(begin_call(ctx));
+    double *dX = nullptr;
+    SD_TRY(upload_pooled(ctx, cudaMemcpyHostToDevice, S, nS, ldS, Y, nY, ldY, T, &dX));
+    SD_TRY(ctx->buf[BUF_OUT].reserve((size_t)(nY > 0 ? nY : 1) * sizeof(i64)));
+    i64 *d_out = ctx->buf[BUF_OUT].as<i64>();
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(band_depth_oos_device(ctx, dX, T, nS, nY, nS + nY, j, relax, d_out));
+    SD_TRY(mark(ctx, 2));
+    if (nY > 0)
+        SD_CUDA(cudaMemcpyAsync(count_out, d_out, (size_t)nY * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
+    return end_call(ctx, true);
+}
+
+int sd_band_depth_oos_f64_dev(sd_ctx *ctx, const double *dS, int64_t T, int64_t nS, int64_t ldS, const double *dY,
+                              int64_t nY, int64_t ldY, int j, int relax, int64_t *d_count_out) {
+    SD_TRY(check_common(ctx, dS, d_count_out, "sd_band_depth_oos_f64_dev"));
+    SD_REQUIRE(dY || nY == 0, "sd_band_depth_oos_f64_dev: NULL Y");
+    SD_REQUIRE(T >= 1 && nS >= 1 && nY >= 0 && ldS >= nS && ldY >= nY, "sd_band_depth_oos_f64_dev: bad sizes");
+    SD_TRY(begin_call(ctx));
+    SD_TRY(mark(ctx, 1));
+    const double *dX = dS;
+    i64 ld = ldS;
+    if (nY > 0 && !(dY == dS + nS && ldY == ldS)) {  // not already the columns after the sample: pool them
+        double *dP = nullptr;
+        SD_TRY(upload_pooled(ctx, cudaMemcpyDeviceToDevice, dS, nS, ldS, dY, nY, ldY, T, &dP));
+        dX = dP;
+        ld = nS + nY;
+    }
+    SD_TRY(band_depth_oos_device(ctx, dX, T, nS, nY, ld, j, relax, (i64 *)d_count_out));
+    SD_TRY(mark(ctx, 2));
+    return end_call(ctx, false);
+}
+
+// point clouds: [S; Y] rows, query ids nS .. nS + nY - 1
+static int pooled_cloud(sd_ctx *ctx, const double *S, int64_t nS, int d, const double *Y, int64_t nY, double **dP,
+                        const i64 **d_q) {
+    SD_TRY(upload_pooled(ctx, cudaMemcpyHostToDevice, S, nS * d, nS * d, Y, nY * d, nY * d, 1, dP));
+    SD_TRY(ctx->buf[BUF_MISC].reserve((size_t)(nY > 0 ? nY : 1) * sizeof(i64)));
+    i64 *q = ctx->buf[BUF_MISC].as<i64>();
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(finite_check_device(ctx, *dP, 1, (nS + nY) * d, (nS + nY) * d));
+    SD_TRY(iota_from_device(ctx, q, nY, nS));
+    *d_q = q;
+    return SD_OK;
+}
+
+int sd_pointcloud_simplicial_oos_f64(sd_ctx *ctx, const double *S, int64_t nS, int d, const double *Y, int64_t nY,
+                                     double tol, int64_t *count_out) {
+    SD_TRY(check_common(ctx, S, count_out, "sd_pointcloud_simplicial_oos_f64"));
+    SD_REQUIRE(Y || nY == 0, "sd_pointcloud_simplicial_oos_f64: NULL Y");
+    SD_REQUIRE(nS >= 1 && nY >= 0, "sd_pointcloud_simplicial_oos_f64: bad sizes");
+    SD_REQUIRE(d >= 1 && d <= 3, "sd_pointcloud_simplicial_oos_f64: d=%d not supported (1..3)", d);
+    SD_REQUIRE(tol >= 0.0, "sd_pointcloud_simplicial_oos_f64: tol must be >= 0");
+    SD_TRY(begin_call(ctx));
+    double *dP = nullptr;
+    const i64 *d_q = nullptr;
+    SD_TRY(ctx->buf[BUF_OUT].reserve((size_t)(nY > 0 ? nY : 1) * sizeof(i64)));
+    i64 *d_out = ctx->buf[BUF_OUT].as<i64>();
+    SD_TRY(pooled_cloud(ctx, S, nS, d, Y, nY, &dP, &d_q));
+    SD_TRY(simplicial_device(ctx, dP, nS + 1, d, d_q, nY, tol, d_out, true));
+    SD_TRY(mark(ctx, 2));
+    if (nY > 0)
+        SD_CUDA(cudaMemcpyAsync(count_out, d_out, (size_t)nY * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
+    return end_call(ctx, true);
+}
+
+int sd_pointcloud_l1_oos_f64(sd_ctx *ctx, const double *S, int64_t nS, int d, const double *Y, int64_t nY,
+                             double *depth_out) {
+    SD_TRY(check_common(ctx, S, depth_out, "sd_pointcloud_l1_oos_f64"));
+    SD_REQUIRE(Y || nY == 0, "sd_pointcloud_l1_oos_f64: NULL Y");
+    SD_REQUIRE(nS >= 1 && nY >= 0, "sd_pointcloud_l1_oos_f64: bad sizes");
+    SD_REQUIRE(d >= 1 && d <= 16, "sd_pointcloud_l1_oos_f64: d=%d not supported (1..16)", d);
+    SD_TRY(begin_call(ctx));
+    double *dP = nullptr;
+    const i64 *d_q = nullptr;
+    SD_TRY(ctx->buf[BUF_OUT].reserve((size_t)(nY > 0 ? nY : 1) * sizeof(double)));
+    double *d_out = ctx->buf[BUF_OUT].as<double>();
+    SD_TRY(pooled_cloud(ctx, S, nS, d, Y, nY, &dP, &d_q));
+    SD_TRY(l1_device(ctx, dP, nS, d, d_q, nY, d_out, nS + 1));
+    SD_TRY(mark(ctx, 2));
+    if (nY > 0)
+        SD_CUDA(cudaMemcpyAsync(depth_out, d_out, (size_t)nY * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    return end_call(ctx, true);
+}
+
 int sd_pointcloud_oja_f64(sd_ctx *ctx, const double *P, int64_t n, int d, const int64_t *query_idx, int64_t nq,
                           const int64_t *pool, int64_t npool, double hull_volume, double *out) {
     SD_TRY(check_common(ctx, P, out, "sd_pointcloud_oja_f64"));

@@ -151,15 +151,21 @@ int gather_i64_device(sd_ctx *ctx, const i64 *d_src, const i64 *d_idx, i64 nq, i
 int compact_columns_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, const i64 *d_cols, i64 m, double *d_out);
 int compact_batches_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, const i64 *d_cols, i64 m, i64 nb,
                            double *d_out);
-int l1_device(sd_ctx *ctx, const double *dP, i64 n, int d, const i64 *d_q, i64 nq, double *d_out);
+int l1_device(sd_ctx *ctx, const double *dP, i64 n, int d, const i64 *d_q, i64 nq, double *d_out,
+              i64 n_pop = 0);
 int oja_device(sd_ctx *ctx, const double *dP, i64 n, int d, const i64 *d_q, i64 nq, const i64 *d_pool,
                i64 npool, double hull_volume, double *d_out);
 int cloud_blocks_device(sd_ctx *ctx, const double *dP, int d, const i64 *d_member, const i64 *d_off,
                         const i64 *d_qpos, i64 B, int kind, double tol, const double *d_volume, double *d_out);
 int simplicial_device(sd_ctx *ctx, const double *dP, i64 n, int d, const i64 *d_q, i64 nq, double tol,
-                      i64 *d_out);
+                      i64 *d_out, bool oos = false);
 int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride_j, i64 T, const i64 *d_q, i64 nq,
-                             double tol, i64 *d_out);
+                             double tol, i64 *d_out, i64 m_others = -1);
+// out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
+int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
+                          i64 *d_out);
+int iota_from_device(sd_ctx *ctx, i64 *d_p, i64 count, i64 base);
+int finite_check_device(sd_ctx *ctx, const double *dX, i64 rows, i64 cols, i64 ld);
 int oja2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, const i64 *d_q, i64 nq, double hull_volume,
                       double *d_out);
 int simplex_depth_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, const i64 *d_q, i64 nq,

@@ -34,7 +34,7 @@ constexpr int L1_THREADS = 128;
 template <int D>
 __global__ void __launch_bounds__(L1_THREADS) l1_kernel(const double *__restrict__ P, const i64 n, const int d_rt,
                                                         const i64 *__restrict__ q, const i64 nq,
-                                                        double *__restrict__ out) {
+                                                        const double denom, double *__restrict__ out) {
     extern __shared__ double s_pts[];  // L1_TILE * d
     const int d = D > 0 ? D : d_rt;
     const int part = threadIdx.x % L1_LANES;
@@ -97,22 +97,25 @@ __global__ void __launch_bounds__(L1_THREADS) l1_kernel(const double *__restrict
             tot += v * v;
         }
     }
-    if (active && part == 0) out[qi] = 1.0 - sqrt(tot) / (double)n;
+    if (active && part == 0) out[qi] = 1.0 - sqrt(tot) / denom;
 }
 
-int l1_device(sd_ctx *ctx, const double *dP, i64 n, int d, const i64 *d_q, i64 nq, double *d_out) {
+// The others are the first n points, skipping the query when it is one of them.  n_pop = population size of the
+// divisor: n for queries among the points, n + 1 for out-of-sample queries (ids >= n, never skipped).
+int l1_device(sd_ctx *ctx, const double *dP, i64 n, int d, const i64 *d_q, i64 nq, double *d_out, i64 n_pop) {
     if (nq == 0) return SD_OK;
+    const double denom = (double)(n_pop > 0 ? n_pop : n);
     const unsigned grid = (unsigned)ceil_div(nq, L1_THREADS / L1_LANES);
     const size_t smem = (size_t)L1_TILE * d * sizeof(double);
     cudaStream_t st = ctx->stream;
     switch (d) {
-        case 1: l1_kernel<1><<<grid, L1_THREADS, smem, st>>>(dP, n, d, d_q, nq, d_out); break;
-        case 2: l1_kernel<2><<<grid, L1_THREADS, smem, st>>>(dP, n, d, d_q, nq, d_out); break;
-        case 3: l1_kernel<3><<<grid, L1_THREADS, smem, st>>>(dP, n, d, d_q, nq, d_out); break;
+        case 1: l1_kernel<1><<<grid, L1_THREADS, smem, st>>>(dP, n, d, d_q, nq, denom, d_out); break;
+        case 2: l1_kernel<2><<<grid, L1_THREADS, smem, st>>>(dP, n, d, d_q, nq, denom, d_out); break;
+        case 3: l1_kernel<3><<<grid, L1_THREADS, smem, st>>>(dP, n, d, d_q, nq, denom, d_out); break;
         default:
             SD_CUDA(cudaFuncSetAttribute(l1_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          L1_TILE * L1_MAXD * (int)sizeof(double)));
-            l1_kernel<0><<<grid, L1_THREADS, smem, st>>>(dP, n, d, d_q, nq, d_out);
+            l1_kernel<0><<<grid, L1_THREADS, smem, st>>>(dP, n, d, d_q, nq, denom, d_out);
             break;
     }
     ctx->last.launches++;
@@ -212,12 +215,17 @@ __global__ void __launch_bounds__(256) simplicial_kernel(const double *__restric
 constexpr i64 SIMPLICIAL_ENUM_MAX_N = 64;
 constexpr i64 SIMPLEX_ENUM_MAX_N = 64;
 
+// oos: the queries (ids >= n - 1) are not among the first n - 1 points, which are all the others (out-of-sample
+// depth of a point appended to a sample of n - 1).  The enumeration kernel needs nothing else: its others are
+// positions 0 .. n - 2 shifted past the query, and no position reaches a query id.  n is the population size
+// either way, so both forms switch to counting at the same size.
 int simplicial_device(sd_ctx *ctx, const double *dP, i64 n, int d, const i64 *d_q, i64 nq, double tol,
-                      i64 *d_out) {
+                      i64 *d_out, bool oos) {
     if (nq == 0) return SD_OK;
     if (d == 2 && (ctx->simplicial_impl == SD_SIMPLICIAL_COUNT ||
                    (ctx->simplicial_impl == SD_SIMPLICIAL_AUTO && n > SIMPLICIAL_ENUM_MAX_N)))
-        return simplicial2_count_device(ctx, dP, n, 2, 1, d_q, nq, tol, d_out);
+        return oos ? simplicial2_count_device(ctx, dP, n - 1, 2, 1, d_q, nq, tol, d_out, n - 1)
+                   : simplicial2_count_device(ctx, dP, n, 2, 1, d_q, nq, tol, d_out);
     cudaStream_t st = ctx->stream;
     const unsigned grid = (unsigned)nq;
     switch (d) {

@@ -97,7 +97,8 @@ __global__ void __launch_bounds__(256) sc_reduce_kernel(const ScGeom g, const i6
                                                         const double *__restrict__ KB,
                                                         const int *__restrict__ bA, const int *__restrict__ aA,
                                                         const int *__restrict__ bB, const int *__restrict__ aB,
-                                                        int *__restrict__ claim, i64 *__restrict__ out) {
+                                                        int *__restrict__ claim, const i64 m_others,
+                                                        i64 *__restrict__ out) {
     __shared__ i64 s_red[8];
     __shared__ i64 s_cnt[2];
     const i64 li = blockIdx.x;
@@ -160,18 +161,20 @@ __global__ void __launch_bounds__(256) sc_reduce_kernel(const ScGeom g, const i6
     if (threadIdx.x == 0) {
         i64 tot = 0;
         for (int w = 0; w < (int)(blockDim.x >> 5); ++w) tot += s_red[w];
-        const i64 m = n - 1;
-        atomicAdd((u64 *)&out[inst / g.T], (u64)(c3(m) - tot));
+        atomicAdd((u64 *)&out[inst / g.T], (u64)(c3(m_others) - tot));
     }
 }
 
 // Counts for `nq` queries x `T` instances each (T = 1 for point clouds).  d_out[nq] is zeroed here.
+// m_others < 0: the queries are among the n points (n - 1 others); m_others = n: out-of-sample queries (ids >= n,
+// coordinates read from the same array), every one of the n points is an other.
 int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride_j, i64 T, const i64 *d_q, i64 nq,
-                             double tol, i64 *d_out) {
+                             double tol, i64 *d_out, i64 m_others) {
     cudaStream_t st = ctx->stream;
     SD_CUDA(cudaMemsetAsync(d_out, 0, (size_t)nq * sizeof(i64), st));
     const i64 ninst_total = nq * T;
-    if (ninst_total == 0 || n < 4) return SD_OK;  // fewer than 3 other points: no triangle
+    if (m_others < 0) m_others = n - 1;
+    if (ninst_total == 0 || m_others < 3) return SD_OK;  // fewer than 3 other points: no triangle
     if (2 * n >= (1ll << 31)) {
         set_error("simplicial counting: n=%lld too large", (long long)n);
         return SD_ERR_UNSUPPORTED;
@@ -213,8 +216,8 @@ int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride
         SD_CUDA(cudaMemsetAsync(claim, 0, (size_t)ni * n * sizeof(int), st));
         SD_TRY(mbd_all_device(ctx, KA, ni, n, n, false, nullptr, nullptr, bA, aA));  // ranks only
         SD_TRY(mbd_all_device(ctx, KB, ni, 2 * n, 2 * n, false, nullptr, nullptr, bB, tol > 0.0 ? aB : nullptr));
-        if (tol > 0.0) sc_reduce_kernel<true><<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, claim, d_out);
-        else sc_reduce_kernel<false><<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, claim, d_out);
+        if (tol > 0.0) sc_reduce_kernel<true><<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, claim, m_others, d_out);
+        else sc_reduce_kernel<false><<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, claim, m_others, d_out);
         ctx->last.launches++;
         SD_CUDA(cudaGetLastError());
     }

@@ -10,11 +10,11 @@ from typing import List, Union
 
 import pandas as pd
 
-from ._functional import _functionaldepth, _samplefunctionaldepth
+from ._functional import _functionaldepth, _functionaldepth_of, _samplefunctionaldepth
 from ._helper import DepthDegeneracy  # noqa: F401  (re-exported like the reference's `from ._helper import *`)
-from ._pointcloud import _pointwisedepth, _samplepointwisedepth
+from ._pointcloud import _pointwisedepth, _pointwisedepth_of, _samplepointwisedepth
 
-__all__ = ['FunctionalDepth', 'PointcloudDepth', 'AbstractDepth']
+__all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'AbstractDepth']
 
 
 def _go():
@@ -253,3 +253,34 @@ def FunctionalDepth(
         return _FunctionalDepthUnivariate(df=data[0], depths=depth)
     else:
         return _FunctionalDepthSeries(df=data[0], depths=depth)
+
+
+def FunctionalDepthOf(
+    data: List[pd.DataFrame],
+    sample: List[pd.DataFrame],
+    J=2,
+    containment='r2',
+    relax=False,
+    deep_check=False,
+    quiet=True,
+) -> _FunctionalDepthUnivariate:
+    """Out-of-sample band depth: the depth of every curve (column) of data[0] against the reference sample
+    sample[0] (both T x n DataFrames with the same T rows).  Each curve gets the depth FunctionalDepth would give it
+    after it alone is appended to the sample; the other curves of data never take part.  The result is indexed by
+    data[0].columns (positions decide, so a label may also occur in the sample).  J = 2 or 3, containment 'r2'."""
+    depth = _functionaldepth_of(data=data, sample=sample, J=J, containment=containment, relax=relax,
+                                deep_check=deep_check, quiet=quiet)
+    return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+
+
+def PointcloudDepthOf(
+    data: pd.DataFrame,
+    sample: pd.DataFrame,
+    containment='simplex',
+    quiet=True,
+) -> _PointwiseDepth:
+    """Out-of-sample point-cloud depth: the depth of every row of data (m x d) against the reference cloud sample
+    (n x d), as PointcloudDepth would give it after that row alone is appended to the sample.  containment is
+    'simplex' (d <= 3) or 'l1' (d <= 16).  Indexed by data.index."""
+    depth = _pointwisedepth_of(data=data, sample=sample, containment=containment, quiet=quiet)
+    return _PointwiseDepth(df=data, depths=depth)
