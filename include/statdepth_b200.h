@@ -246,6 +246,40 @@ int sd_pointcloud_l1_oos_f64(sd_ctx *ctx, const double *S, int64_t nS, int d, co
                              int64_t nY, double *depth_out);
 
 /*
+ * Functional outlier detection (functional boxplot, outliergram).  X [T, n] in `layout`, as sd_band_depth_f64.
+ *
+ * Rank sums.  With b_t(c) / a_t(c) the number of OTHER curves strictly below / above curve c at row t:
+ *   q_out[c]         = sum_t [C(n-1,2) - C(b_t,2) - C(a_t,2)]   (== sd_band_depth_f64(relax = 1, j = 2))
+ *   below_sum_out[c] = sum_t b_t,   above_sum_out[c] = sum_t a_t  (above_sum_out may be NULL)
+ * exact int64; SD_ERR_OVERFLOW when T * C(n-1, 2) exceeds int64.  All three are additive over disjoint blocks of
+ * time rows.  The modified epigraph index of the outliergram is 1 - below_sum / (n T).
+ */
+int sd_band_rank_sums_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_t ld, int layout,
+                          int64_t *q_out, int64_t *below_sum_out, int64_t *above_sum_out);
+
+/* same with DEVICE pointers, SD_LAYOUT_TN only */
+int sd_band_rank_sums_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n, int64_t ld,
+                              int64_t *d_q_out, int64_t *d_below_sum_out, int64_t *d_above_sum_out);
+
+/*
+ * Masked envelope.  member[c] != 0 selects the curves the envelope is taken over (SD_ERR_INVALID if it selects
+ * none).  Per row t: lower_out[t] / upper_out[t] = min / max of X[t, c] over the member curves.
+ * outside_out[c] (may be NULL) = #rows t with X[t, c] < lo_t - f or X[t, c] > hi_t + f, f = factor * (hi_t - lo_t)
+ * (factor finite and >= 0); each of the four operations is one correctly rounded double operation (no fused
+ * multiply-add), so a caller rebuilds the same fences from lower_out / upper_out.  A value on a fence is not
+ * outside.  Rows are independent: a block of time rows gives those rows' envelope and its share of outside_out,
+ * which is additive over disjoint row blocks.
+ */
+int sd_band_envelope_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_t ld, int layout,
+                         const uint8_t *member, double factor, double *lower_out, double *upper_out,
+                         int64_t *outside_out);
+
+/* same with DEVICE pointers (member and outputs too), SD_LAYOUT_TN only */
+int sd_band_envelope_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n, int64_t ld,
+                             const uint8_t *d_member, double factor, double *d_lower_out, double *d_upper_out,
+                             int64_t *d_outside_out);
+
+/*
  * Batched band depth over sub-populations of one matrix (K-sampled blocks, homogeneity
  * permutations): membership[b*n + c] != 0 selects the curves of batch b; queries[b*nqb + i] is
  * the i-th query curve of batch b (must be a member).  count_out[b*nqb + i] as in

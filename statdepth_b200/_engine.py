@@ -86,6 +86,14 @@ SIGNATURES = {
                                                    C.c_int64, C.c_double, C.c_void_p]),
     "sd_pointcloud_l1_oos_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int64,
                                            C.c_void_p]),
+    "sd_band_rank_sums_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_void_p,
+                                        C.c_void_p, C.c_void_p]),
+    "sd_band_rank_sums_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
+                                            C.c_void_p, C.c_void_p]),
+    "sd_band_envelope_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_void_p,
+                                       C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sd_band_envelope_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
+                                           C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sd_band_depth_batched_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                             C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -271,6 +279,47 @@ class Engine:
         self._check(self.lib.sd_band_depth_batched_f64(self._ctx, _ptr(X), T, n, n, _ptr(mem), B, _ptr(qs), nqb,
                                                        int(j), int(bool(relax)), _ptr(out)))
         return out
+
+    # -- outlier detection ------------------------------------------------------------------------------
+    def band_rank_sums(self, X, want_above=False):
+        """(Q, B[, A]) int64 [n]: the relaxed J = 2 numerator and the per-curve sums over time rows of the curves
+        strictly below (and above) each curve.  X is [T, n]; an F-ordered X is passed with SD_LAYOUT_NT."""
+        X, is_f = self._matrix(X)
+        T, n = X.shape
+        q, b = np.empty(n, dtype=np.int64), np.empty(n, dtype=np.int64)
+        a = np.empty(n, dtype=np.int64) if want_above else None
+        self._check(self.lib.sd_band_rank_sums_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, T if is_f else n,
+                                                   LAYOUT_NT if is_f else LAYOUT_TN, _ptr(q), _ptr(b), _ptr(a)))
+        return (q, b, a) if want_above else (q, b)
+
+    def band_rank_sums_dev(self, dX_ptr, T, n, ld, d_q_ptr, d_b_ptr, d_a_ptr=None):
+        """Device-pointer variant (SD_LAYOUT_TN): int64 [n] outputs stay on the device."""
+        self._check(self.lib.sd_band_rank_sums_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
+                                                       C.c_void_p(int(d_q_ptr)), C.c_void_p(int(d_b_ptr)),
+                                                       C.c_void_p(int(d_a_ptr)) if d_a_ptr else None))
+
+    def band_envelope(self, X, member, factor, want_outside=True):
+        """(lo [T], hi [T], outside [n] or None): per-row min / max of the member curves, and per curve the number of
+        rows outside the fences lo - factor * (hi - lo), hi + factor * (hi - lo)."""
+        X, is_f = self._matrix(X)
+        T, n = X.shape
+        mem = np.ascontiguousarray(member, dtype=np.uint8)
+        if mem.shape != (n,):
+            raise ValueError("member must have one entry per curve")
+        lower, upper = np.empty(T), np.empty(T)
+        outside = np.empty(n, dtype=np.int64) if want_outside else None
+        self._check(self.lib.sd_band_envelope_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, T if is_f else n,
+                                                  LAYOUT_NT if is_f else LAYOUT_TN, _ptr(mem), float(factor),
+                                                  _ptr(lower), _ptr(upper), _ptr(outside)))
+        return lower, upper, outside
+
+    def band_envelope_dev(self, dX_ptr, T, n, ld, d_member_ptr, factor, d_lower_ptr, d_upper_ptr,
+                          d_outside_ptr=None):
+        """Device-pointer variant (SD_LAYOUT_TN): member uint8 [n], lo / hi float64 [T], outside int64 [n]."""
+        self._check(self.lib.sd_band_envelope_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
+                                                      C.c_void_p(int(d_member_ptr)), float(factor),
+                                                      C.c_void_p(int(d_lower_ptr)), C.c_void_p(int(d_upper_ptr)),
+                                                      C.c_void_p(int(d_outside_ptr)) if d_outside_ptr else None))
 
     # -- out-of-sample depth ----------------------------------------------------------------------------
     @staticmethod

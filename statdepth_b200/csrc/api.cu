@@ -452,6 +452,94 @@ int sd_band_depth_oos_f64_dev(sd_ctx *ctx, const double *dS, int64_t T, int64_t 
     return end_call(ctx, false);
 }
 
+// ---------------------------------------------------------------------------------------------
+// outlier detection: per-curve rank sums and masked envelopes, see outliers.cu
+// ---------------------------------------------------------------------------------------------
+// host matrix in either layout -> dense device [T, n] (SD_LAYOUT_NT is uploaded, then transposed)
+static int upload_tn(sd_ctx *ctx, const double *X, i64 T, i64 n, i64 ld, int layout, double **dX) {
+    if (layout == SD_LAYOUT_TN) return upload_matrix(ctx, BUF_IN, X, T, n, ld, dX);
+    double *dN = nullptr;
+    SD_TRY(upload_matrix(ctx, BUF_IN2, X, n, T, ld, &dN));
+    SD_TRY(ctx->buf[BUF_IN].reserve((size_t)T * n * sizeof(double)));
+    *dX = ctx->buf[BUF_IN].as<double>();
+    return transpose_device(ctx, dN, n, T, T, *dX);
+}
+
+static int check_matrix(const char *who, i64 T, i64 n, i64 ld, int layout) {
+    SD_REQUIRE(T >= 1 && n >= 1, "%s: bad sizes T=%lld n=%lld", who, (long long)T, (long long)n);
+    SD_REQUIRE(layout == SD_LAYOUT_TN || layout == SD_LAYOUT_NT, "%s: bad layout %d", who, layout);
+    SD_REQUIRE(ld >= (layout == SD_LAYOUT_TN ? n : T), "%s: ld=%lld too small", who, (long long)ld);
+    return SD_OK;
+}
+
+int sd_band_rank_sums_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_t ld, int layout, int64_t *q_out,
+                          int64_t *below_sum_out, int64_t *above_sum_out) {
+    SD_TRY(check_common(ctx, X, q_out, "sd_band_rank_sums_f64"));
+    SD_REQUIRE(below_sum_out, "sd_band_rank_sums_f64: NULL below_sum_out");
+    SD_TRY(check_matrix("sd_band_rank_sums_f64", T, n, ld, layout));
+    SD_TRY(begin_call(ctx));
+    double *dX = nullptr;
+    SD_TRY(upload_tn(ctx, X, T, n, ld, layout, &dX));
+    SD_TRY(ctx->buf[BUF_OUT].reserve((size_t)n * 3 * sizeof(i64)));
+    i64 *d_q = ctx->buf[BUF_OUT].as<i64>(), *d_b = d_q + n, *d_a = above_sum_out ? d_b + n : nullptr;
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(rank_sums_device(ctx, dX, T, n, n, d_q, d_b, d_a));
+    SD_TRY(mark(ctx, 2));
+    SD_CUDA(cudaMemcpyAsync(q_out, d_q, (size_t)n * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
+    SD_CUDA(cudaMemcpyAsync(below_sum_out, d_b, (size_t)n * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
+    if (d_a) SD_CUDA(cudaMemcpyAsync(above_sum_out, d_a, (size_t)n * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
+    return end_call(ctx, true);
+}
+
+int sd_band_rank_sums_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n, int64_t ld, int64_t *d_q_out,
+                              int64_t *d_below_sum_out, int64_t *d_above_sum_out) {
+    SD_TRY(check_common(ctx, dX, d_q_out, "sd_band_rank_sums_f64_dev"));
+    SD_REQUIRE(d_below_sum_out, "sd_band_rank_sums_f64_dev: NULL below_sum_out");
+    SD_TRY(check_matrix("sd_band_rank_sums_f64_dev", T, n, ld, SD_LAYOUT_TN));
+    SD_TRY(begin_call(ctx));
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(rank_sums_device(ctx, dX, T, n, ld, (i64 *)d_q_out, (i64 *)d_below_sum_out, (i64 *)d_above_sum_out));
+    SD_TRY(mark(ctx, 2));
+    return end_call(ctx, false);
+}
+
+int sd_band_envelope_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_t ld, int layout,
+                         const uint8_t *member, double factor, double *lower_out, double *upper_out,
+                         int64_t *outside_out) {
+    SD_TRY(check_common(ctx, X, lower_out, "sd_band_envelope_f64"));
+    SD_REQUIRE(member && upper_out, "sd_band_envelope_f64: NULL member or upper_out");
+    SD_TRY(check_matrix("sd_band_envelope_f64", T, n, ld, layout));
+    SD_TRY(begin_call(ctx));
+    double *dX = nullptr;
+    SD_TRY(upload_tn(ctx, X, T, n, ld, layout, &dX));
+    // member | lower | upper | outside
+    SD_TRY(ctx->buf[BUF_OUT].reserve((size_t)(2 * T + n) * 8 + (size_t)n));
+    double *d_lo = ctx->buf[BUF_OUT].as<double>(), *d_hi = d_lo + T;
+    i64 *d_out = outside_out ? reinterpret_cast<i64 *>(d_hi + T) : nullptr;
+    uint8_t *d_member = reinterpret_cast<uint8_t *>(d_hi + T + n);
+    SD_CUDA(cudaMemcpyAsync(d_member, member, (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(envelope_device(ctx, dX, T, n, n, d_member, factor, d_lo, d_hi, d_out));
+    SD_TRY(mark(ctx, 2));
+    SD_CUDA(cudaMemcpyAsync(lower_out, d_lo, (size_t)T * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    SD_CUDA(cudaMemcpyAsync(upper_out, d_hi, (size_t)T * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    if (d_out) SD_CUDA(cudaMemcpyAsync(outside_out, d_out, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    return end_call(ctx, true);
+}
+
+int sd_band_envelope_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n, int64_t ld,
+                             const uint8_t *d_member, double factor, double *d_lower_out, double *d_upper_out,
+                             int64_t *d_outside_out) {
+    SD_TRY(check_common(ctx, dX, d_lower_out, "sd_band_envelope_f64_dev"));
+    SD_REQUIRE(d_member && d_upper_out, "sd_band_envelope_f64_dev: NULL member or upper_out");
+    SD_TRY(check_matrix("sd_band_envelope_f64_dev", T, n, ld, SD_LAYOUT_TN));
+    SD_TRY(begin_call(ctx));
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(envelope_device(ctx, dX, T, n, ld, d_member, factor, d_lower_out, d_upper_out, (i64 *)d_outside_out));
+    SD_TRY(mark(ctx, 2));
+    return end_call(ctx, false);
+}
+
 // point clouds: [S; Y] rows, query ids nS .. nS + nY - 1
 static int pooled_cloud(sd_ctx *ctx, const double *S, int64_t nS, int d, const double *Y, int64_t nY, double **dP,
                         const i64 **d_q) {

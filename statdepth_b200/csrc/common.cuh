@@ -70,7 +70,7 @@ enum BufId {
 };
 
 // status bits written by kernels into ctx->d_status
-enum { ST_NONFINITE = 1, ST_INTERNAL = 2 };
+enum { ST_NONFINITE = 1, ST_INTERNAL = 2, ST_NO_MEMBER = 4 };
 
 __host__ __device__ static inline i64 ceil_div(i64 a, i64 b) { return (a + b - 1) / b; }
 
@@ -164,6 +164,12 @@ int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride
 // out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out);
+// int32 workspace for rank-only passes in row blocks of *RB rows (ints_per_row each) within a fixed budget
+int rank_block_workspace(sd_ctx *ctx, i64 T, i64 ints_per_row, i64 *RB, int **ws);
+// outlier detection (outliers.cu)
+int rank_sums_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, i64 *d_q, i64 *d_b, i64 *d_a);
+int envelope_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const uint8_t *d_member, double factor,
+                    double *d_lower, double *d_upper, i64 *d_outside);
 int iota_from_device(sd_ctx *ctx, i64 *d_p, i64 count, i64 base);
 int finite_check_device(sd_ctx *ctx, const double *dX, i64 rows, i64 cols, i64 ld);
 int oja2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, const i64 *d_q, i64 nq, double hull_volume,

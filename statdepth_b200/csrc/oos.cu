@@ -90,8 +90,18 @@ __global__ void __launch_bounds__(OOS_THREADS) oos_terms_kernel(const int *__res
     if (sum) atomicAdd((u64 *)&acc[g], (u64)sum);
 }
 
-// Rank workspace (int32 below / above of both passes) per row block.
-constexpr size_t OOS_RANK_BUDGET = 1ull << 30;
+// Rank workspace of the rank-only passes, split into row blocks (also used by rank_sums_device, outliers.cu).
+constexpr size_t RANK_BLOCK_BUDGET = 1ull << 30;
+
+int rank_block_workspace(sd_ctx *ctx, i64 T, i64 ints_per_row, i64 *RB, int **ws) {
+    i64 rb = (i64)(RANK_BLOCK_BUDGET / ((size_t)ints_per_row * sizeof(int)));
+    if (rb < 1) rb = 1;
+    if (rb > T) rb = T;
+    SD_TRY(ctx->buf[BUF_RANKS].reserve((size_t)rb * ints_per_row * sizeof(int)));
+    *RB = rb;
+    *ws = ctx->buf[BUF_RANKS].as<int>();
+    return SD_OK;
+}
 
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out) {
@@ -128,12 +138,9 @@ int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, 
     }
     const i64 n = nS + nY;
     const i64 ny_ranks = nY > 1 ? nY : 0;  // one new curve: nothing to subtract, no second pass
-    const size_t per_row = (size_t)(n + ny_ranks) * 2 * sizeof(int);
-    i64 RB = (i64)(OOS_RANK_BUDGET / per_row);
-    if (RB < 1) RB = 1;
-    if (RB > T) RB = T;
-    SD_TRY(ctx->buf[BUF_RANKS].reserve((size_t)RB * per_row));
-    int *bP = ctx->buf[BUF_RANKS].as<int>();
+    i64 RB = 0;
+    int *bP = nullptr;
+    SD_TRY(rank_block_workspace(ctx, T, (n + ny_ranks) * 2, &RB, &bP));
     int *aP = bP + (size_t)RB * n;
     int *bY = ny_ranks ? aP + (size_t)RB * n : nullptr;
     int *aY = ny_ranks ? bY + (size_t)RB * nY : nullptr;

@@ -8,13 +8,16 @@ module top, depth.py:4, which makes `import statdepth` fail where plotly is not 
 from abc import ABC, abstractmethod
 from typing import List, Union
 
+import numpy as np
 import pandas as pd
 
 from ._functional import _functionaldepth, _functionaldepth_of, _samplefunctionaldepth
 from ._helper import DepthDegeneracy  # noqa: F401  (re-exported like the reference's `from ._helper import *`)
+from ._outliers import _check_central, _checked_values, _functional_boxplot, _outliergram
 from ._pointcloud import _pointwisedepth, _pointwisedepth_of, _samplepointwisedepth
 
-__all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'AbstractDepth']
+__all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'FunctionalBoxplot',
+           'Outliergram', 'AbstractDepth']
 
 
 def _go():
@@ -284,3 +287,97 @@ def PointcloudDepthOf(
     'simplex' (d <= 3) or 'l1' (d <= 16).  Indexed by data.index."""
     depth = _pointwisedepth_of(data=data, sample=sample, containment=containment, quiet=quiet)
     return _PointwiseDepth(df=data, depths=depth)
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# functional outlier detection (drivers in _outliers.py)
+# ---------------------------------------------------------------------------------------------------------------
+class _OutlierResult:
+    """What both outlier rules share: the curves' modified band depth."""
+
+    def __init__(self, df: pd.DataFrame, r: dict):
+        self._df = df
+        self._r = r
+
+    def _series(self, values) -> pd.Series:
+        return pd.Series(index=self._df.columns, data=values)
+
+    def _labels(self, positions) -> list:
+        return [self._df.columns[p] for p in positions]
+
+    def _rows(self, pair) -> pd.DataFrame:
+        return pd.DataFrame({'lower': pair[0], 'upper': pair[1]}, index=self._df.index)
+
+    def depths(self) -> _FunctionalDepthUnivariate:
+        """Modified band depth of every curve, bit-identical to FunctionalDepth([df], J=2, relax=True)."""
+        return _FunctionalDepthUnivariate(df=self._df, depths=self._series(self._r['depth']))
+
+    def outliers(self) -> list:
+        """Labels of the flagged curves, in column order."""
+        return self._labels(np.flatnonzero(self._outlier_mask()))
+
+
+class _FunctionalBoxplot(_OutlierResult):
+    """Functional boxplot (Sun & Genton 2011): central region, envelope, fences, whiskers, magnitude outliers."""
+
+    def median(self):
+        """Label of the deepest curve (first of the central region)."""
+        return self._df.columns[self._r['central'][0]]
+
+    def central_region(self) -> list:
+        """Labels of the central curves, deepest first; ties in depth by column position."""
+        return self._labels(self._r['central'])
+
+    def envelope(self) -> pd.DataFrame:
+        """Per time row, min ('lower') and max ('upper') of the central curves."""
+        return self._rows(self._r['envelope'])
+
+    def fences(self) -> pd.DataFrame:
+        """The envelope inflated by factor x its width on both sides."""
+        return self._rows(self._r['fences'])
+
+    def whiskers(self) -> pd.DataFrame:
+        """Per time row, min and max of the curves that are not outliers."""
+        return self._rows(self._r['whiskers'])
+
+    def outside_counts(self) -> pd.Series:
+        """Per curve, the number of time rows at which it is strictly outside the fences."""
+        return self._series(self._r['outside'])
+
+    def _outlier_mask(self):
+        return self._r['outside'] > 0
+
+
+class _Outliergram(_OutlierResult):
+    """Outliergram (Arribas-Gil & Romo 2014): MBD against the modified epigraph index, shape outliers."""
+
+    def mei(self) -> pd.Series:
+        """Modified epigraph index: the share of (curve, time) pairs at or above the curve, itself included."""
+        return self._series(self._r['mei'])
+
+    def distance(self) -> pd.Series:
+        """How far below the parabola a0 + a1 MEI + a2 n^2 MEI^2 the curve's MBD lies (>= 0 without ties)."""
+        return self._series(self._r['distance'])
+
+    def _outlier_mask(self):
+        return self._r['outlier']
+
+
+def FunctionalBoxplot(data: List[pd.DataFrame], factor=1.5, central=0.5, deep_check=False) -> _FunctionalBoxplot:
+    """Functional boxplot of the curves (columns) of data[0], a T x n DataFrame.
+
+    The central region is the ceil(central * n) curves of largest modified band depth (ties by column position;
+    under ties this can differ from ordered(), whose sort is not stable).  Its per-row envelope, inflated by
+    factor x its width, gives the fences; a curve strictly outside them at any time point is a magnitude outlier.
+    Non-finite values are rejected."""
+    X = _checked_values(data, factor, deep_check)
+    _check_central(central)
+    return _FunctionalBoxplot(data[0], _functional_boxplot(X, float(factor), float(central)))
+
+
+def Outliergram(data: List[pd.DataFrame], factor=1.5, deep_check=False) -> _Outliergram:
+    """Outliergram of the curves (columns) of data[0], a T x n DataFrame: a curve whose distance below the
+    MBD-MEI parabola is at least q3 + factor * (q3 - q1) of all distances is a shape outlier.
+    Non-finite values are rejected."""
+    X = _checked_values(data, factor, deep_check)
+    return _Outliergram(data[0], _outliergram(X, float(factor)))
