@@ -233,6 +233,25 @@ int sd_band_depth_oos_f64_dev(sd_ctx *ctx, const double *dS, int64_t T, int64_t 
                               const double *dY, int64_t nY, int64_t ldY, int j, int relax,
                               int64_t *d_count_out);
 
+/*
+ * A fitted reference: the same relaxed counts from the sample's sorted rows, so that a sample scored against again
+ * and again is sorted once and only the new curves cross to the device on each call.
+ *
+ * Sorted reference rows (the index of a fitted reference): d_sorted_out[t*nS + k] = the k-th smallest of
+ * dX[t*ld + 0 .. nS), ties repeated.  Device pointers, SD_LAYOUT_TN, d_sorted_out holds T*nS doubles.
+ * SD_ERR_NONFINITE when the sample holds NaN or +-inf.
+ */
+int sd_band_sort_rows_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t nS, int64_t ld,
+                              double *d_sorted_out);
+
+/* Relaxed out-of-sample band depth numerators from sorted rows, J = 2 or 3:
+ * d_count_out[(j-2)*nY + g] = sum_t [C(nS,j) - C(b_t,j) - C(a_t,j)], j = 2..J, b_t / a_t = #values of sorted row t
+ * strictly below / above dY[t*ldY + g] -- equal to sd_band_depth_oos_f64_dev(relax = 1, j).  Device pointers,
+ * d_count_out holds (J - 1)*nY int64.  SD_ERR_NONFINITE when Y holds NaN or +-inf, SD_ERR_OVERFLOW when
+ * T * C(nS, J) exceeds int64. */
+int sd_band_depth_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t T, int64_t nS,
+                                 const double *dY, int64_t nY, int64_t ldY, int J, int64_t *d_count_out);
+
 /* Point clouds S[i*d + c] (nS points) and Y[g*d + c] (nY points), d in 1..3:
  * count_out[g] = #{(d+1)-subsets of S whose closed simplex contains Y[g]} with the tolerance band `tol` of
  * sd_pointcloud_simplicial_f64 (enumerated, or counted for d = 2 when nS + 1 > 64, as there).

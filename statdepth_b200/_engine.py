@@ -6,6 +6,7 @@ compute entry point raises :class:`EngineUnavailable`.
 import ctypes as C
 import os
 import threading
+import warnings
 
 import numpy as np
 
@@ -82,6 +83,9 @@ SIGNATURES = {
                                         C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
     "sd_band_depth_oos_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                             C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
+    "sd_band_sort_rows_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]),
+    "sd_band_depth_sorted_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
+                                               C.c_int64, C.c_int, C.c_void_p]),
     "sd_pointcloud_simplicial_oos_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p,
                                                    C.c_int64, C.c_double, C.c_void_p]),
     "sd_pointcloud_l1_oos_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int64,
@@ -355,6 +359,18 @@ class Engine:
                                                        C.c_void_p(int(dY_ptr)), int(nY), int(ldY), int(j),
                                                        int(bool(relax)), C.c_void_p(int(d_out_ptr))))
 
+    def band_sort_rows_dev(self, dX_ptr, T, nS, ld, d_sorted_ptr):
+        """The index of a fitted reference: float64 [T, nS] rows of X (SD_LAYOUT_TN) sorted ascending, on the device."""
+        self._check(self.lib.sd_band_sort_rows_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(nS), int(ld),
+                                                       C.c_void_p(int(d_sorted_ptr))))
+
+    def band_depth_sorted_counts_dev(self, d_sorted_ptr, T, nS, dY_ptr, nY, ldY, J, d_out_ptr):
+        """Relaxed numerators of the new curves Y [T, nY] against sorted rows: int64 [(J - 1), nY] on the device,
+        row j - 2 equal to band_depth_oos_counts_dev(relax=True) for j."""
+        self._check(self.lib.sd_band_depth_sorted_f64_dev(self._ctx, C.c_void_p(int(d_sorted_ptr)), int(T), int(nS),
+                                                          C.c_void_p(int(dY_ptr)), int(nY), int(ldY), int(J),
+                                                          C.c_void_p(int(d_out_ptr))))
+
     def simplicial_oos_counts(self, S, Y, tol=1e-7):
         S = np.ascontiguousarray(S, dtype=np.float64)
         Y = np.ascontiguousarray(Y, dtype=np.float64)
@@ -432,6 +448,23 @@ class Engine:
         self._check(self.lib.sd_pointcloud_blocks_f64(self._ctx, _ptr(P), n, d, _ptr(mem), _ptr(off), _ptr(qp), B,
                                                       int(self.BLOCK_KINDS[kind]), float(tol), _ptr(hv), _ptr(out)))
         return out
+
+
+def device_rows(eng, X):
+    """(stream, dX): the rows X [T, n] as a C-order float64 tensor on eng's device, uploaded on eng's stream (so the
+    upload, later outputs and the engine's kernels are ordered on it).  A DataFrame's values are usually curve-major
+    (F order): that memory is uploaded as it is and transposed on the device, as sd_band_depth_f64 does with
+    SD_LAYOUT_NT (a host transpose of 819 MB takes over a second)."""
+    import torch
+    device = torch.device("cuda", eng.device)
+    stream = torch.cuda.ExternalStream(eng.stream(), device=device)
+    curve_major = X.strides[0] == X.itemsize and X.strides[1] != X.itemsize
+    host = np.ascontiguousarray(X.T if curve_major else X, dtype=np.float64)
+    with warnings.catch_warnings():
+        warnings.filterwarnings("ignore", message="The given NumPy array is not writable")  # only read here
+        with torch.cuda.stream(stream):
+            d = torch.from_numpy(host).to(device)
+            return stream, (d.t().contiguous() if curve_major else d)
 
 
 _engines = {}

@@ -18,7 +18,7 @@ from . import _dist, settings
 from ._engine import get_engine
 from ._helper import DepthDegeneracy, _check_containment, _handle_depth_errors
 
-__all__ = ['_functionaldepth', '_samplefunctionaldepth', '_functionaldepth_of']
+__all__ = ['_functionaldepth', '_samplefunctionaldepth', '_functionaldepth_of', '_relaxed_depths_of']
 
 
 def _positions(labels, axis_index: pd.Index, what: str) -> np.ndarray:
@@ -145,23 +145,28 @@ def _univariate_depths_of(S: np.ndarray, Y: np.ndarray, J: int, relax: bool) -> 
     if nY == 0:
         return depth
     ys = np.arange(nY, dtype=np.int64)
-    X = None
+    if relax:
+        # additive over time rows: shard the rows of the pooled [S | Y] matrix, split it at nS per block
+        X = np.ascontiguousarray(np.concatenate([S, Y], axis=1))
+        return _relaxed_depths_of([_dist.relaxed_counts(
+            lambda Xr, q, jj: eng.band_depth_oos_counts(Xr[:, :nS], Xr[:, nS:], jj, True)[q], X, ys, j)
+            for j in range(2, J + 1)], T, nS)
     for j in range(2, J + 1):
-        if relax:
-            # additive over time rows: shard the rows of the pooled [S | Y] matrix, split it at nS per block
-            if X is None:
-                X = np.ascontiguousarray(np.concatenate([S, Y], axis=1))
-            cnt = _dist.relaxed_counts(lambda Xr, q, jj: eng.band_depth_oos_counts(Xr[:, :nS], Xr[:, nS:], jj, True)[q],
-                                       X, ys, j)
-        else:
-            if j == 3:  # bd_triple_kernel enumerates the C(nS, 3) sample triples of every new curve
-                settings.check_enumeration(float(nY) * binom(nS, 3),
-                                           'out-of-sample strict band depth with J=3 (n=%d)' % (nS + 1))
-            cnt = _dist.query_sharded(lambda qb: eng.band_depth_oos_counts(S, Y[:, qb], j, False), ys, np.int64)
-        s_nj = cnt.astype(np.float64)
-        if relax:
-            s_nj = s_nj / float(T)
-        depth = depth + s_nj / binom(nS + 1, j)
+        if j == 3:  # bd_triple_kernel enumerates the C(nS, 3) sample triples of every new curve
+            settings.check_enumeration(float(nY) * binom(nS, 3),
+                                       'out-of-sample strict band depth with J=3 (n=%d)' % (nS + 1))
+        cnt = _dist.query_sharded(lambda qb: eng.band_depth_oos_counts(S, Y[:, qb], j, False), ys, np.int64)
+        depth = depth + cnt.astype(np.float64) / binom(nS + 1, j)
+    return depth
+
+
+def _relaxed_depths_of(counts, T: int, nS: int) -> np.ndarray:
+    """Relaxed out-of-sample depth from the numerators counts[j - 2] (j = 2..J): sum_j cnt_j / T / binom(nS + 1, j),
+    the arithmetic of _univariate_depths with n = nS + 1.  Every out-of-sample path forms its floats here, so equal
+    counts give bit-identical depths."""
+    depth = np.zeros(len(counts[0]), dtype=np.float64)
+    for j, cnt in enumerate(counts, start=2):
+        depth = depth + (np.asarray(cnt).astype(np.float64) / float(T)) / binom(nS + 1, j)
     return depth
 
 

@@ -11,7 +11,6 @@ per-row envelopes all-gathered, and the whisker pass runs after the outside coun
 """
 import math
 import numbers
-import warnings
 from fractions import Fraction
 from typing import List
 
@@ -20,7 +19,7 @@ import pandas as pd
 from scipy.special import binom
 
 from . import _dist
-from ._engine import get_engine
+from ._engine import device_rows, get_engine
 from ._functional import _values
 from ._helper import _handle_depth_errors
 
@@ -62,17 +61,7 @@ class _Rows:
         import torch
         self.torch = torch
         self.device = torch.device('cuda', eng.device)
-        # the engine's stream: the upload, the outputs and the engine's kernels are ordered on it
-        self.stream = torch.cuda.ExternalStream(eng.stream(), device=self.device)
-        # a DataFrame's values are usually curve-major (F order): upload that memory as it is and transpose on the
-        # device, as sd_band_depth_f64 does with SD_LAYOUT_NT (a host transpose of 819 MB takes over a second)
-        curve_major = X.strides[0] == X.itemsize and X.strides[1] != X.itemsize
-        host = np.ascontiguousarray(X.T if curve_major else X, dtype=np.float64)
-        with warnings.catch_warnings():
-            warnings.filterwarnings('ignore', message='The given NumPy array is not writable')  # only read here
-            with torch.cuda.stream(self.stream):
-                d = torch.from_numpy(host).to(self.device)
-                self.dX = d.t().contiguous() if curve_major else d
+        self.stream, self.dX = device_rows(eng, X)
 
     def _empty(self, size, dtype):
         return self.torch.empty(size, dtype=dtype, device=self.device)

@@ -30,6 +30,7 @@ SOURCES = {
     "bd_gemm.cu": [],
     "bd_match.cu": [],
     "oos.cu": [],
+    "reference.cu": [],
     "outliers.cu": ["-fmad=false"],
     "pointcloud.cu": ["-fmad=false"],
     "simplicial_count.cu": ["-fmad=false"],

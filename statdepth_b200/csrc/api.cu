@@ -452,6 +452,30 @@ int sd_band_depth_oos_f64_dev(sd_ctx *ctx, const double *dS, int64_t T, int64_t 
     return end_call(ctx, false);
 }
 
+// a fitted reference: sorted sample rows, and out-of-sample counts from them (reference.cu)
+int sd_band_sort_rows_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t nS, int64_t ld,
+                              double *d_sorted_out) {
+    SD_TRY(check_common(ctx, dX, d_sorted_out, "sd_band_sort_rows_f64_dev"));
+    SD_REQUIRE(T >= 1 && nS >= 1 && ld >= nS, "sd_band_sort_rows_f64_dev: bad sizes");
+    SD_TRY(begin_call(ctx));
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(sort_rows_device(ctx, dX, T, nS, ld, d_sorted_out));
+    SD_TRY(mark(ctx, 2));
+    return end_call(ctx, false);
+}
+
+int sd_band_depth_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t T, int64_t nS, const double *dY,
+                                 int64_t nY, int64_t ldY, int J, int64_t *d_count_out) {
+    SD_TRY(check_common(ctx, d_sorted, d_count_out, "sd_band_depth_sorted_f64_dev"));
+    SD_REQUIRE(dY || nY == 0, "sd_band_depth_sorted_f64_dev: NULL Y");
+    SD_REQUIRE(T >= 1 && nS >= 1 && nY >= 0 && ldY >= nY, "sd_band_depth_sorted_f64_dev: bad sizes");
+    SD_TRY(begin_call(ctx));
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(depth_sorted_device(ctx, d_sorted, T, nS, dY, nY, ldY, J, (i64 *)d_count_out));
+    SD_TRY(mark(ctx, 2));
+    return end_call(ctx, false);
+}
+
 // ---------------------------------------------------------------------------------------------
 // outlier detection: per-curve rank sums and masked envelopes, see outliers.cu
 // ---------------------------------------------------------------------------------------------

@@ -74,6 +74,12 @@ enum { ST_NONFINITE = 1, ST_INTERNAL = 2, ST_NO_MEMBER = 4 };
 
 __host__ __device__ static inline i64 ceil_div(i64 a, i64 b) { return (a + b - 1) / b; }
 
+// C(m, J) for J = 2, 3 in int64 (the band-depth j-terms of the out-of-sample kernels)
+__device__ __forceinline__ i64 oos_comb(const i64 m, const int J) {
+    if (J == 2) return m * (m - 1) / 2;
+    return m < 3 ? 0 : (m * (m - 1) / 2) * (m - 2) / 3;  // as comb3_dev (mbd.cu): the product is divisible by 3
+}
+
 // order-preserving map double -> u64 (with -0.0 folded onto +0.0 so that == ties stay ties)
 __host__ __device__ static inline u64 sortable_key(double x) {
     if (x == 0.0) x = 0.0;
@@ -164,8 +170,14 @@ int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride
 // out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out);
+// SD_ERR_OVERFLOW (message prefixed by who) unless T * C(nS, j) fits in int64
+int oos_overflow_check(i64 T, i64 nS, int j, const char *who);
 // int32 workspace for rank-only passes in row blocks of *RB rows (ints_per_row each) within a fixed budget
 int rank_block_workspace(sd_ctx *ctx, i64 T, i64 ints_per_row, i64 *RB, int **ws);
+// sorted reference rows and out-of-sample counts from them (reference.cu)
+int sort_rows_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 ld, double *d_sorted);
+int depth_sorted_device(sd_ctx *ctx, const double *d_sorted, i64 T, i64 nS, const double *dY, i64 nY, i64 ldY,
+                        int J, i64 *d_out);
 // outlier detection (outliers.cu)
 int rank_sums_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, i64 *d_q, i64 *d_b, i64 *d_a);
 int envelope_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const uint8_t *d_member, double factor,

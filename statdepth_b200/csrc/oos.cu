@@ -54,11 +54,6 @@ int finite_check_device(sd_ctx *ctx, const double *dX, i64 rows, i64 cols, i64 l
 constexpr int OOS_THREADS = 256;
 constexpr int OOS_ROWS = 32;  // time rows summed per thread before its one atomic
 
-__device__ __forceinline__ i64 oos_comb(const i64 m, const int J) {
-    if (J == 2) return m * (m - 1) / 2;
-    return m < 3 ? 0 : (m * (m - 1) / 2) * (m - 2) / 3;  // as comb3_dev (mbd.cu): the product is divisible by 3
-}
-
 // grid (new-curve tiles, row tiles).  One thread per (new curve g, OOS_ROWS rows): the rank rows are read
 // coalesced along g.  bY / aY == nullptr: a single new curve (no other new curve to subtract).
 template <int J>
@@ -88,6 +83,17 @@ __global__ void __launch_bounds__(OOS_THREADS) oos_terms_kernel(const int *__res
     }
     if (bad) atomicOr(status, ST_INTERNAL);
     if (sum) atomicAdd((u64 *)&acc[g], (u64)sum);
+}
+
+// overflow guard of band_depth_device with n - 1 = nS others: T * C(nS, j) (and 3 * C(nS, 3)) fit in int64
+int oos_overflow_check(i64 T, i64 nS, int j, const char *who) {
+    const long double full = (j == 2) ? (long double)nS * (nS - 1) / 2.0L
+                                      : (long double)nS * (nS - 1) * (nS - 2) / 6.0L;
+    if (full * (long double)T >= 9.0e18L || (j == 3 && 3.0L * full >= 9.0e18L)) {
+        set_error("%s: T*C(nS,%d) overflows int64 for T=%lld nS=%lld", who, j, (long long)T, (long long)nS);
+        return SD_ERR_OVERFLOW;
+    }
+    return SD_OK;
 }
 
 // Rank workspace of the rank-only passes, split into row blocks (also used by rank_sums_device, outliers.cu).
@@ -126,16 +132,7 @@ int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, 
         ctx->last.bd_impl_used = SD_BD_BITS;
         return bd_strict_device(ctx, dX, T, nS + 1, ld, d_q, nY, j, d_out);
     }
-    // overflow guard of band_depth_device with n - 1 = nS others: T * C(nS, j) (and 3 * C(nS, 3)) fit in int64
-    {
-        const long double full = (j == 2) ? (long double)nS * (nS - 1) / 2.0L
-                                          : (long double)nS * (nS - 1) * (nS - 2) / 6.0L;
-        if (full * (long double)T >= 9.0e18L || (j == 3 && 3.0L * full >= 9.0e18L)) {
-            set_error("out-of-sample band depth: T*C(nS,%d) overflows int64 for T=%lld nS=%lld", j, (long long)T,
-                      (long long)nS);
-            return SD_ERR_OVERFLOW;
-        }
-    }
+    SD_TRY(oos_overflow_check(T, nS, j, "out-of-sample band depth"));
     const i64 n = nS + nY;
     const i64 ny_ranks = nY > 1 ? nY : 0;  // one new curve: nothing to subtract, no second pass
     i64 RB = 0;

@@ -11,13 +11,14 @@ from typing import List, Union
 import numpy as np
 import pandas as pd
 
-from ._functional import _functionaldepth, _functionaldepth_of, _samplefunctionaldepth
+from ._functional import _functionaldepth, _functionaldepth_of, _samplefunctionaldepth, _values
 from ._helper import DepthDegeneracy  # noqa: F401  (re-exported like the reference's `from ._helper import *`)
 from ._outliers import _check_central, _checked_values, _functional_boxplot, _outliergram
 from ._pointcloud import _pointwisedepth, _pointwisedepth_of, _samplepointwisedepth
+from ._reference import _checked_reference, _query_values, _SortedReference
 
 __all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'FunctionalBoxplot',
-           'Outliergram', 'AbstractDepth']
+           'Outliergram', 'FunctionalReference', 'DepthClassifier', 'AbstractDepth']
 
 
 def _go():
@@ -381,3 +382,95 @@ def Outliergram(data: List[pd.DataFrame], factor=1.5, deep_check=False) -> _Outl
     Non-finite values are rejected."""
     X = _checked_values(data, factor, deep_check)
     return _Outliergram(data[0], _outliergram(X, float(factor)))
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# fitted references and depth-based classification (driver in _reference.py)
+# ---------------------------------------------------------------------------------------------------------------
+class FunctionalReference:
+    """A reference sample (sample[0], a T x n_S DataFrame) fitted once for relaxed out-of-sample band depth.
+
+    Construction sorts every time row of the sample on the GPU and keeps only that index; each depth_of() call then
+    uploads only the new curves and binary-searches them in the sorted rows.  depth_of([df]) equals
+    FunctionalDepthOf([df], sample, J=J, relax=True) bit for bit.  Only relaxed (modified) band depth, J = 2 or 3, on
+    univariate data is offered: a strict band must hold a curve at all T points jointly, which sorted rows cannot
+    decide.  Non-finite values are rejected.  close() (or leaving a `with` block) frees the index."""
+
+    def __init__(self, sample: List[pd.DataFrame], J=2, deep_check=False):
+        _checked_reference(sample, J, deep_check)
+        self.J = J
+        self._T = sample[0].shape[0]
+        self._index = sample[0].index
+        self._ref = _SortedReference(_values(sample[0]), J)
+
+    def depth_of(self, data: List[pd.DataFrame], deep_check=False) -> _FunctionalDepthUnivariate:
+        """Depth of every curve (column) of data[0] against the reference, indexed by data[0].columns (a label may
+        repeat a sample label)."""
+        if self._ref is None:
+            raise ValueError('the reference is closed')
+        Y = _query_values(data, self.J, deep_check, self._T, self._index)
+        depth = pd.Series(index=data[0].columns, data=self._ref.depths(Y))
+        return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+
+    def close(self) -> None:
+        if self._ref is not None:
+            self._ref.close()
+            self._ref = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+        return False
+
+
+class DepthClassifier:
+    """Maximum-depth classifier (Lopez-Pintado & Romo 2006): a curve belongs to the class in which it is deepest.
+
+    references maps each class label to its training curves ([DataFrame], T x n_k, the same T for every class); each
+    class is fitted once as a FunctionalReference.  depths([df]) are the DD-plot coordinates (one column per class,
+    equal to FunctionalDepthOf([df], references[label], J=J, relax=True)); predict([df]) takes the class of largest
+    depth, ties going to the class listed first."""
+
+    def __init__(self, references: dict, J=2, deep_check=False):
+        if not isinstance(references, dict) or len(references) < 2:
+            raise ValueError('references must be a dict of at least two classes.')
+        for sample in references.values():
+            _checked_reference(sample, J, deep_check)
+        if len({sample[0].shape[0] for sample in references.values()}) > 1:
+            raise ValueError('every class must have the same number of time points.')
+        self.labels = list(references)
+        self._refs = []
+        try:
+            for label in self.labels:
+                self._refs.append(FunctionalReference(references[label], J=J, deep_check=deep_check))
+        except BaseException:
+            self.close()
+            raise
+
+    def depths(self, data: List[pd.DataFrame], deep_check=False) -> pd.DataFrame:
+        """Depth of every curve of data[0] in every class: rows data[0].columns, one column per class label."""
+        if not self._refs:
+            raise ValueError('the classifier is closed')
+        cols = [ref.depth_of(data, deep_check=deep_check).values for ref in self._refs]
+        return pd.DataFrame(np.column_stack(cols), index=data[0].columns,
+                            columns=pd.Index(self.labels, tupleize_cols=False))
+
+    def predict(self, data: List[pd.DataFrame], deep_check=False) -> pd.Series:
+        """Label of the class of largest depth for every curve of data[0] (ties: the class listed first)."""
+        d = self.depths(data, deep_check=deep_check)
+        best = np.argmax(d.to_numpy(), axis=1)  # the first maximum
+        return pd.Series([self.labels[k] for k in best], index=d.index, dtype=object)
+
+    def close(self) -> None:
+        for ref in self._refs:
+            ref.close()
+        self._refs = []
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+        return False
