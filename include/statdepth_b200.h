@@ -299,6 +299,22 @@ int sd_band_envelope_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n
                              int64_t *d_outside_out);
 
 /*
+ * Extremal depth (Narisetty & Nair 2016).  b_t(c) / a_t(c) as for the rank sums above.
+ *
+ * Pointwise extremity: d_m_out[t*n + c] = |b_t(c) - a_t(c)| in [0, n - 1] (int32, row-major; the paper's pointwise
+ * depth is 1 - m / n).  Device pointers, SD_LAYOUT_TN.  Rows are independent: a block of time rows gives those rows
+ * of m.  SD_ERR_NONFINITE when X holds NaN or +-inf.
+ */
+int sd_band_extremity_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n, int64_t ld, int32_t *d_m_out);
+
+/* Numerators from the full extremity matrix d_m [T, n] (row-major): with key(c) = (m_t(c))_t sorted descending and
+ * keys compared lexicographically (larger = more extreme), d_num_out[c] = #{h : key(h) >= key(c)} in [1, n];
+ * ED = d_num_out / n, equal keys get equal numerators.  Device pointers, d_num_out holds n int64.  SD_ERR_INVALID
+ * when an m value lies outside [0, n - 1], when n > INT32_MAX, or when T > SD_EXTREMAL_T_MAX. */
+#define SD_EXTREMAL_T_MAX 16384
+int sd_extremal_depth_dev(sd_ctx *ctx, const int32_t *d_m, int64_t T, int64_t n, int64_t *d_num_out);
+
+/*
  * Batched band depth over sub-populations of one matrix (K-sampled blocks, homogeneity
  * permutations): membership[b*n + c] != 0 selects the curves of batch b; queries[b*nqb + i] is
  * the i-th query curve of batch b (must be a member).  count_out[b*nqb + i] as in

@@ -98,6 +98,8 @@ SIGNATURES = {
                                        C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sd_band_envelope_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                            C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sd_band_extremity_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]),
+    "sd_extremal_depth_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]),
     "sd_band_depth_batched_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                             C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -324,6 +326,17 @@ class Engine:
                                                       C.c_void_p(int(d_member_ptr)), float(factor),
                                                       C.c_void_p(int(d_lower_ptr)), C.c_void_p(int(d_upper_ptr)),
                                                       C.c_void_p(int(d_outside_ptr)) if d_outside_ptr else None))
+
+    # -- extremal depth ---------------------------------------------------------------------------------
+    def band_extremity_dev(self, dX_ptr, T, n, ld, d_m_ptr):
+        """Pointwise extremities |b - a| of the rows X [T, n] (SD_LAYOUT_TN): int32 [T, n] on the device."""
+        self._check(self.lib.sd_band_extremity_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
+                                                       C.c_void_p(int(d_m_ptr))))
+
+    def extremal_depth_dev(self, d_m_ptr, T, n, d_num_ptr):
+        """Extremal-depth numerators int64 [n] from the full extremity matrix int32 [T, n], on the device."""
+        self._check(self.lib.sd_extremal_depth_dev(self._ctx, C.c_void_p(int(d_m_ptr)), int(T), int(n),
+                                                   C.c_void_p(int(d_num_ptr))))
 
     # -- out-of-sample depth ----------------------------------------------------------------------------
     @staticmethod

@@ -1,5 +1,6 @@
-"""Functional outlier detection drivers: functional boxplot (Sun & Genton 2011) and outliergram (Arribas-Gil &
-Romo 2014), built on the integers K1 ranks with (csrc/outliers.cu, DESIGN.md K8).
+"""Functional outlier detection drivers: functional boxplot (Sun & Genton 2011), outliergram (Arribas-Gil & Romo
+2014) and extremal depth (Narisetty & Nair 2016), built on the integers K1 ranks with (csrc/outliers.cu, DESIGN.md
+K8; csrc/extremal.cu, K10).
 
 Both take univariate data X [T, n] (time rows x curves) and return plain arrays; depth.py wraps them in result
 objects.  Every per-curve quantity is exact int64 from the engine; floats are formed here once, at the end.
@@ -7,7 +8,9 @@ objects.  Every per-curve quantity is exact int64 from the engine; floats are fo
 On one GPU the matrix crosses PCIe once per call: the rows are uploaded once and every engine call reads them in
 place through the `_dev` entry points.  An engine without them (the CPU test double) gets the host matrix.  Under
 `enable_distributed()` every rank takes a block of time rows: the rank sums and outside counts are all-reduced, the
-per-row envelopes all-gathered, and the whisker pass runs after the outside counts are reduced.
+per-row envelopes all-gathered, and the whisker pass runs after the outside counts are reduced.  Extremal depth is
+not additive over rows: every rank computes the extremities of its rows, they are all-gathered through the host, and
+every rank orders the curves on the full matrix.
 """
 import math
 import numbers
@@ -23,24 +26,38 @@ from ._engine import device_rows, get_engine
 from ._functional import _values
 from ._helper import _handle_depth_errors
 
-__all__ = ['_checked_values', '_check_central', '_functional_boxplot', '_outliergram']
+__all__ = ['_checked_values', '_check_central', '_check_extremal_rows', '_functional_boxplot', '_outliergram',
+           '_extremal_depth']
+
+EXTREMAL_T_MAX = 16384  # SD_EXTREMAL_T_MAX (include/statdepth_b200.h): the bound of the per-curve sort on the GPU
 
 
 def _real(x) -> bool:
     return isinstance(x, numbers.Real) and not isinstance(x, bool)
 
 
-def _checked_values(data: List[pd.DataFrame], factor, deep_check=False) -> np.ndarray:
-    """The validation of FunctionalDepth([df], J=2, relax=True), then the outlier factor; X [T, n]."""
+NO_FACTOR = object()  # _checked_values without the outlier factor (None is a bad factor, not a missing one)
+
+
+def _checked_values(data: List[pd.DataFrame], factor, deep_check=False,
+                    what='functional outlier detection') -> np.ndarray:
+    """The validation of FunctionalDepth([df], J=2, relax=True), then the outlier factor (unless NO_FACTOR);
+    X [T, n]."""
     if isinstance(data, list) and len(data) > 1:
-        raise NotImplementedError('functional outlier detection is implemented for univariate data ([DataFrame])')
+        raise NotImplementedError('%s is implemented for univariate data ([DataFrame])' % what)
     _handle_depth_errors(data=data, J=2, containment='r2', relax=True, deep_check=deep_check)
-    if not (_real(factor) and math.isfinite(factor) and factor >= 0):
+    if factor is not NO_FACTOR and not (_real(factor) and math.isfinite(factor) and factor >= 0):
         raise ValueError('factor must be a finite number >= 0.')
     X = _values(data[0])
     if X.shape[1] < 2:
-        raise ValueError('functional outlier detection needs at least two curves.')
+        raise ValueError('%s needs at least two curves.' % what)
     return X
+
+
+def _check_extremal_rows(T: int) -> None:
+    if T > EXTREMAL_T_MAX:
+        raise NotImplementedError('extremal depth is implemented for up to %d time points (got %d)'
+                                  % (EXTREMAL_T_MAX, T))
 
 
 def _check_central(central) -> None:
@@ -91,6 +108,30 @@ class _Rows:
             qb = qb.cpu().numpy()
             return qb[0], qb[1]
 
+    def extremity(self) -> np.ndarray:
+        """m [T, n] int32: the pointwise extremities |b - a| of these rows, on the host."""
+        if self.T == 0:
+            return np.zeros((0, self.n), dtype=np.int32)
+        if not self.on_device:
+            return np.asarray(self.eng.band_extremity(self.X), dtype=np.int32)
+        with self.torch.cuda.stream(self.stream):
+            return self._extremity_dev().cpu().numpy()
+
+    def _extremity_dev(self):
+        m = self._empty((self.T, self.n), self.torch.int32)
+        self.eng.band_extremity_dev(self.dX.data_ptr(), self.T, self.n, self.n, m.data_ptr())
+        return m
+
+    def extremal_numerators(self) -> np.ndarray:
+        """e [n] with these rows as the whole matrix; on the device the extremities never leave it."""
+        if not self.on_device:
+            return _numerators_of(self.eng, self.extremity())
+        with self.torch.cuda.stream(self.stream):
+            m = self._extremity_dev()
+            e = self._empty(self.n, self.torch.int64)
+            self.eng.extremal_depth_dev(m.data_ptr(), self.T, self.n, e.data_ptr())
+            return e.cpu().numpy()
+
     def envelope(self, member: np.ndarray, factor: float, want_outside: bool):
         """(lo [T], hi [T], outside [n] or None) of these rows over the member curves."""
         if self.T == 0:
@@ -107,6 +148,21 @@ class _Rows:
                                        env[0].data_ptr(), env[1].data_ptr(), None if out is None else out.data_ptr())
             env = env.cpu().numpy()
             return env[0], env[1], None if out is None else out.cpu().numpy()
+
+
+def _numerators_of(eng, m: np.ndarray) -> np.ndarray:
+    """Extremal-depth numerators e [n] from the full extremity matrix m [T, n] (uploaded once on a GPU engine)."""
+    if not hasattr(eng, 'extremal_depth_dev'):
+        return np.asarray(eng.extremal_depth(m), dtype=np.int64)
+    import torch
+    device = torch.device('cuda', eng.device)
+    stream = torch.cuda.ExternalStream(eng.stream(), device=device)
+    T, n = m.shape
+    with torch.cuda.stream(stream):
+        dm = torch.from_numpy(np.ascontiguousarray(m, dtype=np.int32)).to(device)
+        e = torch.empty(n, dtype=torch.int64, device=device)
+        eng.extremal_depth_dev(dm.data_ptr(), T, n, e.data_ptr())
+        return e.cpu().numpy()
 
 
 def _local_rows(X: np.ndarray):
@@ -142,14 +198,33 @@ def central_count(central: float, n: int) -> int:
     return max(1, math.ceil(Fraction(central) * n))
 
 
-def _functional_boxplot(X: np.ndarray, factor: float, central: float) -> dict:
-    """Central region: the ceil(central * n) curves of largest MBD numerator Q, ties by column position.  Envelope
-    of the central region per row, fences inflated by factor * its width, outside counts against the fences, and the
-    whiskers: the envelope of every curve that never leaves the fences."""
+def _extremal_numerators(rows: _Rows, T: int, size: int) -> np.ndarray:
+    """e [n] of the whole matrix X [T, n] from this rank's rows (a collective when size > 1)."""
+    if size == 1:
+        return rows.extremal_numerators()
+    return _numerators_of(rows.eng, _dist.allgather_blocks(rows.extremity(), T))
+
+
+def _extremal_depth(X: np.ndarray) -> np.ndarray:
+    """Extremal-depth numerators e [n] of the curves of X [T, n]: ED = e / n."""
+    rows, size = _local_rows(X)
+    return _extremal_numerators(rows, X.shape[0], size)
+
+
+def _functional_boxplot(X: np.ndarray, factor: float, central: float, depth: str = 'mbd') -> dict:
+    """Central region: the ceil(central * n) curves of largest MBD numerator Q (depth='mbd') or extremal-depth
+    numerator e (depth='extremal'), ties by column position.  Envelope of the central region per row, fences inflated
+    by factor * its width, outside counts against the fences, and the whiskers: the envelope of every curve that
+    never leaves the fences."""
     T, n = X.shape
     rows, size = _local_rows(X)
-    q = _summed(rows.mbd_counts(), size)
-    order = np.argsort(-q, kind='stable')  # Q descending, then column position ascending
+    if depth == 'extremal':
+        q = _extremal_numerators(rows, T, size)
+        depths = q.astype(np.float64) / n
+    else:
+        q = _summed(rows.mbd_counts(), size)
+        depths = _mbd(q, T, n)
+    order = np.argsort(-q, kind='stable')  # Q (or e) descending, then column position ascending
     central_pos = order[:central_count(central, n)]
     member = np.zeros(n, dtype=np.uint8)
     member[central_pos] = 1
@@ -159,7 +234,7 @@ def _functional_boxplot(X: np.ndarray, factor: float, central: float) -> dict:
     inside = (outside == 0).astype(np.uint8)  # never empty for factor >= 0: the central curves are inside
     wlo, whi, _ = rows.envelope(inside, 0.0, False)
     lower, upper = fences(lo, hi, factor)
-    return dict(depth=_mbd(q, T, n), q=q, central=central_pos, envelope=(lo, hi), fences=(lower, upper),
+    return dict(depth=depths, q=q, central=central_pos, envelope=(lo, hi), fences=(lower, upper),
                 whiskers=(_gathered(wlo, T, size), _gathered(whi, T, size)), outside=outside)
 
 

@@ -31,6 +31,7 @@ SOURCES = {
     "bd_match.cu": [],
     "oos.cu": [],
     "reference.cu": [],
+    "extremal.cu": [],
     "outliers.cu": ["-fmad=false"],
     "pointcloud.cu": ["-fmad=false"],
     "simplicial_count.cu": ["-fmad=false"],

@@ -564,6 +564,27 @@ int sd_band_envelope_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n
     return end_call(ctx, false);
 }
 
+// extremal depth: pointwise extremities of a block of rows, numerators from the full matrix (extremal.cu)
+int sd_band_extremity_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n, int64_t ld, int32_t *d_m_out) {
+    SD_TRY(check_common(ctx, dX, d_m_out, "sd_band_extremity_f64_dev"));
+    SD_TRY(check_matrix("sd_band_extremity_f64_dev", T, n, ld, SD_LAYOUT_TN));
+    SD_TRY(begin_call(ctx));
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(extremity_device(ctx, dX, T, n, ld, (int *)d_m_out));
+    SD_TRY(mark(ctx, 2));
+    return end_call(ctx, false);
+}
+
+int sd_extremal_depth_dev(sd_ctx *ctx, const int32_t *d_m, int64_t T, int64_t n, int64_t *d_num_out) {
+    SD_TRY(check_common(ctx, d_m, d_num_out, "sd_extremal_depth_dev"));
+    SD_REQUIRE(T >= 1 && n >= 1, "sd_extremal_depth_dev: bad sizes T=%lld n=%lld", (long long)T, (long long)n);
+    SD_TRY(begin_call(ctx));
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(extremal_depth_device(ctx, (const int *)d_m, T, n, (i64 *)d_num_out));
+    SD_TRY(mark(ctx, 2));
+    return end_call(ctx, false);
+}
+
 // point clouds: [S; Y] rows, query ids nS .. nS + nY - 1
 static int pooled_cloud(sd_ctx *ctx, const double *S, int64_t nS, int d, const double *Y, int64_t nY, double **dP,
                         const i64 **d_q) {

@@ -66,11 +66,13 @@ enum BufId {
     BUF_RANKS,      // strict BD matcher: per-time-point ranks of all curves (packed pairs)
     BUF_GEOM,       // Oja counting: the pool's points and the queries' positions inside the pool
     BUF_SLAB,       // MBD slab path: per-row maps, bucket tables, bin starts
+    BUF_KEYS,       // extremal depth: per-curve sorted extremities, u32 [n][T] (none of the above is used with it)
+    BUF_ORDER,      // extremal depth: curve ids, group starts, merge-sort / scan temp storage
     NUM_BUFS
 };
 
 // status bits written by kernels into ctx->d_status
-enum { ST_NONFINITE = 1, ST_INTERNAL = 2, ST_NO_MEMBER = 4 };
+enum { ST_NONFINITE = 1, ST_INTERNAL = 2, ST_NO_MEMBER = 4, ST_BAD_INPUT = 8 };  // ST_BAD_INPUT: caller data out of range
 
 __host__ __device__ static inline i64 ceil_div(i64 a, i64 b) { return (a + b - 1) / b; }
 
@@ -182,6 +184,9 @@ int depth_sorted_device(sd_ctx *ctx, const double *d_sorted, i64 T, i64 nS, cons
 int rank_sums_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, i64 *d_q, i64 *d_b, i64 *d_a);
 int envelope_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const uint8_t *d_member, double factor,
                     double *d_lower, double *d_upper, i64 *d_outside);
+// extremal depth (extremal.cu): m = |b - a| of rows, and the numerators e from the full m
+int extremity_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, int *d_m);
+int extremal_depth_device(sd_ctx *ctx, const int *d_m, i64 T, i64 n, i64 *d_e);
 int iota_from_device(sd_ctx *ctx, i64 *d_p, i64 count, i64 base);
 int finite_check_device(sd_ctx *ctx, const double *dX, i64 rows, i64 cols, i64 ld);
 int oja2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, const i64 *d_q, i64 nq, double hull_volume,

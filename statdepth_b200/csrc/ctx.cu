@@ -87,6 +87,10 @@ int check_status(sd_ctx *ctx) {
         set_error("the member mask selects no curve");
         return SD_ERR_INVALID;
     }
+    if (st & ST_BAD_INPUT) {
+        set_error("input value out of range (extremities must lie in [0, n - 1])");
+        return SD_ERR_INVALID;
+    }
     if (st & ST_INTERNAL) {
         set_error("internal consistency check failed on the device (status=%d)", st);
         return SD_ERR_CUDA;

@@ -13,12 +13,13 @@ import pandas as pd
 
 from ._functional import _functionaldepth, _functionaldepth_of, _samplefunctionaldepth, _values
 from ._helper import DepthDegeneracy  # noqa: F401  (re-exported like the reference's `from ._helper import *`)
-from ._outliers import _check_central, _checked_values, _functional_boxplot, _outliergram
+from ._outliers import (NO_FACTOR, _check_central, _check_extremal_rows, _checked_values, _extremal_depth,
+                        _functional_boxplot, _outliergram)
 from ._pointcloud import _pointwisedepth, _pointwisedepth_of, _samplepointwisedepth
 from ._reference import _checked_reference, _query_values, _SortedReference
 
-__all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'FunctionalBoxplot',
-           'Outliergram', 'FunctionalReference', 'DepthClassifier', 'AbstractDepth']
+__all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'ExtremalDepth',
+           'FunctionalBoxplot', 'Outliergram', 'FunctionalReference', 'DepthClassifier', 'AbstractDepth']
 
 
 def _go():
@@ -290,6 +291,21 @@ def PointcloudDepthOf(
     return _PointwiseDepth(df=data, depths=depth)
 
 
+def ExtremalDepth(data: List[pd.DataFrame], deep_check=False) -> _FunctionalDepthUnivariate:
+    """Extremal depth (Narisetty & Nair 2016) of the curves (columns) of data[0], a T x n DataFrame.
+
+    At every time point a curve's extremity is |#curves strictly below - #curves strictly above|.  Curves are ordered
+    by their extremities sorted from largest down, compared lexicographically, so a curve that is extreme somewhere,
+    even for a short stretch, ranks as extreme (modified band depth averages such a stretch away).  The depth is the
+    share of curves at least as extreme: the deepest curve has 1, equally extreme curves have equal depth.  Indexed
+    by data[0].columns.  Univariate data with at most 16 384 time points; non-finite values are rejected."""
+    X = _checked_values(data, NO_FACTOR, deep_check, what='extremal depth')
+    _check_extremal_rows(X.shape[0])
+    e = _extremal_depth(X)
+    return _FunctionalDepthUnivariate(df=data[0], depths=pd.Series(index=data[0].columns,
+                                                                   data=e.astype(np.float64) / X.shape[1]))
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # functional outlier detection (drivers in _outliers.py)
 # ---------------------------------------------------------------------------------------------------------------
@@ -310,7 +326,8 @@ class _OutlierResult:
         return pd.DataFrame({'lower': pair[0], 'upper': pair[1]}, index=self._df.index)
 
     def depths(self) -> _FunctionalDepthUnivariate:
-        """Modified band depth of every curve, bit-identical to FunctionalDepth([df], J=2, relax=True)."""
+        """Modified band depth of every curve, bit-identical to FunctionalDepth([df], J=2, relax=True) (the
+        boxplot with depth='extremal': extremal depth, equal to ExtremalDepth([df]))."""
         return _FunctionalDepthUnivariate(df=self._df, depths=self._series(self._r['depth']))
 
     def outliers(self) -> list:
@@ -364,16 +381,23 @@ class _Outliergram(_OutlierResult):
         return self._r['outlier']
 
 
-def FunctionalBoxplot(data: List[pd.DataFrame], factor=1.5, central=0.5, deep_check=False) -> _FunctionalBoxplot:
+def FunctionalBoxplot(data: List[pd.DataFrame], factor=1.5, central=0.5, deep_check=False,
+                      depth='mbd') -> _FunctionalBoxplot:
     """Functional boxplot of the curves (columns) of data[0], a T x n DataFrame.
 
-    The central region is the ceil(central * n) curves of largest modified band depth (ties by column position;
-    under ties this can differ from ordered(), whose sort is not stable).  Its per-row envelope, inflated by
-    factor x its width, gives the fences; a curve strictly outside them at any time point is a magnitude outlier.
+    The central region is the ceil(central * n) curves of largest depth (ties by column position; under ties this
+    can differ from ordered(), whose sort is not stable): modified band depth with depth='mbd', extremal depth
+    (ExtremalDepth) with depth='extremal', which keeps curves that leave the bulk for a short stretch out of the
+    central region.  Its per-row envelope, inflated by factor x its width, gives the fences; a curve strictly
+    outside them at any time point is a magnitude outlier.  depths() returns the depth the region was ranked by.
     Non-finite values are rejected."""
     X = _checked_values(data, factor, deep_check)
     _check_central(central)
-    return _FunctionalBoxplot(data[0], _functional_boxplot(X, float(factor), float(central)))
+    if not (isinstance(depth, str) and depth in ('mbd', 'extremal')):
+        raise ValueError("depth must be 'mbd' or 'extremal'.")
+    if depth == 'extremal':
+        _check_extremal_rows(X.shape[0])
+    return _FunctionalBoxplot(data[0], _functional_boxplot(X, float(factor), float(central), depth))
 
 
 def Outliergram(data: List[pd.DataFrame], factor=1.5, deep_check=False) -> _Outliergram:
