@@ -315,6 +315,28 @@ int sd_band_extremity_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t 
 int sd_extremal_depth_dev(sd_ctx *ctx, const int32_t *d_m, int64_t T, int64_t n, int64_t *d_num_out);
 
 /*
+ * Halfspace (Tukey) depth numerators, exact int64 (decisions: exact angular keys, no tolerance band).
+ * h(p) = min over closed half-planes H whose boundary passes through p of #{i : x_i in H}, p itself counted; the host
+ * divides by n.  d = 1: h = n - max(b, a), b / a the other points strictly below / above p.  d = 2: with z = #points
+ * equal to p (p included), the m directions v_i = x_i - p != 0 and k_i = #{directions in the half-turn
+ * (phi_i, phi_i + pi]}, h = z + min_i min(k_i, m - k_i), and h = n when m = 0.  Directions are compared by the exact
+ * angular keys of the computed float64 differences (the tol = 0 decisions of the simplicial counting).
+ * SD_ERR_NONFINITE when the input holds NaN or +-inf; SD_ERR_UNSUPPORTED for another d, and beyond the size limits
+ * of the angular counting (2n < 2^31, d = 2) and of the rank pipeline (n < 2^31).
+ */
+int sd_pointcloud_halfspace_f64(sd_ctx *ctx, const double *P, int64_t n, int d, const int64_t *query_idx,
+                                int64_t nq, int64_t *count_out);             /* d in {1,2}; count in [1, n] */
+int sd_functional_halfspace_f64(sd_ctx *ctx, const double *F, int64_t N, int64_t T, int d,
+                                const int64_t *query_idx, int64_t nq, int64_t *count_out);
+                                /* F[(i*T + t)*d + c] as sd_simplex_depth_f64, d = 2; sum_t h_t in [T, T*N] */
+int sd_band_halfspace_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_t ld, int layout,
+                          int64_t *count_out);                               /* univariate, all n curves */
+
+/* same with DEVICE pointers, SD_LAYOUT_TN only; additive over disjoint blocks of time rows */
+int sd_band_halfspace_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n, int64_t ld,
+                              int64_t *d_count_out);
+
+/*
  * Batched band depth over sub-populations of one matrix (K-sampled blocks, homogeneity
  * permutations): membership[b*n + c] != 0 selects the curves of batch b; queries[b*nqb + i] is
  * the i-th query curve of batch b (must be a member).  count_out[b*nqb + i] as in

@@ -100,6 +100,13 @@ SIGNATURES = {
                                            C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sd_band_extremity_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]),
     "sd_extremal_depth_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]),
+    "sd_pointcloud_halfspace_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int64,
+                                              C.c_void_p]),
+    "sd_functional_halfspace_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p,
+                                              C.c_int64, C.c_void_p]),
+    "sd_band_halfspace_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int,
+                                        C.c_void_p]),
+    "sd_band_halfspace_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]),
     "sd_band_depth_batched_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                             C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -337,6 +344,41 @@ class Engine:
         """Extremal-depth numerators int64 [n] from the full extremity matrix int32 [T, n], on the device."""
         self._check(self.lib.sd_extremal_depth_dev(self._ctx, C.c_void_p(int(d_m_ptr)), int(T), int(n),
                                                    C.c_void_p(int(d_num_ptr))))
+
+    # -- halfspace (Tukey) depth -----------------------------------------------------------------------
+    def halfspace_counts(self, P, queries=None):
+        """Numerators h in [1, n] of the points of the cloud P [n, d], d = 1 or 2: the fewest points, p itself
+        included, in a closed half-plane (half-line) whose boundary passes through p.  HD = h / n."""
+        P = np.ascontiguousarray(P, dtype=np.float64)
+        n, d = P.shape
+        q, nq = self._queries(queries, n)
+        out = np.empty(nq, dtype=np.int64)
+        self._check(self.lib.sd_pointcloud_halfspace_f64(self._ctx, _ptr(P), n, d, _ptr(q), nq, _ptr(out)))
+        return out
+
+    def functional_halfspace_counts(self, F, queries=None):
+        """sum over t of the numerator of curve c at time t among the N values F[:, t] (F [N, T, 2]), per query."""
+        F = np.ascontiguousarray(F, dtype=np.float64)
+        N, T, d = F.shape
+        q, nq = self._queries(queries, N)
+        out = np.empty(nq, dtype=np.int64)
+        self._check(self.lib.sd_functional_halfspace_f64(self._ctx, _ptr(F), N, T, d, _ptr(q), nq, _ptr(out)))
+        return out
+
+    def band_halfspace_counts(self, X):
+        """int64 [n]: sum over the time rows of X [T, n] of n - max(b_t, a_t), b_t / a_t the other curves strictly
+        below / above.  An F-ordered X is passed with SD_LAYOUT_NT."""
+        X, is_f = self._matrix(X)
+        T, n = X.shape
+        out = np.empty(n, dtype=np.int64)
+        self._check(self.lib.sd_band_halfspace_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, T if is_f else n,
+                                                   LAYOUT_NT if is_f else LAYOUT_TN, _ptr(out)))
+        return out
+
+    def band_halfspace_counts_dev(self, dX_ptr, T, n, ld, d_out_ptr):
+        """Device-pointer variant (SD_LAYOUT_TN): int64 [n] stays on the device."""
+        self._check(self.lib.sd_band_halfspace_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
+                                                       C.c_void_p(int(d_out_ptr))))
 
     # -- out-of-sample depth ----------------------------------------------------------------------------
     @staticmethod

@@ -32,6 +32,7 @@ SOURCES = {
     "oos.cu": [],
     "reference.cu": [],
     "extremal.cu": [],
+    "halfspace.cu": [],
     "outliers.cu": ["-fmad=false"],
     "pointcloud.cu": ["-fmad=false"],
     "simplicial_count.cu": ["-fmad=false"],

@@ -585,6 +585,91 @@ int sd_extremal_depth_dev(sd_ctx *ctx, const int32_t *d_m, int64_t T, int64_t n,
     return end_call(ctx, false);
 }
 
+// halfspace (Tukey) depth numerators (K11): d = 1 from K1's ranks (halfspace.cu), d = 2 from the angular keys
+// (hs_reduce_kernel, simplicial_count.cu).  Every value is finite-checked whatever the queries; the row lengths are
+// checked by the rank pipeline (n < 2^31) and the angular counting (2n < 2^31).
+
+int sd_pointcloud_halfspace_f64(sd_ctx *ctx, const double *P, int64_t n, int d, const int64_t *query_idx,
+                                int64_t nq, int64_t *count_out) {
+    SD_TRY(check_common(ctx, P, count_out, "sd_pointcloud_halfspace_f64"));
+    SD_REQUIRE(n >= 1 && nq >= 0, "sd_pointcloud_halfspace_f64: bad sizes");
+    if (d != 1 && d != 2) {
+        set_error("sd_pointcloud_halfspace_f64: d=%d not supported (1 or 2)", d);
+        return SD_ERR_UNSUPPORTED;
+    }
+    SD_TRY(begin_call(ctx));
+    double *dP = nullptr;
+    SD_TRY(upload_matrix(ctx, BUF_IN, P, 1, n * d, n * d, &dP));
+    const i64 *d_q = nullptr;
+    SD_TRY(upload_queries(ctx, query_idx, nq, n, &d_q, "sd_pointcloud_halfspace_f64"));
+    SD_TRY(ctx->buf[BUF_OUT].reserve((size_t)(nq + (d == 1 ? n : 0) + 1) * sizeof(i64)));
+    i64 *d_out = ctx->buf[BUF_OUT].as<i64>();
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(finite_check_device(ctx, dP, 1, n * d, n * d));
+    if (d == 2) {
+        SD_TRY(simplicial2_count_device(ctx, dP, n, 2, 1, d_q, nq, 0.0, d_out, -1, SC_HALFSPACE));
+    } else {  // one row of n values: every point's numerator, then the queries'
+        i64 *d_all = d_out + nq;
+        SD_TRY(halfspace1_device(ctx, dP, 1, n, n, d_all));
+        SD_TRY(gather_i64_device(ctx, d_all, d_q, nq, d_out));
+    }
+    SD_TRY(mark(ctx, 2));
+    if (nq > 0)
+        SD_CUDA(cudaMemcpyAsync(count_out, d_out, (size_t)nq * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
+    return end_call(ctx, true);
+}
+
+int sd_functional_halfspace_f64(sd_ctx *ctx, const double *F, int64_t N, int64_t T, int d, const int64_t *query_idx,
+                                int64_t nq, int64_t *count_out) {
+    SD_TRY(check_common(ctx, F, count_out, "sd_functional_halfspace_f64"));
+    SD_REQUIRE(N >= 1 && T >= 1 && nq >= 0, "sd_functional_halfspace_f64: bad sizes");
+    if (d != 2) {
+        set_error("sd_functional_halfspace_f64: d=%d not supported (2)", d);
+        return SD_ERR_UNSUPPORTED;
+    }
+    SD_TRY(begin_call(ctx));
+    double *dF = nullptr;
+    SD_TRY(upload_matrix(ctx, BUF_IN, F, 1, N * T * d, N * T * d, &dF));
+    const i64 *d_q = nullptr;
+    SD_TRY(upload_queries(ctx, query_idx, nq, N, &d_q, "sd_functional_halfspace_f64"));
+    SD_TRY(ctx->buf[BUF_OUT].reserve((size_t)(nq > 0 ? nq : 1) * sizeof(i64)));
+    i64 *d_out = ctx->buf[BUF_OUT].as<i64>();
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(finite_check_device(ctx, dF, 1, N * T * d, N * T * d));
+    SD_TRY(simplicial2_count_device(ctx, dF, N, 2 * T, T, d_q, nq, 0.0, d_out, -1, SC_HALFSPACE));
+    SD_TRY(mark(ctx, 2));
+    if (nq > 0)
+        SD_CUDA(cudaMemcpyAsync(count_out, d_out, (size_t)nq * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
+    return end_call(ctx, true);
+}
+
+int sd_band_halfspace_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_t ld, int layout,
+                          int64_t *count_out) {
+    SD_TRY(check_common(ctx, X, count_out, "sd_band_halfspace_f64"));
+    SD_TRY(check_matrix("sd_band_halfspace_f64", T, n, ld, layout));
+    SD_TRY(begin_call(ctx));
+    double *dX = nullptr;
+    SD_TRY(upload_tn(ctx, X, T, n, ld, layout, &dX));
+    SD_TRY(ctx->buf[BUF_OUT].reserve((size_t)n * sizeof(i64)));
+    i64 *d_out = ctx->buf[BUF_OUT].as<i64>();
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(halfspace1_device(ctx, dX, T, n, n, d_out));
+    SD_TRY(mark(ctx, 2));
+    SD_CUDA(cudaMemcpyAsync(count_out, d_out, (size_t)n * sizeof(i64), cudaMemcpyDeviceToHost, ctx->stream));
+    return end_call(ctx, true);
+}
+
+int sd_band_halfspace_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n, int64_t ld,
+                              int64_t *d_count_out) {
+    SD_TRY(check_common(ctx, dX, d_count_out, "sd_band_halfspace_f64_dev"));
+    SD_TRY(check_matrix("sd_band_halfspace_f64_dev", T, n, ld, SD_LAYOUT_TN));
+    SD_TRY(begin_call(ctx));
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(halfspace1_device(ctx, dX, T, n, ld, (i64 *)d_count_out));
+    SD_TRY(mark(ctx, 2));
+    return end_call(ctx, false);
+}
+
 // point clouds: [S; Y] rows, query ids nS .. nS + nY - 1
 static int pooled_cloud(sd_ctx *ctx, const double *S, int64_t nS, int d, const double *Y, int64_t nY, double **dP,
                         const i64 **d_q) {

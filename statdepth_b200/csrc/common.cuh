@@ -167,8 +167,12 @@ int cloud_blocks_device(sd_ctx *ctx, const double *dP, int d, const i64 *d_membe
                         const i64 *d_qpos, i64 B, int kind, double tol, const double *d_volume, double *d_out);
 int simplicial_device(sd_ctx *ctx, const double *dP, i64 n, int d, const i64 *d_q, i64 nq, double tol,
                       i64 *d_out, bool oos = false);
+// what simplicial2_count_device reduces the two rank passes of the angular keys to (simplicial_count.cu)
+enum ScReduce { SC_TRIANGLES, SC_HALFSPACE };
 int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride_j, i64 T, const i64 *d_q, i64 nq,
-                             double tol, i64 *d_out, i64 m_others = -1);
+                             double tol, i64 *d_out, i64 m_others = -1, ScReduce reduce = SC_TRIANGLES);
+// halfspace depth, d = 1 (halfspace.cu): d_out[c] = sum_t (n - max(b_t(c), a_t(c))) over the rows of X [T, n]
+int halfspace1_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, i64 *d_out);
 // out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out);

@@ -34,6 +34,8 @@
 // the open half-turns of the exact formula.  Angles here come from atan2 / acos (a few ulp): decisions can
 // differ from the enumeration predicate only for triangles whose distance to p is within ~1e-15 |x - p| of
 // tol, far inside the documented tie band of the LP itself (DESIGN.md "Oracle and parity").
+// Halfspace (Tukey) depth (K11) reduces the same keys and rank passes (tol = 0) to a minimum of half-turn counts
+// instead: hs_reduce_kernel, selected by simplicial2_count_device's `reduce`.
 #include "angular_key.cuh"
 #include "common.cuh"
 
@@ -90,6 +92,34 @@ __global__ void __launch_bounds__(256) sc_keys_kernel(const ScGeom g, const i64 
 
 __device__ __forceinline__ i64 c3(i64 m) { return m < 3 ? 0 : (m * (m - 1) / 2) * (m - 2) / 3; }
 
+// pass 1 of the reductions, block-wide: the number of real directions m' and how many of them lie in [0, pi)
+// (key < 12); ARCS: `low` counts the arcs that wrap past 2 pi (end below start).  kb_hi = second half of row B.
+template <bool ARCS>
+__device__ __forceinline__ void sc_count_real(const double *__restrict__ ka, const double *__restrict__ kb_hi,
+                                              const i64 n, i64 *s_cnt, i64 &mreal, i64 &low_out) {
+    i64 real = 0, low = 0;
+    for (i64 j = threadIdx.x; j < n; j += blockDim.x) {
+        const double u = ka[j];
+        real += u < 16.0;
+        if (ARCS) low += u < 16.0 && kb_hi[j] < u;
+        else low += u < 12.0;
+    }
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) {
+        real += __shfl_xor_sync(0xffffffffu, real, s);
+        low += __shfl_xor_sync(0xffffffffu, low, s);
+    }
+    if (threadIdx.x == 0) { s_cnt[0] = 0; s_cnt[1] = 0; }
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0) {
+        atomicAdd((u64 *)&s_cnt[0], (u64)real);
+        atomicAdd((u64 *)&s_cnt[1], (u64)low);
+    }
+    __syncthreads();
+    mreal = s_cnt[0];
+    low_out = s_cnt[1];
+}
+
 // one CTA per instance.  bA/aA: ranks of row A; bB/aB: ranks (strictly below / above) of row B.
 // out[query slot] += #triangles of other points containing the query point (ARCS: meeting the disk D(p, tol)).
 template <bool ARCS>
@@ -106,28 +136,9 @@ __global__ void __launch_bounds__(256) sc_reduce_kernel(const ScGeom g, const i6
     const double *ka = KA + li * n;
     const int *ba = bA + li * n, *aa = aA + li * n, *bb = bB + li * 2 * n, *ab = aB + li * 2 * n;
     int *cl = claim + li * n;
-    // pass 1: number of real directions m' and how many of them lie in [0, pi)  (key < 12);
-    // ARCS: `low` counts the arcs that wrap past 2 pi (end below start)
-    i64 real = 0, low = 0;
-    for (i64 j = threadIdx.x; j < n; j += blockDim.x) {
-        const double u = ka[j];
-        real += u < 16.0;
-        if (ARCS) low += u < 16.0 && KB[li * 2 * n + n + j] < u;
-        else low += u < 12.0;
-    }
-#pragma unroll
-    for (int s = 16; s > 0; s >>= 1) {
-        real += __shfl_xor_sync(0xffffffffu, real, s);
-        low += __shfl_xor_sync(0xffffffffu, low, s);
-    }
-    if (threadIdx.x == 0) { s_cnt[0] = 0; s_cnt[1] = 0; }
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) {
-        atomicAdd((u64 *)&s_cnt[0], (u64)real);
-        atomicAdd((u64 *)&s_cnt[1], (u64)low);
-    }
-    __syncthreads();
-    const i64 mreal = s_cnt[0], L4 = s_cnt[1], H = mreal - L4;
+    i64 mreal, L4;
+    sc_count_real<ARCS>(ka, KB + li * 2 * n + n, n, s_cnt, mreal, L4);
+    const i64 H = mreal - L4;
     // pass 2: every class of equal directions contributes C(g + c, 3) - C(c, 3) once
     i64 noncontain = 0;
     for (i64 j = threadIdx.x; j < n; j += blockDim.x) {
@@ -165,16 +176,70 @@ __global__ void __launch_bounds__(256) sc_reduce_kernel(const ScGeom g, const i6
     }
 }
 
+// Halfspace (Tukey) depth numerator, one CTA per instance (tolerance 0 keys only):
+//     h = z + min over real directions j of min(k_j, m' - k_j),   k_j = #{real directions in (phi_j, phi_j + pi]}
+// z = n - m' counts the query itself and the points equal to it; h = n when no direction is real (the min starts at
+// m').  k_j = c + g_anti: c = directions strictly inside the half-turn (as the tol = 0 branch of sc_reduce_kernel),
+// g_anti = entries of row B equal to the antipode (2n - bB - aB at n + j) less the g antipodes of j's own class.
+// Every member of a class gives the same k and min is idempotent: no claim array.  out[inst] = h for point clouds
+// (T = 1), out[inst / T] += h for curves.  A k outside [0, m'] sets ST_INTERNAL.
+__global__ void __launch_bounds__(256) hs_reduce_kernel(const ScGeom g, const i64 n, const double *__restrict__ KA,
+                                                        const double *__restrict__ KB,
+                                                        const int *__restrict__ bA, const int *__restrict__ aA,
+                                                        const int *__restrict__ bB, const int *__restrict__ aB,
+                                                        i64 *__restrict__ out, int *__restrict__ status) {
+    __shared__ i64 s_red[8];
+    __shared__ i64 s_cnt[2];
+    const i64 li = blockIdx.x;
+    const i64 inst = g.inst0 + li;
+    const double *ka = KA + li * n;
+    const int *ba = bA + li * n, *aa = aA + li * n, *bb = bB + li * 2 * n, *ab = aB + li * 2 * n;
+    i64 mreal, L4;
+    sc_count_real<false>(ka, KB + li * 2 * n + n, n, s_cnt, mreal, L4);
+    const i64 H = mreal - L4;
+    i64 best = mreal;
+    bool bad = false;
+    for (i64 j = threadIdx.x; j < n; j += blockDim.x) {
+        const double u = ka[j];
+        if (!(u < 16.0)) continue;
+        const i64 L = ba[j];
+        const i64 gsz = n - L - (i64)aa[j];
+        const i64 b2w = bb[n + j];
+        const i64 c = u < 12.0 ? (b2w - L - H) - L - gsz : (mreal - L - gsz) + (b2w - L + L4);
+        const i64 k = c + (2 * n - b2w - (i64)ab[n + j]) - gsz;
+        bad |= k < 0 || k > mreal;
+        const i64 side = k < mreal - k ? k : mreal - k;
+        best = side < best ? side : best;
+    }
+    if (bad) atomicOr(status, ST_INTERNAL);
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) {
+        const i64 o = __shfl_xor_sync(0xffffffffu, best, s);
+        best = o < best ? o : best;
+    }
+    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = best;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < (int)(blockDim.x >> 5); ++w) best = s_red[w] < best ? s_red[w] : best;
+        const i64 h = n - mreal + best;
+        if (g.T == 1) out[inst] = h;
+        else atomicAdd((u64 *)&out[inst / g.T], (u64)h);
+    }
+}
+
 // Counts for `nq` queries x `T` instances each (T = 1 for point clouds).  d_out[nq] is zeroed here.
 // m_others < 0: the queries are among the n points (n - 1 others); m_others = n: out-of-sample queries (ids >= n,
 // coordinates read from the same array), every one of the n points is an other.
+// reduce: SC_TRIANGLES (sc_reduce_kernel) or SC_HALFSPACE (hs_reduce_kernel: tol = 0, in-sample queries).
 int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride_j, i64 T, const i64 *d_q, i64 nq,
-                             double tol, i64 *d_out, i64 m_others) {
+                             double tol, i64 *d_out, i64 m_others, ScReduce reduce) {
     cudaStream_t st = ctx->stream;
     SD_CUDA(cudaMemsetAsync(d_out, 0, (size_t)nq * sizeof(i64), st));
     const i64 ninst_total = nq * T;
+    const bool hs = reduce == SC_HALFSPACE;
     if (m_others < 0) m_others = n - 1;
-    if (ninst_total == 0 || m_others < 3) return SD_OK;  // fewer than 3 other points: no triangle
+    if (ninst_total == 0) return SD_OK;
+    if (!hs && m_others < 3) return SD_OK;  // fewer than 3 other points: no triangle
     if (2 * n >= (1ll << 31)) {
         set_error("simplicial counting: n=%lld too large", (long long)n);
         return SD_ERR_UNSUPPORTED;
@@ -213,10 +278,11 @@ int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride
         }
         sc_keys_kernel<<<dim3(gx, (unsigned)ni), 256, 0, st>>>(g, n, ni, tol, KA, KB, ctx->d_status);
         ctx->last.launches++;
-        SD_CUDA(cudaMemsetAsync(claim, 0, (size_t)ni * n * sizeof(int), st));
+        if (!hs) SD_CUDA(cudaMemsetAsync(claim, 0, (size_t)ni * n * sizeof(int), st));
         SD_TRY(mbd_all_device(ctx, KA, ni, n, n, false, nullptr, nullptr, bA, aA));  // ranks only
-        SD_TRY(mbd_all_device(ctx, KB, ni, 2 * n, 2 * n, false, nullptr, nullptr, bB, tol > 0.0 ? aB : nullptr));
-        if (tol > 0.0) sc_reduce_kernel<true><<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, claim, m_others, d_out);
+        SD_TRY(mbd_all_device(ctx, KB, ni, 2 * n, 2 * n, false, nullptr, nullptr, bB, tol > 0.0 || hs ? aB : nullptr));
+        if (hs) hs_reduce_kernel<<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, d_out, ctx->d_status);
+        else if (tol > 0.0) sc_reduce_kernel<true><<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, claim, m_others, d_out);
         else sc_reduce_kernel<false><<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, claim, m_others, d_out);
         ctx->last.launches++;
         SD_CUDA(cudaGetLastError());

@@ -13,13 +13,15 @@ import pandas as pd
 
 from ._functional import _functionaldepth, _functionaldepth_of, _samplefunctionaldepth, _values
 from ._helper import DepthDegeneracy  # noqa: F401  (re-exported like the reference's `from ._helper import *`)
+from ._halfspace import _functional_halfspace, _pointcloud_halfspace
 from ._outliers import (NO_FACTOR, _check_central, _check_extremal_rows, _checked_values, _extremal_depth,
                         _functional_boxplot, _outliergram)
 from ._pointcloud import _pointwisedepth, _pointwisedepth_of, _samplepointwisedepth
 from ._reference import _checked_reference, _query_values, _SortedReference
 
 __all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'ExtremalDepth',
-           'FunctionalBoxplot', 'Outliergram', 'FunctionalReference', 'DepthClassifier', 'AbstractDepth']
+           'HalfspaceDepth', 'FunctionalHalfspaceDepth', 'FunctionalBoxplot', 'Outliergram', 'FunctionalReference',
+           'DepthClassifier', 'AbstractDepth']
 
 
 def _go():
@@ -304,6 +306,30 @@ def ExtremalDepth(data: List[pd.DataFrame], deep_check=False) -> _FunctionalDept
     e = _extremal_depth(X)
     return _FunctionalDepthUnivariate(df=data[0], depths=pd.Series(index=data[0].columns,
                                                                    data=e.astype(np.float64) / X.shape[1]))
+
+
+def HalfspaceDepth(data: pd.DataFrame, to_compute=None) -> _PointwiseDepth:
+    """Halfspace (Tukey) depth of the rows of an n x d DataFrame, d = 1 or 2.
+
+    A point's depth is the smallest share of the n points, itself included, that a closed half-plane (a half-line
+    for d = 1) whose boundary passes through the point can hold: at least 1 / n, at most 1.  Directions are compared
+    exactly in float64 (no tolerance band; set_simplex_tolerance does not apply).  Indexed by to_compute (row labels)
+    or data.index.  Non-finite values are rejected."""
+    return _PointwiseDepth(df=data, depths=_pointcloud_halfspace(data, to_compute))
+
+
+def FunctionalHalfspaceDepth(data: List[pd.DataFrame],
+                             to_compute=None) -> Union[_FunctionalDepthSeries, _FunctionalDepthUnivariate]:
+    """Integrated halfspace depth of curves (Claeskens, Hubert, Slaets & Vakili 2014, uniform weights): the mean
+    over time points of the halfspace depth of each curve's value among all curves' values at that time.
+
+    `[df]` (T rows x n curve columns) is the univariate case, to_compute are column labels; a list of N DataFrames
+    (T rows x 2 channels) the bivariate one, to_compute are list positions (as FunctionalDepth).  Other channel
+    counts raise NotImplementedError.  Non-finite values are rejected."""
+    depth = _functional_halfspace(data, to_compute)
+    if len(data) == 1:
+        return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+    return _FunctionalDepthSeries(df=data[0], depths=depth)
 
 
 # ---------------------------------------------------------------------------------------------------------------
