@@ -337,6 +337,40 @@ int sd_band_halfspace_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t 
                               int64_t *d_count_out);
 
 /*
+ * Random projection depths of curves F [N, T, d] (F[(i*T + t)*d + c] as sd_simplex_depth_f64; a point cloud is
+ * T = 1) along K directions U [K, d] (row-major, used as given: rows must be finite and non-zero; U is HOST memory
+ * in every variant, checked before it is uploaded).  Each (t, k) gives N projections
+ *     y_k(i, t) = (...((U[k,0] F[i,t,0]) + U[k,1] F[i,t,1]) + ...) + U[k,d-1] F[i,t,d-1]
+ * summed in this order with correctly rounded products and sums (no FMA, no tensor cores).
+ *
+ * Random Tukey depth: count_out[i] = sum_t min_k (N - max(b, a)) in [T, T*N], b / a the other projections of the
+ * row strictly below / above; depth = count / (T N).  Equal to the exact halfspace depth numerator when U holds a
+ * direction inside every cell of the arrangement, an upper bound on it otherwise.
+ * Projection outlyingness: o_out[t*N + i] = max_k |y - med| / MAD with med = np.median of the row and the unscaled
+ * MAD = np.median(|y - med|); MAD = 0 gives 0 where y == med and +inf elsewhere.  med_out / mad_out [T, K]
+ * (t-major) may be NULL.  Projection depth is 1 / (1 + O).
+ *
+ * SD_ERR_INVALID for N, T, d or K < 1 and for a zero or non-finite direction row; SD_ERR_NONFINITE when F holds NaN
+ * or +-inf or a projection overflows; SD_ERR_UNSUPPORTED for N >= 2^31.
+ */
+int sd_projection_tukey_f64(sd_ctx *ctx, const double *F, int64_t N, int64_t T, int d, const double *U, int64_t K,
+                            int64_t *count_out);
+int sd_projection_outlyingness_f64(sd_ctx *ctx, const double *F, int64_t N, int64_t T, int d, const double *U,
+                                   int64_t K, double *o_out, double *med_out, double *mad_out);
+/* univariate curves X [T, n] in either layout: the single direction u = 1 (y = x), o_out [T, n], med / mad [T] */
+int sd_band_outlyingness_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_t ld, int layout,
+                             double *o_out, double *med_out, double *mad_out);
+
+/* same with DEVICE pointers for F / X and the outputs (U stays host memory); SD_LAYOUT_TN only */
+int sd_projection_tukey_f64_dev(sd_ctx *ctx, const double *dF, int64_t N, int64_t T, int d, const double *U,
+                                int64_t K, int64_t *d_count_out);
+int sd_projection_outlyingness_f64_dev(sd_ctx *ctx, const double *dF, int64_t N, int64_t T, int d,
+                                       const double *U, int64_t K, double *d_o_out, double *d_med_out,
+                                       double *d_mad_out);
+int sd_band_outlyingness_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n, int64_t ld, double *d_o_out,
+                                 double *d_med_out, double *d_mad_out);
+
+/*
  * Batched band depth over sub-populations of one matrix (K-sampled blocks, homogeneity
  * permutations): membership[b*n + c] != 0 selects the curves of batch b; queries[b*nqb + i] is
  * the i-th query curve of batch b (must be a member).  count_out[b*nqb + i] as in

@@ -5,6 +5,7 @@
 * strict band depth / simplex / point-cloud depths have independent queries -> every rank takes a
   contiguous block of queries and the results are joined with ONE all-gather;
 * homogeneity permutations are independent -> split by permutation, all-gathered.
+* random projection depths of point clouds -> split by direction, MIN / MAX all-reduced (exact, order-free).
 
 Sharding is OPT-IN: `statdepth_b200.enable_distributed()` (or STATDEPTH_DISTRIBUTED=1 in the environment) makes
 every depth call of this process a COLLECTIVE over the default process group.  Every rank must then make the
@@ -83,11 +84,12 @@ def _device_for_collectives():
     return torch.device("cpu")
 
 
-def allreduce_sum(arr: np.ndarray) -> np.ndarray:
+def allreduce(arr: np.ndarray, op: str = "sum") -> np.ndarray:
+    """Element-wise reduction of arr over all ranks; op is "sum", "min" or "max"."""
     import torch
     import torch.distributed as dist
     t = torch.from_numpy(np.ascontiguousarray(arr)).to(_device_for_collectives())
-    dist.all_reduce(t, op=dist.ReduceOp.SUM)
+    dist.all_reduce(t, op={"sum": dist.ReduceOp.SUM, "min": dist.ReduceOp.MIN, "max": dist.ReduceOp.MAX}[op])
     return t.cpu().numpy()
 
 
@@ -148,7 +150,7 @@ def relaxed_counts(compute, X, queries, j, eng=None):
     lo, hi = block(T, rank, size)
     nq = X.shape[1] if queries is None else len(queries)
     local = compute(X[lo:hi], queries, j) if hi > lo else np.zeros(nq, dtype=np.int64)
-    return allreduce_sum(np.asarray(local, dtype=np.int64))
+    return allreduce(np.asarray(local, dtype=np.int64))
 
 
 def query_sharded(compute, queries, dtype):

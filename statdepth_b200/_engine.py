@@ -107,6 +107,18 @@ SIGNATURES = {
     "sd_band_halfspace_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int,
                                         C.c_void_p]),
     "sd_band_halfspace_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]),
+    "sd_projection_tukey_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p,
+                                          C.c_int64, C.c_void_p]),
+    "sd_projection_outlyingness_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p,
+                                                 C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sd_band_outlyingness_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int,
+                                           C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sd_projection_tukey_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p,
+                                              C.c_int64, C.c_void_p]),
+    "sd_projection_outlyingness_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int,
+                                                     C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sd_band_outlyingness_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
+                                               C.c_void_p, C.c_void_p]),
     "sd_band_depth_batched_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                             C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -379,6 +391,69 @@ class Engine:
         """Device-pointer variant (SD_LAYOUT_TN): int64 [n] stays on the device."""
         self._check(self.lib.sd_band_halfspace_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
                                                        C.c_void_p(int(d_out_ptr))))
+
+    # -- random projection depths --------------------------------------------------------------------------
+    @staticmethod
+    def _curves_and_directions(F, U):
+        F = np.ascontiguousarray(F, dtype=np.float64)
+        U = np.ascontiguousarray(U, dtype=np.float64)
+        if F.ndim != 3 or U.ndim != 2 or U.shape[1] != F.shape[2]:
+            raise ValueError("expected curves F [N, T, d] and directions U [K, d]")
+        return F, U
+
+    def projection_tukey_counts(self, F, U):
+        """Random Tukey numerators int64 [N] of the curves F [N, T, d] (a cloud is T = 1) along the directions
+        U [K, d]: sum over t of min over k of N - max(b, a), b / a the other projections strictly below / above."""
+        F, U = self._curves_and_directions(F, U)
+        N, T, d = F.shape
+        out = np.empty(N, dtype=np.int64)
+        self._check(self.lib.sd_projection_tukey_f64(self._ctx, _ptr(F), N, T, d, _ptr(U), U.shape[0], _ptr(out)))
+        return out
+
+    def projection_outlyingness(self, F, U, want_medmad=False):
+        """O [T, N]: per time point the max over the directions U [K, d] of |u.x - med| / MAD of the curves
+        F [N, T, d]; with want_medmad also med and MAD [T, K] of every projected row."""
+        F, U = self._curves_and_directions(F, U)
+        N, T, d = F.shape
+        K = U.shape[0]
+        o = np.empty((T, N))
+        med, mad = (np.empty((T, K)), np.empty((T, K))) if want_medmad else (None, None)
+        self._check(self.lib.sd_projection_outlyingness_f64(self._ctx, _ptr(F), N, T, d, _ptr(U), K, _ptr(o),
+                                                            _ptr(med), _ptr(mad)))
+        return (o, med, mad) if want_medmad else o
+
+    def band_outlyingness(self, X, want_medmad=False):
+        """O [T, n] = |x - med_t| / MAD_t of the univariate curves X [T, n] (and med, MAD [T]).  An F-ordered X is
+        passed with SD_LAYOUT_NT."""
+        X, is_f = self._matrix(X)
+        T, n = X.shape
+        o = np.empty((T, n))
+        med, mad = (np.empty(T), np.empty(T)) if want_medmad else (None, None)
+        self._check(self.lib.sd_band_outlyingness_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, T if is_f else n,
+                                                      LAYOUT_NT if is_f else LAYOUT_TN, _ptr(o), _ptr(med),
+                                                      _ptr(mad)))
+        return (o, med, mad) if want_medmad else o
+
+    def projection_tukey_counts_dev(self, dF_ptr, N, T, d, U, d_out_ptr):
+        """Device-pointer variant (F and the int64 [N] output on the device; U is host memory)."""
+        U = np.ascontiguousarray(U, dtype=np.float64)
+        self._check(self.lib.sd_projection_tukey_f64_dev(self._ctx, C.c_void_p(int(dF_ptr)), int(N), int(T), int(d),
+                                                         _ptr(U), U.shape[0], C.c_void_p(int(d_out_ptr))))
+
+    def projection_outlyingness_dev(self, dF_ptr, N, T, d, U, d_o_ptr, d_med_ptr=None, d_mad_ptr=None):
+        """Device-pointer variant (F, O [T, N] and med / MAD [T, K] on the device; U is host memory)."""
+        U = np.ascontiguousarray(U, dtype=np.float64)
+        self._check(self.lib.sd_projection_outlyingness_f64_dev(
+            self._ctx, C.c_void_p(int(dF_ptr)), int(N), int(T), int(d), _ptr(U), U.shape[0],
+            C.c_void_p(int(d_o_ptr)), C.c_void_p(int(d_med_ptr)) if d_med_ptr else None,
+            C.c_void_p(int(d_mad_ptr)) if d_mad_ptr else None))
+
+    def band_outlyingness_dev(self, dX_ptr, T, n, ld, d_o_ptr, d_med_ptr=None, d_mad_ptr=None):
+        """Device-pointer variant (SD_LAYOUT_TN): O [T, n] and med / MAD [T] stay on the device."""
+        self._check(self.lib.sd_band_outlyingness_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
+                                                          C.c_void_p(int(d_o_ptr)),
+                                                          C.c_void_p(int(d_med_ptr)) if d_med_ptr else None,
+                                                          C.c_void_p(int(d_mad_ptr)) if d_mad_ptr else None))
 
     # -- out-of-sample depth ----------------------------------------------------------------------------
     @staticmethod

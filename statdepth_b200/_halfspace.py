@@ -75,4 +75,4 @@ def _univariate_counts(X: np.ndarray) -> np.ndarray:
     lo, hi = _dist.block(T, rank, size)
     cnt = get_engine().band_halfspace_counts(X[lo:hi]) if hi > lo else np.zeros(n, dtype=np.int64)
     cnt = np.asarray(cnt, dtype=np.int64)
-    return cnt if size == 1 else _dist.allreduce_sum(cnt)
+    return cnt if size == 1 else _dist.allreduce(cnt)

@@ -173,7 +173,7 @@ def _local_rows(X: np.ndarray):
 
 
 def _summed(a: np.ndarray, size: int) -> np.ndarray:
-    return a if size == 1 else _dist.allreduce_sum(np.asarray(a, dtype=np.int64))
+    return a if size == 1 else _dist.allreduce(np.asarray(a, dtype=np.int64))
 
 
 def _gathered(a: np.ndarray, T: int, size: int) -> np.ndarray:

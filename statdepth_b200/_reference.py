@@ -74,7 +74,7 @@ class _SortedReference:
                 self.eng.band_depth_sorted_counts_dev(self.index.data_ptr(), self.hi - self.lo, self.nS, dY.data_ptr(),
                                                       nY, nY, self.J, out.data_ptr())
                 local = out.cpu().numpy()
-        return local if self.size == 1 else _dist.allreduce_sum(local)
+        return local if self.size == 1 else _dist.allreduce(local)
 
     def depths(self, Y: np.ndarray) -> np.ndarray:
         """Relaxed depth of every new curve (column of Y [T, nY]), bit-identical to FunctionalDepthOf(relax=True)."""

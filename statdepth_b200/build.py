@@ -33,6 +33,7 @@ SOURCES = {
     "reference.cu": [],
     "extremal.cu": [],
     "halfspace.cu": [],
+    "projection.cu": ["-fmad=false"],
     "outliers.cu": ["-fmad=false"],
     "pointcloud.cu": ["-fmad=false"],
     "simplicial_count.cu": ["-fmad=false"],

@@ -670,6 +670,115 @@ int sd_band_halfspace_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t 
     return end_call(ctx, false);
 }
 
+// random projection depths (K12, projection.cu).  The directions are small host memory in every variant: checked
+// here (finite, non-zero rows), then uploaded to BUF_MISC.
+static int upload_directions(sd_ctx *ctx, const double *U, i64 K, int d, const double **dU, const char *who) {
+    SD_REQUIRE(U, "%s: NULL directions", who);
+    SD_REQUIRE(K >= 1 && d >= 1, "%s: bad sizes K=%lld d=%d", who, (long long)K, d);
+    for (i64 k = 0; k < K; ++k) {
+        bool nonzero = false;
+        for (int c = 0; c < d; ++c) {
+            const double u = U[k * d + c];
+            SD_REQUIRE(isfinite(u), "%s: direction %lld is not finite", who, (long long)k);
+            nonzero |= u != 0.0;
+        }
+        SD_REQUIRE(nonzero, "%s: direction %lld is zero", who, (long long)k);
+    }
+    SD_TRY(ctx->buf[BUF_MISC].reserve((size_t)K * d * sizeof(double)));
+    double *p = ctx->buf[BUF_MISC].as<double>();
+    SD_CUDA(cudaMemcpyAsync(p, U, (size_t)K * d * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    *dU = p;
+    return SD_OK;
+}
+
+static int projection_call(sd_ctx *ctx, const double *F, int64_t N, int64_t T, int d, const double *U, int64_t K,
+                           ProjKind kind, void *out, double *med_out, double *mad_out, bool dev, const char *who) {
+    SD_TRY(check_common(ctx, F, out, who));
+    SD_REQUIRE(N >= 1 && T >= 1 && d >= 1 && K >= 1, "%s: bad sizes N=%lld T=%lld d=%d K=%lld", who, (long long)N,
+               (long long)T, d, (long long)K);
+    if (N >= (1ll << 31)) {  // the rank pipeline's limit, refused before anything is uploaded
+        set_error("%s: N=%lld exceeds 2^31-1", who, (long long)N);
+        return SD_ERR_UNSUPPORTED;
+    }
+    SD_TRY(begin_call(ctx));
+    const double *dU = nullptr;
+    SD_TRY(upload_directions(ctx, U, K, d, &dU, who));
+    const double *dF = F;
+    void *d_out = out;
+    const size_t out_bytes = (size_t)N * (kind == PJ_TUKEY ? 1 : T) * 8;
+    if (!dev) {
+        double *up = nullptr;
+        SD_TRY(upload_matrix(ctx, BUF_IN, F, 1, N * T * d, N * T * d, &up));
+        dF = up;
+        SD_TRY(ctx->buf[BUF_OUT].reserve(out_bytes));
+        d_out = ctx->buf[BUF_OUT].p;
+    }
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(projection_device(ctx, dF, N, T, d, N * T * d, dU, K, kind, (i64 *)d_out, (double *)d_out, med_out,
+                             mad_out, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost));
+    SD_TRY(mark(ctx, 2));
+    if (!dev) SD_CUDA(cudaMemcpyAsync(out, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    return end_call(ctx, !dev);
+}
+
+int sd_projection_tukey_f64(sd_ctx *ctx, const double *F, int64_t N, int64_t T, int d, const double *U, int64_t K,
+                            int64_t *count_out) {
+    return projection_call(ctx, F, N, T, d, U, K, PJ_TUKEY, count_out, nullptr, nullptr, false,
+                           "sd_projection_tukey_f64");
+}
+
+int sd_projection_tukey_f64_dev(sd_ctx *ctx, const double *dF, int64_t N, int64_t T, int d, const double *U,
+                                int64_t K, int64_t *d_count_out) {
+    return projection_call(ctx, dF, N, T, d, U, K, PJ_TUKEY, d_count_out, nullptr, nullptr, true,
+                           "sd_projection_tukey_f64_dev");
+}
+
+int sd_projection_outlyingness_f64(sd_ctx *ctx, const double *F, int64_t N, int64_t T, int d, const double *U,
+                                   int64_t K, double *o_out, double *med_out, double *mad_out) {
+    return projection_call(ctx, F, N, T, d, U, K, PJ_OUTLYING, o_out, med_out, mad_out, false,
+                           "sd_projection_outlyingness_f64");
+}
+
+int sd_projection_outlyingness_f64_dev(sd_ctx *ctx, const double *dF, int64_t N, int64_t T, int d,
+                                       const double *U, int64_t K, double *d_o_out, double *d_med_out,
+                                       double *d_mad_out) {
+    return projection_call(ctx, dF, N, T, d, U, K, PJ_OUTLYING, d_o_out, d_med_out, d_mad_out, true,
+                           "sd_projection_outlyingness_f64_dev");
+}
+
+int sd_band_outlyingness_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_t ld, int layout,
+                             double *o_out, double *med_out, double *mad_out) {
+    SD_TRY(check_common(ctx, X, o_out, "sd_band_outlyingness_f64"));
+    SD_TRY(check_matrix("sd_band_outlyingness_f64", T, n, ld, layout));
+    if (n >= (1ll << 31)) {
+        set_error("sd_band_outlyingness_f64: n=%lld exceeds 2^31-1", (long long)n);
+        return SD_ERR_UNSUPPORTED;
+    }
+    SD_TRY(begin_call(ctx));
+    double *dX = nullptr;
+    SD_TRY(upload_tn(ctx, X, T, n, ld, layout, &dX));
+    SD_TRY(ctx->buf[BUF_OUT].reserve((size_t)T * n * sizeof(double)));
+    double *d_o = ctx->buf[BUF_OUT].as<double>();
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(projection_device(ctx, dX, n, T, 1, n, nullptr, 1, PJ_OUTLYING, nullptr, d_o, med_out, mad_out,
+                             cudaMemcpyDeviceToHost));
+    SD_TRY(mark(ctx, 2));
+    SD_CUDA(cudaMemcpyAsync(o_out, d_o, (size_t)T * n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    return end_call(ctx, true);
+}
+
+int sd_band_outlyingness_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64_t n, int64_t ld, double *d_o_out,
+                                 double *d_med_out, double *d_mad_out) {
+    SD_TRY(check_common(ctx, dX, d_o_out, "sd_band_outlyingness_f64_dev"));
+    SD_TRY(check_matrix("sd_band_outlyingness_f64_dev", T, n, ld, SD_LAYOUT_TN));
+    SD_TRY(begin_call(ctx));
+    SD_TRY(mark(ctx, 1));
+    SD_TRY(projection_device(ctx, dX, n, T, 1, ld, nullptr, 1, PJ_OUTLYING, nullptr, d_o_out, d_med_out, d_mad_out,
+                             cudaMemcpyDeviceToDevice));
+    SD_TRY(mark(ctx, 2));
+    return end_call(ctx, false);
+}
+
 // point clouds: [S; Y] rows, query ids nS .. nS + nY - 1
 static int pooled_cloud(sd_ctx *ctx, const double *S, int64_t nS, int d, const double *Y, int64_t nY, double **dP,
                         const i64 **d_q) {

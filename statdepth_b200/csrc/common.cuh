@@ -68,6 +68,9 @@ enum BufId {
     BUF_SLAB,       // MBD slab path: per-row maps, bucket tables, bin starts
     BUF_KEYS,       // extremal depth: per-curve sorted extremities, u32 [n][T] (none of the above is used with it)
     BUF_ORDER,      // extremal depth: curve ids, group starts, merge-sort / scan temp storage
+    BUF_PROJ,       // projection depths: projected rows Y
+    BUF_PSORT,      // projection depth: sorted rows of Y
+    BUF_PRED,       // projection depths: running min / max across direction blocks, per-row med / MAD
     NUM_BUFS
 };
 
@@ -173,6 +176,13 @@ int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride
                              double tol, i64 *d_out, i64 m_others = -1, ScReduce reduce = SC_TRIANGLES);
 // halfspace depth, d = 1 (halfspace.cu): d_out[c] = sum_t (n - max(b_t(c), a_t(c))) over the rows of X [T, n]
 int halfspace1_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, i64 *d_out);
+// random projection depths (projection.cu): dU == nullptr takes the rows of X [T, N] (leading dimension ldX) as
+// the projections of the single direction u = 1.  PJ_TUKEY: d_count [N] = sum_t min_k (N - max(b, a)).
+// PJ_OUTLYING: d_o [T][N] = max_k |y - med| / MAD; med_out / mad_out [T][K] (copied with out_kind) may be NULL.
+enum ProjKind { PJ_TUKEY, PJ_OUTLYING };
+int projection_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, i64 ldX, const double *dU, i64 K,
+                      ProjKind kind, i64 *d_count, double *d_o, double *med_out, double *mad_out,
+                      cudaMemcpyKind out_kind);
 // out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out);

@@ -17,10 +17,12 @@ from ._halfspace import _functional_halfspace, _pointcloud_halfspace
 from ._outliers import (NO_FACTOR, _check_central, _check_extremal_rows, _checked_values, _extremal_depth,
                         _functional_boxplot, _outliergram)
 from ._pointcloud import _pointwisedepth, _pointwisedepth_of, _samplepointwisedepth
+from ._projection import _functional_projection, _pointcloud_projection
 from ._reference import _checked_reference, _query_values, _SortedReference
 
 __all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'ExtremalDepth',
-           'HalfspaceDepth', 'FunctionalHalfspaceDepth', 'FunctionalBoxplot', 'Outliergram', 'FunctionalReference',
+           'HalfspaceDepth', 'FunctionalHalfspaceDepth', 'ProjectionDepth', 'FunctionalProjectionDepth',
+           'FunctionalBoxplot', 'Outliergram', 'FunctionalReference',
            'DepthClassifier', 'AbstractDepth']
 
 
@@ -327,6 +329,34 @@ def FunctionalHalfspaceDepth(data: List[pd.DataFrame],
     (T rows x 2 channels) the bivariate one, to_compute are list positions (as FunctionalDepth).  Other channel
     counts raise NotImplementedError.  Non-finite values are rejected."""
     depth = _functional_halfspace(data, to_compute)
+    if len(data) == 1:
+        return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+    return _FunctionalDepthSeries(df=data[0], depths=depth)
+
+
+def ProjectionDepth(data: pd.DataFrame, kind='projection', directions=None, seed=0,
+                    to_compute=None) -> _PointwiseDepth:
+    """Random projection depth of the rows of an n x d DataFrame, any d.
+
+    kind='projection': projection depth (Zuo & Serfling 2000), 1 / (1 + O) with O the largest |u.x - med| / MAD
+    over the directions u (med and the unscaled MAD of the projected sample).  kind='tukey': random Tukey depth
+    (Cuesta-Albertos & Nieto-Reyes 2008), the smallest share of points, the point included, in a closed half-line
+    of one projection; an upper bound on the exact halfspace depth.  directions: None (1000), an int K (K random
+    unit directions from np.random.default_rng(seed)) or an array [K, d] used as given (finite, non-zero rows).
+    Indexed by to_compute (row labels) or data.index.  Non-finite values are rejected."""
+    return _PointwiseDepth(df=data, depths=_pointcloud_projection(data, kind, directions, seed, to_compute))
+
+
+def FunctionalProjectionDepth(data: List[pd.DataFrame], kind='projection', directions=None, seed=0,
+                              to_compute=None) -> Union[_FunctionalDepthSeries, _FunctionalDepthUnivariate]:
+    """Integrated random projection depth of curves: the mean over time points of ProjectionDepth of each curve's
+    value among all curves' values at that time (kind='tukey': sum of numerators over time, divided once by T n).
+
+    `[df]` (T rows x n curve columns) is the univariate case, with the single direction 1.0 (directions must be
+    None; kind='tukey' is FunctionalHalfspaceDepth([df])), to_compute are column labels; a list of N DataFrames
+    (T rows x d channels, any d) the multivariate one, to_compute are list positions.  directions and seed as for
+    ProjectionDepth.  Non-finite values are rejected."""
+    depth = _functional_projection(data, kind, directions, seed, to_compute)
     if len(data) == 1:
         return _FunctionalDepthUnivariate(df=data[0], depths=depth)
     return _FunctionalDepthSeries(df=data[0], depths=depth)
