@@ -152,6 +152,11 @@ def _ptr(a):
     return None if a is None else C.c_void_p(a.ctypes.data)
 
 
+def _dptr(p):
+    """A device (or raw host) address as passed to the C ABI: 0 and None are NULL."""
+    return C.c_void_p(int(p)) if p else None
+
+
 def mbd_plan(n: int, ld: int = None) -> dict:
     """Rank pipeline relaxed depth takes for rows of n curves (host arithmetic of the library, no GPU needed)."""
     out = np.zeros(6, dtype=np.int64)
@@ -236,33 +241,28 @@ class Engine:
 
     @staticmethod
     def _matrix(X):
-        """float64 view + layout of a 2-D array: C-order -> [rows, cols]; F-order -> transposed."""
+        """(X, ld, layout) of a 2-D float64 array [T, n]: a C-order X is SD_LAYOUT_TN with ld = n; an F-order X (what a
+        column-built DataFrame gives) is passed as-is, its memory [n, T] row-major: SD_LAYOUT_NT with ld = T."""
         X = np.asarray(X)
         if X.dtype != np.float64:
             X = X.astype(np.float64)
         if X.ndim != 2:
             raise ValueError("expected a 2-D array")
-        if X.flags.c_contiguous:
-            return X, False
-        if X.flags.f_contiguous:
-            return X, True
-        return np.ascontiguousarray(X), False
+        if X.flags.f_contiguous and not X.flags.c_contiguous:
+            return X, X.shape[0], LAYOUT_NT
+        X = np.ascontiguousarray(X)
+        return X, X.shape[1], LAYOUT_TN
 
     # -- band depth -------------------------------------------------------------------------------
     def band_depth_counts(self, X, queries=None, j=2, relax=False):
         """Integer numerators for subset size j.  X is [T, n] (rows = time points, columns = curves);
         an F-ordered X (what a column-built DataFrame gives) is passed as-is with SD_LAYOUT_NT."""
-        X, is_f = self._matrix(X)
+        X, ld, layout = self._matrix(X)
         T, n = X.shape
         q, nq = self._queries(queries, n)
         out = np.empty(nq, dtype=np.int64)
-        if is_f:  # memory is [n, T] row-major
-            st = self.lib.sd_band_depth_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, T, LAYOUT_NT, _ptr(q), nq,
-                                            int(j), int(bool(relax)), _ptr(out))
-        else:
-            st = self.lib.sd_band_depth_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, n, LAYOUT_TN, _ptr(q), nq,
-                                            int(j), int(bool(relax)), _ptr(out))
-        self._check(st)
+        self._check(self.lib.sd_band_depth_f64(self._ctx, _ptr(X), T, n, ld, layout, _ptr(q), nq, int(j),
+                                               int(bool(relax)), _ptr(out)))
         return out
 
     def band_depth_counts_ptr(self, host_ptr, T, n, ld, queries=None, j=2, relax=False, out=None):
@@ -270,26 +270,23 @@ class Engine:
         q, nq = self._queries(queries, n)
         if out is None:
             out = np.empty(nq, dtype=np.int64)
-        self._check(self.lib.sd_band_depth_f64(self._ctx, C.c_void_p(int(host_ptr)), int(T), int(n), int(ld),
-                                               LAYOUT_TN, _ptr(q), nq, int(j), int(bool(relax)), _ptr(out)))
+        self._check(self.lib.sd_band_depth_f64(self._ctx, _dptr(host_ptr), int(T), int(n), int(ld), LAYOUT_TN,
+                                               _ptr(q), nq, int(j), int(bool(relax)), _ptr(out)))
         return out
 
     def band_depth_counts_dev(self, dX_ptr, T, n, ld, d_out_ptr, d_query_ptr=None, nq=None, j=2, relax=False):
         """Device-pointer variant: no copies; result stays on the device."""
         nq = int(n if nq is None else nq)
-        self._check(self.lib.sd_band_depth_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
-                                                   C.c_void_p(int(d_query_ptr)) if d_query_ptr else None, nq,
-                                                   int(j), int(bool(relax)), C.c_void_p(int(d_out_ptr))))
+        self._check(self.lib.sd_band_depth_f64_dev(self._ctx, _dptr(dX_ptr), int(T), int(n), int(ld),
+                                                   _dptr(d_query_ptr), nq, int(j), int(bool(relax)), _dptr(d_out_ptr)))
 
     def band_ranks(self, X):
         """(below, above) int32 [T, n]: strict ranks of every curve at every time point."""
-        X, is_f = self._matrix(X)
+        X, ld, layout = self._matrix(X)
         T, n = X.shape
         below = np.empty((T, n), dtype=np.int32)
         above = np.empty((T, n), dtype=np.int32)
-        st = self.lib.sd_band_ranks_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, T if is_f else n,
-                                        LAYOUT_NT if is_f else LAYOUT_TN, _ptr(below), _ptr(above))
-        self._check(st)
+        self._check(self.lib.sd_band_ranks_f64(self._ctx, _ptr(X), T, n, ld, layout, _ptr(below), _ptr(above)))
         return below, above
 
     def band_depth_counts_batched(self, X, membership, queries, j=2, relax=False):
@@ -309,53 +306,48 @@ class Engine:
     def band_rank_sums(self, X, want_above=False):
         """(Q, B[, A]) int64 [n]: the relaxed J = 2 numerator and the per-curve sums over time rows of the curves
         strictly below (and above) each curve.  X is [T, n]; an F-ordered X is passed with SD_LAYOUT_NT."""
-        X, is_f = self._matrix(X)
+        X, ld, layout = self._matrix(X)
         T, n = X.shape
         q, b = np.empty(n, dtype=np.int64), np.empty(n, dtype=np.int64)
         a = np.empty(n, dtype=np.int64) if want_above else None
-        self._check(self.lib.sd_band_rank_sums_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, T if is_f else n,
-                                                   LAYOUT_NT if is_f else LAYOUT_TN, _ptr(q), _ptr(b), _ptr(a)))
+        self._check(self.lib.sd_band_rank_sums_f64(self._ctx, _ptr(X), T, n, ld, layout, _ptr(q), _ptr(b), _ptr(a)))
         return (q, b, a) if want_above else (q, b)
 
     def band_rank_sums_dev(self, dX_ptr, T, n, ld, d_q_ptr, d_b_ptr, d_a_ptr=None):
         """Device-pointer variant (SD_LAYOUT_TN): int64 [n] outputs stay on the device."""
-        self._check(self.lib.sd_band_rank_sums_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
-                                                       C.c_void_p(int(d_q_ptr)), C.c_void_p(int(d_b_ptr)),
-                                                       C.c_void_p(int(d_a_ptr)) if d_a_ptr else None))
+        self._check(self.lib.sd_band_rank_sums_f64_dev(self._ctx, _dptr(dX_ptr), int(T), int(n), int(ld),
+                                                       _dptr(d_q_ptr), _dptr(d_b_ptr), _dptr(d_a_ptr)))
 
     def band_envelope(self, X, member, factor, want_outside=True):
         """(lo [T], hi [T], outside [n] or None): per-row min / max of the member curves, and per curve the number of
         rows outside the fences lo - factor * (hi - lo), hi + factor * (hi - lo)."""
-        X, is_f = self._matrix(X)
+        X, ld, layout = self._matrix(X)
         T, n = X.shape
         mem = np.ascontiguousarray(member, dtype=np.uint8)
         if mem.shape != (n,):
             raise ValueError("member must have one entry per curve")
         lower, upper = np.empty(T), np.empty(T)
         outside = np.empty(n, dtype=np.int64) if want_outside else None
-        self._check(self.lib.sd_band_envelope_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, T if is_f else n,
-                                                  LAYOUT_NT if is_f else LAYOUT_TN, _ptr(mem), float(factor),
+        self._check(self.lib.sd_band_envelope_f64(self._ctx, _ptr(X), T, n, ld, layout, _ptr(mem), float(factor),
                                                   _ptr(lower), _ptr(upper), _ptr(outside)))
         return lower, upper, outside
 
     def band_envelope_dev(self, dX_ptr, T, n, ld, d_member_ptr, factor, d_lower_ptr, d_upper_ptr,
                           d_outside_ptr=None):
         """Device-pointer variant (SD_LAYOUT_TN): member uint8 [n], lo / hi float64 [T], outside int64 [n]."""
-        self._check(self.lib.sd_band_envelope_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
-                                                      C.c_void_p(int(d_member_ptr)), float(factor),
-                                                      C.c_void_p(int(d_lower_ptr)), C.c_void_p(int(d_upper_ptr)),
-                                                      C.c_void_p(int(d_outside_ptr)) if d_outside_ptr else None))
+        self._check(self.lib.sd_band_envelope_f64_dev(self._ctx, _dptr(dX_ptr), int(T), int(n), int(ld),
+                                                      _dptr(d_member_ptr), float(factor), _dptr(d_lower_ptr),
+                                                      _dptr(d_upper_ptr), _dptr(d_outside_ptr)))
 
     # -- extremal depth ---------------------------------------------------------------------------------
     def band_extremity_dev(self, dX_ptr, T, n, ld, d_m_ptr):
         """Pointwise extremities |b - a| of the rows X [T, n] (SD_LAYOUT_TN): int32 [T, n] on the device."""
-        self._check(self.lib.sd_band_extremity_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
-                                                       C.c_void_p(int(d_m_ptr))))
+        self._check(self.lib.sd_band_extremity_f64_dev(self._ctx, _dptr(dX_ptr), int(T), int(n), int(ld),
+                                                       _dptr(d_m_ptr)))
 
     def extremal_depth_dev(self, d_m_ptr, T, n, d_num_ptr):
         """Extremal-depth numerators int64 [n] from the full extremity matrix int32 [T, n], on the device."""
-        self._check(self.lib.sd_extremal_depth_dev(self._ctx, C.c_void_p(int(d_m_ptr)), int(T), int(n),
-                                                   C.c_void_p(int(d_num_ptr))))
+        self._check(self.lib.sd_extremal_depth_dev(self._ctx, _dptr(d_m_ptr), int(T), int(n), _dptr(d_num_ptr)))
 
     # -- halfspace (Tukey) depth -----------------------------------------------------------------------
     def halfspace_counts(self, P, queries=None):
@@ -380,17 +372,16 @@ class Engine:
     def band_halfspace_counts(self, X):
         """int64 [n]: sum over the time rows of X [T, n] of n - max(b_t, a_t), b_t / a_t the other curves strictly
         below / above.  An F-ordered X is passed with SD_LAYOUT_NT."""
-        X, is_f = self._matrix(X)
+        X, ld, layout = self._matrix(X)
         T, n = X.shape
         out = np.empty(n, dtype=np.int64)
-        self._check(self.lib.sd_band_halfspace_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, T if is_f else n,
-                                                   LAYOUT_NT if is_f else LAYOUT_TN, _ptr(out)))
+        self._check(self.lib.sd_band_halfspace_f64(self._ctx, _ptr(X), T, n, ld, layout, _ptr(out)))
         return out
 
     def band_halfspace_counts_dev(self, dX_ptr, T, n, ld, d_out_ptr):
         """Device-pointer variant (SD_LAYOUT_TN): int64 [n] stays on the device."""
-        self._check(self.lib.sd_band_halfspace_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
-                                                       C.c_void_p(int(d_out_ptr))))
+        self._check(self.lib.sd_band_halfspace_f64_dev(self._ctx, _dptr(dX_ptr), int(T), int(n), int(ld),
+                                                       _dptr(d_out_ptr)))
 
     # -- random projection depths --------------------------------------------------------------------------
     @staticmethod
@@ -425,35 +416,31 @@ class Engine:
     def band_outlyingness(self, X, want_medmad=False):
         """O [T, n] = |x - med_t| / MAD_t of the univariate curves X [T, n] (and med, MAD [T]).  An F-ordered X is
         passed with SD_LAYOUT_NT."""
-        X, is_f = self._matrix(X)
+        X, ld, layout = self._matrix(X)
         T, n = X.shape
         o = np.empty((T, n))
         med, mad = (np.empty(T), np.empty(T)) if want_medmad else (None, None)
-        self._check(self.lib.sd_band_outlyingness_f64(self._ctx, C.c_void_p(X.ctypes.data), T, n, T if is_f else n,
-                                                      LAYOUT_NT if is_f else LAYOUT_TN, _ptr(o), _ptr(med),
+        self._check(self.lib.sd_band_outlyingness_f64(self._ctx, _ptr(X), T, n, ld, layout, _ptr(o), _ptr(med),
                                                       _ptr(mad)))
         return (o, med, mad) if want_medmad else o
 
     def projection_tukey_counts_dev(self, dF_ptr, N, T, d, U, d_out_ptr):
         """Device-pointer variant (F and the int64 [N] output on the device; U is host memory)."""
         U = np.ascontiguousarray(U, dtype=np.float64)
-        self._check(self.lib.sd_projection_tukey_f64_dev(self._ctx, C.c_void_p(int(dF_ptr)), int(N), int(T), int(d),
-                                                         _ptr(U), U.shape[0], C.c_void_p(int(d_out_ptr))))
+        self._check(self.lib.sd_projection_tukey_f64_dev(self._ctx, _dptr(dF_ptr), int(N), int(T), int(d), _ptr(U),
+                                                         U.shape[0], _dptr(d_out_ptr)))
 
     def projection_outlyingness_dev(self, dF_ptr, N, T, d, U, d_o_ptr, d_med_ptr=None, d_mad_ptr=None):
         """Device-pointer variant (F, O [T, N] and med / MAD [T, K] on the device; U is host memory)."""
         U = np.ascontiguousarray(U, dtype=np.float64)
-        self._check(self.lib.sd_projection_outlyingness_f64_dev(
-            self._ctx, C.c_void_p(int(dF_ptr)), int(N), int(T), int(d), _ptr(U), U.shape[0],
-            C.c_void_p(int(d_o_ptr)), C.c_void_p(int(d_med_ptr)) if d_med_ptr else None,
-            C.c_void_p(int(d_mad_ptr)) if d_mad_ptr else None))
+        self._check(self.lib.sd_projection_outlyingness_f64_dev(self._ctx, _dptr(dF_ptr), int(N), int(T), int(d),
+                                                                _ptr(U), U.shape[0], _dptr(d_o_ptr), _dptr(d_med_ptr),
+                                                                _dptr(d_mad_ptr)))
 
     def band_outlyingness_dev(self, dX_ptr, T, n, ld, d_o_ptr, d_med_ptr=None, d_mad_ptr=None):
         """Device-pointer variant (SD_LAYOUT_TN): O [T, n] and med / MAD [T] stay on the device."""
-        self._check(self.lib.sd_band_outlyingness_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(n), int(ld),
-                                                          C.c_void_p(int(d_o_ptr)),
-                                                          C.c_void_p(int(d_med_ptr)) if d_med_ptr else None,
-                                                          C.c_void_p(int(d_mad_ptr)) if d_mad_ptr else None))
+        self._check(self.lib.sd_band_outlyingness_f64_dev(self._ctx, _dptr(dX_ptr), int(T), int(n), int(ld),
+                                                          _dptr(d_o_ptr), _dptr(d_med_ptr), _dptr(d_mad_ptr)))
 
     # -- out-of-sample depth ----------------------------------------------------------------------------
     @staticmethod
@@ -478,28 +465,26 @@ class Engine:
         out = np.empty(nY, dtype=np.int64)
         if nY == 0:
             return out
-        self._check(self.lib.sd_band_depth_oos_f64(self._ctx, C.c_void_p(S.ctypes.data), T, nS, ldS,
-                                                   C.c_void_p(Y.ctypes.data), nY, ldY, int(j), int(bool(relax)),
-                                                   _ptr(out)))
+        self._check(self.lib.sd_band_depth_oos_f64(self._ctx, _ptr(S), T, nS, ldS, _ptr(Y), nY, ldY, int(j),
+                                                   int(bool(relax)), _ptr(out)))
         return out
 
     def band_depth_oos_counts_dev(self, dS_ptr, T, nS, ldS, dY_ptr, nY, ldY, d_out_ptr, j=2, relax=False):
         """Device-pointer variant: no host copies; int64 counts [nY] stay on the device."""
-        self._check(self.lib.sd_band_depth_oos_f64_dev(self._ctx, C.c_void_p(int(dS_ptr)), int(T), int(nS), int(ldS),
-                                                       C.c_void_p(int(dY_ptr)), int(nY), int(ldY), int(j),
-                                                       int(bool(relax)), C.c_void_p(int(d_out_ptr))))
+        self._check(self.lib.sd_band_depth_oos_f64_dev(self._ctx, _dptr(dS_ptr), int(T), int(nS), int(ldS),
+                                                       _dptr(dY_ptr), int(nY), int(ldY), int(j), int(bool(relax)),
+                                                       _dptr(d_out_ptr)))
 
     def band_sort_rows_dev(self, dX_ptr, T, nS, ld, d_sorted_ptr):
         """The index of a fitted reference: float64 [T, nS] rows of X (SD_LAYOUT_TN) sorted ascending, on the device."""
-        self._check(self.lib.sd_band_sort_rows_f64_dev(self._ctx, C.c_void_p(int(dX_ptr)), int(T), int(nS), int(ld),
-                                                       C.c_void_p(int(d_sorted_ptr))))
+        self._check(self.lib.sd_band_sort_rows_f64_dev(self._ctx, _dptr(dX_ptr), int(T), int(nS), int(ld),
+                                                       _dptr(d_sorted_ptr)))
 
     def band_depth_sorted_counts_dev(self, d_sorted_ptr, T, nS, dY_ptr, nY, ldY, J, d_out_ptr):
         """Relaxed numerators of the new curves Y [T, nY] against sorted rows: int64 [(J - 1), nY] on the device,
         row j - 2 equal to band_depth_oos_counts_dev(relax=True) for j."""
-        self._check(self.lib.sd_band_depth_sorted_f64_dev(self._ctx, C.c_void_p(int(d_sorted_ptr)), int(T), int(nS),
-                                                          C.c_void_p(int(dY_ptr)), int(nY), int(ldY), int(J),
-                                                          C.c_void_p(int(d_out_ptr))))
+        self._check(self.lib.sd_band_depth_sorted_f64_dev(self._ctx, _dptr(d_sorted_ptr), int(T), int(nS),
+                                                          _dptr(dY_ptr), int(nY), int(ldY), int(J), _dptr(d_out_ptr)))
 
     def simplicial_oos_counts(self, S, Y, tol=1e-7):
         S = np.ascontiguousarray(S, dtype=np.float64)

@@ -143,6 +143,11 @@ int prof_end(sd_ctx *ctx);
 // kernels / drivers implemented in the other translation units (all stream-ordered on ctx->stream)
 int band_depth_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq, int j,
                       int relax, i64 *d_out);
+// The int64 guard of relaxed band depth with `others` curves besides the one ranked (n - 1 within a sample, nS out
+// of sample): T * C(others, j) must fit, and for j = 3 also 3 * C(others, 3).  relaxed_overflow_check sets the error
+// (prefixed by who) and returns SD_ERR_OVERFLOW (api.cu).
+bool relaxed_overflows(i64 T, i64 others, int j);
+int relaxed_overflow_check(i64 T, i64 others, int j, const char *who);
 int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool want_j3, i64 *d_acc2,
                    i64 *d_acc3, int *d_rank_b, int *d_rank_a, bool accumulate = false, i64 group_rows = 0);
 int bd_strict_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq, int j,
@@ -186,8 +191,6 @@ int projection_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, i64 ld
 // out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out);
-// SD_ERR_OVERFLOW (message prefixed by who) unless T * C(nS, j) fits in int64
-int oos_overflow_check(i64 T, i64 nS, int j, const char *who);
 // int32 workspace for rank-only passes in row blocks of *RB rows (ints_per_row each) within a fixed budget
 int rank_block_workspace(sd_ctx *ctx, i64 T, i64 ints_per_row, i64 *RB, int **ws);
 // sorted reference rows and out-of-sample counts from them (reference.cu)

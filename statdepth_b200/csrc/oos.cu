@@ -85,17 +85,6 @@ __global__ void __launch_bounds__(OOS_THREADS) oos_terms_kernel(const int *__res
     if (sum) atomicAdd((u64 *)&acc[g], (u64)sum);
 }
 
-// overflow guard of band_depth_device with n - 1 = nS others: T * C(nS, j) (and 3 * C(nS, 3)) fit in int64
-int oos_overflow_check(i64 T, i64 nS, int j, const char *who) {
-    const long double full = (j == 2) ? (long double)nS * (nS - 1) / 2.0L
-                                      : (long double)nS * (nS - 1) * (nS - 2) / 6.0L;
-    if (full * (long double)T >= 9.0e18L || (j == 3 && 3.0L * full >= 9.0e18L)) {
-        set_error("%s: T*C(nS,%d) overflows int64 for T=%lld nS=%lld", who, j, (long long)T, (long long)nS);
-        return SD_ERR_OVERFLOW;
-    }
-    return SD_OK;
-}
-
 // Rank workspace of the rank-only passes, split into row blocks (also used by rank_sums_device, outliers.cu).
 constexpr size_t RANK_BLOCK_BUDGET = 1ull << 30;
 
@@ -132,7 +121,7 @@ int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, 
         ctx->last.bd_impl_used = SD_BD_BITS;
         return bd_strict_device(ctx, dX, T, nS + 1, ld, d_q, nY, j, d_out);
     }
-    SD_TRY(oos_overflow_check(T, nS, j, "out-of-sample band depth"));
+    SD_TRY(relaxed_overflow_check(T, nS, j, "out-of-sample band depth"));
     const i64 n = nS + nY;
     const i64 ny_ranks = nY > 1 ? nY : 0;  // one new curve: nothing to subtract, no second pass
     i64 RB = 0;

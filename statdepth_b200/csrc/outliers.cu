@@ -62,11 +62,7 @@ int rank_sums_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, i64 *d
         set_error("rank sums: bad shape T=%lld n=%lld ld=%lld", (long long)T, (long long)n, (long long)ld);
         return SD_ERR_INVALID;
     }
-    // overflow guard of band_depth_device: T * C(n-1, 2) must fit in int64 (B and A are smaller)
-    if ((long double)(n - 1) * (n - 2) / 2.0L * (long double)T >= 9.0e18L) {
-        set_error("rank sums: T*C(n-1,2) overflows int64 for T=%lld n=%lld", (long long)T, (long long)n);
-        return SD_ERR_OVERFLOW;
-    }
+    SD_TRY(relaxed_overflow_check(T, n - 1, 2, "rank sums"));  // the J = 2 numerator; B and A are smaller
     cudaStream_t st = ctx->stream;
     SD_CUDA(cudaMemsetAsync(d_q, 0, (size_t)n * sizeof(i64), st));
     SD_CUDA(cudaMemsetAsync(d_b, 0, (size_t)n * sizeof(i64), st));

@@ -201,7 +201,7 @@ int depth_sorted_device(sd_ctx *ctx, const double *d_sorted, i64 T, i64 nS, cons
                   (long long)nS, (long long)nY, (long long)ldY);
         return SD_ERR_INVALID;
     }
-    for (int j = 2; j <= J; ++j) SD_TRY(oos_overflow_check(T, nS, j, "sorted-reference band depth"));
+    for (int j = 2; j <= J; ++j) SD_TRY(relaxed_overflow_check(T, nS, j, "sorted-reference band depth"));
     cudaStream_t st = ctx->stream;
     if (nY == 0) return SD_OK;
     SD_CUDA(cudaMemsetAsync(d_out, 0, (size_t)(J - 1) * nY * sizeof(i64), st));
