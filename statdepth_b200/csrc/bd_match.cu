@@ -516,9 +516,13 @@ int bd_strict_match_batched_device(sd_ctx *ctx, const double *dXg, i64 nb, i64 T
     u32 *Rp = reinterpret_cast<u32 *>(rank_b + (size_t)nb * T * n);
     SD_TRY(mbd_all_device(ctx, dXg, nb * T, n, n, false, nullptr, nullptr, rank_b, nullptr));  // ranks only
     SD_TRY(prof_begin(ctx, SD_PHASE_BD_MASKS));
-    bd_pack_ranks_kernel<<<dim3((unsigned)ceil_div(TP * n, 256), (unsigned)nb), 256, 0, st>>>(rank_b, T, n, TP, Rp);
+    for (i64 b0 = 0; b0 < nb; b0 += 65535) {  // gridDim.y = batch: at most 65 535 per launch
+        const i64 cb = nb - b0 < 65535 ? nb - b0 : 65535;
+        bd_pack_ranks_kernel<<<dim3((unsigned)ceil_div(TP * n, 256), (unsigned)cb), 256, 0, st>>>(
+            rank_b + b0 * T * n, T, n, TP, Rp + b0 * TP * n);
+        ctx->last.launches++;
+    }
     SD_TRY(prof_end(ctx));
-    ctx->last.launches++;
     const size_t per_b = (size_t)nqb * ((size_t)W * m * sizeof(uint2) + (size_t)m * (sizeof(ulonglong2) + 1));
     i64 CB = (i64)((3ull << 29) / (per_b > 0 ? per_b : 1));  // matrices per launch pair: ~1.5 GB of sign words
     if (CB < 1) CB = 1;
