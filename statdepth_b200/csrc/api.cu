@@ -91,8 +91,8 @@ int band_depth_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const
     i64 *acc2 = ctx->buf[BUF_ACC].as<i64>();
     i64 *acc3 = acc2 + n;
     if (!d_q && j == 2)  // all curves, in order: the finish kernel writes the caller's buffer, no gather launch
-        return mbd_all_device(ctx, dX, T, n, ld, false, d_out, nullptr, nullptr, nullptr);
-    SD_TRY(mbd_all_device(ctx, dX, T, n, ld, j == 3, acc2, acc3, nullptr, nullptr));
+        return mbd_all_device(ctx, dX, T, n, ld, d_out, nullptr);
+    SD_TRY(mbd_all_device(ctx, dX, T, n, ld, acc2, j == 3 ? acc3 : nullptr));
     return gather_i64_device(ctx, j == 2 ? acc2 : acc3, d_q, nq, d_out);
 }
 
@@ -327,7 +327,7 @@ static int band_depth_pipelined(sd_ctx *ctx, const double *X, i64 T, i64 n, i64 
                 }
                 SD_CUDA(cudaEventRecord(ctx->ev_pipe[s], ctx->copy_stream));
                 SD_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_pipe[s], 0));
-                SD_TRY(mbd_all_device(ctx, dbuf[s], rows, n, n, j == 3, acc2, acc3, nullptr, nullptr, k > 0));
+                SD_TRY(mbd_all_device(ctx, dbuf[s], rows, n, n, acc2, j == 3 ? acc3 : nullptr, k > 0));
                 SD_CUDA(cudaEventRecord(ctx->ev_pipe[2 + s], ctx->stream));
             }
             return SD_OK;
@@ -450,7 +450,7 @@ int sd_band_ranks_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_
         s.download(below_out, d_b, (size_t)T * n * sizeof(int));
         s.download(above_out, d_b + (size_t)T * n, (size_t)T * n * sizeof(int));
         return SD_OK;
-    }, [&] { return mbd_all_device(ctx, dX, T, n, n, false, nullptr, nullptr, d_b, d_b + (size_t)T * n); });
+    }, [&] { return rank_rows_device(ctx, dX, T, n, n, d_b, d_b + (size_t)T * n); });
 }
 
 int sd_band_depth_batched_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_t ld,
@@ -530,8 +530,8 @@ int sd_band_depth_batched_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n
                 const i64 nb = B - b0 < BB ? B - b0 : BB;
                 SD_TRY(compact_batches_device(ctx, dX, T, n, d_cols + b0 * m0, m0, nb, dXg));
                 if (relax) {
-                    SD_TRY(mbd_all_device(ctx, dXg, nb * T, m0, m0, j == 3, acc2 + b0 * m0, acc3 + b0 * m0, nullptr,
-                                          nullptr, false, T));
+                    SD_TRY(mbd_all_device(ctx, dXg, nb * T, m0, m0, acc2 + b0 * m0, j == 3 ? acc3 + b0 * m0 : nullptr,
+                                          false, T));
                 } else {  // strict: sign-vector matcher over all sub-populations of the pass
                     ctx->last.bd_impl_used = SD_BD_MATCH;
                     SD_TRY(bd_strict_match_batched_device(ctx, dXg, nb, T, m0, d_ql + b0 * nqb, nqb, d_out + b0 * nqb,

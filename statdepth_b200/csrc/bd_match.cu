@@ -449,7 +449,7 @@ int bd_strict_match_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, 
         SD_TRY(ctx->buf[BUF_RANKS].reserve((size_t)T * n * sizeof(int) + (size_t)TP * n * sizeof(u32)));
         int *rank_b = ctx->buf[BUF_RANKS].as<int>();
         Rp = reinterpret_cast<u32 *>(rank_b + (size_t)T * n);
-        SD_TRY(mbd_all_device(ctx, dX, T, n, ld, false, nullptr, nullptr, rank_b, nullptr));  // ranks only
+        SD_TRY(rank_rows_device(ctx, dX, T, n, ld, rank_b, nullptr));
         SD_TRY(prof_begin(ctx, SD_PHASE_BD_MASKS));
         bd_pack_ranks_kernel<<<dim3((unsigned)ceil_div(TP * n, 256), 1), 256, 0, st>>>(rank_b, T, n, TP, Rp);
         SD_TRY(prof_end(ctx));
@@ -514,7 +514,7 @@ int bd_strict_match_batched_device(sd_ctx *ctx, const double *dXg, i64 nb, i64 T
     SD_TRY(ctx->buf[BUF_RANKS].reserve((size_t)nb * T * n * sizeof(int) + (size_t)nb * TP * n * sizeof(u32)));
     int *rank_b = ctx->buf[BUF_RANKS].as<int>();
     u32 *Rp = reinterpret_cast<u32 *>(rank_b + (size_t)nb * T * n);
-    SD_TRY(mbd_all_device(ctx, dXg, nb * T, n, n, false, nullptr, nullptr, rank_b, nullptr));  // ranks only
+    SD_TRY(rank_rows_device(ctx, dXg, nb * T, n, n, rank_b, nullptr));
     SD_TRY(prof_begin(ctx, SD_PHASE_BD_MASKS));
     for (i64 b0 = 0; b0 < nb; b0 += 65535) {  // gridDim.y = batch: at most 65 535 per launch
         const i64 cb = nb - b0 < 65535 ? nb - b0 : 65535;

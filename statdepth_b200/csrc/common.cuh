@@ -4,6 +4,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
+#include <functional>
 
 #include "../../include/statdepth_b200.h"
 
@@ -148,8 +149,20 @@ int band_depth_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const
 // (prefixed by who) and returns SD_ERR_OVERFLOW (api.cu).
 bool relaxed_overflows(i64 T, i64 others, int j);
 int relaxed_overflow_check(i64 T, i64 others, int j, const char *who);
-int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool want_j3, i64 *d_acc2,
-                   i64 *d_acc3, int *d_rank_b, int *d_rank_a, bool accumulate = false, i64 group_rows = 0);
+// K1, the per-row strict ranks of X [T, n] (mbd.cu).  mbd_all_device: d_acc2[c] (and d_acc3[c], if given) = the
+// relaxed j = 2 (3) numerator summed over the rows, added to the old value if `accumulate` (row blocks of one
+// matrix); group_rows = g > 0: T / g matrices of g rows accumulate into the rows of [T / g][n] (batched permutations).
+int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, i64 *d_acc2, i64 *d_acc3,
+                   bool accumulate = false, i64 group_rows = 0);
+// d_rank_b / d_rank_a[t*n + c] = #other values of row t strictly below / above X[t, c]; d_rank_a may be null.
+int rank_rows_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, int *d_rank_b, int *d_rank_a);
+// int32 workspace for rank-only passes in row blocks of *RB rows (ints_per_row each) within a fixed budget
+int rank_block_workspace(sd_ctx *ctx, i64 T, i64 ints_per_row, i64 *RB, int **ws);
+// Rank-only passes in blocks of that workspace, at most max_rows each: consume(r0, rows, rb, ra) queues the caller's
+// reduction of one block's ranks (ra null unless want_a) and counts its launches.
+using RankBlockFn = std::function<void(i64 r0, i64 rows, const int *rb, const int *ra)>;
+int for_each_rank_block(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool want_a, i64 max_rows,
+                        const RankBlockFn &consume);
 int bd_strict_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq, int j,
                      i64 *d_out, u64 *d_hits = nullptr);
 int bd_strict_gemm_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq,
@@ -191,8 +204,6 @@ int projection_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, i64 ld
 // out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out);
-// int32 workspace for rank-only passes in row blocks of *RB rows (ints_per_row each) within a fixed budget
-int rank_block_workspace(sd_ctx *ctx, i64 T, i64 ints_per_row, i64 *RB, int **ws);
 // sorted reference rows and out-of-sample counts from them (reference.cu)
 int sort_rows_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 ld, double *d_sorted);
 int depth_sorted_device(sd_ctx *ctx, const double *d_sorted, i64 T, i64 nS, const double *dY, i64 nY, i64 ldY,

@@ -7,10 +7,10 @@
 // extreme (the first depth level at which two depth CDFs differ decides, and that is the first differing key
 // element).  The numerator e(c) = #{h : key(h) >= key(c)} in [1, n]; ED = e / n, the deepest curve has e = n.
 //
-// Stage 1 (extremity_device): rank-only passes of the rank pipeline (mbd.cu) in row blocks of the rank workspace
-//   (rank_block_workspace, oos.cu); extremity_kernel writes m[t*n + c] as int32, row-major.  A rank outside
-//   0 <= b, a, b + a <= n - 1 sets ST_INTERNAL (never a trap); the finite check is K1's.  Rows are independent, so
-//   a block of time rows gives those rows of m (the multi-GPU split).
+// Stage 1 (extremity_device): rank-only passes of the rank pipeline in row blocks (for_each_rank_block, mbd.cu);
+//   extremity_kernel writes m[t*n + c] as int32, row-major.  A rank outside 0 <= b, a, b + a <= n - 1 sets
+//   ST_INTERNAL (never a trap); the finite check is K1's.  Rows are independent, so a block of time rows gives those
+//   rows of m (the multi-GPU split).
 // Stage 2a (extremal_keys_kernel): one CTA per group of G consecutive curves.  It reads rows of m coalesced along c,
 //   places curve g's T values in segment g (2^ceil(log2 T) slots, padded with 0, which sorts last) of a shared tile,
 //   sorts every segment descending with one segmented bitonic network (compare-exchanges never cross a segment),
@@ -56,21 +56,13 @@ int extremity_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, int *d
         return SD_ERR_INVALID;
     }
     cudaStream_t st = ctx->stream;
-    i64 RB = 0;
-    int *rb = nullptr;
-    SD_TRY(rank_block_workspace(ctx, T, 2 * n, &RB, &rb));
-    if (RB > EXT_MAX_ROWS) RB = EXT_MAX_ROWS;
-    int *ra = rb + (size_t)RB * n;
-    for (i64 r0 = 0; r0 < T; r0 += RB) {
-        const i64 rows = T - r0 < RB ? T - r0 : RB;
-        SD_TRY(mbd_all_device(ctx, dX + r0 * ld, rows, n, ld, false, nullptr, nullptr, rb, ra));  // ranks only
+    return for_each_rank_block(ctx, dX, T, n, ld, true, EXT_MAX_ROWS,
+                               [&](i64 r0, i64 rows, const int *rb, const int *ra) {
         i64 grid = ceil_div(rows * n, EXT_THREADS);
         if (grid > 8 * (i64)ctx->sm_count) grid = 8 * (i64)ctx->sm_count;
         extremity_kernel<<<(unsigned)grid, EXT_THREADS, 0, st>>>(rb, ra, n, rows * n, d_m + r0 * n, ctx->d_status);
         ctx->last.launches++;
-        SD_CUDA(cudaGetLastError());
-    }
-    return SD_OK;
+    });
 }
 
 // grid: one CTA per G = tile >> seg_log curves; dynamic shared memory: tile u32

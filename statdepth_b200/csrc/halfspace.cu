@@ -44,20 +44,12 @@ int halfspace1_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, i64 *
     }
     cudaStream_t st = ctx->stream;
     SD_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n * sizeof(i64), st));
-    i64 RB = 0;
-    int *rb = nullptr;
-    SD_TRY(rank_block_workspace(ctx, T, 2 * n, &RB, &rb));
-    if (RB > HS_MAX_ROW_TILES * HS_ROWS) RB = HS_MAX_ROW_TILES * HS_ROWS;
-    int *ra = rb + (size_t)RB * n;
-    for (i64 r0 = 0; r0 < T; r0 += RB) {
-        const i64 rows = T - r0 < RB ? T - r0 : RB;
-        SD_TRY(mbd_all_device(ctx, dX + r0 * ld, rows, n, ld, false, nullptr, nullptr, rb, ra));  // ranks only
+    return for_each_rank_block(ctx, dX, T, n, ld, true, HS_MAX_ROW_TILES * HS_ROWS,
+                               [&](i64, i64 rows, const int *rb, const int *ra) {
         const dim3 grid((unsigned)ceil_div(n, HS_THREADS), (unsigned)ceil_div(rows, HS_ROWS));
         halfspace_terms_kernel<<<grid, HS_THREADS, 0, st>>>(rb, ra, n, rows, d_out, ctx->d_status);
         ctx->last.launches++;
-        SD_CUDA(cudaGetLastError());
-    }
-    return SD_OK;
+    });
 }
 
 }  // namespace sd

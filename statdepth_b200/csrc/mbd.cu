@@ -9,7 +9,8 @@
 // Two pipelines produce the same integers.  Rows of 16 384 .. 131 072 curves take the SLAB path of mbd_slab.cuh
 // (included below: the row stays on the chip, three CTAs per row sort whole bins per thread); this file holds the
 // PART pipeline, which ranks every other row length, the rows the slab path declines (ties, wild tails; under a row
-// mask) and everything under SD_MBD_PATH=parts, and the driver that chooses (mbd_all_device).
+// mask) and everything under SD_MBD_PATH=parts, and the driver that chooses (rank_pipeline).  It has two fronts:
+// mbd_all_device accumulates the relaxed numerators, rank_rows_device writes the ranks b and a of every value.
 //
 // Part pipeline per block of time rows (all kernels on ctx->stream, no host sync):
 //   1. mbd_splitters_kernel : one CTA per row sorts a strided sample (u32 images of float(x - ref), register
@@ -38,7 +39,7 @@
 //                             almost always none is flagged).  Correct for any finite input; slower.
 //   5. mbd_finish_kernel    : numerator += rows * C(n-1,2) - raw / 2, once per call.
 // Row groups (mbd_all_device(..., group_rows)): the rows may be G stacked matrices of equal shape that accumulate
-// into [G][n] (batched permutations); rank-only calls (no accumulator) skip the REDs.
+// into [G][n] (batched permutations); rank_rows_device (no accumulator) skips the REDs.
 // HBM layout: X[t*ld + c] float64 (time-major rows are contiguous and streamed with coalesced
 // loads); raw uint64[n] -> acc int64[n] (mbd_finish_kernel); part lists [row][part][CAP] float32 + uint32.
 #include <stdlib.h>
@@ -1393,13 +1394,137 @@ static SlabPlan slab_plan(const double *dX, const i64 n, const i64 ld) {
     return p;
 }
 
-// d_acc2 == nullptr (with d_rank_b given): ranks only, nothing is accumulated.
-// Sum over ALL curves of one matrix: d_acc2[c] (and d_acc3[c]) += sum_t term_j(b,a).  The
-// accumulators are zeroed here unless `accumulate` (row blocks of one matrix).  Optional per-(t,c) rank output.
-// group_rows = g > 0: the T rows are G = T / g independent matrices of g rows each (same n); d_acc2 / d_acc3
-// are [G][n] and matrix k accumulates into row k (batched permutations: one launch sequence for all of them).
-int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool want_j3, i64 *d_acc2, i64 *d_acc3,
-                   int *d_rank_b, int *d_rank_a, bool accumulate, i64 group_rows) {
+// The part pipeline's geometry and workspaces for one call (blocks of at most Tc rows)
+struct PartPlan {
+    int P, S;
+    i64 NP, row_stride, Tc;
+    bool rank_subbin;
+    float *part_x, *splitters_f;
+    unsigned short *tables;
+    u32 *part_j, *pbase;
+    int *cursor, *rowflag;
+    int2 *biglist;
+};
+
+// The slab path on rows [r0, r0 + rows).  Once its rank kernel is queued, *only is the mask of the rows it skipped
+// (left to the part pipeline), and *done is set when the host has seen that it skipped none.
+static int slab_block(sd_ctx *ctx, const SlabPlan &sp, SlabArgs sa, const RankOut &o, const bool extra,
+                      const double *Xb, const i64 r0, const i64 rows, const int **only, bool *done) {
+    cudaStream_t st = ctx->stream;
+    sa.X = Xb;
+    sa.row0 = r0;
+    SD_CUDA(cudaMemsetAsync(sa.failcount, 0, sizeof(int), st));
+    for (int k = 0; k < 2; ++k)
+        if (!ctx->ev_slab[k]) SD_CUDA(cudaEventCreateWithFlags(&ctx->ev_slab[k], cudaEventDisableTiming));
+    SD_TRY(prof_begin(ctx, SD_PHASE_MBD_SLAB_HIST));
+    mbd_slab_table_kernel<<<(unsigned)rows, SL_TABLE_THREADS, 0, st>>>(sa);
+    // Rows this path cannot take are counted twice: after the table kernel (ties, degenerate ranges) and after the
+    // hist kernel (a bin, a CTA's share or the pair work over its limit: wild tails, adversarial spreads).  Both
+    // counts come back while later kernels run or are already queued, so the host decides without leaving the GPU
+    // idle.  Many unfit rows after the first count (tie-heavy data) send the whole block to the part pipeline;
+    // otherwise the rank kernel skips the flagged rows and the part pipeline ranks just those.
+    // A pipelined host call (row blocks copied on a second stream while earlier blocks are ranked) must not stall the
+    // host: it skips the counts and always queues the masked part pipeline behind the rank kernel (its CTAs exit at
+    // once when no row is flagged: ~50 us per block).  An SD_OPT_ASYNC_DEVICE call does wait: its waits end with the
+    // first two kernels, while the rank kernel is still running.
+    const bool ask = !ctx->mbd_no_wait;
+    if (ask) {
+        SD_CUDA(cudaMemcpyAsync(ctx->h_status + 3, sa.failcount, sizeof(int), cudaMemcpyDeviceToHost, st));
+        SD_CUDA(cudaEventRecord(ctx->ev_slab[0], st));
+    }
+    if (env_int("SD_MBD_SLAB_HIST_THREADS", rows <= (i64)ctx->sm_count ? 1024 : SL_HIST_THREADS) == 1024)
+        mbd_slab_hist_kernel<1024><<<(unsigned)rows, 1024, sp.smem_hist, st>>>(sa);
+    else
+        mbd_slab_hist_kernel<SL_HIST_THREADS><<<(unsigned)rows, SL_HIST_THREADS, sp.smem_hist, st>>>(sa);
+    SD_TRY(prof_end(ctx));
+    ctx->last.launches += 2;
+    if (ask) {
+        SD_CUDA(cudaMemcpyAsync(ctx->h_status + 2, sa.failcount, sizeof(int), cudaMemcpyDeviceToHost, st));
+        SD_CUDA(cudaEventRecord(ctx->ev_slab[1], st));
+        SD_CUDA(cudaEventSynchronize(ctx->ev_slab[0]));
+        if ((i64)ctx->h_status[3] * 16 > rows) return SD_OK;  // all unfit
+    }
+    const dim3 sgrid((unsigned)sp.G, (unsigned)rows);
+    SD_TRY(prof_begin(ctx, SD_PHASE_MBD_SLAB_RANK));
+    if (extra) mbd_slab_rank_kernel<true><<<sgrid, sp.threads, sp.smem_rank, st>>>(sa, o);
+    else mbd_slab_rank_kernel<false><<<sgrid, sp.threads, sp.smem_rank, st>>>(sa, o);
+    SD_TRY(prof_end(ctx));
+    ctx->last.launches++;
+    *only = sa.rowflag;  // the flagged rows: part pipeline (the generic path costs ~2 ms per long row)
+    if (ask) {
+        SD_CUDA(cudaEventSynchronize(ctx->ev_slab[1]));  // the rank kernel is queued behind the hist kernel
+        *done = ctx->h_status[2] == 0;
+    }
+    return SD_OK;
+}
+
+// Steps 1-3 of the part pipeline on rows [r0, r0 + rows): all of them, or those the mask `only` flags
+template <bool EXTRA>
+static int part_block(sd_ctx *ctx, const PartPlan &pp, const RankOut &o, const double *Xb, const i64 ld,
+                      const i64 r0, const i64 rows, const int *only) {
+    cudaStream_t st = ctx->stream;
+    const i64 n = o.n;
+    SD_CUDA(cudaMemsetAsync(pp.cursor, 0, (size_t)pp.Tc * (pp.P + 1) * sizeof(int), st));
+    if (pp.P > 1) {
+        SD_TRY(prof_begin(ctx, SD_PHASE_MBD_SPLITTERS));
+        mbd_splitters_kernel<<<(unsigned)rows, SP_THREADS, 0, st>>>(Xb, n, ld, pp.P, pp.S, pp.splitters_f, pp.tables,
+                                                                    pp.rowflag, ctx->d_status, only);
+        SD_TRY(prof_end(ctx));
+        ctx->last.launches++;
+    }
+    dim3 pgrid((unsigned)ceil_div(n, PT_CHUNK), (unsigned)rows);
+    SD_TRY(prof_begin(ctx, SD_PHASE_MBD_PARTITION));
+    mbd_partition_kernel<<<pgrid, PT_THREADS, PT_SMEM, st>>>(Xb, n, ld, pp.P, pp.splitters_f, pp.tables, pp.cursor,
+                                                             pp.rowflag, pp.part_x, pp.part_j, pp.row_stride,
+                                                             ctx->d_status, only);
+    SD_TRY(prof_end(ctx));
+    ctx->last.launches++;
+    SD_TRY(prof_begin(ctx, SD_PHASE_MBD_RANK));
+    // rows with parts of more than CAP values (heavy ties): those parts are ranked from value tables
+    // one thread per part for the prefix; rows with heavy parts scan their values with the same block
+    int hv_threads = 128;
+    while (hv_threads < pp.P) hv_threads <<= 1;
+    if (n > 16384) hv_threads = HV_THREADS;  // long rows: a heavy row scans n values
+    mbd_heavy_kernel<<<(unsigned)rows, hv_threads, 0, st>>>(Xb, n, ld, pp.P, pp.splitters_f, pp.tables, pp.cursor,
+                                                            pp.rowflag, pp.pbase, r0, o, only);
+    const RankArgs ra = {pp.P,      pp.cursor, pp.pbase,      pp.rowflag, pp.splitters_f, pp.part_x,   pp.part_j,
+                         Xb,        ld,        pp.row_stride, r0,         only,           pp.biglist, ctx->d_status + 2};
+    SD_CUDA(cudaMemsetAsync(ctx->d_status + 2, 0, 4 * sizeof(int), st));  // appended | claimed (big) | - | claimed (overflow)
+    const dim3 rgrid((unsigned)ceil_div(pp.P, RANK_WARPS), (unsigned)rows);
+    const unsigned bgrid = (unsigned)(ctx->sm_count * 4);
+    const unsigned ogrid = (unsigned)(ctx->sm_count * 8);
+    // many parts: the overflowed small parts get their own full-occupancy kernel (-15 us at 256 k parts);
+    // few parts (one rank's rows at 8 GPUs): one more persistent launch costs more than it saves (+10 us)
+    const bool subbin = pp.rank_subbin, split_overflow = subbin && rows * (i64)pp.P >= 100000;
+    if (subbin) mbd_rank_subbin_kernel<EXTRA><<<rgrid, RANK_WARPS * 32, 0, st>>>(ra, o);
+    else mbd_rank_kernel<EXTRA><<<rgrid, RANK_WARPS * 32, 0, st>>>(ra, o);
+    if (split_overflow) mbd_rank_overflow_kernel<EXTRA><<<ogrid, RANK_WARPS * 32, 0, st>>>(ra, o);
+    mbd_rank_big_kernel<EXTRA><<<bgrid, RANK_WARPS * 32, 0, st>>>(ra, o, subbin ? (split_overflow ? 2 : 1) : 0);
+    SD_TRY(prof_end(ctx));
+    ctx->last.launches += split_overflow ? 4 : 3;
+    return SD_OK;
+}
+
+// Step 4 on the rows of [r0, r0 + rows) flagged as overflowing, or all of them when forced; idle CTAs exit at once
+static int generic_block(sd_ctx *ctx, const PartPlan &pp, const RankOut &o, const double *Xb, const i64 ld,
+                         const i64 r0, const i64 rows) {
+    if (ctx->mbd_force_fallback) {
+        fill_int_kernel<<<(unsigned)ceil_div(rows, 256), 256, 0, ctx->stream>>>(pp.rowflag, rows, 2);
+        ctx->last.launches++;
+    }
+    SD_TRY(prof_begin(ctx, SD_PHASE_MBD_GENERIC));
+    const i64 fgrid = rows < 2 * (i64)ctx->sm_count ? rows : 2 * (i64)ctx->sm_count;
+    mbd_fallback_kernel<<<(unsigned)fgrid, 1024, 0, ctx->stream>>>(Xb, o.n, ld, pp.NP, pp.rowflag, rows,
+                                                                   (u64 *)pp.part_x, pp.NP, r0, o, ctx->d_status,
+                                                                   ctx->d_status + 1);
+    SD_TRY(prof_end(ctx));
+    ctx->last.launches++;
+    return SD_OK;
+}
+
+// The driver behind mbd_all_device and rank_rows_device; o brings the j = 3 accumulator, rank outputs and row groups.
+static int rank_pipeline(sd_ctx *ctx, const double *dX, const i64 T, const i64 n, const i64 ld, i64 *d_acc2,
+                         const bool accumulate, RankOut o) {
     if (n < 1 || T < 0 || ld < n) {
         set_error("mbd: bad shape T=%lld n=%lld ld=%lld", (long long)T, (long long)n, (long long)ld);
         return SD_ERR_INVALID;
@@ -1408,6 +1533,7 @@ int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool wan
         set_error("mbd: n=%lld exceeds 2^31-1", (long long)n);
         return SD_ERR_UNSUPPORTED;
     }
+    const i64 group_rows = o.group_rows;
     if (group_rows < 0 || (group_rows > 0 && T % group_rows != 0)) {
         set_error("mbd: %lld rows are not a multiple of the group size %lld", (long long)T, (long long)group_rows);
         return SD_ERR_INVALID;
@@ -1415,12 +1541,8 @@ int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool wan
     const i64 groups = group_rows > 0 ? T / group_rows : 1;
     const i64 acc_len = n * (groups > 0 ? groups : 1);
     cudaStream_t st = ctx->stream;
-    if (!d_acc2 && !d_rank_b) {
-        set_error("mbd: neither an accumulator nor a rank output was given");
-        return SD_ERR_INVALID;
-    }
     if (!accumulate && d_acc2) {  // d_acc2 itself is WRITTEN by mbd_finish_kernel
-        if (want_j3) SD_CUDA(cudaMemsetAsync(d_acc3, 0, (size_t)acc_len * sizeof(i64), st));
+        if (o.acc3) SD_CUDA(cudaMemsetAsync(o.acc3, 0, (size_t)acc_len * sizeof(i64), st));
         if (T == 0) SD_CUDA(cudaMemsetAsync(d_acc2, 0, (size_t)acc_len * sizeof(i64), st));
     }
     if (T == 0) return SD_OK;
@@ -1463,7 +1585,6 @@ int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool wan
     u32 *pbase = reinterpret_cast<u32 *>(rowflag + Tc);
     float *splitters_f = ctx->buf[BUF_SPLIT].as<float>();
     unsigned short *tables = reinterpret_cast<unsigned short *>(splitters_f + (size_t)Tc * (P > 1 ? P - 1 : 1));
-    int *fb_count = ctx->d_status + 1;
     SD_TRY(ctx->buf[BUF_WORK].reserve((size_t)Tc * P * sizeof(int2) + (size_t)acc_len * sizeof(u64)));
     int2 *biglist = ctx->buf[BUF_WORK].as<int2>();
     u64 *raw2 = reinterpret_cast<u64 *>(biglist + (size_t)Tc * P);
@@ -1473,8 +1594,7 @@ int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool wan
 
     // slab path (mbd_slab.cuh): per-value codes, bin starts, per-CTA offsets, row flags
     const SlabPlan sp = ctx->mbd_force_fallback ? SlabPlan{} : slab_plan(dX, n, ld);
-    SlabArgs sa;
-    memset(&sa, 0, sizeof(sa));
+    SlabArgs sa = {};
     if (sp.ok) {
         const size_t rows_cap = (size_t)Tc;
         const size_t cpitch = (size_t)((n + 3) & ~(i64)3);
@@ -1509,151 +1629,23 @@ int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool wan
                                      (int)sp.smem_rank));
     }
 
-    RankOut o;
+    const PartPlan pp = {P, S, NP, row_stride, Tc, rank_subbin, part_x, splitters_f, tables, part_j, pbase, cursor,
+                         rowflag, biglist};
     o.raw2 = d_acc2 ? raw2 : nullptr;
-    o.acc3 = want_j3 ? d_acc3 : nullptr;
-    o.rank_b = d_rank_b;
-    o.rank_a = d_rank_a;
     o.n = n;
     o.full2 = (n - 1) * (n - 2) / 2;
     o.full3 = n - 1 < 3 ? 0 : ((n - 1) * (n - 2) / 2) * (n - 3) / 3;
-    o.group_rows = group_rows;
-
+    const bool extra = o.acc3 || o.rank_b || o.group_rows;
     for (i64 r0 = 0; r0 < T; r0 += Tc) {
         const i64 rows = T - r0 < Tc ? T - r0 : Tc;
         const double *Xb = dX + r0 * ld;
         const int *only = nullptr;  // part pipeline restricted to the rows the slab path gave up
-        bool slab_done = false, need_generic = true;
-        if (sp.ok) {
-            sa.X = Xb;
-            sa.row0 = r0;
-            SD_CUDA(cudaMemsetAsync(sa.failcount, 0, sizeof(int), st));
-            for (int k = 0; k < 2; ++k)
-                if (!ctx->ev_slab[k]) SD_CUDA(cudaEventCreateWithFlags(&ctx->ev_slab[k], cudaEventDisableTiming));
-            SD_TRY(prof_begin(ctx, SD_PHASE_MBD_SLAB_HIST));
-            mbd_slab_table_kernel<<<(unsigned)rows, SL_TABLE_THREADS, 0, st>>>(sa);
-            // Rows this path cannot take are counted twice: after the table kernel (ties, degenerate ranges) and
-            // after the hist kernel (a bin, a CTA's share or the pair work over its limit: wild tails, adversarial
-            // spreads).  Both counts come back while later kernels run or are already queued, so the host decides
-            // without leaving the GPU idle.  Many unfit rows after the first count (tie-heavy data) send the whole
-            // block to the part pipeline; otherwise the rank kernel skips the flagged rows and the part pipeline
-            // ranks just those.
-            // A pipelined host call (row blocks copied on a second stream while earlier blocks are ranked) must not
-            // stall the host: it skips the counts and always queues the masked part pipeline behind the rank kernel
-            // (its CTAs exit at once when no row is flagged: ~50 us per block).  An SD_OPT_ASYNC_DEVICE call does wait:
-            // its waits end with the first two kernels, while the rank kernel is still running.
-            const bool ask = !ctx->mbd_no_wait;
-            if (ask) {
-                SD_CUDA(cudaMemcpyAsync(ctx->h_status + 3, sa.failcount, sizeof(int), cudaMemcpyDeviceToHost, st));
-                SD_CUDA(cudaEventRecord(ctx->ev_slab[0], st));
-            }
-            if (env_int("SD_MBD_SLAB_HIST_THREADS", rows <= (i64)ctx->sm_count ? 1024 : SL_HIST_THREADS) == 1024)
-                mbd_slab_hist_kernel<1024><<<(unsigned)rows, 1024, sp.smem_hist, st>>>(sa);
-            else
-                mbd_slab_hist_kernel<SL_HIST_THREADS><<<(unsigned)rows, SL_HIST_THREADS, sp.smem_hist, st>>>(sa);
-            SD_TRY(prof_end(ctx));
-            ctx->last.launches += 2;
-            bool all_unfit = false;
-            if (ask) {
-                SD_CUDA(cudaMemcpyAsync(ctx->h_status + 2, sa.failcount, sizeof(int), cudaMemcpyDeviceToHost, st));
-                SD_CUDA(cudaEventRecord(ctx->ev_slab[1], st));
-                SD_CUDA(cudaEventSynchronize(ctx->ev_slab[0]));
-                all_unfit = (i64)ctx->h_status[3] * 16 > rows;
-            }
-            if (!all_unfit) {
-                const dim3 sgrid((unsigned)sp.G, (unsigned)rows);
-                SD_TRY(prof_begin(ctx, SD_PHASE_MBD_SLAB_RANK));
-                if (o.acc3 || o.rank_b || o.group_rows)
-                    mbd_slab_rank_kernel<true><<<sgrid, sp.threads, sp.smem_rank, st>>>(sa, o);
-                else
-                    mbd_slab_rank_kernel<false><<<sgrid, sp.threads, sp.smem_rank, st>>>(sa, o);
-                SD_TRY(prof_end(ctx));
-                ctx->last.launches++;
-                only = sa.rowflag;  // the flagged rows: part pipeline (the generic path costs ~2 ms per long row)
-                if (ask) {
-                    SD_CUDA(cudaEventSynchronize(ctx->ev_slab[1]));  // the rank kernel is queued behind the hist kernel
-                    if (ctx->h_status[2] == 0) {
-                        slab_done = true;
-                        need_generic = false;
-                    }
-                }
-            }
-        }
-        if (slab_done) {
-            // every row of the block has been ranked by the slab path
-        } else if (ctx->mbd_force_fallback) {
-            fill_int_kernel<<<(unsigned)ceil_div(rows, 256), 256, 0, st>>>(rowflag, rows, 2);
-            ctx->last.launches++;
-        } else {
-            SD_CUDA(cudaMemsetAsync(cursor, 0, (size_t)Tc * (P + 1) * sizeof(int), st));
-            if (P > 1) {
-                SD_TRY(prof_begin(ctx, SD_PHASE_MBD_SPLITTERS));
-                mbd_splitters_kernel<<<(unsigned)rows, SP_THREADS, 0, st>>>(Xb, n, ld, P, S, splitters_f,
-                                                                            tables, rowflag, ctx->d_status, only);
-                SD_TRY(prof_end(ctx));
-                ctx->last.launches++;
-            }
-            dim3 pgrid((unsigned)ceil_div(n, PT_CHUNK), (unsigned)rows);
-            SD_TRY(prof_begin(ctx, SD_PHASE_MBD_PARTITION));
-            mbd_partition_kernel<<<pgrid, PT_THREADS, PT_SMEM, st>>>(Xb, n, ld, P, splitters_f, tables, cursor,
-                                                                     rowflag, part_x, part_j, row_stride,
-                                                                     ctx->d_status, only);
-            SD_TRY(prof_end(ctx));
-            ctx->last.launches++;
-            SD_TRY(prof_begin(ctx, SD_PHASE_MBD_RANK));
-            // rows with parts of more than CAP values (heavy ties): those parts are ranked from value tables
-            // one thread per part for the prefix; rows with heavy parts scan their values with the same block
-            int hv_threads = 128;
-            while (hv_threads < P) hv_threads <<= 1;
-            if (n > 16384) hv_threads = HV_THREADS;  // long rows: a heavy row scans n values
-            mbd_heavy_kernel<<<(unsigned)rows, hv_threads, 0, st>>>(Xb, n, ld, P, splitters_f, tables, cursor, rowflag, pbase,
-                                                                    r0, o, only);
-            RankArgs ra;
-            ra.P = P;
-            ra.cursor = cursor;
-            ra.pbase = pbase;
-            ra.rowflag = rowflag;
-            ra.only = only;
-            ra.splitters_f = splitters_f;
-            ra.X = Xb;
-            ra.ld = ld;
-            ra.part_x = part_x;
-            ra.part_j = part_j;
-            ra.row_stride = row_stride;
-            ra.row0 = r0;
-            ra.biglist = biglist;
-            ra.bigcount = ctx->d_status + 2;
-            SD_CUDA(cudaMemsetAsync(ctx->d_status + 2, 0, 4 * sizeof(int), st));  // appended | claimed (big) | - | claimed (overflow)
-            const dim3 rgrid((unsigned)ceil_div(P, RANK_WARPS), (unsigned)rows);
-            const unsigned bgrid = (unsigned)(ctx->sm_count * 4);
-            const unsigned ogrid = (unsigned)(ctx->sm_count * 8);
-            // many parts: the overflowed small parts get their own full-occupancy kernel (-15 us at 256 k parts);
-            // few parts (one rank's rows at 8 GPUs): one more persistent launch costs more than it saves (+10 us)
-            const bool split_overflow = rank_subbin && rows * (i64)P >= 100000;
-            const int big_mode = rank_subbin ? (split_overflow ? 2 : 1) : 0;
-            if (o.acc3 || o.rank_b || o.group_rows) {
-                if (rank_subbin) mbd_rank_subbin_kernel<true><<<rgrid, RANK_WARPS * 32, 0, st>>>(ra, o);
-                else mbd_rank_kernel<true><<<rgrid, RANK_WARPS * 32, 0, st>>>(ra, o);
-                if (split_overflow) mbd_rank_overflow_kernel<true><<<ogrid, RANK_WARPS * 32, 0, st>>>(ra, o);
-                mbd_rank_big_kernel<true><<<bgrid, RANK_WARPS * 32, 0, st>>>(ra, o, big_mode);
-            } else {
-                if (rank_subbin) mbd_rank_subbin_kernel<false><<<rgrid, RANK_WARPS * 32, 0, st>>>(ra, o);
-                else mbd_rank_kernel<false><<<rgrid, RANK_WARPS * 32, 0, st>>>(ra, o);
-                if (split_overflow) mbd_rank_overflow_kernel<false><<<ogrid, RANK_WARPS * 32, 0, st>>>(ra, o);
-                mbd_rank_big_kernel<false><<<bgrid, RANK_WARPS * 32, 0, st>>>(ra, o, big_mode);
-            }
-            SD_TRY(prof_end(ctx));
-            ctx->last.launches += split_overflow ? 4 : 3;
-        }
-        // rows flagged as overflowing (or all rows when forced): generic path; idle CTAs exit at once
-        if (need_generic) {
-            SD_TRY(prof_begin(ctx, SD_PHASE_MBD_GENERIC));
-            const i64 fgrid = rows < 2 * (i64)ctx->sm_count ? rows : 2 * (i64)ctx->sm_count;
-            mbd_fallback_kernel<<<(unsigned)fgrid, 1024, 0, st>>>(Xb, n, ld, NP, rowflag, rows, (u64 *)part_x, NP, r0, o,
-                                                                  ctx->d_status, fb_count);
-            SD_TRY(prof_end(ctx));
-            ctx->last.launches++;
-        }
+        bool done = false;
+        if (sp.ok) SD_TRY(slab_block(ctx, sp, sa, o, extra, Xb, r0, rows, &only, &done));
+        if (!done && !ctx->mbd_force_fallback)
+            SD_TRY(extra ? part_block<true>(ctx, pp, o, Xb, ld, r0, rows, only)
+                         : part_block<false>(ctx, pp, o, Xb, ld, r0, rows, only));
+        if (!done) SD_TRY(generic_block(ctx, pp, o, Xb, ld, r0, rows));
         SD_CUDA(cudaGetLastError());
     }
     if (d_acc2) {
@@ -1663,6 +1655,45 @@ int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool wan
         ctx->last.launches++;
     }
     SD_CUDA(cudaGetLastError());
+    return SD_OK;
+}
+
+int mbd_all_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, i64 *d_acc2, i64 *d_acc3, bool accumulate,
+                   i64 group_rows) {
+    RankOut o = {nullptr, d_acc3};
+    o.group_rows = group_rows;
+    return rank_pipeline(ctx, dX, T, n, ld, d_acc2, accumulate, o);
+}
+
+int rank_rows_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, int *d_rank_b, int *d_rank_a) {
+    return rank_pipeline(ctx, dX, T, n, ld, nullptr, false, RankOut{nullptr, nullptr, d_rank_b, d_rank_a});
+}
+
+constexpr size_t RANK_BLOCK_BUDGET = 1ull << 30;
+
+int rank_block_workspace(sd_ctx *ctx, i64 T, i64 ints_per_row, i64 *RB, int **ws) {
+    i64 rb = (i64)(RANK_BLOCK_BUDGET / ((size_t)ints_per_row * sizeof(int)));
+    if (rb < 1) rb = 1;
+    if (rb > T) rb = T;
+    SD_TRY(ctx->buf[BUF_RANKS].reserve((size_t)rb * ints_per_row * sizeof(int)));
+    *RB = rb;
+    *ws = ctx->buf[BUF_RANKS].as<int>();
+    return SD_OK;
+}
+
+int for_each_rank_block(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool want_a, i64 max_rows,
+                        const RankBlockFn &consume) {
+    i64 RB = 0;
+    int *rb = nullptr;
+    SD_TRY(rank_block_workspace(ctx, T, want_a ? 2 * n : n, &RB, &rb));
+    if (RB > max_rows) RB = max_rows;
+    int *ra = want_a ? rb + (size_t)RB * n : nullptr;
+    for (i64 r0 = 0; r0 < T; r0 += RB) {
+        const i64 rows = T - r0 < RB ? T - r0 : RB;
+        SD_TRY(rank_rows_device(ctx, dX + r0 * ld, rows, n, ld, rb, ra));
+        consume(r0, rows, rb, ra);
+        SD_CUDA(cudaGetLastError());
+    }
     return SD_OK;
 }
 

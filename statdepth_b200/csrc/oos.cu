@@ -85,19 +85,6 @@ __global__ void __launch_bounds__(OOS_THREADS) oos_terms_kernel(const int *__res
     if (sum) atomicAdd((u64 *)&acc[g], (u64)sum);
 }
 
-// Rank workspace of the rank-only passes, split into row blocks (also used by rank_sums_device, outliers.cu).
-constexpr size_t RANK_BLOCK_BUDGET = 1ull << 30;
-
-int rank_block_workspace(sd_ctx *ctx, i64 T, i64 ints_per_row, i64 *RB, int **ws) {
-    i64 rb = (i64)(RANK_BLOCK_BUDGET / ((size_t)ints_per_row * sizeof(int)));
-    if (rb < 1) rb = 1;
-    if (rb > T) rb = T;
-    SD_TRY(ctx->buf[BUF_RANKS].reserve((size_t)rb * ints_per_row * sizeof(int)));
-    *RB = rb;
-    *ws = ctx->buf[BUF_RANKS].as<int>();
-    return SD_OK;
-}
-
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out) {
     if (j != 2 && j != 3) {
@@ -133,8 +120,8 @@ int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, 
     for (i64 r0 = 0; r0 < T; r0 += RB) {
         const i64 rows = T - r0 < RB ? T - r0 : RB;
         const double *Xb = dX + r0 * ld;
-        SD_TRY(mbd_all_device(ctx, Xb, rows, n, ld, false, nullptr, nullptr, bP, aP));  // ranks only
-        if (ny_ranks) SD_TRY(mbd_all_device(ctx, Xb + nS, rows, nY, ld, false, nullptr, nullptr, bY, aY));
+        SD_TRY(rank_rows_device(ctx, Xb, rows, n, ld, bP, aP));
+        if (ny_ranks) SD_TRY(rank_rows_device(ctx, Xb + nS, rows, nY, ld, bY, aY));
         const dim3 grid((unsigned)ceil_div(nY, OOS_THREADS), (unsigned)ceil_div(rows, OOS_ROWS));
         if (j == 2) oos_terms_kernel<2><<<grid, OOS_THREADS, 0, st>>>(bP, aP, bY, aY, nS, nY, rows, d_out, ctx->d_status);
         else oos_terms_kernel<3><<<grid, OOS_THREADS, 0, st>>>(bP, aP, bY, aY, nS, nY, rows, d_out, ctx->d_status);

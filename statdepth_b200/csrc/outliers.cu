@@ -67,20 +67,12 @@ int rank_sums_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, i64 *d
     SD_CUDA(cudaMemsetAsync(d_q, 0, (size_t)n * sizeof(i64), st));
     SD_CUDA(cudaMemsetAsync(d_b, 0, (size_t)n * sizeof(i64), st));
     if (d_a) SD_CUDA(cudaMemsetAsync(d_a, 0, (size_t)n * sizeof(i64), st));
-    i64 RB = 0;
-    int *rb = nullptr;
-    SD_TRY(rank_block_workspace(ctx, T, 2 * n, &RB, &rb));
-    if (RB > RS_MAX_ROW_TILES * RS_ROWS) RB = RS_MAX_ROW_TILES * RS_ROWS;
-    int *ra = rb + (size_t)RB * n;
-    for (i64 r0 = 0; r0 < T; r0 += RB) {
-        const i64 rows = T - r0 < RB ? T - r0 : RB;
-        SD_TRY(mbd_all_device(ctx, dX + r0 * ld, rows, n, ld, false, nullptr, nullptr, rb, ra));  // ranks only
+    return for_each_rank_block(ctx, dX, T, n, ld, true, RS_MAX_ROW_TILES * RS_ROWS,
+                               [&](i64, i64 rows, const int *rb, const int *ra) {
         const dim3 grid((unsigned)ceil_div(n, RS_THREADS), (unsigned)ceil_div(rows, RS_ROWS));
         rank_sums_kernel<<<grid, RS_THREADS, 0, st>>>(rb, ra, n, rows, d_q, d_b, d_a, ctx->d_status);
         ctx->last.launches++;
-        SD_CUDA(cudaGetLastError());
-    }
-    return SD_OK;
+    });
 }
 
 constexpr int ENV_THREADS = 256;

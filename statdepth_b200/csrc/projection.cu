@@ -18,7 +18,7 @@
 //   projection_kernel   register-tiled like a small GEMM: a CTA computes 128 points x 32 directions, 4 x 4 per
 //                       thread, for TT consecutive time points; it stages each point's record of TT * d values
 //                       (contiguous in F) through shared memory, or for d > 32 one time point in chunks of 32.
-//   RT: mbd_all_device  rank-only passes (as halfspace1_device), then rt_min_kernel: one thread per (i, up to 32 time
+//   RT: rank_rows_device passes (as halfspace1_device), then rt_min_kernel: one thread per (i, up to 32 time
 //                       points) reads the block's kb rows of each t coalesced along i and keeps a running int32 min;
 //                       after the last direction block it adds sum_t with one int64 atomic.
 //   PD: sort_rows_device (K9) into sorted rows, medmad_kernel (one thread per row: median, then the MAD as the k-th
@@ -288,7 +288,7 @@ int projection_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, i64 ld
             }
             const int first = k0 == 0, last = k0 + kb == K;
             if (rt) {
-                SD_TRY(mbd_all_device(ctx, Yb, rows, N, ldY, false, nullptr, nullptr, rb, ra));  // ranks only
+                SD_TRY(rank_rows_device(ctx, Yb, rows, N, ldY, rb, ra));
                 rt_min_kernel<<<rgrid, RD_THREADS, 0, st>>>(rb, ra, N, kb, tb, tpt, (int *)pred, first, last, d_count,
                                                             ctx->d_status);
                 ctx->last.launches++;

@@ -5,8 +5,8 @@
 // scored against again and again is sorted once and kept on the device; each later call reads only the new curves.
 //
 // Build (sort_rows_device): sorted[t*nS + k] = the k-th smallest of row t, ties repeated.
-//   1. K1 rank-only passes (mbd.cu) give every value its below-rank b (exact, finite check included), in row
-//      blocks of the rank workspace (rank_block_workspace, oos.cu).
+//   1. K1 rank-only passes in row blocks (for_each_rank_block, mbd.cu) give every value its below-rank b (exact,
+//      finite check included).
 //   2. sort_scatter_kernel  sorted[t][b] = X[t, c].  All curves of a tie run share b and write equal values to the
 //                           run's first slot (benign race; -0.0 and +0.0 compare equal, either may land).  The other
 //                           slots of the run keep the gap sentinel the rows were filled with before: an all-ones NaN
@@ -130,18 +130,12 @@ int sort_rows_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 ld, doubl
     }
     cudaStream_t st = ctx->stream;
     SD_CUDA(cudaMemsetAsync(d_sorted, 0xff, (size_t)T * nS * sizeof(double), st));  // gap sentinel: a NaN
-    i64 RB = 0;
-    int *below = nullptr;
-    SD_TRY(rank_block_workspace(ctx, T, nS, &RB, &below));
-    if (RB > SORT_MAX_ROWS) RB = SORT_MAX_ROWS;
-    for (i64 r0 = 0; r0 < T; r0 += RB) {
-        const i64 rows = T - r0 < RB ? T - r0 : RB;
-        SD_TRY(mbd_all_device(ctx, dX + r0 * ld, rows, nS, ld, false, nullptr, nullptr, below, nullptr));  // ranks only
+    SD_TRY(for_each_rank_block(ctx, dX, T, nS, ld, false, SORT_MAX_ROWS,
+                               [&](i64 r0, i64 rows, const int *below, const int *) {
         sort_scatter_kernel<<<dim3((unsigned)ceil_div(nS, SORT_THREADS), (unsigned)rows), SORT_THREADS, 0, st>>>(
             dX + r0 * ld, ld, below, nS, d_sorted + r0 * nS, ctx->d_status);
         ctx->last.launches++;
-        SD_CUDA(cudaGetLastError());
-    }
+    }));
     i64 chunks = ceil_div(4 * (i64)ctx->sm_count, T);
     const i64 most = ceil_div(nS, FILL_MIN_CHUNK);
     if (chunks > most) chunks = most;

@@ -279,8 +279,8 @@ int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride
         sc_keys_kernel<<<dim3(gx, (unsigned)ni), 256, 0, st>>>(g, n, ni, tol, KA, KB, ctx->d_status);
         ctx->last.launches++;
         if (!hs) SD_CUDA(cudaMemsetAsync(claim, 0, (size_t)ni * n * sizeof(int), st));
-        SD_TRY(mbd_all_device(ctx, KA, ni, n, n, false, nullptr, nullptr, bA, aA));  // ranks only
-        SD_TRY(mbd_all_device(ctx, KB, ni, 2 * n, 2 * n, false, nullptr, nullptr, bB, tol > 0.0 || hs ? aB : nullptr));
+        SD_TRY(rank_rows_device(ctx, KA, ni, n, n, bA, aA));
+        SD_TRY(rank_rows_device(ctx, KB, ni, 2 * n, 2 * n, bB, tol > 0.0 || hs ? aB : nullptr));
         if (hs) hs_reduce_kernel<<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, d_out, ctx->d_status);
         else if (tol > 0.0) sc_reduce_kernel<true><<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, claim, m_others, d_out);
         else sc_reduce_kernel<false><<<(unsigned)ni, 256, 0, st>>>(g, n, KA, KB, bA, aA, bB, aB, claim, m_others, d_out);
@@ -446,8 +446,8 @@ int oja2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, const i64 *d_q, i
         if (gx < 1) gx = 1;
         sc_keys_kernel<<<dim3(gx, (unsigned)ni), 256, 0, st>>>(g, n, ni, 0.0, KA, KB, ctx->d_status);
         ctx->last.launches++;
-        SD_TRY(mbd_all_device(ctx, KA, ni, n, n, false, nullptr, nullptr, bA, aA));
-        SD_TRY(mbd_all_device(ctx, KB, ni, 2 * n, 2 * n, false, nullptr, nullptr, bB, nullptr));
+        SD_TRY(rank_rows_device(ctx, KA, ni, n, n, bA, aA));
+        SD_TRY(rank_rows_device(ctx, KB, ni, 2 * n, 2 * n, bB, nullptr));
         oja2_reduce_kernel<<<(unsigned)ni, OJ_THREADS, 0, st>>>(g, n, KA, bA, aA, bB, bucket, hull_volume, d_out);
         ctx->last.launches++;
         SD_CUDA(cudaGetLastError());
