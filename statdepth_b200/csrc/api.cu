@@ -30,16 +30,6 @@ static int strict_enumerate(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld,
     SD_TRY(ctx->buf[BUF_WORK].reserve(sizeof(u64)));
     u64 *d_hits = ctx->buf[BUF_WORK].as<u64>();
     SD_CUDA(cudaMemsetAsync(d_hits, 0, sizeof(u64), ctx->stream));
-    i64 *iq = nullptr;
-    if (!d_q) {  // materialise the identity so that the probe and the remainder can be offset
-        SD_TRY(ctx->buf[BUF_QIDX].reserve((size_t)nq * sizeof(i64) * 2));
-        iq = ctx->buf[BUF_QIDX].as<i64>() + nq;
-        std::vector<i64> h((size_t)nq);
-        for (i64 i = 0; i < nq; ++i) h[(size_t)i] = i;
-        SD_CUDA(cudaMemcpyAsync(iq, h.data(), (size_t)nq * sizeof(i64), cudaMemcpyHostToDevice, ctx->stream));
-        SD_CUDA(cudaStreamSynchronize(ctx->stream));
-        d_q = iq;
-    }
     SD_TRY(bd_strict_device(ctx, dX, T, n, ld, d_q, PROBE, 2, d_out, d_hits));
     u64 h_hits = 0;
     SD_CUDA(cudaMemcpyAsync(&h_hits, d_hits, sizeof(u64), cudaMemcpyDeviceToHost, ctx->stream));
@@ -74,6 +64,12 @@ int band_depth_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const
         return SD_ERR_UNSUPPORTED;
     }
     if (!relax) {
+        if (!d_q) {  // all curves: the strict drivers take an explicit list (the probe and the chunks offset it)
+            SD_TRY(ctx->buf[BUF_QIDX].reserve((size_t)nq * sizeof(i64)));
+            i64 *q = ctx->buf[BUF_QIDX].as<i64>();
+            SD_TRY(iota_from_device(ctx, q, nq, 0));
+            d_q = q;
+        }
         if (j == 3) {
             ctx->last.bd_impl_used = SD_BD_BITS;
             return bd_strict_device(ctx, dX, T, n, ld, d_q, nq, 3, d_out);

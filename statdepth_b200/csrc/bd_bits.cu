@@ -211,12 +211,7 @@ __global__ void __launch_bounds__(256) bd_triple_kernel(const uint2 *__restrict_
     if ((threadIdx.x & 31) == 0 && count) atomicAdd((u64 *)&out[q], count);
 }
 
-__global__ void iota_i64_kernel(i64 *p, i64 count) {
-    const i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < count) p[i] = i;
-}
-
-// d_q == nullptr means all curves.  d_out[nq] receives the strict numerator for subset size j.
+// d_out[nq] receives the strict numerator for subset size j.
 int bd_strict_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq, int j,
                      i64 *d_out, u64 *d_hits) {
     if (n < 1 || T < 1 || ld < n || nq < 0) {
@@ -232,13 +227,6 @@ int bd_strict_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const 
     SD_CUDA(cudaMemsetAsync(d_out, 0, (size_t)nq * sizeof(i64), st));
     const i64 m = n - 1;  // other curves
     if (nq == 0 || m < j) return SD_OK;
-    if (!d_q) {
-        SD_TRY(ctx->buf[BUF_QIDX].reserve((size_t)nq * sizeof(i64)));
-        i64 *iq = ctx->buf[BUF_QIDX].as<i64>();
-        iota_i64_kernel<<<(unsigned)ceil_div(nq, 256), 256, 0, st>>>(iq, nq);
-        ctx->last.launches++;
-        d_q = iq;
-    }
     const i64 W = ceil_div(T, 32);
     if (W > 65535) {
         set_error("strict band depth: T=%lld too large (max %d)", (long long)T, 65535 * 32);

@@ -408,11 +408,6 @@ int probe_int8_peak(sd_ctx *ctx, double *ops_per_s) {
     return SD_OK;
 }
 
-__global__ void iota_i64_kernel2(i64 *p, i64 count) {
-    const i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < count) p[i] = i;
-}
-
 int bd_strict_gemm_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq,
                           i64 *d_out) {
     if (n < 1 || T < 1 || ld < n || nq < 0) {
@@ -426,13 +421,6 @@ int bd_strict_gemm_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, c
     cudaStream_t st = ctx->stream;
     SD_CUDA(cudaMemsetAsync(d_out, 0, (size_t)nq * sizeof(i64), st));
     if (nq == 0) return SD_OK;
-    if (!d_q) {
-        SD_TRY(ctx->buf[BUF_QIDX].reserve((size_t)nq * sizeof(i64)));
-        i64 *iq = ctx->buf[BUF_QIDX].as<i64>();
-        iota_i64_kernel2<<<(unsigned)ceil_div(nq, 256), 256, 0, st>>>(iq, nq);
-        ctx->last.launches++;
-        d_q = iq;
-    }
     const int NB = (int)ceil_div(n, GM_TILE);
     const int KS = (int)ceil_div(T, GM_TSTEP);
     if (2 * KS > 65535) {

@@ -18,6 +18,10 @@
 //                     curves that tie with q somewhere (set Z, at most 64) are tested against everybody.
 // Exactness does not rest on the hash: a run with two different vectors, a hash hit whose words differ, or
 // more than 64 tied curves flags the query, and flagged queries are recomputed by the enumerating kernels.
+// Both drivers, for one matrix and for nb equally shaped matrices (permutation tests), take their ranks from
+// packed_ranks (one rank pass, ranks packed in pairs; the single driver skips it for long series or few queries)
+// and end in recompute_flagged (flags read back once, flagged queries recomputed matrix by matrix).  They differ
+// in how they chunk the signature and match launches.
 #include <vector>
 
 #include "common.cuh"
@@ -385,19 +389,10 @@ __global__ void __launch_bounds__(NT, NT == 512 ? 2 : 8) bd_match_kernel(const u
     }
 }
 
-__global__ void bm_gather_kernel(const i64 *__restrict__ src, const i64 *__restrict__ pos, i64 cnt,
-                                 i64 *__restrict__ dst) {
-    const i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < cnt) dst[i] = src[pos[i]];
-}
 __global__ void bm_scatter_kernel(const i64 *__restrict__ src, const i64 *__restrict__ pos, i64 cnt,
                                   i64 *__restrict__ dst) {
     const i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < cnt) dst[pos[i]] = src[i];
-}
-__global__ void bm_iota_kernel(i64 *p, i64 count) {
-    const i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < count) p[i] = i;
 }
 
 // picks the smallest sort capacity that holds the m other curves of a query
@@ -418,43 +413,75 @@ static int launch_match(cudaStream_t st, dim3 grid, i64 m, const uint2 *Mw, cons
 
 bool bd_match_supported(i64 T, i64 n) { return n - 1 <= BM_MAXM && n >= 3 && ceil_div(T, 32) <= 4096; }
 
-// d_out[nq] = strict J=2 numerators.  Queries the matcher cannot certify are recomputed with `fallback`
-// (the enumerating path).  Synchronises the stream once (to read the flags).
+// Ranks of all curves at every time point of nb matrices of T rows (matrix b starts at row b·T of dX), from one pass
+// of the rank pipeline, packed in pairs for the signature kernel: *Rp = [nb][TP][n] words in BUF_RANKS.
+static int packed_ranks(sd_ctx *ctx, const double *dX, i64 ld, i64 nb, i64 T, i64 n, u32 **Rp) {
+    const i64 TP = ceil_div(T, 32) * 16;
+    SD_TRY(ctx->buf[BUF_RANKS].reserve((size_t)nb * T * n * sizeof(int) + (size_t)nb * TP * n * sizeof(u32)));
+    int *rank_b = ctx->buf[BUF_RANKS].as<int>();
+    *Rp = reinterpret_cast<u32 *>(rank_b + (size_t)nb * T * n);
+    SD_TRY(rank_rows_device(ctx, dX, nb * T, n, ld, rank_b, nullptr));
+    SD_TRY(prof_begin(ctx, SD_PHASE_BD_MASKS));
+    for (i64 b0 = 0; b0 < nb; b0 += 65535) {  // gridDim.y = batch: at most 65 535 per launch
+        const i64 cb = nb - b0 < 65535 ? nb - b0 : 65535;
+        bd_pack_ranks_kernel<<<dim3((unsigned)ceil_div(TP * n, 256), (unsigned)cb), 256, 0, ctx->stream>>>(
+            rank_b + b0 * T * n, T, n, TP, *Rp + b0 * TP * n);
+        ctx->last.launches++;
+    }
+    SD_TRY(prof_end(ctx));
+    return SD_OK;
+}
+
+// Recomputes the queries the match kernel flagged with `fallback` (the enumerating path), matrix by matrix: nb
+// matrices of T rows (matrix b starts at row b·T of dX), nqb queries each, d_flag / d_q / d_out laid out [nb][nqb].
+// Reads the flags back with one synchronisation; *n_fallback (if given) grows by the number of flagged queries.
+static int recompute_flagged(sd_ctx *ctx, const double *dX, i64 nb, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nqb,
+                             const unsigned char *d_flag, i64 *d_out, StrictFallback fallback, i64 *n_fallback) {
+    cudaStream_t st = ctx->stream;
+    std::vector<unsigned char> h_flag((size_t)(nb * nqb));
+    SD_CUDA(cudaMemcpyAsync(h_flag.data(), d_flag, h_flag.size(), cudaMemcpyDeviceToHost, st));
+    SD_CUDA(cudaStreamSynchronize(st));
+    std::vector<i64> pos;
+    for (i64 b = 0; b < nb; ++b) {
+        pos.clear();
+        for (i64 i = 0; i < nqb; ++i)
+            if (h_flag[(size_t)(b * nqb + i)]) pos.push_back(i);
+        if (n_fallback) *n_fallback += (i64)pos.size();
+        if (pos.empty()) continue;
+        const i64 nf = (i64)pos.size();
+        SD_TRY(ctx->buf[BUF_SPLIT].reserve((size_t)nf * 3 * sizeof(i64)));
+        i64 *d_pos = ctx->buf[BUF_SPLIT].as<i64>();
+        i64 *d_qsub = d_pos + nf, *d_osub = d_qsub + nf;
+        SD_CUDA(cudaMemcpyAsync(d_pos, pos.data(), (size_t)nf * sizeof(i64), cudaMemcpyHostToDevice, st));
+        SD_TRY(gather_i64_device(ctx, d_q + b * nqb, d_pos, nf, d_qsub));
+        SD_CUDA(cudaStreamSynchronize(st));  // pos is a pageable host vector
+        SD_TRY(fallback(ctx, dX + b * T * ld, T, n, ld, d_qsub, nf, d_osub));
+        bm_scatter_kernel<<<(unsigned)ceil_div(nf, 256), 256, 0, st>>>(d_osub, d_pos, nf, d_out + b * nqb);
+        ctx->last.launches++;
+        SD_CUDA(cudaGetLastError());
+    }
+    return SD_OK;
+}
+
+// d_out[nq] = strict J=2 numerators.  Queries the matcher cannot certify are recomputed with `fallback`;
+// *n_fallback counts them.
 int bd_strict_match_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq, i64 *d_out,
-                           int (*fallback)(sd_ctx *, const double *, i64, i64, i64, const i64 *, i64, i64 *),
-                           i64 *n_fallback) {
+                           StrictFallback fallback, i64 *n_fallback) {
     cudaStream_t st = ctx->stream;
     if (n_fallback) *n_fallback = 0;
     if (nq == 0) return SD_OK;
     const i64 m = n - 1;
     const i64 W = ceil_div(T, 32);
-    if (!d_q) {
-        SD_TRY(ctx->buf[BUF_QIDX].reserve((size_t)nq * sizeof(i64) * 2));
-        i64 *iq = ctx->buf[BUF_QIDX].as<i64>() + nq;
-        bm_iota_kernel<<<(unsigned)ceil_div(nq, 256), 256, 0, st>>>(iq, nq);
-        ctx->last.launches++;
-        d_q = iq;
-    }
     const size_t per_q = (size_t)W * m * sizeof(uint2) + (size_t)m * (sizeof(ulonglong2) + 1) + 64;
     i64 QB = (i64)((2ull << 30) / per_q);
     if (QB < BM_SQ) QB = BM_SQ;
     if (QB > 32768) QB = 32768;
     if (QB > nq) QB = nq;
-    // ranks of all curves at every time point (one pass of the rank pipeline), packed in pairs for the signature
-    // kernel; very long series keep the float64 signature kernel (the rank matrix would not pay)
-    const i64 TP = W * 16;
+    // signatures from packed ranks; very long series or few queries keep the float64 signature kernel (the rank
+    // matrix would not pay)
     const bool by_ranks = T * n <= (1ll << 26) && nq >= 64;
     u32 *Rp = nullptr;
-    if (by_ranks) {
-        SD_TRY(ctx->buf[BUF_RANKS].reserve((size_t)T * n * sizeof(int) + (size_t)TP * n * sizeof(u32)));
-        int *rank_b = ctx->buf[BUF_RANKS].as<int>();
-        Rp = reinterpret_cast<u32 *>(rank_b + (size_t)T * n);
-        SD_TRY(rank_rows_device(ctx, dX, T, n, ld, rank_b, nullptr));
-        SD_TRY(prof_begin(ctx, SD_PHASE_BD_MASKS));
-        bd_pack_ranks_kernel<<<dim3((unsigned)ceil_div(TP * n, 256), 1), 256, 0, st>>>(rank_b, T, n, TP, Rp);
-        SD_TRY(prof_end(ctx));
-        ctx->last.launches++;
-    }
+    if (by_ranks) SD_TRY(packed_ranks(ctx, dX, ld, 1, T, n, &Rp));
     // signature / flag storage borrows rank-pipeline buffers (after the rank pass, stream ordered)
     SD_TRY(ctx->buf[BUF_MASK].reserve((size_t)QB * W * m * sizeof(uint2)));
     SD_TRY(ctx->buf[BUF_PART_X].reserve((size_t)QB * m * sizeof(ulonglong2) + (size_t)QB * m + (size_t)nq + 64));
@@ -477,52 +504,20 @@ int bd_strict_match_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, 
         ctx->last.launches += 2;
         SD_CUDA(cudaGetLastError());
     }
-    // flagged queries -> enumerating kernels
-    std::vector<unsigned char> h_flag((size_t)nq);
-    SD_CUDA(cudaMemcpyAsync(h_flag.data(), flag, (size_t)nq, cudaMemcpyDeviceToHost, st));
-    SD_CUDA(cudaStreamSynchronize(st));
-    std::vector<i64> pos;
-    for (i64 i = 0; i < nq; ++i)
-        if (h_flag[(size_t)i]) pos.push_back(i);
-    if (n_fallback) *n_fallback = (i64)pos.size();
-    if (pos.empty()) return SD_OK;
-    const i64 nf = (i64)pos.size();
-    SD_TRY(ctx->buf[BUF_SPLIT].reserve((size_t)nf * 3 * sizeof(i64)));
-    i64 *d_pos = ctx->buf[BUF_SPLIT].as<i64>();
-    i64 *d_qsub = d_pos + nf, *d_osub = d_qsub + nf;
-    SD_CUDA(cudaMemcpyAsync(d_pos, pos.data(), (size_t)nf * sizeof(i64), cudaMemcpyHostToDevice, st));
-    bm_gather_kernel<<<(unsigned)ceil_div(nf, 256), 256, 0, st>>>(d_q, d_pos, nf, d_qsub);
-    ctx->last.launches++;
-    SD_CUDA(cudaStreamSynchronize(st));  // pos is a pageable host vector
-    SD_TRY(fallback(ctx, dX, T, n, ld, d_qsub, nf, d_osub));
-    bm_scatter_kernel<<<(unsigned)ceil_div(nf, 256), 256, 0, st>>>(d_osub, d_pos, nf, d_out);
-    ctx->last.launches++;
-    SD_CUDA(cudaGetLastError());
-    return SD_OK;
+    return recompute_flagged(ctx, dX, 1, T, n, ld, d_q, nq, flag, d_out, fallback, n_fallback);
 }
 
 // Strict J = 2 numerators of nb equally shaped matrices (dXg = [nb][T][n], nqb queries each: d_ql[nb][nqb] are
 // positions inside their matrix).  One rank pass, one pack, and one signature + one match launch per chunk of
 // matrices instead of ~9 launches and two host synchronisations per matrix (permutation tests).
 int bd_strict_match_batched_device(sd_ctx *ctx, const double *dXg, i64 nb, i64 T, i64 n, const i64 *d_ql, i64 nqb,
-                                   i64 *d_out,
-                                   int (*fallback)(sd_ctx *, const double *, i64, i64, i64, const i64 *, i64, i64 *)) {
+                                   i64 *d_out, StrictFallback fallback) {
     cudaStream_t st = ctx->stream;
     if (nb == 0 || nqb == 0) return SD_OK;
     const i64 m = n - 1;
     const i64 W = ceil_div(T, 32), TP = W * 16;
-    SD_TRY(ctx->buf[BUF_RANKS].reserve((size_t)nb * T * n * sizeof(int) + (size_t)nb * TP * n * sizeof(u32)));
-    int *rank_b = ctx->buf[BUF_RANKS].as<int>();
-    u32 *Rp = reinterpret_cast<u32 *>(rank_b + (size_t)nb * T * n);
-    SD_TRY(rank_rows_device(ctx, dXg, nb * T, n, n, rank_b, nullptr));
-    SD_TRY(prof_begin(ctx, SD_PHASE_BD_MASKS));
-    for (i64 b0 = 0; b0 < nb; b0 += 65535) {  // gridDim.y = batch: at most 65 535 per launch
-        const i64 cb = nb - b0 < 65535 ? nb - b0 : 65535;
-        bd_pack_ranks_kernel<<<dim3((unsigned)ceil_div(TP * n, 256), (unsigned)cb), 256, 0, st>>>(
-            rank_b + b0 * T * n, T, n, TP, Rp + b0 * TP * n);
-        ctx->last.launches++;
-    }
-    SD_TRY(prof_end(ctx));
+    u32 *Rp = nullptr;
+    SD_TRY(packed_ranks(ctx, dXg, n, nb, T, n, &Rp));
     const size_t per_b = (size_t)nqb * ((size_t)W * m * sizeof(uint2) + (size_t)m * (sizeof(ulonglong2) + 1));
     i64 CB = (i64)((3ull << 29) / (per_b > 0 ? per_b : 1));  // matrices per launch pair: ~1.5 GB of sign words
     if (CB < 1) CB = 1;
@@ -547,30 +542,7 @@ int bd_strict_match_batched_device(sd_ctx *ctx, const double *dXg, i64 nb, i64 T
         ctx->last.launches += 2;
         SD_CUDA(cudaGetLastError());
     }
-    // flagged queries -> enumerating kernels, matrix by matrix
-    std::vector<unsigned char> h_flag((size_t)(nb * nqb));
-    SD_CUDA(cudaMemcpyAsync(h_flag.data(), flag, h_flag.size(), cudaMemcpyDeviceToHost, st));
-    SD_CUDA(cudaStreamSynchronize(st));
-    std::vector<i64> pos;
-    for (i64 b = 0; b < nb; ++b) {
-        pos.clear();
-        for (i64 i = 0; i < nqb; ++i)
-            if (h_flag[(size_t)(b * nqb + i)]) pos.push_back(i);
-        if (pos.empty()) continue;
-        const i64 nf = (i64)pos.size();
-        SD_TRY(ctx->buf[BUF_SPLIT].reserve((size_t)nf * 3 * sizeof(i64)));
-        i64 *d_pos = ctx->buf[BUF_SPLIT].as<i64>();
-        i64 *d_qsub = d_pos + nf, *d_osub = d_qsub + nf;
-        SD_CUDA(cudaMemcpyAsync(d_pos, pos.data(), (size_t)nf * sizeof(i64), cudaMemcpyHostToDevice, st));
-        bm_gather_kernel<<<(unsigned)ceil_div(nf, 256), 256, 0, st>>>(d_ql + b * nqb, d_pos, nf, d_qsub);
-        ctx->last.launches++;
-        SD_CUDA(cudaStreamSynchronize(st));  // pos is a pageable host vector
-        SD_TRY(fallback(ctx, dXg + b * T * n, T, n, n, d_qsub, nf, d_osub));
-        bm_scatter_kernel<<<(unsigned)ceil_div(nf, 256), 256, 0, st>>>(d_osub, d_pos, nf, d_out + b * nqb);
-        ctx->last.launches++;
-        SD_CUDA(cudaGetLastError());
-    }
-    return SD_OK;
+    return recompute_flagged(ctx, dXg, nb, T, n, n, d_ql, nqb, flag, d_out, fallback, nullptr);
 }
 
 }  // namespace sd

@@ -163,18 +163,22 @@ int rank_block_workspace(sd_ctx *ctx, i64 T, i64 ints_per_row, i64 *RB, int **ws
 using RankBlockFn = std::function<void(i64 r0, i64 rows, const int *rb, const int *ra)>;
 int for_each_rank_block(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, bool want_a, i64 max_rows,
                         const RankBlockFn &consume);
+// K2, strict band depth (bd_bits.cu, bd_gemm.cu, bd_match.cu; strict_enumerate in api.cu): d_q must not be null.
+// The strict branch of band_depth_device writes the ids 0 .. nq - 1 into BUF_QIDX when the caller gives no query
+// list, so no strict driver may reserve BUF_QIDX (growing it would free that list).
 int bd_strict_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq, int j,
                      i64 *d_out, u64 *d_hits = nullptr);
 int bd_strict_gemm_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq,
                           i64 *d_out);
 int probe_int8_peak(sd_ctx *ctx, double *ops_per_s);
 bool bd_match_supported(i64 T, i64 n);
+// the enumerating strict J = 2 path (strict_enumerate) that recomputes the queries the matcher cannot certify
+using StrictFallback = int (*)(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq,
+                               i64 *d_out);
 int bd_strict_match_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, i64 ld, const i64 *d_q, i64 nq, i64 *d_out,
-                           int (*fallback)(sd_ctx *, const double *, i64, i64, i64, const i64 *, i64, i64 *),
-                           i64 *n_fallback);
+                           StrictFallback fallback, i64 *n_fallback);
 int bd_strict_match_batched_device(sd_ctx *ctx, const double *dXg, i64 nb, i64 T, i64 n, const i64 *d_ql, i64 nqb,
-                                   i64 *d_out,
-                                   int (*fallback)(sd_ctx *, const double *, i64, i64, i64, const i64 *, i64, i64 *));
+                                   i64 *d_out, StrictFallback fallback);
 int transpose_device(sd_ctx *ctx, const double *d_in, i64 rows, i64 cols, i64 ld_in, double *d_out);
 int gather_i64_device(sd_ctx *ctx, const i64 *d_src, const i64 *d_idx, i64 nq, i64 *d_out);
 int compact_columns_device(sd_ctx *ctx, const double *dX, i64 T, i64 n, const i64 *d_cols, i64 m, double *d_out);

@@ -427,6 +427,28 @@ def test_strict_auto_policy(engine, oracle):
     assert (engine.band_depth_counts(smooth, None, 2, False)[q] == oracle.bd_counts(smooth, q)).all()
 
 
+def test_strict_null_queries(engine):
+    """queries=None means the ids 0 .. n-1, written once on the device before the strict route is chosen: on every
+    route the counts and the route equal those of an explicit np.arange(n), at exactly one launch more.  n = 8200 is
+    above the matcher's limit, so SD_BD_AUTO reaches the probe of the enumerating path, which offsets that list."""
+    from statdepth_b200 import _engine as E
+    walk = walks(31, 96, 1300)
+    cases = [(walk, E.BD_BITS, (E.BD_BITS,)), (walk, E.BD_GEMM, (E.BD_GEMM,)), (walk, E.BD_MATCH, (E.BD_MATCH,)),
+             (walks(37, 8, 8200), E.BD_AUTO, (E.BD_BITS, E.BD_GEMM))]
+    for X, impl, used in cases:
+        try:
+            engine.set_option(E.OPT_BD_IMPL, impl)
+            got = engine.band_depth_counts(X, None, 2, False)
+            t_null = engine.timings()
+            exp = engine.band_depth_counts(X, np.arange(X.shape[1]), 2, False)
+            t_list = engine.timings()
+        finally:
+            engine.set_option(E.OPT_BD_IMPL, E.BD_AUTO)
+        assert (got == exp).all()
+        assert t_null["bd_impl_used"] == t_list["bd_impl_used"] and t_list["bd_impl_used"] in used
+        assert t_null["launches"] == t_list["launches"] + 1
+
+
 def test_strict_match_edge_shapes(engine, oracle):
     """Sign-vector matcher on ragged shapes: T not a multiple of 32, n = 3 .. 8193, a few tied curves (set Z)."""
     from statdepth_b200 import _engine as E
