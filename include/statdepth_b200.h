@@ -371,6 +371,42 @@ int sd_band_outlyingness_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64
                                  double *d_med_out, double *d_mad_out);
 
 /*
+ * Fitted references for random projection depths: the depth of NEW observations against a reference sample S, with
+ * the out-of-sample convention above (new observation g gets what the in-sample entry point returns for g after g
+ * alone is appended to S, with the same directions).  The reference's projections are sorted once; each query reads
+ * only the new observations and binary-searches them in the sorted rows.
+ *
+ * Index: d_sorted_out[(t*K + k)*nS + j] = the j-th smallest of the projections y_k(i, t) of the nS curves dF [nS, T, d]
+ * (as sd_projection_*: a point cloud is T = 1, U host memory checked there), ties repeated.  Device pointers;
+ * d_sorted_out holds T*K*nS doubles (2.05 GB at nS = 5 000, T = 256, K = 200).  SD_ERR_NONFINITE when F holds NaN or
+ * +-inf or a projection overflows; SD_ERR_UNSUPPORTED for nS >= 2^31.
+ */
+int sd_projection_sort_rows_f64_dev(sd_ctx *ctx, const double *dF, int64_t nS, int64_t T, int d, const double *U,
+                                    int64_t K, double *d_sorted_out);
+
+/* New curves dF_new [nY, T, d] against that index, the same U [K, d].  With b / a the reference projections of row
+ * (t, k) strictly below / above the new projection y:
+ *   tukey:        d_count_out[g] = sum_t min_k (nS + 1 - max(b, a))  == sd_projection_tukey_f64 of S + [g], entry nS
+ *   outlyingness: d_o_out[t*nY + g] = max_k |y - med'| / MAD', med' / MAD' of the row with y appended
+ *                 == sd_projection_outlyingness_f64 of S + [g], column nS, bit for bit.
+ * Device pointers.  SD_ERR_NONFINITE when F_new holds NaN or +-inf or a projection of it overflows;
+ * SD_ERR_UNSUPPORTED for nS + 1 >= 2^31. */
+int sd_projection_tukey_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t nS, int64_t T,
+                                       const double *dF_new, int64_t nY, int d, const double *U, int64_t K,
+                                       int64_t *d_count_out);
+int sd_projection_outlyingness_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t nS, int64_t T,
+                                              const double *dF_new, int64_t nY, int d, const double *U, int64_t K,
+                                              double *d_o_out);
+
+/* Univariate curves dY [T, nY] (dY[t*ldY + g]) against sorted rows from sd_band_sort_rows_f64_dev (the single
+ * direction u = 1): d_count_out[g] == sd_band_halfspace_f64 of [S | g], entry nS; d_o_out [T, nY] ==
+ * sd_band_outlyingness_f64 of [S | g], column nS.  Errors as above. */
+int sd_band_halfspace_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t T, int64_t nS, const double *dY,
+                                     int64_t nY, int64_t ldY, int64_t *d_count_out);
+int sd_band_outlyingness_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t T, int64_t nS,
+                                        const double *dY, int64_t nY, int64_t ldY, double *d_o_out);
+
+/*
  * Batched band depth over sub-populations of one matrix (K-sampled blocks, homogeneity
  * permutations): membership[b*n + c] != 0 selects the curves of batch b; queries[b*nqb + i] is
  * the i-th query curve of batch b (must be a member).  count_out[b*nqb + i] as in

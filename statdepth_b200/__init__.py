@@ -7,6 +7,7 @@
     from statdepth_b200 import HalfspaceDepth, FunctionalHalfspaceDepth  # halfspace (Tukey) depth, d = 1 or 2
     from statdepth_b200 import ProjectionDepth, FunctionalProjectionDepth  # random projection depths, any d
     from statdepth_b200 import FunctionalReference, DepthClassifier  # a reference fitted once; max-depth classes
+    from statdepth_b200 import FunctionalProjectionDepthOf, ProjectionDepthOf  # projection depths of new data
     from statdepth_b200.homogeneity import FunctionalHomogeneity     # == statdepth.homogeneity
     from statdepth_b200.testing import generate_noisy_univariate     # == statdepth.testing
 
@@ -19,11 +20,12 @@ from ._dist import enable_distributed
 from ._engine import Engine, EngineError, EngineUnavailable, get_engine
 from ._helper import DepthDegeneracy
 from .depth import (DepthClassifier, ExtremalDepth, FunctionalBoxplot, FunctionalDepth, FunctionalDepthOf,
-                    FunctionalHalfspaceDepth, FunctionalProjectionDepth, FunctionalReference, HalfspaceDepth,
-                    Outliergram, PointcloudDepth, PointcloudDepthOf, ProjectionDepth)
+                    FunctionalHalfspaceDepth, FunctionalProjectionDepth, FunctionalProjectionDepthOf,
+                    FunctionalReference, HalfspaceDepth, Outliergram, PointcloudDepth, PointcloudDepthOf,
+                    ProjectionDepth, ProjectionDepthOf)
 from .settings import get_simplex_tolerance, set_simplex_tolerance
 
 __version__ = "0.1.0"
 __all__ = ["FunctionalDepth", "PointcloudDepth", "FunctionalDepthOf", "PointcloudDepthOf", "FunctionalBoxplot",
-           "Outliergram", "ExtremalDepth", "HalfspaceDepth", "FunctionalHalfspaceDepth", "ProjectionDepth", "FunctionalProjectionDepth", "FunctionalReference", "DepthClassifier", "DepthDegeneracy", "Engine", "EngineError", "EngineUnavailable",
+           "Outliergram", "ExtremalDepth", "HalfspaceDepth", "FunctionalHalfspaceDepth", "ProjectionDepth", "FunctionalProjectionDepth", "FunctionalReference", "DepthClassifier", "FunctionalProjectionDepthOf", "ProjectionDepthOf", "DepthDegeneracy", "Engine", "EngineError", "EngineUnavailable",
            "get_engine", "get_simplex_tolerance", "set_simplex_tolerance", "enable_distributed"]

@@ -119,6 +119,16 @@ SIGNATURES = {
                                                      C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "sd_band_outlyingness_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                                C.c_void_p, C.c_void_p]),
+    "sd_projection_sort_rows_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p,
+                                                  C.c_int64, C.c_void_p]),
+    "sd_projection_tukey_sorted_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
+                                                     C.c_int64, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),
+    "sd_projection_outlyingness_sorted_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
+                                                            C.c_int64, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),
+    "sd_band_halfspace_sorted_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
+                                                   C.c_int64, C.c_int64, C.c_void_p]),
+    "sd_band_outlyingness_sorted_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
+                                                      C.c_int64, C.c_int64, C.c_void_p]),
     "sd_band_depth_batched_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                             C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -485,6 +495,42 @@ class Engine:
         row j - 2 equal to band_depth_oos_counts_dev(relax=True) for j."""
         self._check(self.lib.sd_band_depth_sorted_f64_dev(self._ctx, _dptr(d_sorted_ptr), int(T), int(nS),
                                                           _dptr(dY_ptr), int(nY), int(ldY), int(J), _dptr(d_out_ptr)))
+
+    # -- fitted references for random projection depths ----------------------------------------------------------
+    def projection_sort_rows_dev(self, dF_ptr, nS, T, d, U, d_sorted_ptr):
+        """The index of a projected reference: float64 [T, K, nS], the projections of the curves F [nS, T, d] (on the
+        device) along U [K, d] (host memory) sorted ascending per (t, k), on the device."""
+        U = np.ascontiguousarray(U, dtype=np.float64)
+        self._check(self.lib.sd_projection_sort_rows_f64_dev(self._ctx, _dptr(dF_ptr), int(nS), int(T), int(d), _ptr(U),
+                                                             U.shape[0], _dptr(d_sorted_ptr)))
+
+    def projection_tukey_sorted_counts_dev(self, d_sorted_ptr, nS, T, dF_ptr, nY, d, U, d_out_ptr):
+        """Random Tukey numerators int64 [nY] of the new curves F [nY, T, d] against a projected index, each equal to
+        projection_tukey_counts of the reference with that curve appended (its entry nS)."""
+        U = np.ascontiguousarray(U, dtype=np.float64)
+        self._check(self.lib.sd_projection_tukey_sorted_f64_dev(self._ctx, _dptr(d_sorted_ptr), int(nS), int(T),
+                                                                _dptr(dF_ptr), int(nY), int(d), _ptr(U), U.shape[0],
+                                                                _dptr(d_out_ptr)))
+
+    def projection_outlyingness_sorted_dev(self, d_sorted_ptr, nS, T, dF_ptr, nY, d, U, d_o_ptr):
+        """O [T, nY] of the new curves F [nY, T, d] against a projected index, each column equal to
+        projection_outlyingness of the reference with that curve appended (its column nS)."""
+        U = np.ascontiguousarray(U, dtype=np.float64)
+        self._check(self.lib.sd_projection_outlyingness_sorted_f64_dev(self._ctx, _dptr(d_sorted_ptr), int(nS),
+                                                                       int(T), _dptr(dF_ptr), int(nY), int(d),
+                                                                       _ptr(U), U.shape[0], _dptr(d_o_ptr)))
+
+    def band_halfspace_sorted_counts_dev(self, d_sorted_ptr, T, nS, dY_ptr, nY, ldY, d_out_ptr):
+        """Integrated halfspace numerators int64 [nY] of the univariate new curves Y [T, nY] against sorted rows
+        (band_sort_rows_dev), each equal to band_halfspace_counts of [S | g] (its entry nS)."""
+        self._check(self.lib.sd_band_halfspace_sorted_f64_dev(self._ctx, _dptr(d_sorted_ptr), int(T), int(nS),
+                                                              _dptr(dY_ptr), int(nY), int(ldY), _dptr(d_out_ptr)))
+
+    def band_outlyingness_sorted_dev(self, d_sorted_ptr, T, nS, dY_ptr, nY, ldY, d_o_ptr):
+        """O [T, nY] of the univariate new curves Y [T, nY] against sorted rows, each column equal to
+        band_outlyingness of [S | g] (its column nS)."""
+        self._check(self.lib.sd_band_outlyingness_sorted_f64_dev(self._ctx, _dptr(d_sorted_ptr), int(T), int(nS),
+                                                                 _dptr(dY_ptr), int(nY), int(ldY), _dptr(d_o_ptr)))
 
     def simplicial_oos_counts(self, S, Y, tol=1e-7):
         S = np.ascontiguousarray(S, dtype=np.float64)

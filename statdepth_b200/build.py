@@ -31,6 +31,7 @@ SOURCES = {
     "bd_match.cu": [],
     "oos.cu": [],
     "reference.cu": [],
+    "reference_proj.cu": ["-fmad=false"],
     "extremal.cu": [],
     "halfspace.cu": [],
     "projection.cu": ["-fmad=false"],

@@ -1015,4 +1015,68 @@ int sd_band_outlyingness_f64_dev(sd_ctx *ctx, const double *dX, int64_t T, int64
                                   "sd_band_outlyingness_f64_dev");
 }
 
+// ---------------------------------------------------------------------------------------------
+// fitted references for random projection depths (K13, reference_proj.cu)
+// ---------------------------------------------------------------------------------------------
+int sd_projection_sort_rows_f64_dev(sd_ctx *ctx, const double *dF, int64_t nS, int64_t T, int d, const double *U,
+                                    int64_t K, double *d_sorted_out) {
+    const char *who = "sd_projection_sort_rows_f64_dev";
+    SD_REQUIRE(nS >= 1 && T >= 1 && d >= 1 && K >= 1, "%s: bad sizes nS=%lld T=%lld d=%d K=%lld", who,
+               (long long)nS, (long long)T, d, (long long)K);
+    if (nS >= (1ll << 31)) {  // the rank pipeline's limit, refused before anything is uploaded
+        set_error("%s: nS=%lld exceeds 2^31-1", who, (long long)nS);
+        return SD_ERR_UNSUPPORTED;
+    }
+    const double *dU = nullptr;
+    return call(ctx, who, dF, d_sorted_out, false,
+                [&](Staging &) { return upload_directions(ctx, U, K, d, &dU, who); },
+                [&] { return projection_sort_rows_device(ctx, dF, nS, T, d, dU, K, d_sorted_out); });
+}
+
+// new observations against a sorted index: U == NULL takes the univariate rows dY [T, nY] (ldY) against K9's index
+static int sorted_query_call(sd_ctx *ctx, const double *d_sorted, i64 nS, i64 T, const double *dY, i64 nY, i64 ldY,
+                             int d, const double *U, i64 K, ProjKind kind, void *out, const char *who) {
+    SD_REQUIRE(dY || nY == 0, "%s: NULL new data", who);
+    SD_REQUIRE(nS >= 1 && T >= 1 && nY >= 0 && d >= 1 && K >= 1 && ldY >= nY,
+               "%s: bad sizes nS=%lld T=%lld nY=%lld d=%d K=%lld ldY=%lld", who, (long long)nS, (long long)T,
+               (long long)nY, d, (long long)K, (long long)ldY);
+    if (nS + 1 >= (1ll << 31)) {
+        set_error("%s: nS + 1 = %lld exceeds 2^31-1", who, (long long)(nS + 1));
+        return SD_ERR_UNSUPPORTED;
+    }
+    const double *dU = nullptr;
+    return call(ctx, who, d_sorted, out, false,
+                [&](Staging &) { return U ? upload_directions(ctx, U, K, d, &dU, who) : SD_OK; },
+                [&] {
+                    return projection_sorted_device(ctx, d_sorted, nS, T, dY, nY, ldY, d, dU, K, kind, (i64 *)out,
+                                                    (double *)out);
+                });
+}
+
+int sd_projection_tukey_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t nS, int64_t T,
+                                       const double *dF_new, int64_t nY, int d, const double *U, int64_t K,
+                                       int64_t *d_count_out) {
+    return sorted_query_call(ctx, d_sorted, nS, T, dF_new, nY, nY, d, U, K, PJ_TUKEY, d_count_out,
+                             "sd_projection_tukey_sorted_f64_dev");
+}
+
+int sd_projection_outlyingness_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t nS, int64_t T,
+                                              const double *dF_new, int64_t nY, int d, const double *U, int64_t K,
+                                              double *d_o_out) {
+    return sorted_query_call(ctx, d_sorted, nS, T, dF_new, nY, nY, d, U, K, PJ_OUTLYING, d_o_out,
+                             "sd_projection_outlyingness_sorted_f64_dev");
+}
+
+int sd_band_halfspace_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t T, int64_t nS, const double *dY,
+                                     int64_t nY, int64_t ldY, int64_t *d_count_out) {
+    return sorted_query_call(ctx, d_sorted, nS, T, dY, nY, ldY, 1, nullptr, 1, PJ_TUKEY, d_count_out,
+                             "sd_band_halfspace_sorted_f64_dev");
+}
+
+int sd_band_outlyingness_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t T, int64_t nS,
+                                        const double *dY, int64_t nY, int64_t ldY, double *d_o_out) {
+    return sorted_query_call(ctx, d_sorted, nS, T, dY, nY, ldY, 1, nullptr, 1, PJ_OUTLYING, d_o_out,
+                             "sd_band_outlyingness_sorted_f64_dev");
+}
+
 }  // extern "C"

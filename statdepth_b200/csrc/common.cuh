@@ -205,6 +205,23 @@ enum ProjKind { PJ_TUKEY, PJ_OUTLYING };
 int projection_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, i64 ldX, const double *dU, i64 K,
                       ProjKind kind, i64 *d_count, double *d_o, double *med_out, double *mad_out,
                       cudaMemcpyKind out_kind);
+// projection.cu's row blocks, shared by the fitted projected references (reference_proj.cu): rows of N projections
+// (leading dimension N rounded up to even) that fit PJ_BUDGET; kb_max directions by tb_max time points per block (a
+// time block keeps all K directions when K rows fit); project_device writes the block (t0 .. t0 + tb, kb directions
+// from dU) as Y[(tt * kb + kk) * ldY + i].
+i64 projection_rows_max(i64 N);
+void projection_blocks(i64 rows_max, i64 T, i64 K, i64 *kb_max, i64 *tb_max);
+int project_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, const double *dU, i64 kb, i64 t0, i64 tb,
+                   double *Y, i64 ldY);
+// fitted projected references (reference_proj.cu, K13): d_sorted[(t * K + k) * nS + j] = the j-th smallest of the
+// projections y_k(., t) of the nS reference curves F [nS, T, d]
+int projection_sort_rows_device(sd_ctx *ctx, const double *dF, i64 nS, i64 T, int d, const double *dU, i64 K,
+                                double *d_sorted);
+// new observations against such an index: dU == nullptr takes the rows of Y [T, nY] (leading dimension ldY) against
+// K9's sorted rows (K = 1, y = x); else dY holds new curves [nY, T, d].  PJ_TUKEY: d_count [nY] = sum_t min_k
+// (nS + 1 - max(b, a)); PJ_OUTLYING: d_o [T][nY] = max_k |y - med'| / MAD' of the row with y appended.
+int projection_sorted_device(sd_ctx *ctx, const double *d_sorted, i64 nS, i64 T, const double *dY, i64 nY, i64 ldY,
+                             int d, const double *dU, i64 K, ProjKind kind, i64 *d_count, double *d_o);
 // out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out);

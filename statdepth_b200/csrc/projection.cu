@@ -21,10 +21,11 @@
 //   RT: rank_rows_device passes (as halfspace1_device), then rt_min_kernel: one thread per (i, up to 32 time
 //                       points) reads the block's kb rows of each t coalesced along i and keeps a running int32 min;
 //                       after the last direction block it adds sum_t with one int64 atomic.
-//   PD: sort_rows_device (K9) into sorted rows, medmad_kernel (one thread per row: median, then the MAD as the k-th
-//                       smallest of L = |s[m-1..0] - med| and R = |s[m..] - med|, m = #values < med; both are
-//                       non-decreasing because rounding is monotone, so a binary search over how many come from L
-//                       finds it in O(log N)), then pd_max_kernel: a running max per (t, i) over the block's rows,
+//   PD: sort_rows_device (K9) into sorted rows, medmad_kernel (one thread per row: row_median / row_mad of
+//                       sorted_row.cuh, the median, then the MAD as the k-th smallest of L = |s[m-1..0] - med| and
+//                       R = |s[m..] - med|, m = #values < med; both are non-decreasing because rounding is monotone,
+//                       so a binary search over how many come from L finds it in O(log N)), then pd_max_kernel: a
+//                       running max per (t, i) over the block's rows,
 //                       compared as u64 bit patterns (non-negative doubles and +inf order like them).
 // Direction blocks continue the running min / max (BUF_PRED), since K N 8 bytes need not fit the workspace (and a
 // projection launch takes at most PJ_MAX_KB directions); a time block keeps all K directions whenever K rows fit.
@@ -35,9 +36,7 @@
 // finite check in the rank passes (SD_ERR_NONFINITE).  A rank outside 0 <= b, a, b + a <= N - 1 sets ST_INTERNAL
 // (never a trap).  Univariate outlyingness (dU == nullptr) skips the projection: the rows of X [T, N] are the
 // single direction's rows (u = 1, y = x).
-#include <math.h>
-
-#include "common.cuh"
+#include "sorted_row.cuh"
 
 namespace sd {
 
@@ -145,50 +144,16 @@ __global__ void __launch_bounds__(RD_THREADS) rt_min_kernel(const int *__restric
     if (last && s) atomicAdd((u64 *)&count[i], (u64)s);
 }
 
-// k-th smallest (0-based) of L ∪ R, L[j] = |s[m-1-j] - med| (j < m), R[j] = |s[m+j] - med| (j < n - m): i = how
-// many of the k + 1 smallest come from L, the least i with R[k - i] <= L[i]
-__device__ __forceinline__ double kth_deviation(const double *__restrict__ s, const i64 n, const i64 m,
-                                                const double med, const i64 k) {
-    const i64 nL = m, nR = n - m;
-    i64 lo = k + 1 - nR > 0 ? k + 1 - nR : 0;
-    i64 hi = k + 1 < nL ? k + 1 : nL;
-    while (lo < hi) {
-        const i64 i = (lo + hi) >> 1, j = k + 1 - i;
-        if (j > 0 && i < nL && fabs(__dsub_rn(s[m + j - 1], med)) > fabs(__dsub_rn(s[m - 1 - i], med))) lo = i + 1;
-        else hi = i;
-    }
-    const i64 j = k + 1 - lo;
-    double v = 0.0;
-    if (lo > 0) v = fabs(__dsub_rn(s[m - lo], med));
-    if (j > 0) {
-        const double r = fabs(__dsub_rn(s[m + j - 1], med));
-        if (lo == 0 || r > v) v = r;
-    }
-    return v;
-}
-
 // one thread per sorted row: med[r], mad[r] as np.median and np.median(np.abs(y - med))
 __global__ void __launch_bounds__(MM_THREADS) medmad_kernel(const double *__restrict__ sorted, const i64 R,
                                                             const i64 n, double *__restrict__ med,
                                                             double *__restrict__ mad) {
     const i64 r = (i64)blockIdx.x * MM_THREADS + threadIdx.x;
     if (r >= R) return;
-    const double *s = sorted + r * n;
-    const i64 h = n >> 1;
-    const double md = (n & 1) ? s[h] : __ddiv_rn(__dadd_rn(s[h - 1], s[h]), 2.0);
-    i64 m = 0;  // #values < md: lower bound
-    for (i64 len = n; len > 0;) {
-        const i64 half = len >> 1;
-        if (s[m + half] < md) {
-            m += half + 1;
-            len -= half + 1;
-        } else {
-            len = half;
-        }
-    }
+    const PlainRow s{sorted + r * n};
+    const double md = row_median(s, n), v = row_mad(s, n, md);
     med[r] = md;
-    mad[r] = (n & 1) ? kth_deviation(s, n, m, md, h)
-                     : __ddiv_rn(__dadd_rn(kth_deviation(s, n, m, md, h - 1), kth_deviation(s, n, m, md, h)), 2.0);
+    mad[r] = v;
 }
 
 // grid (point tiles, time tiles of tpt time points).  Y rows r = tt * kb + kk (leading dimension ldY), med / mad
@@ -209,12 +174,37 @@ __global__ void __launch_bounds__(RD_THREADS) pd_max_kernel(const double *__rest
         for (i64 kk = 0; kk < kb; ++kk) {
             const i64 r = t * kb + kk;
             const double y = Y[r * ldY + i], md = med[r], s = mad[r];
-            const double o = s == 0.0 ? (y == md ? 0.0 : (double)INFINITY) : __ddiv_rn(fabs(__dsub_rn(y, md)), s);
-            const u64 ob = (u64)__double_as_longlong(o);
+            const u64 ob = (u64)__double_as_longlong(outlyingness(y, md, s));
             m = ob > m ? ob : m;
         }
         (out ? out : run)[t * N + i] = __longlong_as_double((long long)m);
     }
+}
+
+i64 projection_rows_max(i64 N) {
+    const i64 rows = (i64)(PJ_BUDGET / ((size_t)(N + (N & 1)) * sizeof(double)));
+    return rows < 1 ? 1 : rows;
+}
+
+void projection_blocks(i64 rows_max, i64 T, i64 K, i64 *kb_max, i64 *tb_max) {
+    // a time block keeps all K directions when K rows fit
+    i64 kb = K <= rows_max ? K : rows_max;
+    if (kb > PJ_MAX_KB) kb = PJ_MAX_KB;
+    i64 tb = kb == K ? rows_max / K : 1;
+    if (tb > T) tb = T;
+    if (tb > PJ_MAX_TB) tb = PJ_MAX_TB;
+    *kb_max = kb;
+    *tb_max = tb;
+}
+
+int project_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, const double *dU, i64 kb, i64 t0, i64 tb,
+                   double *Y, i64 ldY) {
+    const int TT = d <= PJ_W ? PJ_W / d : 1;
+    const dim3 pgrid((unsigned)ceil_div(N, PJ_PTS), (unsigned)ceil_div(kb, PJ_DIRS), (unsigned)ceil_div(tb, TT));
+    projection_kernel<<<pgrid, PJ_THREADS, 0, ctx->stream>>>(dF, N, T, d, dU, kb, t0, tb, TT, Y, ldY);
+    ctx->last.launches++;
+    SD_CUDA(cudaGetLastError());
+    return SD_OK;
 }
 
 int projection_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, i64 ldX, const double *dU, i64 K,
@@ -234,20 +224,15 @@ int projection_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, i64 ld
     if (dU) SD_TRY(finite_check_device(ctx, dF, 1, N * T * d, N * T * d));
     else SD_TRY(finite_check_device(ctx, dF, T, N, ldX));
     const i64 ldY = dU ? N + (N & 1) : ldX;
-    i64 rows_max = (i64)(PJ_BUDGET / ((size_t)(N + (N & 1)) * sizeof(double)));
-    if (rows_max < 1) rows_max = 1;
+    i64 rows_max = projection_rows_max(N);
     int *rb = nullptr, *ra = nullptr;
     if (rt) {
         i64 RB = 0;
         SD_TRY(rank_block_workspace(ctx, rows_max < T * K ? rows_max : T * K, 2 * N, &RB, &rb));
         if (rows_max > RB) rows_max = RB;
     }
-    // a time block keeps all K directions when K rows fit
-    i64 kb_max = K <= rows_max ? K : rows_max;
-    if (kb_max > PJ_MAX_KB) kb_max = PJ_MAX_KB;
-    i64 tb_max = kb_max == K ? rows_max / K : 1;
-    if (tb_max > T) tb_max = T;
-    if (tb_max > PJ_MAX_TB) tb_max = PJ_MAX_TB;
+    i64 kb_max, tb_max;
+    projection_blocks(rows_max, T, K, &kb_max, &tb_max);
     const i64 R = tb_max * kb_max;
     if (rt) ra = rb + (size_t)R * N;
     double *Y = nullptr;
@@ -266,7 +251,6 @@ int projection_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, i64 ld
     double *pred = ctx->buf[BUF_PRED].as<double>();
     double *d_med = pred + (split ? (size_t)tb_max * N : 0), *d_mad = d_med + R;
     if (rt) SD_CUDA(cudaMemsetAsync(d_count, 0, (size_t)N * sizeof(i64), st));
-    const int TT = d <= PJ_W ? PJ_W / d : 1;
     for (i64 t0 = 0; t0 < T; t0 += tb_max) {
         const i64 tb = T - t0 < tb_max ? T - t0 : tb_max;
         // time points per reduction thread: up to RD_MAX_ROWS while N tb / tpt threads still fill ~2 occupancies
@@ -279,11 +263,7 @@ int projection_device(sd_ctx *ctx, const double *dF, i64 N, i64 T, int d, i64 ld
             const i64 rows = tb * kb;
             const double *Yb = dF + t0 * ldX;
             if (dU) {
-                const dim3 pgrid((unsigned)ceil_div(N, PJ_PTS), (unsigned)ceil_div(kb, PJ_DIRS),
-                                 (unsigned)ceil_div(tb, TT));
-                projection_kernel<<<pgrid, PJ_THREADS, 0, st>>>(dF, N, T, d, dU + k0 * d, kb, t0, tb, TT, Y, ldY);
-                ctx->last.launches++;
-                SD_CUDA(cudaGetLastError());
+                SD_TRY(project_device(ctx, dF, N, T, d, dU + k0 * d, kb, t0, tb, Y, ldY));
                 Yb = Y;
             }
             const int first = k0 == 0, last = k0 + kb == K;

@@ -18,13 +18,14 @@
 //
 // Query (depth_sorted_device): count[(j-2)*nY + g] = sum_t [C(nS,j) - C(b_t,j) - C(a_t,j)], j = 2..J, equal to
 // band_depth_oos_device(relax = 1, j).  sorted_terms_kernel: one thread per (new curve g, block of R rows), Y read
-// coalesced along g; per row a lower and an upper bound search of y in the same loop (their step sizes depend on nS
-// only, so the two chains of dependent loads interleave and no warp diverges).  Every index read stays in [0, nS)
+// coalesced along g; per row sorted_bounds (sorted_row.cuh): a lower and an upper bound search of y in the same loop
+// (their step sizes depend on nS only, so the two chains of dependent loads interleave and no warp diverges).  Every
+// index read stays in [0, nS)
 // and every result in [0, nS] whatever the buffer holds; 0 <= b, a and b + a <= nS is checked all the same (a
 // failure sets ST_INTERNAL, the kernel never traps).  One int64 atomic per (g, row block, j).
 // R is 32 rows when there are enough new curves to fill the GPU; fewer new curves get fewer rows per thread, down to
 // one, so that n_Y * T / R threads still reach ~ 2 full occupancies (each row costs ~2 log2(nS) dependent loads).
-#include "common.cuh"
+#include "sorted_row.cuh"
 
 namespace sd {
 
@@ -161,17 +162,8 @@ __global__ void __launch_bounds__(Q_THREADS) sorted_terms_kernel(const double *_
     i64 s2 = 0, s3 = 0;
     bool bad = false;
     for (i64 t = r0; t < r1; ++t) {
-        const double y = Y[t * ldY + g];
-        const double *row = sorted + t * nS;
-        const double *lo = row, *hi = row;  // lower bound (first >= y), upper bound (first > y)
-        for (i64 len = nS; len > 1;) {
-            const i64 half = len >> 1;
-            lo = lo[half] < y ? lo + half : lo;
-            hi = hi[half] <= y ? hi + half : hi;
-            len -= half;
-        }
-        const i64 b = (lo - row) + (*lo < y);
-        const i64 a = nS - ((hi - row) + (*hi <= y));
+        i64 b, a;
+        sorted_bounds(sorted + t * nS, nS, Y[t * ldY + g], b, a);
         if (b < 0 || a < 0 || b + a > nS) {
             bad = true;
             continue;

@@ -17,13 +17,13 @@ from ._halfspace import _functional_halfspace, _pointcloud_halfspace
 from ._outliers import (NO_FACTOR, _check_central, _check_extremal_rows, _checked_values, _extremal_depth,
                         _functional_boxplot, _outliergram)
 from ._pointcloud import _pointwisedepth, _pointwisedepth_of, _samplepointwisedepth
-from ._projection import _functional_projection, _pointcloud_projection
-from ._reference import _checked_reference, _query_values, _SortedReference
+from ._projection import KINDS, _functional_projection, _pointcloud_projection, draw_directions
+from ._reference import _checked_reference, _curve_values, _ProjectedReference, _query_values, _SortedReference
 
 __all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'ExtremalDepth',
            'HalfspaceDepth', 'FunctionalHalfspaceDepth', 'ProjectionDepth', 'FunctionalProjectionDepth',
-           'FunctionalBoxplot', 'Outliergram', 'FunctionalReference',
-           'DepthClassifier', 'AbstractDepth']
+           'FunctionalBoxplot', 'Outliergram', 'FunctionalReference', 'DepthClassifier',
+           'FunctionalProjectionDepthOf', 'ProjectionDepthOf', 'AbstractDepth']
 
 
 def _go():
@@ -467,30 +467,77 @@ def Outliergram(data: List[pd.DataFrame], factor=1.5, deep_check=False) -> _Outl
 # ---------------------------------------------------------------------------------------------------------------
 # fitted references and depth-based classification (driver in _reference.py)
 # ---------------------------------------------------------------------------------------------------------------
+def _check_reference_depth(depth, J, directions):
+    if not (isinstance(depth, str) and depth in ('mbd',) + KINDS):
+        raise ValueError("depth must be 'mbd', 'projection' or 'tukey' (got %r)" % (depth,))
+    if depth == 'mbd' and directions is not None:
+        raise ValueError("directions apply to depth='projection' or 'tukey'")
+    if depth != 'mbd' and J != 2:
+        raise ValueError('J applies to depth=\'mbd\' only: leave it at 2 for depth=%r' % depth)
+
+
 class FunctionalReference:
-    """A reference sample (sample[0], a T x n_S DataFrame) fitted once for relaxed out-of-sample band depth.
+    """A reference sample fitted once; depth_of() scores new curves against it.
 
-    Construction sorts every time row of the sample on the GPU and keeps only that index; each depth_of() call then
-    uploads only the new curves and binary-searches them in the sorted rows.  depth_of([df]) equals
-    FunctionalDepthOf([df], sample, J=J, relax=True) bit for bit.  Only relaxed (modified) band depth, J = 2 or 3, on
-    univariate data is offered: a strict band must hold a curve at all T points jointly, which sorted rows cannot
-    decide.  Non-finite values are rejected.  close() (or leaving a `with` block) frees the index."""
+    depth='mbd' (relaxed band depth, J = 2 or 3, univariate sample[0], a T x n_S DataFrame): construction sorts every
+    time row of the sample on the GPU and keeps only that index; each depth_of() call then uploads only the new curves
+    and binary-searches them in the sorted rows.  depth_of([df]) equals FunctionalDepthOf([df], sample, J=J,
+    relax=True) bit for bit.  A strict band must hold a curve at all T points jointly, which sorted rows cannot decide.
 
-    def __init__(self, sample: List[pd.DataFrame], J=2, deep_check=False):
-        _checked_reference(sample, J, deep_check)
+    depth='projection' or 'tukey' (J must stay 2): sample is [df] (univariate, directions must be None) or N
+    DataFrames of T x d.  Construction draws the directions once (as FunctionalProjectionDepth: None gives 1000, an
+    int K gives K random unit directions from seed, an array [K, d] is used as given; kept as .directions, None for
+    univariate data) and sorts the sample's projections per (time point, direction) on the GPU: an index of T K n_S
+    doubles (2.05 GB at n_S = 5 000, T = 256, K = 200) kept for as long as the reference.  A new curve g gets the depth
+    FunctionalProjectionDepth(sample + [g], kind=depth, directions=.directions) gives it, bit for bit; the other new
+    curves never take part.
+
+    Non-finite values (and, for the projection kinds, projections that overflow) are rejected.  close() (or leaving a
+    `with` block) frees the index."""
+
+    def __init__(self, sample: List[pd.DataFrame], J=2, deep_check=False, depth='mbd', directions=None, seed=0):
+        _check_reference_depth(depth, J, directions)
         self.J = J
+        self.depth = depth
+        self.directions = None
+        if depth == 'mbd':
+            _checked_reference(sample, J, deep_check)
+            self._T = sample[0].shape[0]
+            self._index = sample[0].index
+            self._ref = _SortedReference(_values(sample[0]), J)
+            return
+        X, F = _curve_values(sample, directions)
+        if X is not None and X.shape[1] == 0:
+            raise ValueError('No data passed.')
         self._T = sample[0].shape[0]
         self._index = sample[0].index
-        self._ref = _SortedReference(_values(sample[0]), J)
+        self._d = None if F is None else F.shape[2]
+        if F is not None:
+            self.directions = draw_directions(self._d, directions, seed)
+        self._ref = _ProjectedReference(depth, X=X, F=F, U=self.directions)
 
-    def depth_of(self, data: List[pd.DataFrame], deep_check=False) -> _FunctionalDepthUnivariate:
-        """Depth of every curve (column) of data[0] against the reference, indexed by data[0].columns (a label may
-        repeat a sample label)."""
+    def depth_of(self, data: List[pd.DataFrame], deep_check=False) -> _FunctionalDepthSeries:
+        """Depth of every new curve against the reference.  Univariate: the columns of data[0], indexed by
+        data[0].columns (a label may repeat a sample label).  Multivariate (projection kinds): M DataFrames of T x d,
+        indexed by list position, as FunctionalProjectionDepth."""
         if self._ref is None:
             raise ValueError('the reference is closed')
-        Y = _query_values(data, self.J, deep_check, self._T, self._index)
-        depth = pd.Series(index=data[0].columns, data=self._ref.depths(Y))
-        return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+        if self.depth == 'mbd':
+            Y = _query_values(data, self.J, deep_check, self._T, self._index)
+            depth = pd.Series(index=data[0].columns, data=self._ref.depths(Y))
+            return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+        X, F = _curve_values(data, frames=self._d is not None)
+        if data[0].shape[0] != self._T:
+            raise ValueError('data and sample must have the same number of time points.')
+        if F is not None and F.shape[2] != self._d:
+            raise ValueError('data and sample must have the same number of channels.')
+        if deep_check and not all(len(df.index) == len(self._index) and all(df.index == self._index) for df in data):
+            raise ValueError('DataFrames indices must be the same')
+        if F is None:
+            return _FunctionalDepthUnivariate(df=data[0], depths=pd.Series(index=data[0].columns,
+                                                                           data=self._ref.depths(X)))
+        return _FunctionalDepthSeries(df=data[0], depths=pd.Series(index=list(range(len(data))),
+                                                                   data=self._ref.depths(F)))
 
     def close(self) -> None:
         if self._ref is not None:
@@ -508,37 +555,54 @@ class FunctionalReference:
 class DepthClassifier:
     """Maximum-depth classifier (Lopez-Pintado & Romo 2006): a curve belongs to the class in which it is deepest.
 
-    references maps each class label to its training curves ([DataFrame], T x n_k, the same T for every class); each
-    class is fitted once as a FunctionalReference.  depths([df]) are the DD-plot coordinates (one column per class,
-    equal to FunctionalDepthOf([df], references[label], J=J, relax=True)); predict([df]) takes the class of largest
-    depth, ties going to the class listed first."""
+    references maps each class label to its training curves, each class fitted once as a FunctionalReference with
+    the given depth.  depth='mbd': [DataFrame] T x n_k, the same T for every class; depths([df]) (one column per class)
+    equal FunctionalDepthOf([df], references[label], J=J, relax=True).  depth='projection' or 'tukey': [df] for every
+    class, or lists of T x d DataFrames with the same T and d for every class; one set of directions, drawn once from
+    d and seed (or given), is shared by all classes (.directions), so that the DD-plot coordinates are comparable.
+    predict(data) takes the class of largest depth, ties going to the class listed first."""
 
-    def __init__(self, references: dict, J=2, deep_check=False):
+    def __init__(self, references: dict, J=2, deep_check=False, depth='mbd', directions=None, seed=0):
         if not isinstance(references, dict) or len(references) < 2:
             raise ValueError('references must be a dict of at least two classes.')
+        _check_reference_depth(depth, J, directions)
         for sample in references.values():
-            _checked_reference(sample, J, deep_check)
+            if depth == 'mbd':
+                _checked_reference(sample, J, deep_check)
+            else:
+                _curve_values(sample, directions)
         if len({sample[0].shape[0] for sample in references.values()}) > 1:
             raise ValueError('every class must have the same number of time points.')
+        self.directions = None
+        if depth != 'mbd':
+            if len({len(sample) == 1 for sample in references.values()}) > 1:
+                raise ValueError('every class must be univariate, or every class multivariate.')
+            dims = {sample[0].shape[1] for sample in references.values() if len(sample) > 1}
+            if len(dims) > 1:
+                raise ValueError('every class must have the same number of channels.')
+            if dims:
+                self.directions = draw_directions(dims.pop(), directions, seed)
         self.labels = list(references)
         self._refs = []
         try:
             for label in self.labels:
-                self._refs.append(FunctionalReference(references[label], J=J, deep_check=deep_check))
+                self._refs.append(FunctionalReference(references[label], J=J, deep_check=deep_check, depth=depth,
+                                                      directions=self.directions))
         except BaseException:
             self.close()
             raise
 
     def depths(self, data: List[pd.DataFrame], deep_check=False) -> pd.DataFrame:
-        """Depth of every curve of data[0] in every class: rows data[0].columns, one column per class label."""
+        """Depth of every new curve in every class: one column per class label, rows indexed as
+        FunctionalReference.depth_of indexes them (data[0].columns, or list positions for multivariate curves)."""
         if not self._refs:
             raise ValueError('the classifier is closed')
-        cols = [ref.depth_of(data, deep_check=deep_check).values for ref in self._refs]
-        return pd.DataFrame(np.column_stack(cols), index=data[0].columns,
+        res = [ref.depth_of(data, deep_check=deep_check) for ref in self._refs]
+        return pd.DataFrame(np.column_stack([r.values for r in res]), index=res[0].index,
                             columns=pd.Index(self.labels, tupleize_cols=False))
 
     def predict(self, data: List[pd.DataFrame], deep_check=False) -> pd.Series:
-        """Label of the class of largest depth for every curve of data[0] (ties: the class listed first)."""
+        """Label of the class of largest depth for every new curve (ties: the class listed first)."""
         d = self.depths(data, deep_check=deep_check)
         best = np.argmax(d.to_numpy(), axis=1)  # the first maximum
         return pd.Series([self.labels[k] for k in best], index=d.index, dtype=object)
@@ -554,3 +618,38 @@ class DepthClassifier:
     def __exit__(self, *exc):
         self.close()
         return False
+
+
+def FunctionalProjectionDepthOf(data: List[pd.DataFrame], sample: List[pd.DataFrame], kind='projection',
+                                directions=None, seed=0) -> _FunctionalDepthSeries:
+    """Out-of-sample integrated projection depth (kind='projection') or random Tukey depth ('tukey') of new curves
+    against the reference curves sample: each new curve gets what FunctionalProjectionDepth(sample + [g], kind,
+    directions, seed) gives it, bit for bit; the other new curves never take part.  Univariate [df] (T x n, indexed by
+    data[0].columns; directions must be None) or lists of T x d DataFrames (indexed by list position).  One call of
+    FunctionalReference(sample, depth=kind, ...).depth_of(data): to score many batches, keep the reference."""
+    with FunctionalReference(sample, depth=kind, directions=directions, seed=seed) as ref:
+        return ref.depth_of(data)
+
+
+def ProjectionDepthOf(data: pd.DataFrame, sample: pd.DataFrame, kind='projection', directions=None,
+                      seed=0) -> _PointwiseDepth:
+    """Out-of-sample projection depth (kind='projection') or random Tukey depth ('tukey') of the rows of data (m x d)
+    against the reference cloud sample (n x d): each row gets what ProjectionDepth(pd.concat([sample, row]), kind,
+    directions, seed) gives it, bit for bit.  The sample's projections are sorted once on the GPU (K n doubles) and
+    every row is binary-searched in them.  Indexed by data.index.  Non-finite values are rejected."""
+    for name, df in (('data', data), ('sample', sample)):
+        if not isinstance(df, pd.DataFrame):
+            raise ValueError('%s must be a DataFrame (points x d columns).' % name)
+    if sample.shape[0] == 0 or sample.shape[1] == 0:
+        raise ValueError('No data passed.')
+    if data.shape[1] != sample.shape[1]:
+        raise ValueError('data and sample must have the same number of columns.')
+    if kind not in KINDS:
+        raise ValueError("kind must be one of %s (got %r)" % (KINDS, kind))
+    U = draw_directions(sample.shape[1], directions, seed)
+    ref = _ProjectedReference(kind, F=np.ascontiguousarray(_values(sample))[:, None, :], U=U, cloud=True)
+    try:
+        depth = ref.depths(np.ascontiguousarray(_values(data))[:, None, :])
+    finally:
+        ref.close()
+    return _PointwiseDepth(df=data, depths=pd.Series(index=data.index, data=depth))
