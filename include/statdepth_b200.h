@@ -175,13 +175,17 @@ int sd_band_ranks_f64(sd_ctx *ctx, const double *X, int64_t T, int64_t n, int64_
  * of the closed simplex test (the reference's LP accepts ~1e-7; pass 0 for exact sign tests).
  *   relax == 0 : #{(d+1)-subsets of the other N-1 curves containing the query at all T rows}
  *   relax != 0 : sum over subsets of #rows contained
+ * SD_ERR_OVERFLOW when relax != 0, d = 2, the counts are counted (enum sd_simplicial_impl) and T * C(N-1, 3)
+ * exceeds int64 (T = 1: N > 3 810 780; T = 64: N > 952 696).
  */
 int sd_simplex_depth_f64(sd_ctx *ctx, const double *F, int64_t N, int64_t T, int d,
                          const int64_t *query_idx, int64_t nq, int relax, double tol,
                          int64_t *count_out);
 
 /* Point cloud P[i*d + c], n points.  Replaces the 'simplex' branch of _pointwisedepth
- * (_pointcloud.py:44-56): #{(d+1)-subsets of the other points whose closed simplex contains p}. */
+ * (_pointcloud.py:44-56): #{(d+1)-subsets of the other points whose closed simplex contains p}.
+ * SD_ERR_OVERFLOW when d = 2, the counts are counted (enum sd_simplicial_impl) and C(n-1, 3) exceeds int64
+ * (n > 3 810 780). */
 int sd_pointcloud_simplicial_f64(sd_ctx *ctx, const double *P, int64_t n, int d,
                                  const int64_t *query_idx, int64_t nq, double tol,
                                  int64_t *count_out);
@@ -255,7 +259,8 @@ int sd_band_depth_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t T,
 /* Point clouds S[i*d + c] (nS points) and Y[g*d + c] (nY points), d in 1..3:
  * count_out[g] = #{(d+1)-subsets of S whose closed simplex contains Y[g]} with the tolerance band `tol` of
  * sd_pointcloud_simplicial_f64 (enumerated, or counted for d = 2 when nS + 1 > 64, as there).
- * The host divides by C(nS + 1, d + 1). */
+ * The host divides by C(nS + 1, d + 1).  SD_ERR_OVERFLOW when d = 2, the counts are counted and C(nS, 3) exceeds
+ * int64 (nS > 3 810 779). */
 int sd_pointcloud_simplicial_oos_f64(sd_ctx *ctx, const double *S, int64_t nS, int d,
                                      const double *Y, int64_t nY, double tol, int64_t *count_out);
 

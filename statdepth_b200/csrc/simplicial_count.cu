@@ -90,7 +90,18 @@ __global__ void __launch_bounds__(256) sc_keys_kernel(const ScGeom g, const i64 
     if (bad || !isfinite(px) || !isfinite(py)) atomicOr(status, ST_NONFINITE);
 }
 
-__device__ __forceinline__ i64 c3(i64 m) { return m < 3 ? 0 : (m * (m - 1) / 2) * (m - 2) / 3; }
+// C(m, 3), exact whenever it fits in int64: the even factor is halved and the multiple of 3 divided by 3 before the
+// product, so no partial product exceeds the result ((m (m - 1) / 2) (m - 2) would wrap from m = 2 642 247).
+__device__ __forceinline__ i64 c3(i64 m) {
+    if (m < 3) return 0;
+    i64 a = m, b = m - 1, c = m - 2;
+    if (a % 2 == 0) a /= 2;
+    else b /= 2;
+    if (a % 3 == 0) a /= 3;
+    else if (b % 3 == 0) b /= 3;
+    else c /= 3;
+    return a * b * c;
+}
 
 // pass 1 of the reductions, block-wide: the number of real directions m' and how many of them lie in [0, pi)
 // (key < 12); ARCS: `low` counts the arcs that wrap past 2 pi (end below start).  kb_hi = second half of row B.
@@ -247,6 +258,15 @@ int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride
     if (!(tol >= 0.0)) {
         set_error("simplicial counting: tolerance %g is negative or NaN", tol);
         return SD_ERR_INVALID;
+    }
+    // a triangle count is at most C(m_others, 3) per instance, and curves add T of them into one int64 (the halfspace
+    // numerators are at most T n).  Exact: m_others < 2^30 here, so C(m_others, 3) < 2^90.
+    if (!hs) {
+        const __int128 c = (__int128)m_others * (m_others - 1) * (m_others - 2) / 6;
+        if (c > (__int128)INT64_MAX / T) {
+            set_error("simplicial counting: T*C(%lld,3) overflows int64 for T=%lld", (long long)m_others, (long long)T);
+            return SD_ERR_OVERFLOW;
+        }
     }
     // batch size: ~52 n bytes of keys and ranks per instance (+ the rank pipeline's part lists)
     i64 IB = (i64)((3ull << 30) / (size_t)(56 * n));
