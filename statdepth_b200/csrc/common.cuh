@@ -110,7 +110,7 @@ struct sd_ctx {
     void *stage[2] = {nullptr, nullptr};                        // pinned staging of pageable host input (api.cu)
     size_t stage_cap[2] = {0, 0};
     cudaEvent_t ev_stage[2] = {nullptr, nullptr};
-    cudaEvent_t ev_slab[2] = {nullptr, nullptr};                // MBD slab path: unfit-row counts copied (mbd.cu)
+    cudaEvent_t ev_slab[2] = {nullptr, nullptr};                // MBD slab path: table / hist kernel done (mbd.cu)
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};  // h2d start | kernels start | kernels end | d2h end
     sd_timings last = {0, 0, 0, 0, 0, 0};
     int bd_impl = SD_BD_AUTO;
@@ -126,8 +126,10 @@ struct sd_ctx {
     int prof_n = 0;
     int64_t phase_ns[SD_PHASE_COUNT] = {};
     sd::DevBuf buf[sd::NUM_BUFS];
-    int *d_status = nullptr;  // device int[4]: [0] status bits, [1] MBD rows ranked by the generic path
+    int *d_status = nullptr;  // device int[8]: [0] status bits, [1] MBD rows ranked by the generic path; [6..7] mbd.cu
     int *h_status = nullptr;  // pinned mirror; [2] and [3] also receive the slab path's unfit-row counts mid-call (mbd.cu)
+    int *h_status_dev = nullptr;  // the mirror as kernels address it (mapped), for the counts the slab kernels store
+    int mbd_attributes_set = 0;   // the rank pipeline's kernel attributes are set on this context's device (mbd.cu)
 };
 
 namespace sd {

@@ -250,7 +250,9 @@ int sd_init(int device, sd_ctx **out) {
     for (int i = 0; i < 4; ++i) SD_CUDA(cudaEventCreateWithFlags(&ctx->ev_pipe[i], cudaEventDisableTiming));
     for (int i = 0; i < 4; ++i) SD_CUDA(cudaEventCreate(&ctx->ev[i]));
     SD_CUDA(cudaMalloc(&ctx->d_status, 8 * sizeof(int)));
-    SD_CUDA(cudaMallocHost(&ctx->h_status, 4 * sizeof(int)));
+    SD_CUDA(cudaMemset(ctx->d_status, 0, 8 * sizeof(int)));  // [6..7]: the slab path's counters, left at zero by every call
+    SD_CUDA(cudaHostAlloc(&ctx->h_status, 4 * sizeof(int), cudaHostAllocMapped));
+    SD_CUDA(cudaHostGetDevicePointer(&ctx->h_status_dev, ctx->h_status, 0));
     memset(ctx->h_status, 0, 4 * sizeof(int));
     *out = ctx;
     return SD_OK;

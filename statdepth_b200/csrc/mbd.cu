@@ -1394,6 +1394,25 @@ static SlabPlan slab_plan(const double *dX, const i64 n, const i64 ld) {
     return p;
 }
 
+// The dynamic shared memory the kernels of the rank pipeline may take, set once per context: the slab kernels may
+// take all an SM offers beside their static arrays (what a launch takes is its plan's size), so that no call of any
+// context on the device lowers a limit another one relies on.
+static int mbd_kernel_attributes(sd_ctx *ctx) {
+    if (ctx->mbd_attributes_set) return SD_OK;
+    int optin = 0;
+    SD_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+    SD_CUDA(cudaFuncSetAttribute(mbd_partition_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PT_SMEM));
+    const void *slab[4] = {(const void *)mbd_slab_hist_kernel<SL_HIST_THREADS>, (const void *)mbd_slab_hist_kernel<1024>,
+                           (const void *)mbd_slab_rank_kernel<false>, (const void *)mbd_slab_rank_kernel<true>};
+    for (const void *f : slab) {
+        cudaFuncAttributes fa;
+        SD_CUDA(cudaFuncGetAttributes(&fa, f));
+        SD_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes));
+    }
+    ctx->mbd_attributes_set = 1;
+    return SD_OK;
+}
+
 // The part pipeline's geometry and workspaces for one call (blocks of at most Tc rows)
 struct PartPlan {
     int P, S;
@@ -1408,41 +1427,38 @@ struct PartPlan {
 
 // The slab path on rows [r0, r0 + rows).  Once its rank kernel is queued, *only is the mask of the rows it skipped
 // (left to the part pipeline), and *done is set when the host has seen that it skipped none.
-static int slab_block(sd_ctx *ctx, const SlabPlan &sp, SlabArgs sa, const RankOut &o, const bool extra,
-                      const double *Xb, const i64 r0, const i64 rows, const int **only, bool *done) {
+static int slab_block(sd_ctx *ctx, const SlabPlan &sp, SlabArgs sa, const SlabReport &rep, const RankOut &o,
+                      const bool extra, const double *Xb, const i64 r0, const i64 rows, const int **only, bool *done) {
     cudaStream_t st = ctx->stream;
     sa.X = Xb;
     sa.row0 = r0;
-    SD_CUDA(cudaMemsetAsync(sa.failcount, 0, sizeof(int), st));
     for (int k = 0; k < 2; ++k)
         if (!ctx->ev_slab[k]) SD_CUDA(cudaEventCreateWithFlags(&ctx->ev_slab[k], cudaEventDisableTiming));
     SD_TRY(prof_begin(ctx, SD_PHASE_MBD_SLAB_HIST));
-    mbd_slab_table_kernel<<<(unsigned)rows, SL_TABLE_THREADS, 0, st>>>(sa);
+    mbd_slab_table_kernel<<<(unsigned)rows, SL_TABLE_THREADS, 0, st>>>(sa, rep);
     // Rows this path cannot take are counted twice: after the table kernel (ties, degenerate ranges) and after the
-    // hist kernel (a bin, a CTA's share or the pair work over its limit: wild tails, adversarial spreads).  Both
-    // counts come back while later kernels run or are already queued, so the host decides without leaving the GPU
-    // idle.  Many unfit rows after the first count (tie-heavy data) send the whole block to the part pipeline;
-    // otherwise the rank kernel skips the flagged rows and the part pipeline ranks just those.
+    // hist kernel (a bin, a CTA's share or the pair work over its limit: wild tails, adversarial spreads).  The last
+    // CTA of each kernel stores its count into the pinned status mirror (slab_report), so the host decides while later
+    // kernels run or are already queued, without leaving the GPU idle.  Many unfit rows after the first count
+    // (tie-heavy data) send the whole block to the part pipeline; otherwise the rank kernel skips the flagged rows and
+    // the part pipeline ranks just those.
     // A pipelined host call (row blocks copied on a second stream while earlier blocks are ranked) must not stall the
     // host: it skips the counts and always queues the masked part pipeline behind the rank kernel (its CTAs exit at
     // once when no row is flagged: ~50 us per block).  An SD_OPT_ASYNC_DEVICE call does wait: its waits end with the
     // first two kernels, while the rank kernel is still running.
     const bool ask = !ctx->mbd_no_wait;
-    if (ask) {
-        SD_CUDA(cudaMemcpyAsync(ctx->h_status + 3, sa.failcount, sizeof(int), cudaMemcpyDeviceToHost, st));
-        SD_CUDA(cudaEventRecord(ctx->ev_slab[0], st));
-    }
+    if (ask) SD_CUDA(cudaEventRecord(ctx->ev_slab[0], st));
     if (env_int("SD_MBD_SLAB_HIST_THREADS", rows <= (i64)ctx->sm_count ? 1024 : SL_HIST_THREADS) == 1024)
-        mbd_slab_hist_kernel<1024><<<(unsigned)rows, 1024, sp.smem_hist, st>>>(sa);
+        mbd_slab_hist_kernel<1024><<<(unsigned)rows, 1024, sp.smem_hist, st>>>(sa, rep);
     else
-        mbd_slab_hist_kernel<SL_HIST_THREADS><<<(unsigned)rows, SL_HIST_THREADS, sp.smem_hist, st>>>(sa);
+        mbd_slab_hist_kernel<SL_HIST_THREADS><<<(unsigned)rows, SL_HIST_THREADS, sp.smem_hist, st>>>(sa, rep);
     SD_TRY(prof_end(ctx));
     ctx->last.launches += 2;
+    const volatile int *counts = ctx->h_status + 2;  // [0] after the hist kernel, [1] after the table kernel
     if (ask) {
-        SD_CUDA(cudaMemcpyAsync(ctx->h_status + 2, sa.failcount, sizeof(int), cudaMemcpyDeviceToHost, st));
         SD_CUDA(cudaEventRecord(ctx->ev_slab[1], st));
         SD_CUDA(cudaEventSynchronize(ctx->ev_slab[0]));
-        if ((i64)ctx->h_status[3] * 16 > rows) return SD_OK;  // all unfit
+        if ((i64)counts[1] * 16 > rows) return SD_OK;  // all unfit
     }
     const dim3 sgrid((unsigned)sp.G, (unsigned)rows);
     SD_TRY(prof_begin(ctx, SD_PHASE_MBD_SLAB_RANK));
@@ -1453,7 +1469,7 @@ static int slab_block(sd_ctx *ctx, const SlabPlan &sp, SlabArgs sa, const RankOu
     *only = sa.rowflag;  // the flagged rows: part pipeline (the generic path costs ~2 ms per long row)
     if (ask) {
         SD_CUDA(cudaEventSynchronize(ctx->ev_slab[1]));  // the rank kernel is queued behind the hist kernel
-        *done = ctx->h_status[2] == 0;
+        *done = counts[0] == 0;
     }
     return SD_OK;
 }
@@ -1588,12 +1604,13 @@ static int rank_pipeline(sd_ctx *ctx, const double *dX, const i64 T, const i64 n
     SD_TRY(ctx->buf[BUF_WORK].reserve((size_t)Tc * P * sizeof(int2) + (size_t)acc_len * sizeof(u64)));
     int2 *biglist = ctx->buf[BUF_WORK].as<int2>();
     u64 *raw2 = reinterpret_cast<u64 *>(biglist + (size_t)Tc * P);
-    if (d_acc2) SD_CUDA(cudaMemsetAsync(raw2, 0, (size_t)acc_len * sizeof(u64), st));
-
-    SD_CUDA(cudaFuncSetAttribute(mbd_partition_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PT_SMEM));
+    SD_TRY(mbd_kernel_attributes(ctx));
 
     // slab path (mbd_slab.cuh): per-value codes, bin starts, per-CTA offsets, row flags
     const SlabPlan sp = ctx->mbd_force_fallback ? SlabPlan{} : slab_plan(dX, n, ld);
+    // raw2 starts at zero: cleared by the slab path's first table kernel, else by a memset
+    SlabReport rep = {ctx->h_status_dev + 2, sp.ok && d_acc2 ? raw2 : nullptr, sp.ok && d_acc2 ? acc_len : 0};
+    if (d_acc2 && !sp.ok) SD_CUDA(cudaMemsetAsync(raw2, 0, (size_t)acc_len * sizeof(u64), st));
     SlabArgs sa = {};
     if (sp.ok) {
         const size_t rows_cap = (size_t)Tc;
@@ -1619,14 +1636,6 @@ static int rank_pipeline(sd_ctx *ctx, const double *dX, const i64 T, const i64 n
         sa.starts = reinterpret_cast<unsigned short *>(base + off_starts);
         sa.failcount = ctx->d_status + 6;
         sa.status = ctx->d_status;
-        SD_CUDA(cudaFuncSetAttribute(mbd_slab_hist_kernel<SL_HIST_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)sp.smem_hist));
-        SD_CUDA(cudaFuncSetAttribute(mbd_slab_hist_kernel<1024>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)sp.smem_hist));
-        SD_CUDA(cudaFuncSetAttribute(mbd_slab_rank_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)sp.smem_rank));
-        SD_CUDA(cudaFuncSetAttribute(mbd_slab_rank_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)sp.smem_rank));
     }
 
     const PartPlan pp = {P, S, NP, row_stride, Tc, rank_subbin, part_x, splitters_f, tables, part_j, pbase, cursor,
@@ -1641,7 +1650,8 @@ static int rank_pipeline(sd_ctx *ctx, const double *dX, const i64 T, const i64 n
         const double *Xb = dX + r0 * ld;
         const int *only = nullptr;  // part pipeline restricted to the rows the slab path gave up
         bool done = false;
-        if (sp.ok) SD_TRY(slab_block(ctx, sp, sa, o, extra, Xb, r0, rows, &only, &done));
+        if (sp.ok) SD_TRY(slab_block(ctx, sp, sa, rep, o, extra, Xb, r0, rows, &only, &done));
+        rep.zero_len = 0;  // later row blocks accumulate
         if (!done && !ctx->mbd_force_fallback)
             SD_TRY(extra ? part_block<true>(ctx, pp, o, Xb, ld, r0, rows, only)
                          : part_block<false>(ctx, pp, o, Xb, ld, r0, rows, only));

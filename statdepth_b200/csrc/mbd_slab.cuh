@@ -63,9 +63,18 @@ struct SlabArgs {
     unsigned short *starts;    // [rows][G*NBc] first entry position of a bin inside its CTA
     u32 *below;                // [rows][G] #values in the bins of lower CTAs
     int *rowflag;              // [rows] 0, or 2: generic path
-    int *failcount;            // rows flagged by the hist kernel
+    int *failcount;            // [0] rows flagged by the table and hist kernels, [1] their CTAs' ticket (slab_report)
     i64 row0;
     int *status;
+};
+
+// What the table and hist kernels hand over beside the rows: the unfit-row counts, stored by the last CTA of each kernel
+// straight into the host's pinned status mirror (mapped: no copy in the stream between the kernels), and the j = 2
+// accumulator of the call, which the table kernel of its first row block clears.
+struct SlabReport {
+    int *host;                 // device view of the mirror: [0] unfit rows after the hist kernel, [1] after the table kernel
+    u64 *zero;                 // [zero_len] cleared by the table kernel, or null
+    i64 zero_len;
 };
 
 // d = fma(x, s, c) = 2^52 + (1 + (x - lo) * (SL_BUCKETS - 2) / (hi - lo)) * 2^32: the mantissa is a fixed-point
@@ -75,10 +84,30 @@ __device__ __forceinline__ int slab_bucket(const double d) {
     return min(max(__double2hiint(d), SL_TOP0), SL_TOP0 + SL_BUCKETS - 1) - SL_TOP0;
 }
 
+// The hist kernel keeps SL_TBL_COPIES copies of the code table, entry k of copy r at word 2 (k * SL_TBL_COPIES + r):
+// copy r lies on banks 2r and 2r + 1 whatever k is, so when lane l reads copy l % 16 the lanes of a half-warp hit 16
+// different bank pairs and a 64-bit lookup takes its 2 wavefronts for any buckets (one shared table: ~3x that, 71 %
+// of the LSU pipe).  tbl points at the lane's copy.
+constexpr int SL_TBL_COPIES = 16;
+
 __device__ __forceinline__ u32 slab_code(const double x, const double s, const double c, const uint2 *tbl) {
     const double d = fma(x, s, c);
-    const uint2 e = tbl[slab_bucket(d)];
+    const uint2 e = tbl[slab_bucket(d) * SL_TBL_COPIES];
     return e.x + __umulhi((u32)__double2loint(d), e.y);
+}
+
+// Thread 0 of every CTA of the table / hist kernel, once its row is decided: the CTA that draws the last ticket stores
+// the unfit-row count to the host's mirror; after the hist kernel (always queued behind the table kernel) it also
+// resets the count and the ticket, so that every call starts from zeros without a memset.
+__device__ __forceinline__ void slab_report(const SlabArgs &a, const SlabReport &r, const bool failed, const bool hist) {
+    if (failed) atomicAdd(a.failcount, 1);
+    __threadfence();
+    if (atomicAdd(a.failcount + 1, 1) != (int)gridDim.x - 1) return;
+    __threadfence();
+    const int count = hist ? atomicExch(a.failcount, 0) : atomicAdd(a.failcount, 0);
+    a.failcount[1] = 0;
+    *(volatile int *)(r.host + (hist ? 0 : 1)) = count;
+    __threadfence_system();
 }
 
 __device__ __forceinline__ bool slab_nonfinite(const double x) {
@@ -148,13 +177,14 @@ __device__ __forceinline__ u32 slab_block_scan(const u32 v, u32 *wsum, u32 &tota
 // table: sample -> range and code table.  One small CTA per row (the 55 barrier stages of the sample sort and the
 // scattered sample loads are latency, hidden by running many of these CTAs per SM).
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(SL_TABLE_THREADS, 4) mbd_slab_table_kernel(const SlabArgs a) {
+__global__ void __launch_bounds__(SL_TABLE_THREADS, 4) mbd_slab_table_kernel(const SlabArgs a, const SlabReport r) {
     __shared__ u32 bh[SL_BUCKETS];
     __shared__ u32 wsum[33];
     __shared__ int s_dups;
     __shared__ float s_q[2];
     const int tid = threadIdx.x;
     const i64 row = blockIdx.x;
+    for (i64 i = row * SL_TABLE_THREADS + tid; i < r.zero_len; i += (i64)gridDim.x * SL_TABLE_THREADS) r.zero[i] = 0ull;
     const int n = (int)a.n;
     const double *xr = a.X + row * a.ld;
     const int NB = a.G * a.NBc;
@@ -206,8 +236,8 @@ __global__ void __launch_bounds__(SL_TABLE_THREADS, 4) mbd_slab_table_kernel(con
     const bool fail = s_dups > SL_DUPS_MAX || !(span > 0.0) || !(s > 0.0) || slab_nonfinite(s) || slab_nonfinite(c);
     if (tid == 0) {
         a.rowflag[row] = fail ? 2 : 0;
-        if (fail) atomicAdd(a.failcount, 1);
-        else a.rowmap[row] = make_double2(s, c);
+        if (!fail) a.rowmap[row] = make_double2(s, c);
+        slab_report(a, r, fail, false);
     }
     if (fail) return;  // uniform
 
@@ -240,23 +270,29 @@ static_assert(SL_TABLE_THREADS == SL_BUCKETS && SL_SORTED == 1024 && SL_SORTED =
 // NT = 512 (two CTAs per SM) when there are rows enough to fill the machine twice over, 1024 (one per SM) for the short
 // blocks of a multi-GPU rank or a pipelined host call: a CTA's warps are what hides its DRAM latency.
 template <int NT>
-__global__ void __launch_bounds__(NT, NT == SL_HIST_THREADS ? SD_SLAB_HIST_MINB : 1) mbd_slab_hist_kernel(const SlabArgs a) {
+__global__ void __launch_bounds__(NT, NT == SL_HIST_THREADS ? SD_SLAB_HIST_MINB : 1)
+    mbd_slab_hist_kernel(const SlabArgs a, const SlabReport r) {
     extern __shared__ __align__(16) unsigned char sl_smem[];
     u32 *bins = reinterpret_cast<u32 *>(sl_smem);  // [NB]
-    __shared__ uint2 tbl[SL_BUCKETS];
+    __shared__ uint2 tbl[SL_BUCKETS * SL_TBL_COPIES];  // 32 KB: two CTAs of 512 threads still fit an SM
     __shared__ u32 wsum[33];
     __shared__ u32 s_pairwork;
-    const int tid = threadIdx.x, nt = NT;
+    __shared__ u32 s_first[32];  // [G] first entry of each rank CTA
+    const int tid = threadIdx.x, nt = NT, lane = tid & 31, wid = tid >> 5;
     const i64 row = blockIdx.x;
-    if (a.rowflag[row] & 2) return;  // the table kernel gave the row up
+    if (a.rowflag[row] & 2) {  // the table kernel gave the row up
+        if (tid == 0) slab_report(a, r, false, true);
+        return;
+    }
     const int n = (int)a.n;
     const double *xr = a.X + row * a.ld;
     const int NB = a.G * a.NBc;
-    for (int k = tid; k < SL_BUCKETS; k += nt) tbl[k] = a.tables[row * SL_BUCKETS + k];
+    for (int k = tid; k < SL_BUCKETS * SL_TBL_COPIES; k += nt) tbl[k] = a.tables[row * SL_BUCKETS + k / SL_TBL_COPIES];
     for (int b = tid; b < NB; b += nt) bins[b] = 0u;
     if (tid == 0) s_pairwork = 0u;
     const double2 sc = a.rowmap[row];
     const double s = sc.x, c = sc.y;
+    const uint2 *tbl_mine = tbl + (lane & (SL_TBL_COPIES - 1));
     __syncthreads();
 
     // 1. the pass
@@ -265,37 +301,45 @@ __global__ void __launch_bounds__(NT, NT == SL_HIST_THREADS ? SD_SLAB_HIST_MINB 
     uint2 *crow2 = reinterpret_cast<uint2 *>(crow);
     slab_stream(reinterpret_cast<const double2 *>(xr), n >> 1, tid, nt, [&](const double2 v, const int p) {
         bad |= slab_nonfinite(v.x) | slab_nonfinite(v.y);
-        const u32 c0 = slab_code(v.x, s, c, tbl), c1 = slab_code(v.y, s, c, tbl);
+        const u32 c0 = slab_code(v.x, s, c, tbl_mine), c1 = slab_code(v.y, s, c, tbl_mine);
         crow2[p] = make_uint2(c0, c1);
         atomicAdd(&bins[c0 >> SL_SHIFT], 1u);
         atomicAdd(&bins[c1 >> SL_SHIFT], 1u);
     });
     if ((n & 1) && tid == 0) {
         bad |= slab_nonfinite(xr[n - 1]);
-        const u32 c0 = slab_code(xr[n - 1], s, c, tbl);
+        const u32 c0 = slab_code(xr[n - 1], s, c, tbl_mine);
         crow[n - 1] = c0;
         atomicAdd(&bins[c0 >> SL_SHIFT], 1u);
     }
     if (bad) atomicOr(a.status, ST_NONFINITE);
     __syncthreads();
 
-    // 2. exclusive prefix over the bins (in place), validation, per-CTA starts
-    const int bpt = (NB + nt - 1) / nt;
-    const int b0 = tid * bpt, b1 = min(b0 + bpt, NB);
+    // 2. exclusive prefix over the bins (in place), validation, per-CTA starts.  Warp w owns the bins
+    //    [w * S, (w + 1) * S) (S a multiple of 32: NB is a multiple of 1024) and its lanes walk them 32 consecutive
+    //    bins at a time, so that every shared-memory access is conflict-free; a warp scan carries the running sum.
+    const int S = NB / (NT / 32);
+    u32 *wbins = bins + wid * S + lane;
     u32 sum = 0u, maxc = 0u, pairwork = 0u;
-    for (int b = b0; b < b1; ++b) {
-        const u32 cnt = bins[b];
+    for (int k = 0; k < S; k += 32) {
+        const u32 cnt = wbins[k];
         sum += cnt;
         maxc = max(maxc, cnt);
         if (cnt > (u32)SL_SORT_CAP) pairwork += min(cnt, 65535u) * min(cnt, 65535u);
     }
     if (pairwork) atomicAdd(&s_pairwork, min(pairwork, SL_PAIRWORK_MAX + 1u));
     u32 total;
-    u32 run = slab_block_scan(sum, wsum, total);
-    for (int b = b0; b < b1; ++b) {
-        const u32 cnt = bins[b];
-        bins[b] = run;
-        run += cnt;
+    u32 run = __shfl_sync(0xffffffffu, slab_block_scan(sum, wsum, total), 0);  // values in lower warps' bins
+    for (int k = 0; k < S; k += 32) {
+        const u32 cnt = wbins[k];
+        u32 incl = cnt;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const u32 up = __shfl_up_sync(0xffffffffu, incl, d);
+            if (lane >= d) incl += up;
+        }
+        wbins[k] = run + incl - cnt;
+        run += __shfl_sync(0xffffffffu, incl, 31);
     }
     __syncthreads();
     bool fail = maxc > (u32)SL_BIN_MAX || total != (u32)n;
@@ -304,34 +348,30 @@ __global__ void __launch_bounds__(NT, NT == SL_HIST_THREADS ? SD_SLAB_HIST_MINB 
         const u32 next = tid + 1 < a.G ? bins[(tid + 1) * a.NBc] : (u32)n;
         fail |= next - first > (u32)a.ecap;
         a.below[row * a.G + tid] = first;
+        s_first[tid] = first;
     }
     if (tid == 0) fail |= s_pairwork > SL_PAIRWORK_MAX;
     fail = __syncthreads_or(fail);
+    if (tid == 0) slab_report(a, r, fail, true);
     if (fail) {
-        if (tid == 0) {
-            a.rowflag[row] = 2;
-            atomicAdd(a.failcount, 1);
-        }
+        if (tid == 0) a.rowflag[row] = 2;
         return;
     }
-    // starts relative to the owning rank CTA's first bin, converted in place and copied out coalesced (two per word)
-    if (b0 < b1) {
-        int edge = (b0 / a.NBc) * a.NBc;  // first bin of the rank CTA that owns bin b
-        u32 first = bins[edge];
-        __syncwarp();
-        for (int b = b0; b < b1; ++b) {
-            if (b == edge + a.NBc) {
-                edge = b;
-                first = bins[b];
-            }
-            if (b != edge) bins[b] -= first;  // the edge bins are read by other threads: zeroed after the barrier
-        }
-    }
-    __syncthreads();
-    if (tid < a.G) bins[tid * a.NBc] = 0u;
-    __syncthreads();
+    // starts relative to the owning rank CTA's first bin, copied out coalesced (two per word; NBc is even, so both
+    // bins of a word belong to the same rank CTA)
+    const uint2 *bins2 = reinterpret_cast<const uint2 *>(bins);
     u32 *st2 = reinterpret_cast<u32 *>(a.starts + row * NB);  // NB is a multiple of 1024
-    for (int w = tid; w < (NB >> 1); w += nt) st2[w] = bins[2 * w] | (bins[2 * w + 1] << 16);
+    const int words_c = a.NBc >> 1;
+    int g = 0, edge = words_c;  // rank CTA of word w, first word of the next one
+    for (int w = tid; w < (NB >> 1); w += nt) {
+        while (w >= edge) {
+            ++g;
+            edge += words_c;
+        }
+        const uint2 v = bins2[w];
+        const u32 first = s_first[g];
+        st2[w] = (v.x - first) | ((v.y - first) << 16);
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
