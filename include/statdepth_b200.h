@@ -44,7 +44,7 @@ enum sd_status {
     SD_ERR_CUDA = 2,        /* a CUDA runtime call failed; text in sd_last_error() */
     SD_ERR_NO_DEVICE = 3,   /* no usable sm_100 device */
     SD_ERR_NONFINITE = 4,   /* NaN or +-inf in the input */
-    SD_ERR_OVERFLOW = 5,    /* integer numerator would exceed int64 for this (n, T, J) */
+    SD_ERR_OVERFLOW = 5,    /* integer numerator would exceed int64 for this (n, T, J); a squared distance overflows */
     SD_ERR_UNSUPPORTED = 6  /* configuration the engine does not implement (no CPU fallback) */
 };
 
@@ -410,6 +410,27 @@ int sd_band_halfspace_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_
                                      int64_t nY, int64_t ldY, int64_t *d_count_out);
 int sd_band_outlyingness_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int64_t T, int64_t nS,
                                         const double *dY, int64_t nY, int64_t ldY, double *d_o_out);
+
+/*
+ * Functional spatial depth (L2 spatial depth of curves, Chakraborty & Chaudhuri 2014).  A curve is the vector of its
+ * F = T*d values in (t, c) order; r_out[q] = || sum_{j : x_j != x_q} (x_j - x_q) / ||x_j - x_q|| || (Euclidean norms
+ * over all F values; duplicates of x_q, and pairs whose squared distance underflows to 0, contribute 0).  The depth is
+ * 1 - r / n_pop with n_pop = n in sample and nS + 1 out of sample; the host forms it.
+ * layout SD_LAYOUT_NT: X[i*F + f], curve i a row (frames [N, T, d]); SD_LAYOUT_TN: X[f*n + i], curve i a column (the
+ * values of a univariate T x n DataFrame), transposed on the device.  Each query's sums run in an order fixed by the
+ * indices and the tile sizes alone, so results never depend on the other queries; out of sample r_out[g] equals the
+ * in-sample r of S + [g] at entry nS bit for bit.
+ * SD_ERR_NONFINITE when an input holds NaN or +-inf, SD_ERR_OVERFLOW when a squared distance overflows (||x_j - x_q||
+ * of about 1.3e154 or more).
+ */
+int sd_spatial_norms_f64(sd_ctx *ctx, const double *X, int64_t n, int64_t F, int layout, const int64_t *query_idx,
+                         int64_t nq, double *r_out);
+/* new curves Y [nY] against the sample S [nS] (same layout, each dense: S[i*F + f] or S[f*nS + i]) */
+int sd_spatial_norms_of_f64(sd_ctx *ctx, const double *S, int64_t nS, const double *Y, int64_t nY, int64_t F,
+                            int layout, double *r_out);
+/* same with DEVICE pointers, curves as rows only (dS [nS, F], dY [nY, F]); d_r_out holds nY doubles */
+int sd_spatial_norms_of_f64_dev(sd_ctx *ctx, const double *dS, int64_t nS, const double *dY, int64_t nY, int64_t F,
+                                double *d_r_out);
 
 /*
  * Batched band depth over sub-populations of one matrix (K-sampled blocks, homogeneity

@@ -8,6 +8,7 @@
     from statdepth_b200 import ProjectionDepth, FunctionalProjectionDepth  # random projection depths, any d
     from statdepth_b200 import FunctionalReference, DepthClassifier  # a reference fitted once; max-depth classes
     from statdepth_b200 import FunctionalProjectionDepthOf, ProjectionDepthOf  # projection depths of new data
+    from statdepth_b200 import FunctionalSpatialDepth, FunctionalSpatialDepthOf  # L2 spatial depth of curves
     from statdepth_b200.homogeneity import FunctionalHomogeneity     # == statdepth.homogeneity
     from statdepth_b200.testing import generate_noisy_univariate     # == statdepth.testing
 
@@ -21,11 +22,11 @@ from ._engine import Engine, EngineError, EngineUnavailable, get_engine
 from ._helper import DepthDegeneracy
 from .depth import (DepthClassifier, ExtremalDepth, FunctionalBoxplot, FunctionalDepth, FunctionalDepthOf,
                     FunctionalHalfspaceDepth, FunctionalProjectionDepth, FunctionalProjectionDepthOf,
-                    FunctionalReference, HalfspaceDepth, Outliergram, PointcloudDepth, PointcloudDepthOf,
-                    ProjectionDepth, ProjectionDepthOf)
+                    FunctionalReference, FunctionalSpatialDepth, FunctionalSpatialDepthOf, HalfspaceDepth,
+                    Outliergram, PointcloudDepth, PointcloudDepthOf, ProjectionDepth, ProjectionDepthOf)
 from .settings import get_simplex_tolerance, set_simplex_tolerance
 
 __version__ = "0.1.0"
 __all__ = ["FunctionalDepth", "PointcloudDepth", "FunctionalDepthOf", "PointcloudDepthOf", "FunctionalBoxplot",
-           "Outliergram", "ExtremalDepth", "HalfspaceDepth", "FunctionalHalfspaceDepth", "ProjectionDepth", "FunctionalProjectionDepth", "FunctionalReference", "DepthClassifier", "FunctionalProjectionDepthOf", "ProjectionDepthOf", "DepthDegeneracy", "Engine", "EngineError", "EngineUnavailable",
+           "Outliergram", "ExtremalDepth", "HalfspaceDepth", "FunctionalHalfspaceDepth", "ProjectionDepth", "FunctionalProjectionDepth", "FunctionalReference", "DepthClassifier", "FunctionalProjectionDepthOf", "ProjectionDepthOf", "FunctionalSpatialDepth", "FunctionalSpatialDepthOf", "DepthDegeneracy", "Engine", "EngineError", "EngineUnavailable",
            "get_engine", "get_simplex_tolerance", "set_simplex_tolerance", "enable_distributed"]

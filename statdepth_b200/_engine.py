@@ -129,6 +129,12 @@ SIGNATURES = {
                                                    C.c_int64, C.c_int64, C.c_void_p]),
     "sd_band_outlyingness_sorted_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
                                                       C.c_int64, C.c_int64, C.c_void_p]),
+    "sd_spatial_norms_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p,
+                                       C.c_int64, C.c_void_p]),
+    "sd_spatial_norms_of_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64,
+                                          C.c_int, C.c_void_p]),
+    "sd_spatial_norms_of_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64,
+                                              C.c_void_p]),
     "sd_band_depth_batched_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                             C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -531,6 +537,49 @@ class Engine:
         band_outlyingness of [S | g] (its column nS)."""
         self._check(self.lib.sd_band_outlyingness_sorted_f64_dev(self._ctx, _dptr(d_sorted_ptr), int(T), int(nS),
                                                                  _dptr(dY_ptr), int(nY), int(ldY), _dptr(d_o_ptr)))
+
+    # -- functional spatial depth ----------------------------------------------------------------------
+    @staticmethod
+    def _curves(A):
+        """(A, layout) of curves as the rows of a 2-D float64 array [n, F]: a C-order A is SD_LAYOUT_NT; an F-order A
+        (the transpose of a univariate DataFrame's C-order values [T, n]) is passed as-is with SD_LAYOUT_TN."""
+        A = np.asarray(A)
+        if A.dtype != np.float64:
+            A = A.astype(np.float64)
+        if A.ndim != 2:
+            raise ValueError("expected curves as a 2-D array [n, F]")
+        if A.flags.f_contiguous and not A.flags.c_contiguous:
+            return A, LAYOUT_TN
+        return np.ascontiguousarray(A), LAYOUT_NT
+
+    def spatial_norms(self, X, queries=None):
+        """r [nq] = || sum_j u(x_j - x_q) || of the curves X [n, F] (rows; u(0) = 0) for the queries (all when None);
+        spatial depth is 1 - r / n."""
+        X, layout = self._curves(X)
+        n, F = X.shape
+        q, nq = self._queries(queries, n)
+        out = np.empty(nq, dtype=np.float64)
+        self._check(self.lib.sd_spatial_norms_f64(self._ctx, _ptr(X), n, F, layout, _ptr(q), nq, _ptr(out)))
+        return out
+
+    def spatial_norms_of(self, S, Y):
+        """r [nY] of the new curves Y [nY, F] against the sample S [nS, F] (rows); the depth is 1 - r / (nS + 1)."""
+        S, ls = self._curves(S)
+        Y = np.asarray(Y, dtype=np.float64)
+        Y = np.asfortranarray(Y) if ls == LAYOUT_TN else np.ascontiguousarray(Y)  # in S's layout
+        if Y.ndim != 2 or S.shape[1] != Y.shape[1]:
+            raise ValueError("S and Y must have the same number of values per curve")
+        out = np.empty(Y.shape[0], dtype=np.float64)
+        if Y.shape[0] == 0:
+            return out
+        self._check(self.lib.sd_spatial_norms_of_f64(self._ctx, _ptr(S), S.shape[0], _ptr(Y), Y.shape[0], S.shape[1],
+                                                     ls, _ptr(out)))
+        return out
+
+    def spatial_norms_of_dev(self, dS_ptr, nS, dY_ptr, nY, F, d_r_ptr):
+        """Device-pointer variant (curves as rows: S [nS, F], Y [nY, F]); r [nY] stays on the device."""
+        self._check(self.lib.sd_spatial_norms_of_f64_dev(self._ctx, _dptr(dS_ptr), int(nS), _dptr(dY_ptr), int(nY),
+                                                         int(F), _dptr(d_r_ptr)))
 
     def simplicial_oos_counts(self, S, Y, tol=1e-7):
         S = np.ascontiguousarray(S, dtype=np.float64)

@@ -38,6 +38,7 @@ SOURCES = {
     "outliers.cu": ["-fmad=false"],
     "pointcloud.cu": ["-fmad=false"],
     "simplicial_count.cu": ["-fmad=false"],
+    "spatial.cu": [],
 }
 EXPORT_MAP = os.path.join(CSRC, "exports.map")
 

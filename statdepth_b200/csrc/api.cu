@@ -390,6 +390,25 @@ static int upload_directions(sd_ctx *ctx, const double *U, i64 K, int d, const d
     return SD_OK;
 }
 
+// spatial depth (K14): [S; Y] as dense device rows [nS + nY, F] (Y may be empty).  SD_LAYOUT_TN memory (curves are
+// columns, [F, n]) is pooled as [F, nS + nY] and transposed once the kernel phase has begun.
+static int upload_curves(Staging &s, const double *S, i64 nS, const double *Y, i64 nY, i64 F, int layout,
+                         const double **dP) {
+    double *d = nullptr;
+    if (layout == SD_LAYOUT_NT) {
+        SD_TRY(upload_pooled(s.ctx, cudaMemcpyHostToDevice, S, nS * F, nS * F, Y, nY * F, nY * F, 1, &d));
+    } else {
+        SD_TRY(upload_pooled(s.ctx, cudaMemcpyHostToDevice, S, nS, nS, Y, nY, nY, F, &d));
+        s.nt = d;
+        s.nt_rows = F;
+        s.nt_cols = nS + nY;
+        SD_TRY(s.ctx->buf[BUF_IN2].reserve((size_t)(nS + nY) * F * sizeof(double)));
+        d = s.nt_out = s.ctx->buf[BUF_IN2].as<double>();
+    }
+    *dP = d;
+    return SD_OK;
+}
+
 }  // namespace sd
 
 using namespace sd;
@@ -1077,6 +1096,61 @@ int sd_band_outlyingness_sorted_f64_dev(sd_ctx *ctx, const double *d_sorted, int
                                         const double *dY, int64_t nY, int64_t ldY, double *d_o_out) {
     return sorted_query_call(ctx, d_sorted, nS, T, dY, nY, ldY, 1, nullptr, 1, PJ_OUTLYING, d_o_out,
                              "sd_band_outlyingness_sorted_f64_dev");
+}
+
+// ---------------------------------------------------------------------------------------------
+// functional spatial depth (K14, spatial.cu)
+// ---------------------------------------------------------------------------------------------
+int sd_spatial_norms_f64(sd_ctx *ctx, const double *X, int64_t n, int64_t F, int layout, const int64_t *query_idx,
+                         int64_t nq, double *r_out) {
+    const char *who = "sd_spatial_norms_f64";
+    SD_REQUIRE(n >= 1 && F >= 1 && nq >= 0, "%s: bad sizes n=%lld F=%lld nq=%lld", who, (long long)n, (long long)F,
+               (long long)nq);
+    SD_REQUIRE(layout == SD_LAYOUT_TN || layout == SD_LAYOUT_NT, "%s: bad layout %d", who, layout);
+    SD_REQUIRE(query_idx || nq == n, "%s: query_idx == NULL requires nq == n", who);
+    const double *dX = nullptr;
+    const i64 *d_q = nullptr;
+    double *d_r = nullptr;
+    return call(ctx, who, X, r_out, true, [&](Staging &s) -> int {
+        SD_TRY(upload_curves(s, X, n, nullptr, 0, F, layout, &dX));
+        SD_TRY(upload_queries(ctx, query_idx, nq, n, &d_q, who));
+        return s.output(BUF_OUT, r_out, nq, &d_r);
+    }, [&]() -> int {
+        SD_TRY(finite_check_device(ctx, dX, 1, n * F, n * F));
+        return spatial_device(ctx, dX, d_q, nq, dX, n, F, d_r);
+    });
+}
+
+static int spatial_of_call(sd_ctx *ctx, const double *S, i64 nS, const double *Y, i64 nY, i64 F, int layout,
+                           double *r, bool dev, const char *who) {
+    SD_REQUIRE(Y || nY == 0, "%s: NULL Y", who);
+    SD_REQUIRE(nS >= 1 && nY >= 0 && F >= 1, "%s: bad sizes nS=%lld nY=%lld F=%lld", who, (long long)nS,
+               (long long)nY, (long long)F);
+    SD_REQUIRE(layout == SD_LAYOUT_TN || layout == SD_LAYOUT_NT, "%s: bad layout %d", who, layout);
+    const double *dS = S, *dY = Y;
+    double *d_r = r;
+    return call(ctx, who, S, r, !dev, [&](Staging &s) -> int {
+        if (dev) return SD_OK;
+        const double *dP = nullptr;
+        SD_TRY(upload_curves(s, S, nS, Y, nY, F, layout, &dP));
+        dS = dP;
+        dY = dP + nS * F;
+        return s.output(BUF_OUT, r, nY, &d_r);
+    }, [&]() -> int {
+        SD_TRY(finite_check_device(ctx, dS, 1, nS * F, nS * F));
+        SD_TRY(finite_check_device(ctx, dY, 1, nY * F, nY * F));
+        return spatial_device(ctx, dY, nullptr, nY, dS, nS, F, d_r);
+    });
+}
+
+int sd_spatial_norms_of_f64(sd_ctx *ctx, const double *S, int64_t nS, const double *Y, int64_t nY, int64_t F,
+                            int layout, double *r_out) {
+    return spatial_of_call(ctx, S, nS, Y, nY, F, layout, r_out, false, "sd_spatial_norms_of_f64");
+}
+
+int sd_spatial_norms_of_f64_dev(sd_ctx *ctx, const double *dS, int64_t nS, const double *dY, int64_t nY, int64_t F,
+                                double *d_r_out) {
+    return spatial_of_call(ctx, dS, nS, dY, nY, F, SD_LAYOUT_NT, d_r_out, true, "sd_spatial_norms_of_f64_dev");
 }
 
 }  // extern "C"

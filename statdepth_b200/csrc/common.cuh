@@ -72,11 +72,12 @@ enum BufId {
     BUF_PROJ,       // projection depths: projected rows Y
     BUF_PSORT,      // projection depth: sorted rows of Y
     BUF_PRED,       // projection depths: running min / max across direction blocks, per-row med / MAD
+    BUF_SPATIAL,    // spatial depth: one row block of weights W [rows][nS] and the per-feature-block partial norms
     NUM_BUFS
 };
 
 // status bits written by kernels into ctx->d_status
-enum { ST_NONFINITE = 1, ST_INTERNAL = 2, ST_NO_MEMBER = 4, ST_BAD_INPUT = 8 };  // ST_BAD_INPUT: caller data out of range
+enum { ST_NONFINITE = 1, ST_INTERNAL = 2, ST_NO_MEMBER = 4, ST_BAD_INPUT = 8, ST_OVERFLOW = 16 };  // ST_BAD_INPUT: caller data out of range
 
 __host__ __device__ static inline i64 ceil_div(i64 a, i64 b) { return (a + b - 1) / b; }
 
@@ -224,6 +225,11 @@ int projection_sort_rows_device(sd_ctx *ctx, const double *dF, i64 nS, i64 T, in
 // (nS + 1 - max(b, a)); PJ_OUTLYING: d_o [T][nY] = max_k |y - med'| / MAD' of the row with y appended.
 int projection_sorted_device(sd_ctx *ctx, const double *d_sorted, i64 nS, i64 T, const double *dY, i64 nY, i64 ldY,
                              int d, const double *dU, i64 K, ProjKind kind, i64 *d_count, double *d_o);
+// functional spatial depth (spatial.cu, K14): d_r[q] = || sum_s u(S_s - Q_q) || of the rows Q[idx(q) * F] (idx = d_qidx
+// or q) against the sample rows dS [nS, F], in an order fixed by q's index and the tile sizes; ST_OVERFLOW when a
+// squared distance overflows
+int spatial_device(sd_ctx *ctx, const double *dQ, const i64 *d_qidx, i64 nq, const double *dS, i64 nS, i64 F,
+                   double *d_r);
 // out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out);

@@ -83,6 +83,10 @@ int check_status(sd_ctx *ctx) {
         set_error("input contains NaN or +-inf (the B200 engine rejects non-finite values)");
         return SD_ERR_NONFINITE;
     }
+    if (st & ST_OVERFLOW) {
+        set_error("a squared distance overflows float64 (differences of about 1.3e154 or more)");
+        return SD_ERR_OVERFLOW;
+    }
     if (st & ST_NO_MEMBER) {
         set_error("the member mask selects no curve");
         return SD_ERR_INVALID;

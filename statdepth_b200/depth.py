@@ -19,11 +19,13 @@ from ._outliers import (NO_FACTOR, _check_central, _check_extremal_rows, _checke
 from ._pointcloud import _pointwisedepth, _pointwisedepth_of, _samplepointwisedepth
 from ._projection import KINDS, _functional_projection, _pointcloud_projection, draw_directions
 from ._reference import _checked_reference, _curve_values, _ProjectedReference, _query_values, _SortedReference
+from ._spatial import _functional_spatial, _functional_spatial_of, _spatial_curves, _SpatialReference
 
 __all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'ExtremalDepth',
            'HalfspaceDepth', 'FunctionalHalfspaceDepth', 'ProjectionDepth', 'FunctionalProjectionDepth',
            'FunctionalBoxplot', 'Outliergram', 'FunctionalReference', 'DepthClassifier',
-           'FunctionalProjectionDepthOf', 'ProjectionDepthOf', 'AbstractDepth']
+           'FunctionalProjectionDepthOf', 'ProjectionDepthOf', 'FunctionalSpatialDepth', 'FunctionalSpatialDepthOf',
+           'AbstractDepth']
 
 
 def _go():
@@ -468,9 +470,9 @@ def Outliergram(data: List[pd.DataFrame], factor=1.5, deep_check=False) -> _Outl
 # fitted references and depth-based classification (driver in _reference.py)
 # ---------------------------------------------------------------------------------------------------------------
 def _check_reference_depth(depth, J, directions):
-    if not (isinstance(depth, str) and depth in ('mbd',) + KINDS):
-        raise ValueError("depth must be 'mbd', 'projection' or 'tukey' (got %r)" % (depth,))
-    if depth == 'mbd' and directions is not None:
+    if not (isinstance(depth, str) and depth in ('mbd', 'spatial') + KINDS):
+        raise ValueError("depth must be 'mbd', 'projection', 'tukey' or 'spatial' (got %r)" % (depth,))
+    if depth in ('mbd', 'spatial') and directions is not None:
         raise ValueError("directions apply to depth='projection' or 'tukey'")
     if depth != 'mbd' and J != 2:
         raise ValueError('J applies to depth=\'mbd\' only: leave it at 2 for depth=%r' % depth)
@@ -492,6 +494,10 @@ class FunctionalReference:
     FunctionalProjectionDepth(sample + [g], kind=depth, directions=.directions) gives it, bit for bit; the other new
     curves never take part.
 
+    depth='spatial' (J must stay 2, directions None): sample is [df] or N DataFrames of T x d, as for the projection
+    kinds.  The sample's n_S x T d values stay on the GPU for as long as the reference; a new curve g gets the depth
+    FunctionalSpatialDepth(sample + [g]) gives it, bit for bit, and each depth_of() call uploads only the new curves.
+
     Non-finite values (and, for the projection kinds, projections that overflow) are rejected.  close() (or leaving a
     `with` block) frees the index."""
 
@@ -506,6 +512,13 @@ class FunctionalReference:
             self._index = sample[0].index
             self._ref = _SortedReference(_values(sample[0]), J)
             return
+        if depth == 'spatial':
+            X, F = _spatial_curves(sample)
+            self._T = sample[0].shape[0]
+            self._index = sample[0].index
+            self._d = None if F is None else F.shape[2]
+            self._ref = _SpatialReference(X=X, F=F)
+            return
         X, F = _curve_values(sample, directions)
         if X is not None and X.shape[1] == 0:
             raise ValueError('No data passed.')
@@ -518,8 +531,8 @@ class FunctionalReference:
 
     def depth_of(self, data: List[pd.DataFrame], deep_check=False) -> _FunctionalDepthSeries:
         """Depth of every new curve against the reference.  Univariate: the columns of data[0], indexed by
-        data[0].columns (a label may repeat a sample label).  Multivariate (projection kinds): M DataFrames of T x d,
-        indexed by list position, as FunctionalProjectionDepth."""
+        data[0].columns (a label may repeat a sample label).  Multivariate (projection kinds, spatial): M DataFrames of
+        T x d, indexed by list position, as FunctionalProjectionDepth."""
         if self._ref is None:
             raise ValueError('the reference is closed')
         if self.depth == 'mbd':
@@ -560,6 +573,7 @@ class DepthClassifier:
     equal FunctionalDepthOf([df], references[label], J=J, relax=True).  depth='projection' or 'tukey': [df] for every
     class, or lists of T x d DataFrames with the same T and d for every class; one set of directions, drawn once from
     d and seed (or given), is shared by all classes (.directions), so that the DD-plot coordinates are comparable.
+    depth='spatial': the same forms of data as the projection kinds, without directions.
     predict(data) takes the class of largest depth, ties going to the class listed first."""
 
     def __init__(self, references: dict, J=2, deep_check=False, depth='mbd', directions=None, seed=0):
@@ -580,7 +594,7 @@ class DepthClassifier:
             dims = {sample[0].shape[1] for sample in references.values() if len(sample) > 1}
             if len(dims) > 1:
                 raise ValueError('every class must have the same number of channels.')
-            if dims:
+            if dims and depth in KINDS:
                 self.directions = draw_directions(dims.pop(), directions, seed)
         self.labels = list(references)
         self._refs = []
@@ -653,3 +667,35 @@ def ProjectionDepthOf(data: pd.DataFrame, sample: pd.DataFrame, kind='projection
     finally:
         ref.close()
     return _PointwiseDepth(df=data, depths=pd.Series(index=data.index, data=depth))
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# functional spatial depth (driver in _spatial.py)
+# ---------------------------------------------------------------------------------------------------------------
+def FunctionalSpatialDepth(data: List[pd.DataFrame],
+                           to_compute=None) -> Union[_FunctionalDepthSeries, _FunctionalDepthUnivariate]:
+    """Functional spatial depth (Chakraborty & Chaudhuri 2014; depth.FSD in fda.usc): a curve is the vector of its
+    T d values, and its depth is 1 - || sum_j u(x_j - x) || / n with u(v) = v / ||v|| (Euclidean norm over all values,
+    (t, c) order, no time weight, channels as given) and u(0) = 0, so duplicates of x contribute nothing; n counts x.
+    Unlike the pointwise depths it sees a curve as one object: a shape that is slightly wrong at every time point
+    gets a low depth.
+
+    `[df]` (T rows x n curve columns) is the univariate case, to_compute are column labels; a list of N DataFrames
+    (T rows x d channels, any d) the multivariate one, to_compute are list positions.  Non-finite values are
+    rejected, and so (EngineError, SD_ERR_OVERFLOW) are curves whose squared distance overflows float64."""
+    depth = _functional_spatial(data, to_compute)
+    if len(data) == 1:
+        return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+    return _FunctionalDepthSeries(df=data[0], depths=depth)
+
+
+def FunctionalSpatialDepthOf(data: List[pd.DataFrame],
+                             sample: List[pd.DataFrame]) -> Union[_FunctionalDepthSeries, _FunctionalDepthUnivariate]:
+    """Out-of-sample functional spatial depth: each new curve g gets what FunctionalSpatialDepth(sample + [g]) gives
+    it (divisor n_S + 1), bit for bit; the other new curves never take part.  Univariate [df] (T x n, indexed by
+    data[0].columns) or lists of T x d DataFrames (indexed by list position).  To score many batches against one
+    sample, keep a FunctionalReference(sample, depth='spatial'), which keeps the sample on the GPU."""
+    depth = _functional_spatial_of(data, sample)
+    if len(sample) == 1:
+        return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+    return _FunctionalDepthSeries(df=data[0], depths=depth)
