@@ -93,18 +93,17 @@ def allreduce(arr: np.ndarray, op: str = "sum") -> np.ndarray:
     return t.cpu().numpy()
 
 
-def allgather_blocks(local: np.ndarray, total: int) -> np.ndarray:
-    """Concatenate per-rank blocks (sizes given by block()) along axis 0."""
+def allgather_blocks(local, total: int) -> np.ndarray:
+    """Concatenate per-rank blocks (sizes given by block()) along axis 0; a block is a host array or a device tensor."""
     import torch
     import torch.distributed as dist
     rank, size = dist.get_rank(), dist.get_world_size()
-    dev = _device_for_collectives()
+    local = torch.as_tensor(local).to(_device_for_collectives())
     sizes = [block(total, r, size) for r in range(size)]
     width = max(hi - lo for lo, hi in sizes)
-    pad = np.zeros((width,) + local.shape[1:], dtype=local.dtype)
-    pad[: local.shape[0]] = local
-    mine = torch.from_numpy(pad).to(dev)
-    joined = torch.empty((size * width,) + tuple(mine.shape[1:]), dtype=mine.dtype, device=dev)
+    mine = local.new_zeros((width,) + tuple(local.shape[1:]))
+    mine[: local.shape[0]] = local
+    joined = torch.empty((size * width,) + tuple(mine.shape[1:]), dtype=mine.dtype, device=mine.device)
     dist.all_gather_into_tensor(joined, mine)  # one collective, one D2H
     joined = joined.cpu().numpy().reshape((size, width) + tuple(mine.shape[1:]))
     return np.concatenate([joined[r][: hi - lo] for r, (lo, hi) in enumerate(sizes)], axis=0)
@@ -126,7 +125,7 @@ def relaxed_counts_device(eng, X, queries, j):
         out = torch.zeros(n, dtype=torch.int64, device=dev)
         Xl = None
         if hi > lo:
-            Xl = torch.from_numpy(np.ascontiguousarray(X[lo:hi], dtype=np.float64)).to(dev)
+            Xl = eng.upload(X[lo:hi])
             eng.set_option(OPT_ASYNC_DEVICE, 1)
             try:
                 eng.band_depth_counts_dev(Xl.data_ptr(), hi - lo, n, n, out.data_ptr(), None, n, j, True)
@@ -144,7 +143,7 @@ def relaxed_counts(compute, X, queries, j, eng=None):
     rank, size = world()
     if size == 1:
         return compute(X, queries, j)
-    if eng is not None and _nccl() and hasattr(eng, "band_depth_counts_dev") and j in (2, 3) and X.flags.c_contiguous:
+    if eng is not None and _nccl() and j in (2, 3) and X.flags.c_contiguous:
         return relaxed_counts_device(eng, X, queries, j)
     T = X.shape[0]
     lo, hi = block(T, rank, size)

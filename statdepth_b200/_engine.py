@@ -5,6 +5,7 @@ compute entry point raises :class:`EngineUnavailable`.
 """
 import ctypes as C
 import os
+import sys
 import threading
 import warnings
 
@@ -248,6 +249,37 @@ class Engine:
         """Wait for the engine's stream; completes a call made under OPT_ASYNC_DEVICE (raises its error)."""
         self._check(self.lib.sd_sync(self._ctx))
 
+    def _on_stream(self):
+        """(torch, device, a context making the engine's stream current): uploads, outputs and copies back are ordered
+        with the engine's kernels on its stream, and the caching allocator keeps their memory on it."""
+        import torch
+        device = torch.device("cuda", self.device)
+        return torch, device, torch.cuda.stream(torch.cuda.ExternalStream(self.stream(), device=device))
+
+    def upload(self, A, dtype=np.float64):
+        """A as a C-order tensor of dtype on the engine's device, uploaded on the engine's stream.  The rows of a
+        DataFrame's values are usually curve-major (F order): that memory is uploaded as it is and transposed on the
+        device, as sd_band_depth_f64 does with SD_LAYOUT_NT (a host transpose of 819 MB takes over a second)."""
+        A = np.asarray(A)
+        torch, device, on_stream = self._on_stream()
+        curve_major = A.ndim == 2 and A.strides[0] == A.itemsize and A.strides[1] != A.itemsize
+        host = np.ascontiguousarray(A.T if curve_major else A, dtype=dtype)
+        with warnings.catch_warnings(), on_stream:
+            warnings.filterwarnings("ignore", message="The given NumPy array is not writable")  # only read here
+            d = torch.from_numpy(host).to(device)
+            return d.t().contiguous() if curve_major else d
+
+    def _staged(self, call, *outputs, host=True):
+        """call(*pointers) on the engine's stream, one device pointer per output (shape, numpy dtype) allocated there
+        (NULL for None); the outputs come back as host arrays, or as device tensors when host is False.  Callers upload
+        their inputs first, so a call holds no device memory beyond its inputs and outputs."""
+        torch, device, on_stream = self._on_stream()
+        with on_stream:
+            outs = [None if o is None else torch.empty(o[0], dtype=getattr(torch, np.dtype(o[1]).name), device=device)
+                    for o in outputs]
+            call(*(None if t is None else t.data_ptr() for t in outs))
+            return [t.cpu().numpy() if host and t is not None else t for t in outs]
+
     @staticmethod
     def _queries(queries, n):
         if queries is None:
@@ -272,7 +304,14 @@ class Engine:
     # -- band depth -------------------------------------------------------------------------------
     def band_depth_counts(self, X, queries=None, j=2, relax=False):
         """Integer numerators for subset size j.  X is [T, n] (rows = time points, columns = curves);
-        an F-ordered X (what a column-built DataFrame gives) is passed as-is with SD_LAYOUT_NT."""
+        an F-ordered X (what a column-built DataFrame gives) is passed as-is with SD_LAYOUT_NT.  X from upload() is
+        read in place, for all curves."""
+        if _on_device(X):
+            if queries is not None:
+                raise ValueError("an uploaded X is scored for all curves")
+            T, n = X.shape
+            return self._staged(lambda out: self.band_depth_counts_dev(X.data_ptr(), T, n, n, out, None, n, j, relax),
+                                ((n,), np.int64))[0]
         X, ld, layout = self._matrix(X)
         T, n = X.shape
         q, nq = self._queries(queries, n)
@@ -321,7 +360,14 @@ class Engine:
     # -- outlier detection ------------------------------------------------------------------------------
     def band_rank_sums(self, X, want_above=False):
         """(Q, B[, A]) int64 [n]: the relaxed J = 2 numerator and the per-curve sums over time rows of the curves
-        strictly below (and above) each curve.  X is [T, n]; an F-ordered X is passed with SD_LAYOUT_NT."""
+        strictly below (and above) each curve.  X is [T, n]; an F-ordered X is passed with SD_LAYOUT_NT, X from upload()
+        is read in place."""
+        if _on_device(X):
+            T, n = X.shape
+            (qba,) = self._staged(lambda p: self.band_rank_sums_dev(X.data_ptr(), T, n, n, p, p + 8 * n,
+                                                                    p + 16 * n if want_above else None),
+                                  ((3 if want_above else 2, n), np.int64))
+            return tuple(qba)
         X, ld, layout = self._matrix(X)
         T, n = X.shape
         q, b = np.empty(n, dtype=np.int64), np.empty(n, dtype=np.int64)
@@ -336,12 +382,20 @@ class Engine:
 
     def band_envelope(self, X, member, factor, want_outside=True):
         """(lo [T], hi [T], outside [n] or None): per-row min / max of the member curves, and per curve the number of
-        rows outside the fences lo - factor * (hi - lo), hi + factor * (hi - lo)."""
-        X, ld, layout = self._matrix(X)
+        rows outside the fences lo - factor * (hi - lo), hi + factor * (hi - lo).  X from upload() is read in place."""
+        on_device = _on_device(X)
+        if not on_device:
+            X, ld, layout = self._matrix(X)
         T, n = X.shape
         mem = np.ascontiguousarray(member, dtype=np.uint8)
         if mem.shape != (n,):
             raise ValueError("member must have one entry per curve")
+        if on_device:
+            d_mem = self.upload(mem, np.uint8)
+            env, outside = self._staged(lambda e, o: self.band_envelope_dev(X.data_ptr(), T, n, n, d_mem.data_ptr(),
+                                                                            factor, e, e + 8 * T, o),
+                                        ((2, T), np.float64), ((n,), np.int64) if want_outside else None)
+            return env[0], env[1], outside
         lower, upper = np.empty(T), np.empty(T)
         outside = np.empty(n, dtype=np.int64) if want_outside else None
         self._check(self.lib.sd_band_envelope_f64(self._ctx, _ptr(X), T, n, ld, layout, _ptr(mem), float(factor),
@@ -356,6 +410,21 @@ class Engine:
                                                       _dptr(d_upper_ptr), _dptr(d_outside_ptr)))
 
     # -- extremal depth ---------------------------------------------------------------------------------
+    def band_extremity(self, X):
+        """Pointwise extremities |b - a| int32 [T, n] of the rows X [T, n], where the rows are: a host array for host
+        rows, a device tensor for rows from upload() (extremal_depth reads it in place)."""
+        on_device = _on_device(X)
+        dX = X if on_device else self.upload(X)
+        T, n = dX.shape
+        return self._staged(lambda m: self.band_extremity_dev(dX.data_ptr(), T, n, n, m), ((T, n), np.int32),
+                            host=not on_device)[0]
+
+    def extremal_depth(self, m):
+        """Extremal-depth numerators int64 [n] from the full extremity matrix m int32 [T, n] (host, or on the device)."""
+        T, n = m.shape
+        dm = m if _on_device(m) else self.upload(m, np.int32)
+        return self._staged(lambda e: self.extremal_depth_dev(dm.data_ptr(), T, n, e), ((n,), np.int64))[0]
+
     def band_extremity_dev(self, dX_ptr, T, n, ld, d_m_ptr):
         """Pointwise extremities |b - a| of the rows X [T, n] (SD_LAYOUT_TN): int32 [T, n] on the device."""
         self._check(self.lib.sd_band_extremity_f64_dev(self._ctx, _dptr(dX_ptr), int(T), int(n), int(ld),
@@ -491,6 +560,22 @@ class Engine:
                                                        _dptr(dY_ptr), int(nY), int(ldY), int(j), int(bool(relax)),
                                                        _dptr(d_out_ptr)))
 
+    def band_sort_rows(self, X):
+        """The index of a fitted reference: the rows X [T, nS] sorted ascending, a float64 tensor [T, nS] on the
+        device (the uploaded rows are freed on return)."""
+        dX = self.upload(X)
+        T, nS = dX.shape
+        return self._staged(lambda s: self.band_sort_rows_dev(dX.data_ptr(), T, nS, nS, s), ((T, nS), np.float64),
+                            host=False)[0]
+
+    def band_depth_sorted_counts(self, index, Y, J):
+        """int64 [J - 1, nY]: the relaxed numerators of the new curves Y [T, nY] against band_sort_rows' index."""
+        T, nS = index.shape
+        dY = self.upload(Y)
+        nY = dY.shape[1]
+        return self._staged(lambda o: self.band_depth_sorted_counts_dev(index.data_ptr(), T, nS, dY.data_ptr(), nY,
+                                                                        nY, J, o), ((J - 1, nY), np.int64))[0]
+
     def band_sort_rows_dev(self, dX_ptr, T, nS, ld, d_sorted_ptr):
         """The index of a fitted reference: float64 [T, nS] rows of X (SD_LAYOUT_TN) sorted ascending, on the device."""
         self._check(self.lib.sd_band_sort_rows_f64_dev(self._ctx, _dptr(dX_ptr), int(T), int(nS), int(ld),
@@ -503,6 +588,50 @@ class Engine:
                                                           _dptr(dY_ptr), int(nY), int(ldY), int(J), _dptr(d_out_ptr)))
 
     # -- fitted references for random projection depths ----------------------------------------------------------
+    def projection_sort_rows(self, F, U):
+        """The index of a projected reference: float64 [T, K, nS] on the device, the projections of the curves
+        F [nS, T, d] along U [K, d] sorted ascending per (t, k) (the uploaded curves are freed on return)."""
+        F, U = self._curves_and_directions(F, U)
+        nS, T, d = F.shape
+        dF = self.upload(F.reshape(nS, -1))
+        return self._staged(lambda s: self.projection_sort_rows_dev(dF.data_ptr(), nS, T, d, U, s),
+                            ((T, len(U), nS), np.float64), host=False)[0]
+
+    def projection_tukey_sorted_counts(self, index, F, U):
+        """Random Tukey numerators int64 [nY] of the new curves F [nY, T, d] against projection_sort_rows' index."""
+        F, U = self._curves_and_directions(F, U)
+        nY, T, d = F.shape
+        dF = self.upload(F.reshape(nY, -1))
+        return self._staged(lambda o: self.projection_tukey_sorted_counts_dev(index.data_ptr(), index.shape[2], T,
+                                                                              dF.data_ptr(), nY, d, U, o),
+                            ((nY,), np.int64))[0]
+
+    def projection_outlyingness_sorted(self, index, F, U):
+        """O [T, nY] of the new curves F [nY, T, d] against projection_sort_rows' index."""
+        F, U = self._curves_and_directions(F, U)
+        nY, T, d = F.shape
+        dF = self.upload(F.reshape(nY, -1))
+        return self._staged(lambda o: self.projection_outlyingness_sorted_dev(index.data_ptr(), index.shape[2], T,
+                                                                              dF.data_ptr(), nY, d, U, o),
+                            ((T, nY), np.float64))[0]
+
+    def band_halfspace_sorted_counts(self, index, Y):
+        """Integrated halfspace numerators int64 [nY] of the univariate new curves Y [T, nY] against band_sort_rows'
+        index."""
+        T, nS = index.shape
+        dY = self.upload(Y)
+        nY = dY.shape[1]
+        return self._staged(lambda o: self.band_halfspace_sorted_counts_dev(index.data_ptr(), T, nS, dY.data_ptr(),
+                                                                            nY, nY, o), ((nY,), np.int64))[0]
+
+    def band_outlyingness_sorted(self, index, Y):
+        """O [T, nY] of the univariate new curves Y [T, nY] against band_sort_rows' index."""
+        T, nS = index.shape
+        dY = self.upload(Y)
+        nY = dY.shape[1]
+        return self._staged(lambda o: self.band_outlyingness_sorted_dev(index.data_ptr(), T, nS, dY.data_ptr(), nY,
+                                                                        nY, o), ((T, nY), np.float64))[0]
+
     def projection_sort_rows_dev(self, dF_ptr, nS, T, d, U, d_sorted_ptr):
         """The index of a projected reference: float64 [T, K, nS], the projections of the curves F [nS, T, d] (on the
         device) along U [K, d] (host memory) sorted ascending per (t, k), on the device."""
@@ -563,17 +692,24 @@ class Engine:
         return out
 
     def spatial_norms_of(self, S, Y):
-        """r [nY] of the new curves Y [nY, F] against the sample S [nS, F] (rows); the depth is 1 - r / (nS + 1)."""
-        S, ls = self._curves(S)
+        """r [nY] of the new curves Y [nY, F] against the sample S [nS, F] (rows; host, or from upload()); the depth is
+        1 - r / (nS + 1)."""
+        on_device = _on_device(S)
+        if not on_device:
+            S, ls = self._curves(S)
         Y = np.asarray(Y, dtype=np.float64)
-        Y = np.asfortranarray(Y) if ls == LAYOUT_TN else np.ascontiguousarray(Y)  # in S's layout
         if Y.ndim != 2 or S.shape[1] != Y.shape[1]:
             raise ValueError("S and Y must have the same number of values per curve")
-        out = np.empty(Y.shape[0], dtype=np.float64)
-        if Y.shape[0] == 0:
-            return out
-        self._check(self.lib.sd_spatial_norms_of_f64(self._ctx, _ptr(S), S.shape[0], _ptr(Y), Y.shape[0], S.shape[1],
-                                                     ls, _ptr(out)))
+        (nS, F), nY = S.shape, Y.shape[0]
+        if nY == 0:
+            return np.empty(0, dtype=np.float64)
+        if on_device:
+            dY = self.upload(Y)
+            return self._staged(lambda r: self.spatial_norms_of_dev(S.data_ptr(), nS, dY.data_ptr(), nY, F, r),
+                                ((nY,), np.float64))[0]
+        Y = np.asfortranarray(Y) if ls == LAYOUT_TN else np.ascontiguousarray(Y)  # in S's layout
+        out = np.empty(nY, dtype=np.float64)
+        self._check(self.lib.sd_spatial_norms_of_f64(self._ctx, _ptr(S), nS, _ptr(Y), nY, F, ls, _ptr(out)))
         return out
 
     def spatial_norms_of_dev(self, dS_ptr, nS, dY_ptr, nY, F, d_r_ptr):
@@ -660,21 +796,16 @@ class Engine:
         return out
 
 
-def device_rows(eng, X):
-    """(stream, dX): the rows X [T, n] as a C-order float64 tensor on eng's device, uploaded on eng's stream (so the
-    upload, later outputs and the engine's kernels are ordered on it).  A DataFrame's values are usually curve-major
-    (F order): that memory is uploaded as it is and transposed on the device, as sd_band_depth_f64 does with
-    SD_LAYOUT_NT (a host transpose of 819 MB takes over a second)."""
-    import torch
-    device = torch.device("cuda", eng.device)
-    stream = torch.cuda.ExternalStream(eng.stream(), device=device)
-    curve_major = X.strides[0] == X.itemsize and X.strides[1] != X.itemsize
-    host = np.ascontiguousarray(X.T if curve_major else X, dtype=np.float64)
-    with warnings.catch_warnings():
-        warnings.filterwarnings("ignore", message="The given NumPy array is not writable")  # only read here
-        with torch.cuda.stream(stream):
-            d = torch.from_numpy(host).to(device)
-            return stream, (d.t().contiguous() if curve_major else d)
+def _on_device(A) -> bool:
+    """A is a device tensor, as Engine.upload returns (torch is imported once there is one)."""
+    torch = sys.modules.get("torch")
+    return torch is not None and isinstance(A, torch.Tensor)
+
+
+def resident(eng, A):
+    """The rows A as eng reads them on every later call: uploaded once to an Engine's device, the host array itself
+    for any other engine (a test double answering from host memory)."""
+    return eng.upload(A) if isinstance(eng, Engine) else A
 
 
 _engines = {}

@@ -5,12 +5,11 @@ K8; csrc/extremal.cu, K10).
 Both take univariate data X [T, n] (time rows x curves) and return plain arrays; depth.py wraps them in result
 objects.  Every per-curve quantity is exact int64 from the engine; floats are formed here once, at the end.
 
-On one GPU the matrix crosses PCIe once per call: the rows are uploaded once and every engine call reads them in
-place through the `_dev` entry points.  An engine without them (the CPU test double) gets the host matrix.  Under
-`enable_distributed()` every rank takes a block of time rows: the rank sums and outside counts are all-reduced, the
-per-row envelopes all-gathered, and the whisker pass runs after the outside counts are reduced.  Extremal depth is
-not additive over rows: every rank computes the extremities of its rows, they are all-gathered through the host, and
-every rank orders the curves on the full matrix.
+On one GPU the matrix crosses PCIe once per call: the rows are uploaded once (Engine.upload) and every engine call
+reads them in place.  Under `enable_distributed()` every rank takes a block of time rows: the rank sums and outside
+counts are all-reduced, the per-row envelopes all-gathered, and the whisker pass runs after the outside counts are
+reduced.  Extremal depth is not additive over rows: every rank computes the extremities of its rows, they are
+all-gathered, and every rank orders the curves on the full matrix.
 """
 import math
 import numbers
@@ -22,7 +21,7 @@ import pandas as pd
 from scipy.special import binom
 
 from . import _dist
-from ._engine import device_rows, get_engine
+from ._engine import get_engine, resident
 from ._functional import _values
 from ._helper import _handle_depth_errors
 
@@ -66,103 +65,37 @@ def _check_central(central) -> None:
 
 
 class _Rows:
-    """A block of time rows X [T, n] on one engine."""
+    """A block of time rows X [T, n], resident on its engine (an empty block is never uploaded)."""
 
     def __init__(self, eng, X):
         self.eng = eng
         self.T, self.n = X.shape
-        self.on_device = hasattr(eng, 'band_envelope_dev') and self.T > 0
-        if not self.on_device:
-            self.X = X
-            return
-        import torch
-        self.torch = torch
-        self.device = torch.device('cuda', eng.device)
-        self.stream, self.dX = device_rows(eng, X)
-
-    def _empty(self, size, dtype):
-        return self.torch.empty(size, dtype=dtype, device=self.device)
+        self.X = resident(eng, X) if self.T > 0 else X
 
     def mbd_counts(self) -> np.ndarray:
         """Q [n]: the relaxed J = 2 numerators of these rows."""
         if self.T == 0:
             return np.zeros(self.n, dtype=np.int64)
-        if not self.on_device:
-            return np.asarray(self.eng.band_depth_counts(self.X, None, 2, True), dtype=np.int64)
-        with self.torch.cuda.stream(self.stream):
-            q = self._empty(self.n, self.torch.int64)
-            self.eng.band_depth_counts_dev(self.dX.data_ptr(), self.T, self.n, self.n, q.data_ptr(), None, self.n, 2,
-                                           True)
-            return q.cpu().numpy()
+        return self.eng.band_depth_counts(self.X, None, 2, True)
 
     def rank_sums(self):
         """(Q, B) [n]: numerators and sums of the curves strictly below, over these rows."""
         if self.T == 0:
             return np.zeros(self.n, dtype=np.int64), np.zeros(self.n, dtype=np.int64)
-        if not self.on_device:
-            q, b = self.eng.band_rank_sums(self.X)
-            return np.asarray(q, dtype=np.int64), np.asarray(b, dtype=np.int64)
-        with self.torch.cuda.stream(self.stream):
-            qb = self._empty((2, self.n), self.torch.int64)
-            self.eng.band_rank_sums_dev(self.dX.data_ptr(), self.T, self.n, self.n, qb[0].data_ptr(), qb[1].data_ptr())
-            qb = qb.cpu().numpy()
-            return qb[0], qb[1]
+        return self.eng.band_rank_sums(self.X)
 
     def extremity(self) -> np.ndarray:
-        """m [T, n] int32: the pointwise extremities |b - a| of these rows, on the host."""
+        """m [T, n] int32: the pointwise extremities |b - a| of these rows, where the rows are (on one GPU they never
+        reach the host)."""
         if self.T == 0:
             return np.zeros((0, self.n), dtype=np.int32)
-        if not self.on_device:
-            return np.asarray(self.eng.band_extremity(self.X), dtype=np.int32)
-        with self.torch.cuda.stream(self.stream):
-            return self._extremity_dev().cpu().numpy()
-
-    def _extremity_dev(self):
-        m = self._empty((self.T, self.n), self.torch.int32)
-        self.eng.band_extremity_dev(self.dX.data_ptr(), self.T, self.n, self.n, m.data_ptr())
-        return m
-
-    def extremal_numerators(self) -> np.ndarray:
-        """e [n] with these rows as the whole matrix; on the device the extremities never leave it."""
-        if not self.on_device:
-            return _numerators_of(self.eng, self.extremity())
-        with self.torch.cuda.stream(self.stream):
-            m = self._extremity_dev()
-            e = self._empty(self.n, self.torch.int64)
-            self.eng.extremal_depth_dev(m.data_ptr(), self.T, self.n, e.data_ptr())
-            return e.cpu().numpy()
+        return self.eng.band_extremity(self.X)
 
     def envelope(self, member: np.ndarray, factor: float, want_outside: bool):
         """(lo [T], hi [T], outside [n] or None) of these rows over the member curves."""
         if self.T == 0:
             return np.zeros(0), np.zeros(0), (np.zeros(self.n, dtype=np.int64) if want_outside else None)
-        if not self.on_device:
-            lo, hi, out = self.eng.band_envelope(self.X, member, factor, want_outside)
-            return np.asarray(lo), np.asarray(hi), None if out is None else np.asarray(out, dtype=np.int64)
-        torch = self.torch
-        with torch.cuda.stream(self.stream):
-            d_member = torch.from_numpy(np.ascontiguousarray(member, dtype=np.uint8)).to(self.device)
-            env = self._empty((2, self.T), torch.float64)
-            out = self._empty(self.n, torch.int64) if want_outside else None
-            self.eng.band_envelope_dev(self.dX.data_ptr(), self.T, self.n, self.n, d_member.data_ptr(), factor,
-                                       env[0].data_ptr(), env[1].data_ptr(), None if out is None else out.data_ptr())
-            env = env.cpu().numpy()
-            return env[0], env[1], None if out is None else out.cpu().numpy()
-
-
-def _numerators_of(eng, m: np.ndarray) -> np.ndarray:
-    """Extremal-depth numerators e [n] from the full extremity matrix m [T, n] (uploaded once on a GPU engine)."""
-    if not hasattr(eng, 'extremal_depth_dev'):
-        return np.asarray(eng.extremal_depth(m), dtype=np.int64)
-    import torch
-    device = torch.device('cuda', eng.device)
-    stream = torch.cuda.ExternalStream(eng.stream(), device=device)
-    T, n = m.shape
-    with torch.cuda.stream(stream):
-        dm = torch.from_numpy(np.ascontiguousarray(m, dtype=np.int32)).to(device)
-        e = torch.empty(n, dtype=torch.int64, device=device)
-        eng.extremal_depth_dev(dm.data_ptr(), T, n, e.data_ptr())
-        return e.cpu().numpy()
+        return self.eng.band_envelope(self.X, member, factor, want_outside)
 
 
 def _local_rows(X: np.ndarray):
@@ -200,9 +133,8 @@ def central_count(central: float, n: int) -> int:
 
 def _extremal_numerators(rows: _Rows, T: int, size: int) -> np.ndarray:
     """e [n] of the whole matrix X [T, n] from this rank's rows (a collective when size > 1)."""
-    if size == 1:
-        return rows.extremal_numerators()
-    return _numerators_of(rows.eng, _dist.allgather_blocks(rows.extremity(), T))
+    m = rows.extremity()
+    return rows.eng.extremal_depth(m if size == 1 else _dist.allgather_blocks(m, T))
 
 
 def _extremal_depth(X: np.ndarray) -> np.ndarray:

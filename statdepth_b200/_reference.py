@@ -6,10 +6,9 @@ once on the device and kept there (the index); every later call uploads only the
 integers sd_band_depth_oos_f64 returns and the floats are formed by _functional._relaxed_depths_of, so the depths are
 bit-identical to FunctionalDepthOf(relax=True).
 
-On one GPU the index lives in a torch tensor on the engine's device.  An engine without the `_dev` entry points (the
-CPU test double) keeps a host index from its `band_sort_rows` and answers `band_depth_sorted_counts`.  Under
-`enable_distributed()` every rank indexes its block of time rows; each call scores the same rows of the new curves and
-all-reduces the counts, so construction and every call are collectives.
+The engine's `band_sort_rows` returns the index on its device, and `band_depth_sorted_counts` answers each call
+from it.  Under `enable_distributed()` every rank indexes its block of time rows; each call scores the same rows of
+the new curves and all-reduces the counts, so construction and every call are collectives.
 
 Projection and random Tukey depth (csrc/reference_proj.cu, DESIGN.md K13).  The reference's projections along the
 directions U are sorted once per (time point, direction): an index of T K n_S doubles (K9's sorted rows for univariate
@@ -26,7 +25,7 @@ import numpy as np
 import pandas as pd
 
 from . import _dist
-from ._engine import device_rows, get_engine
+from ._engine import get_engine
 from ._functional import _relaxed_depths_of, _values
 from ._helper import _handle_depth_errors
 from ._projection import _depth_from_rows
@@ -52,38 +51,14 @@ class _SortedReference:
         rank, self.size = _dist.world()
         self.lo, self.hi = _dist.block(self.T, rank, self.size)
         self.eng = get_engine()
-        self.on_device = hasattr(self.eng, 'band_sort_rows_dev')
-        rows = S[self.lo:self.hi]
-        self.index = None
-        if self.hi == self.lo:
-            return
-        if not self.on_device:
-            self.index = np.asarray(self.eng.band_sort_rows(rows), dtype=np.float64)
-            return
-        import torch
-        self.torch = torch
-        stream, dX = device_rows(self.eng, rows)
-        with torch.cuda.stream(stream):
-            index = torch.empty((self.hi - self.lo, self.nS), dtype=torch.float64, device=dX.device)
-            self.eng.band_sort_rows_dev(dX.data_ptr(), self.hi - self.lo, self.nS, self.nS, index.data_ptr())
-        self.index = index  # the raw rows are dropped on return
+        self.index = self.eng.band_sort_rows(S[self.lo:self.hi]) if self.hi > self.lo else None
 
     def counts(self, Y: np.ndarray) -> np.ndarray:
         """int64 [J - 1, nY]: row j - 2 holds the relaxed numerators of subset size j, summed over the ranks."""
-        nY = Y.shape[1]
-        rows = Y[self.lo:self.hi]
         if self.index is None:
-            local = np.zeros((self.J - 1, nY), dtype=np.int64)
-        elif not self.on_device:
-            local = np.asarray(self.eng.band_depth_sorted_counts(self.index, rows, self.J), dtype=np.int64)
+            local = np.zeros((self.J - 1, Y.shape[1]), dtype=np.int64)
         else:
-            torch = self.torch
-            stream, dY = device_rows(self.eng, rows)
-            with torch.cuda.stream(stream):
-                out = torch.empty((self.J - 1, nY), dtype=torch.int64, device=dY.device)
-                self.eng.band_depth_sorted_counts_dev(self.index.data_ptr(), self.hi - self.lo, self.nS, dY.data_ptr(),
-                                                      nY, nY, self.J, out.data_ptr())
-                local = out.cpu().numpy()
+            local = self.eng.band_depth_sorted_counts(self.index, Y[self.lo:self.hi], self.J)
         return local if self.size == 1 else _dist.allreduce(local)
 
     def depths(self, Y: np.ndarray) -> np.ndarray:
@@ -135,79 +110,38 @@ def _curve_values(data: List[pd.DataFrame], directions=None, frames=None):
 class _ProjectedReference:
     """This rank's share of a reference fitted for projection (kind='projection') or random Tukey depth ('tukey'):
     univariate curves X [T, nS] (U None), or curves F [nS, T, d] along U [K, d]; cloud=True (F [nS, 1, d]) shards the
-    directions instead of the time rows.  The device index is a torch tensor of T K nS doubles that lives as long as
-    the reference."""
+    directions instead of the time rows.  The index, T K nS doubles on the engine's device, lives as long as the
+    reference."""
 
     def __init__(self, kind: str, X=None, F=None, U=None, cloud=False):
         self.kind, self.U, self.cloud = kind, U, cloud
         if U is None:
             self.T, self.nS = X.shape
         else:
-            self.nS, self.T, self.d = F.shape
+            self.nS, self.T = F.shape[:2]
         rank, self.size = _dist.world()
         self.lo, self.hi = _dist.block(len(U) if cloud else self.T, rank, self.size)
         self.eng = get_engine()
-        self.on_device = hasattr(self.eng, 'projection_sort_rows_dev')
         self.index = None
         if self.hi == self.lo:
             return
         if U is None:
-            rows = X[self.lo:self.hi]
+            self.index = self.eng.band_sort_rows(X[self.lo:self.hi])
         else:
-            F = np.ascontiguousarray(F if cloud else F[:, self.lo:self.hi], dtype=np.float64)
             self.Ul = np.ascontiguousarray(U[self.lo:self.hi] if cloud else U)
-        if not self.on_device:
-            self.index = np.asarray(self.eng.band_sort_rows(rows) if U is None
-                                    else self.eng.projection_sort_rows(F, self.Ul), dtype=np.float64)
-            return
-        import torch
-        self.torch = torch
-        if U is None:
-            stream, dX = device_rows(self.eng, rows)
-            with torch.cuda.stream(stream):
-                index = torch.empty((self.hi - self.lo, self.nS), dtype=torch.float64, device=dX.device)
-                self.eng.band_sort_rows_dev(dX.data_ptr(), self.hi - self.lo, self.nS, self.nS, index.data_ptr())
-        else:
-            tb = F.shape[1]
-            stream, dF = device_rows(self.eng, F.reshape(self.nS, -1))
-            with torch.cuda.stream(stream):
-                index = torch.empty((tb, len(self.Ul), self.nS), dtype=torch.float64, device=dF.device)
-                self.eng.projection_sort_rows_dev(dF.data_ptr(), self.nS, tb, self.d, self.Ul, index.data_ptr())
-        self.index = index  # the raw reference is dropped on return
+            self.index = self.eng.projection_sort_rows(F if cloud else F[:, self.lo:self.hi], self.Ul)
 
     def _local(self, Y):
         """This rank's numerators [nY] (Tukey) or outlyingness rows [rows, nY] of the new observations."""
         tukey = self.kind == 'tukey'
-        if self.U is None:
-            nY = Y.shape[1]
-            rows = Y[self.lo:self.hi]
-        else:
-            nY = Y.shape[0]
-            rows = np.ascontiguousarray(Y if self.cloud else Y[:, self.lo:self.hi], dtype=np.float64)
         eng = self.eng
-        if not self.on_device:
-            if self.U is None:
-                out = (eng.band_halfspace_sorted_counts(self.index, rows) if tukey
-                       else eng.band_outlyingness_sorted(self.index, rows))
-            else:
-                out = (eng.projection_tukey_sorted_counts(self.index, rows, self.Ul) if tukey
-                       else eng.projection_outlyingness_sorted(self.index, rows, self.Ul))
-            return np.asarray(out, dtype=np.int64 if tukey else np.float64)
-        torch = self.torch
-        tb = self.index.shape[0]
-        stream, dY = device_rows(eng, rows if self.U is None else rows.reshape(nY, -1))
-        with torch.cuda.stream(stream):
-            if tukey:
-                out = torch.empty(nY, dtype=torch.int64, device=dY.device)
-            else:
-                out = torch.empty((tb, nY), dtype=torch.float64, device=dY.device)
-            if self.U is None:
-                fn = eng.band_halfspace_sorted_counts_dev if tukey else eng.band_outlyingness_sorted_dev
-                fn(self.index.data_ptr(), tb, self.nS, dY.data_ptr(), nY, nY, out.data_ptr())
-            else:
-                fn = eng.projection_tukey_sorted_counts_dev if tukey else eng.projection_outlyingness_sorted_dev
-                fn(self.index.data_ptr(), self.nS, tb, dY.data_ptr(), nY, self.d, self.Ul, out.data_ptr())
-            return out.cpu().numpy()
+        if self.U is None:
+            rows = Y[self.lo:self.hi]
+            return (eng.band_halfspace_sorted_counts(self.index, rows) if tukey
+                    else eng.band_outlyingness_sorted(self.index, rows))
+        rows = Y if self.cloud else Y[:, self.lo:self.hi]
+        return (eng.projection_tukey_sorted_counts(self.index, rows, self.Ul) if tukey
+                else eng.projection_outlyingness_sorted(self.index, rows, self.Ul))
 
     def depths(self, Y: np.ndarray) -> np.ndarray:
         """Depth of every new observation (columns of Y [T, nY] for univariate curves, else Y [nY, T, d]), bit-identical

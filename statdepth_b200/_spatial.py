@@ -21,7 +21,7 @@ import numpy as np
 import pandas as pd
 
 from . import _dist
-from ._engine import device_rows, get_engine
+from ._engine import get_engine, resident
 from ._functional import _positions
 from ._reference import _curve_values
 
@@ -77,32 +77,14 @@ def _checked_new_curves(data, XS, FS):
 
 
 class _SpatialReference:
-    """A sample of curves kept for spatial depth: n_S x F doubles in a torch tensor on the engine's device for as long
-    as the reference lives (a host array for a test double without `_dev` methods).  Every rank holds all of it."""
+    """A sample of curves kept for spatial depth: n_S x F doubles uploaded once to the engine's device, for as long as
+    the reference lives.  Every rank holds all of it."""
 
     def __init__(self, X=None, F=None):
         A = _rows(X, F)
         self.nS, self.F = A.shape
         self.eng = get_engine()
-        self.on_device = hasattr(self.eng, 'spatial_norms_of_dev')
-        if not self.on_device:
-            self.sample = np.ascontiguousarray(A, dtype=np.float64)
-            return
-        import torch
-        self.torch = torch
-        _, self.sample = device_rows(self.eng, A)
-
-    def _norms(self, Y):
-        """r of the new curves Y [m, F] (rows) against the sample."""
-        if not self.on_device:
-            return self.eng.spatial_norms_of(self.sample, Y)
-        torch = self.torch
-        stream, dY = device_rows(self.eng, Y)
-        with torch.cuda.stream(stream):
-            out = torch.empty(Y.shape[0], dtype=torch.float64, device=dY.device)
-            self.eng.spatial_norms_of_dev(self.sample.data_ptr(), self.nS, dY.data_ptr(), Y.shape[0], self.F,
-                                          out.data_ptr())
-            return out.cpu().numpy()
+        self.sample = resident(self.eng, A)
 
     def depths(self, Y: np.ndarray) -> np.ndarray:
         """Depth of every new curve: the columns of Y [T, nY] (univariate), else Y [nY, T, d]; each equals
@@ -112,7 +94,8 @@ class _SpatialReference:
             raise ValueError('data and sample must have the same number of values per curve.')
         if A.shape[0] == 0:
             return np.zeros(0, dtype=np.float64)
-        r = _dist.query_sharded(lambda qb: self._norms(A[qb]), np.arange(A.shape[0]), np.float64)
+        r = _dist.query_sharded(lambda qb: self.eng.spatial_norms_of(self.sample, A[qb]), np.arange(A.shape[0]),
+                                np.float64)
         return 1.0 - np.asarray(r, dtype=np.float64) / (self.nS + 1)
 
     def close(self) -> None:

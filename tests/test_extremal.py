@@ -118,8 +118,8 @@ def _spikes(seed):
 # CPU test double
 # ---------------------------------------------------------------------------------------------------------------
 class ExtremalOracleEngine:
-    """TEST DOUBLE: the host methods the outlier drivers call, answered by numpy (no `_dev` methods, so the drivers
-    take the host path)."""
+    """TEST DOUBLE: the Engine methods the outlier drivers call, answered by numpy (not an Engine, so the drivers hand
+    it the host rows)."""
 
     def __init__(self):
         self.calls = 0

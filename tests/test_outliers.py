@@ -103,8 +103,8 @@ def np_outliergram(X, factor=1.5):
 # CPU test double
 # ---------------------------------------------------------------------------------------------------------------
 class OutlierOracleEngine:
-    """TEST DOUBLE: the host methods the outlier drivers call, answered by numpy (no `_dev` methods, so the drivers
-    take the host path)."""
+    """TEST DOUBLE: the Engine methods the outlier drivers call, answered by numpy (not an Engine, so the drivers hand
+    it the host rows)."""
 
     def __init__(self):
         from oracle import cpu_oracle

@@ -41,8 +41,8 @@ def np_sorted_counts(sorted_rows, Y, J):
 
 
 class SortedOracleEngine:
-    """TEST DOUBLE: the fitted reference answered by np.sort + searchsorted (no `_dev` methods, so the driver takes the
-    host path), and FunctionalDepthOf's relaxed counts answered by the C oracle on S u {g}, one g at a time."""
+    """TEST DOUBLE: the fitted reference answered by np.sort + searchsorted (the index is a host array), and
+    FunctionalDepthOf's relaxed counts answered by the C oracle on S u {g}, one g at a time."""
 
     def __init__(self):
         from oracle import cpu_oracle

@@ -106,7 +106,7 @@ def sorted_outlyingness(index, Y):
 
 class ReferenceOracleEngine(ProjectionOracleEngine):
     """TEST DOUBLE: test_projection's numpy engine (the in-sample calls), plus the fitted-reference calls answered by
-    np.sort and the restated query kernels (no `_dev` methods, so the driver keeps a host index)."""
+    np.sort and the restated query kernels (the index is a host array)."""
 
     def band_sort_rows(self, X):
         self._finite(X)

@@ -69,7 +69,7 @@ def _frames(F):
 
 class SpatialOracleEngine:
     """TEST DOUBLE: the engine methods the spatial drivers call, answered by the numpy oracle, refusing non-finite
-    input with SD_ERR_NONFINITE as the engine does (no `_dev` methods: the reference keeps a host sample)."""
+    input with SD_ERR_NONFINITE as the engine does (not an Engine, so the reference keeps a host sample)."""
 
     def __init__(self):
         self.calls = 0
