@@ -433,6 +433,37 @@ int sd_spatial_norms_of_f64_dev(sd_ctx *ctx, const double *dS, int64_t nS, const
                                 double *d_r_out);
 
 /*
+ * h-modal depth (Cuevas, Febrero & Fraiman 2007).  Curves as for the spatial entry points: the vector of F = T*d values
+ * in (t, c) order, SD_LAYOUT_NT (curve i a row) or SD_LAYOUT_TN (curve i a column, transposed on the device); d2 is
+ * the plain squared Euclidean distance over all F values, accumulated in f order (d2(a, b) == d2(b, a) bit for bit).
+ * The depth is S * phi(0) / n_pop with S = sum_j exp(c d2(x_q, x_j)), c = -1 / (2 h^2), n_pop = n in sample (j over all
+ * n curves, q included) and nS + 1 out of sample; the host forms it, and picks h.
+ *
+ * Pair selection: d2_out[0] and d2_out[1] (HOST memory, both variants) = the k-th and min(k + 1, N - 1)-th smallest
+ * (0-based) of the N = n (n - 1) / 2 squared distances d2(x_i, x_j), i < j: exact order statistics (a radix select over
+ * the bit patterns, the distances recomputed per pass; workspace at most 1 GB at any n).  2 <= n <= 4 194 240.
+ * Sums: s_out[q] = S of the queries (all when query_idx == NULL, query_idx always HOST memory), summed in an order fixed
+ * by the indices and the tile sizes alone, so a query's bits never depend on the other queries; out of sample, s_out[g]
+ * equals the in-sample S of S + [g] at entry nS bit for bit.  c must be finite and < 0.
+ * SD_ERR_NONFINITE when an input holds NaN or +-inf, SD_ERR_OVERFLOW when a squared distance overflows.
+ */
+int sd_modal_pair_select_f64(sd_ctx *ctx, const double *X, int64_t n, int64_t F, int layout, int64_t k,
+                             double *d2_out);
+/* same with DEVICE rows dX [n, F] */
+int sd_modal_pair_select_f64_dev(sd_ctx *ctx, const double *dX, int64_t n, int64_t F, int64_t k, double *d2_out);
+int sd_modal_sums_f64(sd_ctx *ctx, const double *X, int64_t n, int64_t F, int layout, double c,
+                      const int64_t *query_idx, int64_t nq, double *s_out);
+/* same with DEVICE rows dX [n, F] and DEVICE output d_s_out [nq] */
+int sd_modal_sums_f64_dev(sd_ctx *ctx, const double *dX, int64_t n, int64_t F, double c, const int64_t *query_idx,
+                          int64_t nq, double *d_s_out);
+/* new curves Y [nY] against the sample S [nS] (same layout, each dense) */
+int sd_modal_sums_of_f64(sd_ctx *ctx, const double *S, int64_t nS, const double *Y, int64_t nY, int64_t F,
+                         int layout, double c, double *s_out);
+/* same with DEVICE pointers, curves as rows only (dS [nS, F], dY [nY, F]); d_s_out holds nY doubles */
+int sd_modal_sums_of_f64_dev(sd_ctx *ctx, const double *dS, int64_t nS, const double *dY, int64_t nY, int64_t F,
+                             double c, double *d_s_out);
+
+/*
  * Batched band depth over sub-populations of one matrix (K-sampled blocks, homogeneity
  * permutations): membership[b*n + c] != 0 selects the curves of batch b; queries[b*nqb + i] is
  * the i-th query curve of batch b (must be a member).  count_out[b*nqb + i] as in

@@ -136,6 +136,17 @@ SIGNATURES = {
                                           C.c_int, C.c_void_p]),
     "sd_spatial_norms_of_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64,
                                               C.c_void_p]),
+    "sd_modal_pair_select_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_int64,
+                                           C.c_void_p]),
+    "sd_modal_pair_select_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]),
+    "sd_modal_sums_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_double, C.c_void_p,
+                                    C.c_int64, C.c_void_p]),
+    "sd_modal_sums_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_double, C.c_void_p,
+                                        C.c_int64, C.c_void_p]),
+    "sd_modal_sums_of_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int,
+                                       C.c_double, C.c_void_p]),
+    "sd_modal_sums_of_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64,
+                                           C.c_double, C.c_void_p]),
     "sd_band_depth_batched_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                             C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -716,6 +727,73 @@ class Engine:
         """Device-pointer variant (curves as rows: S [nS, F], Y [nY, F]); r [nY] stays on the device."""
         self._check(self.lib.sd_spatial_norms_of_f64_dev(self._ctx, _dptr(dS_ptr), int(nS), _dptr(dY_ptr), int(nY),
                                                          int(F), _dptr(d_r_ptr)))
+
+    # -- h-modal depth ---------------------------------------------------------------------------------------
+    def modal_pair_select(self, X, k):
+        """(d2_k, d2_k1): the k-th and min(k + 1, N - 1)-th smallest (0-based) of the N = n (n - 1) / 2 squared
+        distances between the curves X [n, F] (rows; host, or from upload()), exact."""
+        out = np.empty(2, dtype=np.float64)
+        if _on_device(X):
+            n, F = X.shape
+            return self.modal_pair_select_dev(X.data_ptr(), n, F, k)
+        X, layout = self._curves(X)
+        n, F = X.shape
+        self._check(self.lib.sd_modal_pair_select_f64(self._ctx, _ptr(X), n, F, layout, int(k), _ptr(out)))
+        return out
+
+    def modal_pair_select_dev(self, dX_ptr, n, F, k):
+        """Device-pointer variant (curves as rows dX [n, F]); the two order statistics come back as a host array."""
+        out = np.empty(2, dtype=np.float64)
+        self._check(self.lib.sd_modal_pair_select_f64_dev(self._ctx, _dptr(dX_ptr), int(n), int(F), int(k),
+                                                          _ptr(out)))
+        return out
+
+    def modal_sums(self, X, c, queries=None):
+        """S [nq] = sum_j exp(c d2(x_q, x_j)) over all n curves X [n, F] (rows; host, or from upload()) for the queries
+        (all when None); the h-modal depth is S phi(0) / n."""
+        if _on_device(X):
+            n, F = X.shape
+            q, nq = self._queries(queries, n)
+            return self._staged(lambda out: self.modal_sums_dev(X.data_ptr(), n, F, c, q, out), ((nq,), np.float64))[0]
+        X, layout = self._curves(X)
+        n, F = X.shape
+        q, nq = self._queries(queries, n)
+        out = np.empty(nq, dtype=np.float64)
+        self._check(self.lib.sd_modal_sums_f64(self._ctx, _ptr(X), n, F, layout, float(c), _ptr(q), nq, _ptr(out)))
+        return out
+
+    def modal_sums_dev(self, dX_ptr, n, F, c, queries, d_out_ptr):
+        """Device-pointer variant (curves as rows dX [n, F]; queries a host index array or None); S stays on the
+        device."""
+        q, nq = self._queries(queries, n)
+        self._check(self.lib.sd_modal_sums_f64_dev(self._ctx, _dptr(dX_ptr), int(n), int(F), float(c), _ptr(q), nq,
+                                                   _dptr(d_out_ptr)))
+
+    def modal_sums_of(self, S, Y, c):
+        """S [nY] of the new curves Y [nY, F] against the sample S [nS, F] (rows; host, or from upload()), each with
+        its own term exp(-0) = 1; the depth is S phi(0) / (nS + 1)."""
+        on_device = _on_device(S)
+        if not on_device:
+            S, ls = self._curves(S)
+        Y = np.asarray(Y, dtype=np.float64)
+        if Y.ndim != 2 or S.shape[1] != Y.shape[1]:
+            raise ValueError("S and Y must have the same number of values per curve")
+        (nS, F), nY = S.shape, Y.shape[0]
+        if nY == 0:
+            return np.empty(0, dtype=np.float64)
+        if on_device:
+            dY = self.upload(Y)
+            return self._staged(lambda r: self.modal_sums_of_dev(S.data_ptr(), nS, dY.data_ptr(), nY, F, c, r),
+                                ((nY,), np.float64))[0]
+        Y = np.asfortranarray(Y) if ls == LAYOUT_TN else np.ascontiguousarray(Y)  # in S's layout
+        out = np.empty(nY, dtype=np.float64)
+        self._check(self.lib.sd_modal_sums_of_f64(self._ctx, _ptr(S), nS, _ptr(Y), nY, F, ls, float(c), _ptr(out)))
+        return out
+
+    def modal_sums_of_dev(self, dS_ptr, nS, dY_ptr, nY, F, c, d_out_ptr):
+        """Device-pointer variant (curves as rows: S [nS, F], Y [nY, F]); S [nY] stays on the device."""
+        self._check(self.lib.sd_modal_sums_of_f64_dev(self._ctx, _dptr(dS_ptr), int(nS), _dptr(dY_ptr), int(nY),
+                                                      int(F), float(c), _dptr(d_out_ptr)))
 
     def simplicial_oos_counts(self, S, Y, tol=1e-7):
         S = np.ascontiguousarray(S, dtype=np.float64)

@@ -39,6 +39,7 @@ SOURCES = {
     "pointcloud.cu": ["-fmad=false"],
     "simplicial_count.cu": ["-fmad=false"],
     "spatial.cu": [],
+    "modal.cu": [],
 }
 EXPORT_MAP = os.path.join(CSRC, "exports.map")
 

@@ -9,6 +9,8 @@
 // host / _dev pair shares one static body that takes a `dev` flag: the checks and the device work are written once,
 // and the host side alone stages.  Checks only the host can make (query, pool and member ids in range) stay in its
 // `stage`.
+#include <float.h>
+
 #include <thread>
 #include <vector>
 
@@ -1151,6 +1153,103 @@ int sd_spatial_norms_of_f64(sd_ctx *ctx, const double *S, int64_t nS, const doub
 int sd_spatial_norms_of_f64_dev(sd_ctx *ctx, const double *dS, int64_t nS, const double *dY, int64_t nY, int64_t F,
                                 double *d_r_out) {
     return spatial_of_call(ctx, dS, nS, dY, nY, F, SD_LAYOUT_NT, d_r_out, true, "sd_spatial_norms_of_f64_dev");
+}
+
+// ---------------------------------------------------------------------------------------------
+// h-modal depth (K15, modal.cu)
+// ---------------------------------------------------------------------------------------------
+static int modal_select_call(sd_ctx *ctx, const double *X, i64 n, i64 F, int layout, i64 k, double *d2_out, bool dev,
+                             const char *who) {
+    SD_REQUIRE(n >= 2 && F >= 1, "%s: bad sizes n=%lld F=%lld (n >= 2: at least one pair)", who, (long long)n,
+               (long long)F);
+    SD_REQUIRE(n <= 65535ll * 64, "%s: n=%lld too large (at most 4 194 240 curves)", who, (long long)n);
+    SD_REQUIRE(layout == SD_LAYOUT_TN || layout == SD_LAYOUT_NT, "%s: bad layout %d", who, layout);
+    const i64 npairs = n * (n - 1) / 2;
+    SD_REQUIRE(k >= 0 && k < npairs, "%s: k=%lld out of range [0, %lld)", who, (long long)k, (long long)npairs);
+    const double *dX = X;
+    return call(ctx, who, X, d2_out, !dev, [&](Staging &s) -> int {
+        return dev ? SD_OK : upload_curves(s, X, n, nullptr, 0, F, layout, &dX);
+    }, [&]() -> int {
+        SD_TRY(finite_check_device(ctx, dX, 1, n * F, n * F));
+        return modal_select_device(ctx, dX, n, F, k, k + 1 < npairs ? k + 1 : k, d2_out);
+    });
+}
+
+int sd_modal_pair_select_f64(sd_ctx *ctx, const double *X, int64_t n, int64_t F, int layout, int64_t k,
+                             double *d2_out) {
+    return modal_select_call(ctx, X, n, F, layout, k, d2_out, false, "sd_modal_pair_select_f64");
+}
+
+int sd_modal_pair_select_f64_dev(sd_ctx *ctx, const double *dX, int64_t n, int64_t F, int64_t k, double *d2_out) {
+    return modal_select_call(ctx, dX, n, F, SD_LAYOUT_NT, k, d2_out, true, "sd_modal_pair_select_f64_dev");
+}
+
+static int check_modal_c(double c, const char *who) {
+    SD_REQUIRE(c < 0.0 && c >= -DBL_MAX, "%s: c=%g must be finite and < 0 (c = -1 / (2 h^2))", who, c);
+    return SD_OK;
+}
+
+static int modal_sums_call(sd_ctx *ctx, const double *X, i64 n, i64 F, int layout, double c, const int64_t *query_idx,
+                           i64 nq, double *s_out, bool dev, const char *who) {
+    SD_REQUIRE(n >= 1 && F >= 1 && nq >= 0, "%s: bad sizes n=%lld F=%lld nq=%lld", who, (long long)n, (long long)F,
+               (long long)nq);
+    SD_REQUIRE(layout == SD_LAYOUT_TN || layout == SD_LAYOUT_NT, "%s: bad layout %d", who, layout);
+    SD_REQUIRE(query_idx || nq == n, "%s: query_idx == NULL requires nq == n", who);
+    SD_TRY(check_modal_c(c, who));
+    const double *dX = X;
+    const i64 *d_q = nullptr;
+    double *d_s = s_out;
+    return call(ctx, who, X, s_out, !dev, [&](Staging &s) -> int {
+        if (!dev) SD_TRY(upload_curves(s, X, n, nullptr, 0, F, layout, &dX));
+        SD_TRY(upload_queries(ctx, query_idx, nq, n, &d_q, who));
+        return dev ? SD_OK : s.output(BUF_OUT, s_out, nq, &d_s);
+    }, [&]() -> int {
+        SD_TRY(finite_check_device(ctx, dX, 1, n * F, n * F));
+        return modal_sums_device(ctx, dX, d_q, nq, dX, n, F, false, c, d_s);
+    });
+}
+
+int sd_modal_sums_f64(sd_ctx *ctx, const double *X, int64_t n, int64_t F, int layout, double c,
+                      const int64_t *query_idx, int64_t nq, double *s_out) {
+    return modal_sums_call(ctx, X, n, F, layout, c, query_idx, nq, s_out, false, "sd_modal_sums_f64");
+}
+
+int sd_modal_sums_f64_dev(sd_ctx *ctx, const double *dX, int64_t n, int64_t F, double c, const int64_t *query_idx,
+                          int64_t nq, double *d_s_out) {
+    return modal_sums_call(ctx, dX, n, F, SD_LAYOUT_NT, c, query_idx, nq, d_s_out, true, "sd_modal_sums_f64_dev");
+}
+
+static int modal_sums_of_call(sd_ctx *ctx, const double *S, i64 nS, const double *Y, i64 nY, i64 F, int layout,
+                              double c, double *s_out, bool dev, const char *who) {
+    SD_REQUIRE(Y || nY == 0, "%s: NULL Y", who);
+    SD_REQUIRE(nS >= 1 && nY >= 0 && F >= 1, "%s: bad sizes nS=%lld nY=%lld F=%lld", who, (long long)nS,
+               (long long)nY, (long long)F);
+    SD_REQUIRE(layout == SD_LAYOUT_TN || layout == SD_LAYOUT_NT, "%s: bad layout %d", who, layout);
+    SD_TRY(check_modal_c(c, who));
+    const double *dS = S, *dY = Y;
+    double *d_s = s_out;
+    return call(ctx, who, S, s_out, !dev, [&](Staging &s) -> int {
+        if (dev) return SD_OK;
+        const double *dP = nullptr;
+        SD_TRY(upload_curves(s, S, nS, Y, nY, F, layout, &dP));
+        dS = dP;
+        dY = dP + nS * F;
+        return s.output(BUF_OUT, s_out, nY, &d_s);
+    }, [&]() -> int {
+        SD_TRY(finite_check_device(ctx, dS, 1, nS * F, nS * F));
+        SD_TRY(finite_check_device(ctx, dY, 1, nY * F, nY * F));
+        return modal_sums_device(ctx, dY, nullptr, nY, dS, nS, F, true, c, d_s);
+    });
+}
+
+int sd_modal_sums_of_f64(sd_ctx *ctx, const double *S, int64_t nS, const double *Y, int64_t nY, int64_t F,
+                         int layout, double c, double *s_out) {
+    return modal_sums_of_call(ctx, S, nS, Y, nY, F, layout, c, s_out, false, "sd_modal_sums_of_f64");
+}
+
+int sd_modal_sums_of_f64_dev(sd_ctx *ctx, const double *dS, int64_t nS, const double *dY, int64_t nY, int64_t F,
+                             double c, double *d_s_out) {
+    return modal_sums_of_call(ctx, dS, nS, dY, nY, F, SD_LAYOUT_NT, c, d_s_out, true, "sd_modal_sums_of_f64_dev");
 }
 
 }  // extern "C"

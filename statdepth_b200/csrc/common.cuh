@@ -73,6 +73,7 @@ enum BufId {
     BUF_PSORT,      // projection depth: sorted rows of Y
     BUF_PRED,       // projection depths: running min / max across direction blocks, per-row med / MAD
     BUF_SPATIAL,    // spatial depth: one row block of weights W [rows][nS] and the per-feature-block partial norms
+    BUF_MODAL,      // h-modal depth: gathered candidate keys of the pair selection, or a row block of sum partials
     NUM_BUFS
 };
 
@@ -230,6 +231,13 @@ int projection_sorted_device(sd_ctx *ctx, const double *d_sorted, i64 nS, i64 T,
 // squared distance overflows
 int spatial_device(sd_ctx *ctx, const double *dQ, const i64 *d_qidx, i64 nq, const double *dS, i64 nS, i64 F,
                    double *d_r);
+// h-modal depth (modal.cu, K15): out[0], out[1] = the k0-th and k1-th smallest (0-based) squared distance over the
+// pairs i < j of the rows dX [n, F] (host memory; synchronises the stream between passes)
+int modal_select_device(sd_ctx *ctx, const double *dX, i64 n, i64 F, i64 k0, i64 k1, double *out);
+// d_out[q] = sum_s exp(c d2) of the rows Q[idx(q) * F] (idx = d_qidx or q) against the sample rows dS [nS, F], plus,
+// with self, the query's own row as column nS (exp(-0) = 1); ST_OVERFLOW when a squared distance overflows
+int modal_sums_device(sd_ctx *ctx, const double *dQ, const i64 *d_qidx, i64 nq, const double *dS, i64 nS, i64 F,
+                      bool self, double c, double *d_out);
 // out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out);

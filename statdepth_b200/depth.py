@@ -19,13 +19,14 @@ from ._outliers import (NO_FACTOR, _check_central, _check_extremal_rows, _checke
 from ._pointcloud import _pointwisedepth, _pointwisedepth_of, _samplepointwisedepth
 from ._projection import KINDS, _functional_projection, _pointcloud_projection, draw_directions
 from ._reference import _checked_reference, _curve_values, _ProjectedReference, _query_values, _SortedReference
+from ._modal import DEFAULT_QUANTILE, _checked_bandwidth, _functional_modal, _functional_modal_of, _ModalReference
 from ._spatial import _functional_spatial, _functional_spatial_of, _spatial_curves, _SpatialReference
 
 __all__ = ['FunctionalDepth', 'PointcloudDepth', 'FunctionalDepthOf', 'PointcloudDepthOf', 'ExtremalDepth',
            'HalfspaceDepth', 'FunctionalHalfspaceDepth', 'ProjectionDepth', 'FunctionalProjectionDepth',
            'FunctionalBoxplot', 'Outliergram', 'FunctionalReference', 'DepthClassifier',
            'FunctionalProjectionDepthOf', 'ProjectionDepthOf', 'FunctionalSpatialDepth', 'FunctionalSpatialDepthOf',
-           'AbstractDepth']
+           'FunctionalModalDepth', 'FunctionalModalDepthOf', 'AbstractDepth']
 
 
 def _go():
@@ -469,13 +470,17 @@ def Outliergram(data: List[pd.DataFrame], factor=1.5, deep_check=False) -> _Outl
 # ---------------------------------------------------------------------------------------------------------------
 # fitted references and depth-based classification (driver in _reference.py)
 # ---------------------------------------------------------------------------------------------------------------
-def _check_reference_depth(depth, J, directions):
-    if not (isinstance(depth, str) and depth in ('mbd', 'spatial') + KINDS):
-        raise ValueError("depth must be 'mbd', 'projection', 'tukey' or 'spatial' (got %r)" % (depth,))
-    if depth in ('mbd', 'spatial') and directions is not None:
+def _check_reference_depth(depth, J, directions, quantile=DEFAULT_QUANTILE, bandwidth=None):
+    if not (isinstance(depth, str) and depth in ('mbd', 'spatial', 'modal') + KINDS):
+        raise ValueError("depth must be 'mbd', 'projection', 'tukey', 'spatial' or 'modal' (got %r)" % (depth,))
+    if depth in ('mbd', 'spatial', 'modal') and directions is not None:
         raise ValueError("directions apply to depth='projection' or 'tukey'")
     if depth != 'mbd' and J != 2:
         raise ValueError('J applies to depth=\'mbd\' only: leave it at 2 for depth=%r' % depth)
+    if depth != 'modal' and (quantile != DEFAULT_QUANTILE or bandwidth is not None):
+        raise ValueError("quantile and bandwidth apply to depth='modal' only")
+    if depth == 'modal':
+        _checked_bandwidth(quantile, bandwidth)
 
 
 class FunctionalReference:
@@ -498,26 +503,37 @@ class FunctionalReference:
     kinds.  The sample's n_S x T d values stay on the GPU for as long as the reference; a new curve g gets the depth
     FunctionalSpatialDepth(sample + [g]) gives it, bit for bit, and each depth_of() call uploads only the new curves.
 
+    depth='modal' (J must stay 2, directions None): the same forms of sample as 'spatial', kept on the GPU the same way.
+    Construction fixes the bandwidth once (.bandwidth): the given bandwidth, else the quantile of the sample's own
+    pair distances.  A new curve g gets the depth FunctionalModalDepth(sample + [g], bandwidth=.bandwidth) gives it,
+    bit for bit.  quantile and bandwidth apply to depth='modal' only; .bandwidth is None for the other kinds.
+
     Non-finite values (and, for the projection kinds, projections that overflow) are rejected.  close() (or leaving a
     `with` block) frees the index."""
 
-    def __init__(self, sample: List[pd.DataFrame], J=2, deep_check=False, depth='mbd', directions=None, seed=0):
-        _check_reference_depth(depth, J, directions)
+    def __init__(self, sample: List[pd.DataFrame], J=2, deep_check=False, depth='mbd', directions=None, seed=0,
+                 quantile=DEFAULT_QUANTILE, bandwidth=None):
+        _check_reference_depth(depth, J, directions, quantile, bandwidth)
         self.J = J
         self.depth = depth
         self.directions = None
+        self.bandwidth = None
         if depth == 'mbd':
             _checked_reference(sample, J, deep_check)
             self._T = sample[0].shape[0]
             self._index = sample[0].index
             self._ref = _SortedReference(_values(sample[0]), J)
             return
-        if depth == 'spatial':
+        if depth in ('spatial', 'modal'):
             X, F = _spatial_curves(sample)
             self._T = sample[0].shape[0]
             self._index = sample[0].index
             self._d = None if F is None else F.shape[2]
-            self._ref = _SpatialReference(X=X, F=F)
+            if depth == 'spatial':
+                self._ref = _SpatialReference(X=X, F=F)
+            else:
+                self._ref = _ModalReference(X=X, F=F, quantile=quantile, bandwidth=bandwidth)
+                self.bandwidth = self._ref.bandwidth
             return
         X, F = _curve_values(sample, directions)
         if X is not None and X.shape[1] == 0:
@@ -531,7 +547,7 @@ class FunctionalReference:
 
     def depth_of(self, data: List[pd.DataFrame], deep_check=False) -> _FunctionalDepthSeries:
         """Depth of every new curve against the reference.  Univariate: the columns of data[0], indexed by
-        data[0].columns (a label may repeat a sample label).  Multivariate (projection kinds, spatial): M DataFrames of
+        data[0].columns (a label may repeat a sample label).  Multivariate (projection kinds, spatial, modal): M DataFrames of
         T x d, indexed by list position, as FunctionalProjectionDepth."""
         if self._ref is None:
             raise ValueError('the reference is closed')
@@ -573,13 +589,16 @@ class DepthClassifier:
     equal FunctionalDepthOf([df], references[label], J=J, relax=True).  depth='projection' or 'tukey': [df] for every
     class, or lists of T x d DataFrames with the same T and d for every class; one set of directions, drawn once from
     d and seed (or given), is shared by all classes (.directions), so that the DD-plot coordinates are comparable.
-    depth='spatial': the same forms of data as the projection kinds, without directions.
+    depth='spatial': the same forms of data as the projection kinds, without directions.  depth='modal': the same forms;
+    each class selects its own bandwidth at quantile from its own pair distances unless bandwidth is given for all
+    (.bandwidths maps each label to the bandwidth in use; None for the other kinds).
     predict(data) takes the class of largest depth, ties going to the class listed first."""
 
-    def __init__(self, references: dict, J=2, deep_check=False, depth='mbd', directions=None, seed=0):
+    def __init__(self, references: dict, J=2, deep_check=False, depth='mbd', directions=None, seed=0,
+                 quantile=DEFAULT_QUANTILE, bandwidth=None):
         if not isinstance(references, dict) or len(references) < 2:
             raise ValueError('references must be a dict of at least two classes.')
-        _check_reference_depth(depth, J, directions)
+        _check_reference_depth(depth, J, directions, quantile, bandwidth)
         for sample in references.values():
             if depth == 'mbd':
                 _checked_reference(sample, J, deep_check)
@@ -601,10 +620,13 @@ class DepthClassifier:
         try:
             for label in self.labels:
                 self._refs.append(FunctionalReference(references[label], J=J, deep_check=deep_check, depth=depth,
-                                                      directions=self.directions))
+                                                      directions=self.directions, quantile=quantile,
+                                                      bandwidth=bandwidth))
         except BaseException:
             self.close()
             raise
+        self.bandwidths = ({label: ref.bandwidth for label, ref in zip(self.labels, self._refs)}
+                           if depth == 'modal' else None)
 
     def depths(self, data: List[pd.DataFrame], deep_check=False) -> pd.DataFrame:
         """Depth of every new curve in every class: one column per class label, rows indexed as
@@ -696,6 +718,45 @@ def FunctionalSpatialDepthOf(data: List[pd.DataFrame],
     data[0].columns) or lists of T x d DataFrames (indexed by list position).  To score many batches against one
     sample, keep a FunctionalReference(sample, depth='spatial'), which keeps the sample on the GPU."""
     depth = _functional_spatial_of(data, sample)
+    if len(sample) == 1:
+        return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+    return _FunctionalDepthSeries(df=data[0], depths=depth)
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# h-modal depth (driver in _modal.py)
+# ---------------------------------------------------------------------------------------------------------------
+def FunctionalModalDepth(data: List[pd.DataFrame], to_compute=None, quantile=DEFAULT_QUANTILE,
+                         bandwidth=None) -> Union[_FunctionalDepthSeries, _FunctionalDepthUnivariate]:
+    """h-modal depth (Cuevas, Febrero & Fraiman 2007; depth.mode in fda.usc) with the Gaussian kernel phi:
+    MD(x) = (1 / n) sum_j phi(||x_j - x|| / h), a curve being the vector of its T d values (Euclidean norm over all
+    values, (t, c) order, no time weight, channels as given) and j running over all n curves, x included, so the
+    depth lies in [phi(0) / n, phi(0)].  A curve is deep when many curves lie close to it as a whole.
+
+    The bandwidth h is np.quantile of the n (n - 1) / 2 pair distances at quantile (0.15 by default; numpy's default
+    'linear' method, bit for bit whenever the squared distances are the same), found exactly on the GPU without
+    storing the pairs; or bandwidth, used as given (finite, > 0; quantile must then stay at its default).  ValueError
+    when the selected h is 0 (at least quantile of the pairs are duplicates: pass bandwidth=) and for one curve
+    without a bandwidth.
+
+    `[df]` (T rows x n curve columns) is the univariate case, to_compute are column labels; a list of N DataFrames
+    (T rows x d channels, any d) the multivariate one, to_compute are list positions.  Non-finite values are
+    rejected, and so (EngineError, SD_ERR_OVERFLOW) are curves whose squared distance overflows float64."""
+    depth = _functional_modal(data, to_compute, quantile, bandwidth)
+    if len(data) == 1:
+        return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+    return _FunctionalDepthSeries(df=data[0], depths=depth)
+
+
+def FunctionalModalDepthOf(data: List[pd.DataFrame], sample: List[pd.DataFrame], quantile=DEFAULT_QUANTILE,
+                           bandwidth=None) -> Union[_FunctionalDepthSeries, _FunctionalDepthUnivariate]:
+    """Out-of-sample h-modal depth: the bandwidth comes from sample alone (its pair distances at quantile, or
+    bandwidth as given) and a new curve never moves it; each new curve g then gets what
+    FunctionalModalDepth(sample + [g], bandwidth=h) gives it (divisor n_S + 1), bit for bit.  Univariate [df] (T x n,
+    indexed by data[0].columns) or lists of T x d DataFrames (indexed by list position).  To score many batches
+    against one sample, keep a FunctionalReference(sample, depth='modal'): it keeps the sample on the GPU and selects
+    the bandwidth once (.bandwidth)."""
+    depth = _functional_modal_of(data, sample, quantile, bandwidth)
     if len(sample) == 1:
         return _FunctionalDepthUnivariate(df=data[0], depths=depth)
     return _FunctionalDepthSeries(df=data[0], depths=depth)
