@@ -320,42 +320,114 @@ int simplicial2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, i64 stride
 //     sum = 1/2 sum_a det(v_a, S_a),   S_a = sum of v_b over that half-turn
 //         = prefix sums W[r] = sum of v_b with rank < r, taken at the rank of a's class end and of its antipode.
 // Ranks come from the same two passes of the K1 pipeline as the triangle counting (exact keys, tolerance 0).
-// One CTA per query: bucket sums by rank (float64 atomics; only tied directions share a bucket), a block-wide
-// exclusive scan, one pass over the points.  The summation order differs from the reference's pair loop:
-// agreement is to ~1e-14 relative at n = 200 (tests: 1e-12).
+//
+// Accuracy.  S_a is a difference of prefix sums of magnitude n |v|, and det(v_a, S_a) cancels when S_a is nearly
+// parallel to v_a -- at every query far from the bulk, with float64 sums an error of n (R / spread) u.  So the sums
+// are exact: every component of v is held in fixed point, c 2^(e-64) with 2^e above the query's largest component
+// (from the pool's bounding box) and c = hi 2^32 + lo, hi in [-2^32, 2^32), lo in [0, 2^32]; the limbs add up in
+// int64 without overflow for n < 2^30.  The only roundings left are c itself (2^(e-65), below the last bit of every
+// component within 2^-11 of the largest), S_a to a pair of doubles (exact), det by fma-compensated products
+// (u |det| + O(u^2) |v_a| |S_a|) and the sum of the non-negative dets (compensated per thread).
+// Determinism.  Integer sums do not depend on their order, and the dets are added in a fixed order: the result
+// is a function of the pool and the query alone (not of the call's other queries, their batch or the run).
 // ---------------------------------------------------------------------------------------------
 constexpr int OJ_THREADS = 512;
 
+// bbox = {min x, max x, min y, max y} of the pool: with them fl(x_j - p) is bounded by the ends of the box
+// (rounding is monotone), the largest component of every query's directions without a pass over the points.
+__global__ void __launch_bounds__(1024) oja2_bbox_kernel(const double *__restrict__ pts, const i64 n,
+                                                         double *__restrict__ bbox) {
+    __shared__ double s[4][32];
+    double lo[2] = {INFINITY, INFINITY}, hi[2] = {-INFINITY, -INFINITY};
+    for (i64 j = threadIdx.x; j < n; j += blockDim.x)
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+            lo[c] = fmin(lo[c], pts[2 * j + c]);
+            hi[c] = fmax(hi[c], pts[2 * j + c]);
+        }
+#pragma unroll
+    for (int s2 = 16; s2 > 0; s2 >>= 1)
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+            lo[c] = fmin(lo[c], __shfl_xor_sync(0xffffffffu, lo[c], s2));
+            hi[c] = fmax(hi[c], __shfl_xor_sync(0xffffffffu, hi[c], s2));
+        }
+    const int w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    if ((threadIdx.x & 31) == 0) { s[0][w] = lo[0]; s[1][w] = hi[0]; s[2][w] = lo[1]; s[3][w] = hi[1]; }
+    __syncthreads();
+    if (threadIdx.x < 4) {
+        double r = s[threadIdx.x][0];
+        for (int k = 1; k < nw; ++k) r = threadIdx.x & 1 ? fmax(r, s[threadIdx.x][k]) : fmin(r, s[threadIdx.x][k]);
+        bbox[threadIdx.x] = r;
+    }
+}
+
+// v * 2^(64 - e) = hi 2^32 + lo (lo rounded to nearest), scale = 2^(32 - e), |v| < 2^e
+__device__ __forceinline__ void oj_limbs(const double v, const double scale, u64 &hi, u64 &lo) {
+    const double t = v * scale;  // exact: a power of two, |t| < 2^32
+    const double f = floor(t);
+    hi = (u64)(i64)f;
+    lo = (u64)__double2ll_rn((t - f) * 4294967296.0);  // t - f in [0, 1) is exact
+}
+
+// the fixed-point value of limb sums (hi, lo) (two's complement, |value| < 2^93) as s + t exactly, times unit
+__device__ __forceinline__ void oj_to_dd(const u64 hi, const u64 lo, const double unit, double &s, double &t) {
+    const i64 h = (i64)(hi + (lo >> 32));
+    const double hd = (double)h;                                       // |h - hd| <= 2^9
+    const double a = hd * 4294967296.0;                                // exact
+    const double b = (double)((h - (i64)hd) * 4294967296ll + (i64)(lo & 0xffffffffull));  // |.| < 2^42: exact
+    s = a + b;                                                         // two-sum: s + t == a + b
+    const double bb = s - a;
+    t = (a - (s - bb)) + (b - bb);
+    s *= unit;
+    t *= unit;
+}
+
+// W[r] = {hi x, lo x, hi y, lo y} limb sums: exclusive prefix over ranks after pass 2
+struct OjW { u64 hx, lx, hy, ly; };
+__device__ __forceinline__ OjW oj_load(const u64 *w, const i64 r) {
+    const ulonglong2 a = reinterpret_cast<const ulonglong2 *>(w + 4 * r)[0];
+    const ulonglong2 b = reinterpret_cast<const ulonglong2 *>(w + 4 * r)[1];
+    return OjW{a.x, a.y, b.x, b.y};
+}
+
 __global__ void __launch_bounds__(OJ_THREADS) oja2_reduce_kernel(const ScGeom g, const i64 n, const double *__restrict__ KA,
                                                                  const int *__restrict__ bA, const int *__restrict__ aA,
-                                                                 const int *__restrict__ bB, double *__restrict__ bucket,
+                                                                 const int *__restrict__ bB, u64 *__restrict__ bucket,
+                                                                 const double *__restrict__ bbox,
                                                                  const double hull_volume, double *__restrict__ out) {
-    __shared__ double s_part[2][OJ_THREADS];
+    __shared__ u64 s_part[4][OJ_THREADS];
     __shared__ double s_red[OJ_THREADS / 32];
     __shared__ i64 s_cnt[2];
-    __shared__ double s_tot[2];
     const i64 li = blockIdx.x;
     const i64 inst = g.inst0 + li;
     const i64 q = sc_query(g, inst);
     const double px = g.pts[q * g.stride_j], py = g.pts[q * g.stride_j + 1];
     const double *ka = KA + li * n;
     const int *ba = bA + li * n, *aa = aA + li * n, *bb = bB + li * 2 * n;
-    double *bx = bucket + li * 2 * (n + 1), *by = bx + (n + 1);
+    u64 *W = bucket + li * 4 * (n + 1);
     const int tid = threadIdx.x;
-    for (i64 r = tid; r < 2 * (n + 1); r += OJ_THREADS) bx[r] = 0.0;
-    if (tid == 0) { s_cnt[0] = 0; s_cnt[1] = 0; s_tot[0] = 0.0; s_tot[1] = 0.0; }
+    // the fixed-point scale of this query: 2^e > every |component| of its directions
+    const double M = fmax(fmax(fabs(bbox[0] - px), fabs(bbox[1] - px)), fmax(fabs(bbox[2] - py), fabs(bbox[3] - py)));
+    int e;
+    frexp(M, &e);  // M < 2^e (M == 0: every direction is zero, e = 0)
+    const double scale = ldexp(1.0, 32 - e), unit = ldexp(1.0, e - 64);
+    for (i64 r = tid; r < 2 * (n + 1); r += OJ_THREADS) reinterpret_cast<ulonglong2 *>(W)[r] = make_ulonglong2(0, 0);
+    if (tid == 0) { s_cnt[0] = 0; s_cnt[1] = 0; }
     __syncthreads();
-    // pass 1: bucket sums by rank, totals, #real directions and #directions in [0, pi)
+    // pass 1: limb sums by rank, #real directions and #directions in [0, pi)
     i64 real = 0, low = 0;
-    double tx = 0.0, ty = 0.0;
     for (i64 j = tid; j < n; j += OJ_THREADS) {
         const double u = ka[j];
         if (!(u < 16.0)) continue;
-        const double vx = g.pts[j * g.stride_j] - px, vy = g.pts[j * g.stride_j + 1] - py;
-        atomicAdd(&bx[ba[j]], vx);
-        atomicAdd(&by[ba[j]], vy);
-        tx += vx;
-        ty += vy;
+        u64 hx, lx, hy, ly;
+        oj_limbs(g.pts[j * g.stride_j] - px, scale, hx, lx);
+        oj_limbs(g.pts[j * g.stride_j + 1] - py, scale, hy, ly);
+        u64 *w = W + 4 * (i64)ba[j];
+        atomicAdd(w, hx);
+        atomicAdd(w + 1, lx);
+        atomicAdd(w + 2, hy);
+        atomicAdd(w + 3, ly);
         ++real;
         low += u < 12.0;
     }
@@ -363,69 +435,76 @@ __global__ void __launch_bounds__(OJ_THREADS) oja2_reduce_kernel(const ScGeom g,
     for (int s = 16; s > 0; s >>= 1) {
         real += __shfl_xor_sync(0xffffffffu, real, s);
         low += __shfl_xor_sync(0xffffffffu, low, s);
-        tx += __shfl_xor_sync(0xffffffffu, tx, s);
-        ty += __shfl_xor_sync(0xffffffffu, ty, s);
     }
     if ((tid & 31) == 0) {
         atomicAdd((u64 *)&s_cnt[0], (u64)real);
         atomicAdd((u64 *)&s_cnt[1], (u64)low);
-        atomicAdd(&s_tot[0], tx);
-        atomicAdd(&s_tot[1], ty);
     }
     __syncthreads();
-    // pass 2: exclusive scan of the buckets in place: W[r] = sum of v_b with rank < r   (r = 0 .. n)
+    // pass 2: exclusive scan of the limb sums in place: W[r] = sum of v_b with rank < r   (r = 0 .. n; W[n] = total)
     const i64 len = n + 1, chunk = (len + OJ_THREADS - 1) / OJ_THREADS;
     const i64 c0 = tid * chunk, c1 = c0 + chunk < len ? c0 + chunk : len;
-    double sx = 0.0, sy = 0.0;
-    for (i64 r = c0; r < c1; ++r) { sx += bx[r]; sy += by[r]; }
-    s_part[0][tid] = sx;
-    s_part[1][tid] = sy;
-    __syncthreads();
-    if (tid < 2) {  // 512 partial sums per coordinate: a serial scan by one thread each is negligible
-        double run = 0.0;
-        for (int k = 0; k < OJ_THREADS; ++k) { const double v = s_part[tid][k]; s_part[tid][k] = run; run += v; }
-    }
-    __syncthreads();
-    sx = s_part[0][tid];
-    sy = s_part[1][tid];
+    u64 acc4[4] = {0, 0, 0, 0};
     for (i64 r = c0; r < c1; ++r) {
-        const double vx = bx[r], vy = by[r];
-        bx[r] = sx;
-        by[r] = sy;
-        sx += vx;
-        sy += vy;
+        const OjW v = oj_load(W, r);
+        acc4[0] += v.hx; acc4[1] += v.lx; acc4[2] += v.hy; acc4[3] += v.ly;
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) s_part[k][tid] = acc4[k];
+    __syncthreads();
+    if (tid < 4) {  // 512 partial sums per limb: a serial scan by one thread each is negligible
+        u64 run = 0;
+        for (int k = 0; k < OJ_THREADS; ++k) { const u64 v = s_part[tid][k]; s_part[tid][k] = run; run += v; }
     }
     __syncthreads();
-    // pass 3
+#pragma unroll
+    for (int k = 0; k < 4; ++k) acc4[k] = s_part[k][tid];
+    for (i64 r = c0; r < c1; ++r) {
+        const OjW v = oj_load(W, r);
+        reinterpret_cast<ulonglong2 *>(W + 4 * r)[0] = make_ulonglong2(acc4[0], acc4[1]);
+        reinterpret_cast<ulonglong2 *>(W + 4 * r)[1] = make_ulonglong2(acc4[2], acc4[3]);
+        acc4[0] += v.hx; acc4[1] += v.lx; acc4[2] += v.hy; acc4[3] += v.ly;
+    }
+    __syncthreads();
+    // pass 3: det(v_a, S_a) from the exact half-turn sums
     const i64 mreal = s_cnt[0], L4 = s_cnt[1], H = mreal - L4;
-    const double totx = s_tot[0], toty = s_tot[1];
-    double acc = 0.0;
+    const OjW tot = oj_load(W, n);
+    double acc = 0.0, comp = 0.0;
     for (i64 j = tid; j < n; j += OJ_THREADS) {
         const double u = ka[j];
         if (!(u < 16.0)) continue;
         const double vx = g.pts[j * g.stride_j] - px, vy = g.pts[j * g.stride_j + 1] - py;
         const i64 L = ba[j], R = n - (i64)aa[j];  // ranks [L, R) hold the class of j
         const i64 b2w = bb[n + j];
-        double hx, hy;
+        const OjW wr = oj_load(W, R);
+        OjW S;
         if (u < 12.0) {
-            const i64 Lw = b2w - L - H;           // real directions strictly before the antipode
-            hx = bx[Lw] - bx[R];
-            hy = by[Lw] - by[R];
+            const OjW ww = oj_load(W, b2w - L - H);  // real directions strictly before the antipode
+            S = OjW{ww.hx - wr.hx, ww.lx - wr.lx, ww.hy - wr.hy, ww.ly - wr.ly};
         } else {
-            const i64 Lw = b2w - L + L4;
-            hx = (totx - bx[R]) + bx[Lw];
-            hy = (toty - by[R]) + by[Lw];
+            const OjW ww = oj_load(W, b2w - L + L4);
+            S = OjW{tot.hx - wr.hx + ww.hx, tot.lx - wr.lx + ww.lx, tot.hy - wr.hy + ww.hy, tot.ly - wr.ly + ww.ly};
         }
-        acc += vx * hy - vy * hx;
+        double sx, tx, sy, ty;
+        oj_to_dd(S.hx, S.lx, unit, sx, tx);
+        oj_to_dd(S.hy, S.ly, unit, sy, ty);
+        const double p1 = vx * sy, e1 = fma(vx, sy, -p1);
+        const double p2 = vy * sx, e2 = fma(vy, sx, -p2);
+        const double d = (p1 - p2) + ((e1 - e2) + (vx * ty - vy * tx));
+        const double t = acc + d;  // two-sum
+        const double z = t - acc;
+        comp += (acc - (t - z)) + (d - z);
+        acc = t;
     }
+    acc += comp;
 #pragma unroll
     for (int s = 16; s > 0; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
     if ((tid & 31) == 0) s_red[tid >> 5] = acc;
     __syncthreads();
     if (tid == 0) {
-        double tot = 0.0;
-        for (int w = 0; w < OJ_THREADS / 32; ++w) tot += s_red[w];
-        out[inst] = 0.5 * tot / hull_volume;
+        double sum = 0.0;
+        for (int w = 0; w < OJ_THREADS / 32; ++w) sum += s_red[w];
+        out[inst] = 0.5 * sum / hull_volume;
     }
 }
 
@@ -442,15 +521,17 @@ int oja2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, const i64 *d_q, i
         set_error("oja counting: n=%lld too large", (long long)n);
         return SD_ERR_UNSUPPORTED;
     }
-    i64 IB = (i64)((3ull << 30) / (size_t)(72 * n));
+    // batch size: ~88 n bytes of keys, limb sums and ranks per query (+ the rank pipeline's part lists)
+    i64 IB = (i64)((3ull << 30) / (size_t)(88 * n));
     if (IB < 1) IB = 1;
     if (IB > 32768) IB = 32768;
     if (IB > nq) IB = nq;
-    SD_TRY(ctx->buf[BUF_IN2].reserve((size_t)IB * (3 * n + 2 * (n + 1)) * sizeof(double)));
+    SD_TRY(ctx->buf[BUF_IN2].reserve((size_t)IB * (3 * n + 4 * (n + 1)) * sizeof(double) + 4 * sizeof(double)));
     SD_TRY(ctx->buf[BUF_MASK].reserve((size_t)IB * n * 4 * sizeof(int)));
-    double *KA = ctx->buf[BUF_IN2].as<double>();
+    u64 *bucket = ctx->buf[BUF_IN2].as<u64>();  // first: 16-byte loads and stores, 32 (n + 1) bytes per query
+    double *KA = reinterpret_cast<double *>(bucket + (size_t)IB * 4 * (n + 1));
     double *KB = KA + (size_t)IB * n;
-    double *bucket = KB + (size_t)IB * 2 * n;
+    double *bbox = KB + (size_t)IB * 2 * n;
     int *bA = ctx->buf[BUF_MASK].as<int>();
     int *aA = bA + (size_t)IB * n;
     int *bB = aA + (size_t)IB * n;
@@ -459,6 +540,8 @@ int oja2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, const i64 *d_q, i
     g.stride_j = 2;
     g.qidx = d_q;
     g.T = 1;
+    oja2_bbox_kernel<<<1, 1024, 0, st>>>(d_pts, n, bbox);
+    ctx->last.launches++;
     for (i64 i0 = 0; i0 < nq; i0 += IB) {
         const i64 ni = nq - i0 < IB ? nq - i0 : IB;
         g.inst0 = i0;
@@ -468,7 +551,7 @@ int oja2_count_device(sd_ctx *ctx, const double *d_pts, i64 n, const i64 *d_q, i
         ctx->last.launches++;
         SD_TRY(rank_rows_device(ctx, KA, ni, n, n, bA, aA));
         SD_TRY(rank_rows_device(ctx, KB, ni, 2 * n, 2 * n, bB, nullptr));
-        oja2_reduce_kernel<<<(unsigned)ni, OJ_THREADS, 0, st>>>(g, n, KA, bA, aA, bB, bucket, hull_volume, d_out);
+        oja2_reduce_kernel<<<(unsigned)ni, OJ_THREADS, 0, st>>>(g, n, KA, bA, aA, bB, bucket, bbox, hull_volume, d_out);
         ctx->last.launches++;
         SD_CUDA(cudaGetLastError());
     }

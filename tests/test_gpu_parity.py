@@ -970,6 +970,6 @@ def test_counting_randomized_differential(engine, oracle, seed):
         engine.set_option(E.OPT_SIMPLICIAL_IMPL, E.SIMPLICIAL_COUNT)
         L = rng.integers(0, 7, size=(n, 2)).astype(np.float64)
         assert (engine.simplicial_counts(L, q, 0.0) == oracle.simplicial_counts(L, q, 0.0)).all()  # exact keys
-        np.testing.assert_allclose(engine.oja(P, 3.0, q), oracle.oja(P, 3.0, q), rtol=1e-10, atol=1e-12)
+        np.testing.assert_allclose(engine.oja(P, 3.0, q), oracle.oja(P, 3.0, q), rtol=RTOL, atol=1e-12)
     finally:
         engine.set_option(E.OPT_SIMPLICIAL_IMPL, E.SIMPLICIAL_AUTO)
