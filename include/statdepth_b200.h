@@ -464,6 +464,34 @@ int sd_modal_sums_of_f64_dev(sd_ctx *ctx, const double *dS, int64_t nS, const do
                              double c, double *d_s_out);
 
 /*
+ * Kernelized functional spatial depth (KFSD, Sguera, Galeano & Lillo 2014): spatial depth after the feature map of the
+ * Gaussian kernel k(x, y) = exp(c d2(x, y)), c = -1 / sigma^2 (finite and < 0).  Curves and d2 as for the h-modal
+ * entry points.  With e = -expm1(c d2) = 1 - k and w_qj = 1 / sqrt(2 e_qj) (0 where e_qj = 0: duplicates of x_q, x_q
+ * itself in sample), r_out[q] = sqrt(max(2 A B - Q, 0)), A = sum_j w_qj, B = sum_j w_qj e_qj, Q = w_q^T E w_q, E the
+ * sample's matrix of e_ij: r is the norm of the sum of the feature-space unit vectors.  The depth is 1 - r / n_pop with
+ * n_pop = n in sample and nS + 1 out of sample; the host forms it, and picks sigma.
+ * Gram: dE_out [n][n] (DEVICE, caller-owned, 8 n^2 bytes) = e of the rows dX [n, F]; symmetric bit for bit, zero
+ * diagonal.  Norms: in sample (query_idx HOST memory, all when NULL; E built in the context's workspace) and out of
+ * sample (one-shot from host curves, or DEVICE rows dS with their E from the gram call).  A query's bits depend on its
+ * row, the sample and the tile sizes alone; out of sample r_out[g] equals the in-sample r of S + [g] at entry nS.
+ * SD_ERR_UNSUPPORTED when n (in sample) or nS (out of sample) exceeds SD_KFSD_N_MAX (E would pass 8 GiB);
+ * SD_ERR_NONFINITE when an input holds NaN or +-inf, SD_ERR_OVERFLOW when a squared distance overflows.
+ */
+#define SD_KFSD_N_MAX 32768
+int sd_kfsd_gram_f64_dev(sd_ctx *ctx, const double *dX, int64_t n, int64_t F, double c, double *dE_out);
+int sd_kfsd_norms_f64(sd_ctx *ctx, const double *X, int64_t n, int64_t F, int layout, double c,
+                      const int64_t *query_idx, int64_t nq, double *r_out);
+/* same with DEVICE rows dX [n, F] and DEVICE output d_r_out [nq] */
+int sd_kfsd_norms_f64_dev(sd_ctx *ctx, const double *dX, int64_t n, int64_t F, double c, const int64_t *query_idx,
+                          int64_t nq, double *d_r_out);
+/* new curves Y [nY] against the sample S [nS] (same layout, each dense); E is built and dropped within the call */
+int sd_kfsd_norms_of_f64(sd_ctx *ctx, const double *S, int64_t nS, const double *Y, int64_t nY, int64_t F,
+                         int layout, double c, double *r_out);
+/* DEVICE pointers, curves as rows (dS [nS, F], dY [nY, F]), dE [nS][nS] from sd_kfsd_gram_f64_dev with the same c */
+int sd_kfsd_norms_of_f64_dev(sd_ctx *ctx, const double *dS, int64_t nS, const double *dE, const double *dY,
+                             int64_t nY, int64_t F, double c, double *d_r_out);
+
+/*
  * Batched band depth over sub-populations of one matrix (K-sampled blocks, homogeneity
  * permutations): membership[b*n + c] != 0 selects the curves of batch b; queries[b*nqb + i] is
  * the i-th query curve of batch b (must be a member).  count_out[b*nqb + i] as in

@@ -10,6 +10,7 @@
     from statdepth_b200 import FunctionalProjectionDepthOf, ProjectionDepthOf  # projection depths of new data
     from statdepth_b200 import FunctionalSpatialDepth, FunctionalSpatialDepthOf  # L2 spatial depth of curves
     from statdepth_b200 import FunctionalModalDepth, FunctionalModalDepthOf  # h-modal (kernel) depth of curves
+    from statdepth_b200 import FunctionalKernelSpatialDepth, FunctionalKernelSpatialDepthOf  # KFSD of curves
     from statdepth_b200.homogeneity import FunctionalHomogeneity     # == statdepth.homogeneity
     from statdepth_b200.testing import generate_noisy_univariate     # == statdepth.testing
 
@@ -22,7 +23,8 @@ from ._dist import enable_distributed
 from ._engine import Engine, EngineError, EngineUnavailable, get_engine
 from ._helper import DepthDegeneracy
 from .depth import (DepthClassifier, ExtremalDepth, FunctionalBoxplot, FunctionalDepth, FunctionalDepthOf,
-                    FunctionalHalfspaceDepth, FunctionalProjectionDepth, FunctionalProjectionDepthOf,
+                    FunctionalHalfspaceDepth, FunctionalKernelSpatialDepth, FunctionalKernelSpatialDepthOf,
+                    FunctionalProjectionDepth, FunctionalProjectionDepthOf,
                     FunctionalModalDepth, FunctionalModalDepthOf, FunctionalReference, FunctionalSpatialDepth,
                     FunctionalSpatialDepthOf, HalfspaceDepth, Outliergram, PointcloudDepth, PointcloudDepthOf,
                     ProjectionDepth, ProjectionDepthOf)
@@ -30,5 +32,5 @@ from .settings import get_simplex_tolerance, set_simplex_tolerance
 
 __version__ = "0.1.0"
 __all__ = ["FunctionalDepth", "PointcloudDepth", "FunctionalDepthOf", "PointcloudDepthOf", "FunctionalBoxplot",
-           "Outliergram", "ExtremalDepth", "HalfspaceDepth", "FunctionalHalfspaceDepth", "ProjectionDepth", "FunctionalProjectionDepth", "FunctionalReference", "DepthClassifier", "FunctionalProjectionDepthOf", "ProjectionDepthOf", "FunctionalSpatialDepth", "FunctionalSpatialDepthOf", "FunctionalModalDepth", "FunctionalModalDepthOf", "DepthDegeneracy", "Engine", "EngineError", "EngineUnavailable",
+           "Outliergram", "ExtremalDepth", "HalfspaceDepth", "FunctionalHalfspaceDepth", "ProjectionDepth", "FunctionalProjectionDepth", "FunctionalReference", "DepthClassifier", "FunctionalProjectionDepthOf", "ProjectionDepthOf", "FunctionalSpatialDepth", "FunctionalSpatialDepthOf", "FunctionalModalDepth", "FunctionalModalDepthOf", "FunctionalKernelSpatialDepth", "FunctionalKernelSpatialDepthOf", "DepthDegeneracy", "Engine", "EngineError", "EngineUnavailable",
            "get_engine", "get_simplex_tolerance", "set_simplex_tolerance", "enable_distributed"]

@@ -147,6 +147,15 @@ SIGNATURES = {
                                        C.c_double, C.c_void_p]),
     "sd_modal_sums_of_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64,
                                            C.c_double, C.c_void_p]),
+    "sd_kfsd_gram_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_double, C.c_void_p]),
+    "sd_kfsd_norms_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_double, C.c_void_p,
+                                    C.c_int64, C.c_void_p]),
+    "sd_kfsd_norms_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_double, C.c_void_p,
+                                        C.c_int64, C.c_void_p]),
+    "sd_kfsd_norms_of_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int,
+                                       C.c_double, C.c_void_p]),
+    "sd_kfsd_norms_of_f64_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
+                                           C.c_int64, C.c_double, C.c_void_p]),
     "sd_band_depth_batched_f64": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p,
                                             C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p]),
 }
@@ -794,6 +803,69 @@ class Engine:
         """Device-pointer variant (curves as rows: S [nS, F], Y [nY, F]); S [nY] stays on the device."""
         self._check(self.lib.sd_modal_sums_of_f64_dev(self._ctx, _dptr(dS_ptr), int(nS), _dptr(dY_ptr), int(nY),
                                                       int(F), float(c), _dptr(d_out_ptr)))
+
+    # -- kernelized functional spatial depth -------------------------------------------------------------------
+    def kfsd_gram(self, S, c):
+        """E [n, n] = -expm1(c d2(x_i, x_j)) of the curves S [n, F] (rows; host, or from upload()), as a device tensor
+        on the engine's stream."""
+        if not _on_device(S):
+            S = self.upload(self._curves(S)[0])
+        n, F = S.shape
+        return self._staged(lambda e: self.kfsd_gram_dev(S.data_ptr(), n, F, c, e), ((n, n), np.float64),
+                            host=False)[0]
+
+    def kfsd_gram_dev(self, dS_ptr, n, F, c, dE_ptr):
+        """Device-pointer variant (curves as rows dS [n, F]; dE [n, n] caller-owned)."""
+        self._check(self.lib.sd_kfsd_gram_f64_dev(self._ctx, _dptr(dS_ptr), int(n), int(F), float(c), _dptr(dE_ptr)))
+
+    def kfsd_norms(self, X, c, queries=None):
+        """r [nq] = || sum_j (phi(x_q) - phi(x_j)) / ||.|| || over the curves X [n, F] (rows; host, or from upload()),
+        duplicates of x_q contributing 0, for the queries (all when None); KFSD is 1 - r / n."""
+        if _on_device(X):
+            n, F = X.shape
+            q, nq = self._queries(queries, n)
+            return self._staged(lambda out: self.kfsd_norms_dev(X.data_ptr(), n, F, c, q, out), ((nq,), np.float64))[0]
+        X, layout = self._curves(X)
+        n, F = X.shape
+        q, nq = self._queries(queries, n)
+        out = np.empty(nq, dtype=np.float64)
+        self._check(self.lib.sd_kfsd_norms_f64(self._ctx, _ptr(X), n, F, layout, float(c), _ptr(q), nq, _ptr(out)))
+        return out
+
+    def kfsd_norms_dev(self, dX_ptr, n, F, c, queries, d_out_ptr):
+        """Device-pointer variant (curves as rows dX [n, F]; queries a host index array or None); r stays on the
+        device."""
+        q, nq = self._queries(queries, n)
+        self._check(self.lib.sd_kfsd_norms_f64_dev(self._ctx, _dptr(dX_ptr), int(n), int(F), float(c), _ptr(q), nq,
+                                                   _dptr(d_out_ptr)))
+
+    def kfsd_norms_of(self, S, E, Y, c):
+        """r [nY] of the new curves Y [nY, F] against the sample S [nS, F]; KFSD is 1 - r / (nS + 1).  With E None, S
+        is a host array and E is built and dropped within the call; else S comes from upload() and E from
+        kfsd_gram(S, c)."""
+        on_device = E is not None
+        if not on_device:
+            S, ls = self._curves(S)
+        Y = np.asarray(Y, dtype=np.float64)
+        if Y.ndim != 2 or S.shape[1] != Y.shape[1]:
+            raise ValueError("S and Y must have the same number of values per curve")
+        (nS, F), nY = S.shape, Y.shape[0]
+        if nY == 0:
+            return np.empty(0, dtype=np.float64)
+        if on_device:
+            dY = self.upload(Y)
+            return self._staged(lambda r: self.kfsd_norms_of_dev(S.data_ptr(), nS, E.data_ptr(), dY.data_ptr(), nY, F,
+                                                                 c, r), ((nY,), np.float64))[0]
+        Y = np.asfortranarray(Y) if ls == LAYOUT_TN else np.ascontiguousarray(Y)  # in S's layout
+        out = np.empty(nY, dtype=np.float64)
+        self._check(self.lib.sd_kfsd_norms_of_f64(self._ctx, _ptr(S), nS, _ptr(Y), nY, F, ls, float(c), _ptr(out)))
+        return out
+
+    def kfsd_norms_of_dev(self, dS_ptr, nS, dE_ptr, dY_ptr, nY, F, c, d_out_ptr):
+        """Device-pointer variant (curves as rows: S [nS, F], Y [nY, F]; E [nS, nS] from kfsd_gram); r [nY] stays on
+        the device."""
+        self._check(self.lib.sd_kfsd_norms_of_f64_dev(self._ctx, _dptr(dS_ptr), int(nS), _dptr(dE_ptr), _dptr(dY_ptr),
+                                                      int(nY), int(F), float(c), _dptr(d_out_ptr)))
 
     def simplicial_oos_counts(self, S, Y, tol=1e-7):
         S = np.ascontiguousarray(S, dtype=np.float64)

@@ -40,6 +40,7 @@ SOURCES = {
     "simplicial_count.cu": ["-fmad=false"],
     "spatial.cu": [],
     "modal.cu": [],
+    "kfsd.cu": [],
 }
 EXPORT_MAP = os.path.join(CSRC, "exports.map")
 

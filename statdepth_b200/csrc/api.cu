@@ -1252,4 +1252,93 @@ int sd_modal_sums_of_f64_dev(sd_ctx *ctx, const double *dS, int64_t nS, const do
     return modal_sums_of_call(ctx, dS, nS, dY, nY, F, SD_LAYOUT_NT, c, d_s_out, true, "sd_modal_sums_of_f64_dev");
 }
 
+// ---------------------------------------------------------------------------------------------
+// kernelized functional spatial depth (K16, kfsd.cu)
+// ---------------------------------------------------------------------------------------------
+static int check_kfsd(i64 n, double c, const char *who) {
+    SD_REQUIRE(c < 0.0 && c >= -DBL_MAX, "%s: c=%g must be finite and < 0 (c = -1 / sigma^2)", who, c);
+    if (n > SD_KFSD_N_MAX) {
+        set_error("%s: %lld sample curves exceed SD_KFSD_N_MAX = %d (E holds n^2 doubles)", who, (long long)n,
+                  SD_KFSD_N_MAX);
+        return SD_ERR_UNSUPPORTED;
+    }
+    return SD_OK;
+}
+
+int sd_kfsd_gram_f64_dev(sd_ctx *ctx, const double *dX, int64_t n, int64_t F, double c, double *dE_out) {
+    const char *who = "sd_kfsd_gram_f64_dev";
+    SD_REQUIRE(n >= 1 && F >= 1, "%s: bad sizes n=%lld F=%lld", who, (long long)n, (long long)F);
+    SD_TRY(check_kfsd(n, c, who));
+    return call(ctx, who, dX, dE_out, false, no_stage, [&]() -> int {
+        SD_TRY(finite_check_device(ctx, dX, 1, n * F, n * F));
+        return kfsd_gram_device(ctx, dX, n, F, c, dE_out);
+    });
+}
+
+static int kfsd_norms_call(sd_ctx *ctx, const double *X, i64 n, i64 F, int layout, double c, const int64_t *query_idx,
+                           i64 nq, double *r_out, bool dev, const char *who) {
+    SD_REQUIRE(n >= 1 && F >= 1 && nq >= 0, "%s: bad sizes n=%lld F=%lld nq=%lld", who, (long long)n, (long long)F,
+               (long long)nq);
+    SD_REQUIRE(layout == SD_LAYOUT_TN || layout == SD_LAYOUT_NT, "%s: bad layout %d", who, layout);
+    SD_REQUIRE(query_idx || nq == n, "%s: query_idx == NULL requires nq == n", who);
+    SD_TRY(check_kfsd(n, c, who));
+    const double *dX = X;
+    const i64 *d_q = nullptr;
+    double *d_r = r_out;
+    return call(ctx, who, X, r_out, !dev, [&](Staging &s) -> int {
+        if (!dev) SD_TRY(upload_curves(s, X, n, nullptr, 0, F, layout, &dX));
+        SD_TRY(upload_queries(ctx, query_idx, nq, n, &d_q, who));
+        return dev ? SD_OK : s.output(BUF_OUT, r_out, nq, &d_r);
+    }, [&]() -> int {
+        SD_TRY(finite_check_device(ctx, dX, 1, n * F, n * F));
+        return kfsd_device(ctx, dX, d_q, nq, dX, n, F, c, nullptr, d_r);
+    });
+}
+
+int sd_kfsd_norms_f64(sd_ctx *ctx, const double *X, int64_t n, int64_t F, int layout, double c,
+                      const int64_t *query_idx, int64_t nq, double *r_out) {
+    return kfsd_norms_call(ctx, X, n, F, layout, c, query_idx, nq, r_out, false, "sd_kfsd_norms_f64");
+}
+
+int sd_kfsd_norms_f64_dev(sd_ctx *ctx, const double *dX, int64_t n, int64_t F, double c, const int64_t *query_idx,
+                          int64_t nq, double *d_r_out) {
+    return kfsd_norms_call(ctx, dX, n, F, SD_LAYOUT_NT, c, query_idx, nq, d_r_out, true, "sd_kfsd_norms_f64_dev");
+}
+
+// dE == nullptr: the one-shot host call, which builds E in the workspace
+static int kfsd_norms_of_call(sd_ctx *ctx, const double *S, i64 nS, const double *dE, const double *Y, i64 nY, i64 F,
+                              int layout, double c, double *r_out, bool dev, const char *who) {
+    SD_REQUIRE(Y || nY == 0, "%s: NULL Y", who);
+    SD_REQUIRE(!dev || dE, "%s: NULL E", who);
+    SD_REQUIRE(nS >= 1 && nY >= 0 && F >= 1, "%s: bad sizes nS=%lld nY=%lld F=%lld", who, (long long)nS,
+               (long long)nY, (long long)F);
+    SD_REQUIRE(layout == SD_LAYOUT_TN || layout == SD_LAYOUT_NT, "%s: bad layout %d", who, layout);
+    SD_TRY(check_kfsd(nS, c, who));
+    const double *dS = S, *dY = Y;
+    double *d_r = r_out;
+    return call(ctx, who, S, r_out, !dev, [&](Staging &s) -> int {
+        if (dev) return SD_OK;
+        const double *dP = nullptr;
+        SD_TRY(upload_curves(s, S, nS, Y, nY, F, layout, &dP));
+        dS = dP;
+        dY = dP + nS * F;
+        return s.output(BUF_OUT, r_out, nY, &d_r);
+    }, [&]() -> int {
+        SD_TRY(finite_check_device(ctx, dS, 1, nS * F, nS * F));
+        SD_TRY(finite_check_device(ctx, dY, 1, nY * F, nY * F));
+        return kfsd_device(ctx, dY, nullptr, nY, dS, nS, F, c, dE, d_r);
+    });
+}
+
+int sd_kfsd_norms_of_f64(sd_ctx *ctx, const double *S, int64_t nS, const double *Y, int64_t nY, int64_t F,
+                         int layout, double c, double *r_out) {
+    return kfsd_norms_of_call(ctx, S, nS, nullptr, Y, nY, F, layout, c, r_out, false, "sd_kfsd_norms_of_f64");
+}
+
+int sd_kfsd_norms_of_f64_dev(sd_ctx *ctx, const double *dS, int64_t nS, const double *dE, const double *dY,
+                             int64_t nY, int64_t F, double c, double *d_r_out) {
+    return kfsd_norms_of_call(ctx, dS, nS, dE, dY, nY, F, SD_LAYOUT_NT, c, d_r_out, true,
+                              "sd_kfsd_norms_of_f64_dev");
+}
+
 }  // extern "C"

@@ -74,6 +74,7 @@ enum BufId {
     BUF_PRED,       // projection depths: running min / max across direction blocks, per-row med / MAD
     BUF_SPATIAL,    // spatial depth: one row block of weights W [rows][nS] and the per-feature-block partial norms
     BUF_MODAL,      // h-modal depth: gathered candidate keys of the pair selection, or a row block of sum partials
+    BUF_KFSD,       // KFSD: the sample's E [nS][nS] (in-sample and one-shot calls), one row block of W and its partials
     NUM_BUFS
 };
 
@@ -238,6 +239,12 @@ int modal_select_device(sd_ctx *ctx, const double *dX, i64 n, i64 F, i64 k0, i64
 // with self, the query's own row as column nS (exp(-0) = 1); ST_OVERFLOW when a squared distance overflows
 int modal_sums_device(sd_ctx *ctx, const double *dQ, const i64 *d_qidx, i64 nq, const double *dS, i64 nS, i64 F,
                       bool self, double c, double *d_out);
+// kernelized functional spatial depth (kfsd.cu, K16): dE [n][n] = -expm1(c d2) of the rows dX [n, F]; d_r[q] =
+// sqrt(max(2 A B - Q, 0)) of the rows Q[idx(q) * F] (idx = d_qidx or q) against the sample rows dS [nS, F] and their E
+// (dE; nullptr: built into BUF_KFSD); ST_OVERFLOW when a squared distance overflows
+int kfsd_gram_device(sd_ctx *ctx, const double *dX, i64 n, i64 F, double c, double *dE);
+int kfsd_device(sd_ctx *ctx, const double *dQ, const i64 *d_qidx, i64 nq, const double *dS, i64 nS, i64 F, double c,
+                const double *dE, double *d_r);
 // out-of-sample depth (oos.cu): pooled inputs, sample first, queries after it
 int band_depth_oos_device(sd_ctx *ctx, const double *dX, i64 T, i64 nS, i64 nY, i64 ld, int j, int relax,
                           i64 *d_out);

@@ -19,6 +19,7 @@ from ._outliers import (NO_FACTOR, _check_central, _check_extremal_rows, _checke
 from ._pointcloud import _pointwisedepth, _pointwisedepth_of, _samplepointwisedepth
 from ._projection import KINDS, _functional_projection, _pointcloud_projection, draw_directions
 from ._reference import _checked_reference, _curve_values, _ProjectedReference, _query_values, _SortedReference
+from ._kfsd import _functional_kfsd, _functional_kfsd_of, _KfsdReference
 from ._modal import DEFAULT_QUANTILE, _checked_bandwidth, _functional_modal, _functional_modal_of, _ModalReference
 from ._spatial import _functional_spatial, _functional_spatial_of, _spatial_curves, _SpatialReference
 
@@ -471,15 +472,15 @@ def Outliergram(data: List[pd.DataFrame], factor=1.5, deep_check=False) -> _Outl
 # fitted references and depth-based classification (driver in _reference.py)
 # ---------------------------------------------------------------------------------------------------------------
 def _check_reference_depth(depth, J, directions, quantile=DEFAULT_QUANTILE, bandwidth=None):
-    if not (isinstance(depth, str) and depth in ('mbd', 'spatial', 'modal') + KINDS):
-        raise ValueError("depth must be 'mbd', 'projection', 'tukey', 'spatial' or 'modal' (got %r)" % (depth,))
-    if depth in ('mbd', 'spatial', 'modal') and directions is not None:
+    if not (isinstance(depth, str) and depth in ('mbd', 'spatial', 'modal', 'kfsd') + KINDS):
+        raise ValueError("depth must be 'mbd', 'projection', 'tukey', 'spatial', 'modal' or 'kfsd' (got %r)" % (depth,))
+    if depth in ('mbd', 'spatial', 'modal', 'kfsd') and directions is not None:
         raise ValueError("directions apply to depth='projection' or 'tukey'")
     if depth != 'mbd' and J != 2:
         raise ValueError('J applies to depth=\'mbd\' only: leave it at 2 for depth=%r' % depth)
-    if depth != 'modal' and (quantile != DEFAULT_QUANTILE or bandwidth is not None):
-        raise ValueError("quantile and bandwidth apply to depth='modal' only")
-    if depth == 'modal':
+    if depth not in ('modal', 'kfsd') and (quantile != DEFAULT_QUANTILE or bandwidth is not None):
+        raise ValueError("quantile and bandwidth apply to depth='modal' or 'kfsd' only")
+    if depth in ('modal', 'kfsd'):
         _checked_bandwidth(quantile, bandwidth)
 
 
@@ -506,7 +507,13 @@ class FunctionalReference:
     depth='modal' (J must stay 2, directions None): the same forms of sample as 'spatial', kept on the GPU the same way.
     Construction fixes the bandwidth once (.bandwidth): the given bandwidth, else the quantile of the sample's own
     pair distances.  A new curve g gets the depth FunctionalModalDepth(sample + [g], bandwidth=.bandwidth) gives it,
-    bit for bit.  quantile and bandwidth apply to depth='modal' only; .bandwidth is None for the other kinds.
+    bit for bit.
+
+    depth='kfsd' (J must stay 2, directions None): the same forms of sample, kept on the GPU the same way, with its
+    bandwidth fixed at construction as for 'modal' and the sample's n_S x n_S kernel matrix kept on the GPU as well
+    (8 n_S^2 bytes; n_S at most 32 768).  A new curve g gets the depth FunctionalKernelSpatialDepth(sample + [g],
+    bandwidth=.bandwidth) gives it, bit for bit.  quantile and bandwidth apply to depth='modal' and 'kfsd' only;
+    .bandwidth is None for the other kinds.
 
     Non-finite values (and, for the projection kinds, projections that overflow) are rejected.  close() (or leaving a
     `with` block) frees the index."""
@@ -524,7 +531,7 @@ class FunctionalReference:
             self._index = sample[0].index
             self._ref = _SortedReference(_values(sample[0]), J)
             return
-        if depth in ('spatial', 'modal'):
+        if depth in ('spatial', 'modal', 'kfsd'):
             X, F = _spatial_curves(sample)
             self._T = sample[0].shape[0]
             self._index = sample[0].index
@@ -532,7 +539,8 @@ class FunctionalReference:
             if depth == 'spatial':
                 self._ref = _SpatialReference(X=X, F=F)
             else:
-                self._ref = _ModalReference(X=X, F=F, quantile=quantile, bandwidth=bandwidth)
+                kind = _ModalReference if depth == 'modal' else _KfsdReference
+                self._ref = kind(X=X, F=F, quantile=quantile, bandwidth=bandwidth)
                 self.bandwidth = self._ref.bandwidth
             return
         X, F = _curve_values(sample, directions)
@@ -547,8 +555,8 @@ class FunctionalReference:
 
     def depth_of(self, data: List[pd.DataFrame], deep_check=False) -> _FunctionalDepthSeries:
         """Depth of every new curve against the reference.  Univariate: the columns of data[0], indexed by
-        data[0].columns (a label may repeat a sample label).  Multivariate (projection kinds, spatial, modal): M DataFrames of
-        T x d, indexed by list position, as FunctionalProjectionDepth."""
+        data[0].columns (a label may repeat a sample label).  Multivariate (projection kinds, spatial, modal, kfsd): M
+        DataFrames of T x d, indexed by list position, as FunctionalProjectionDepth."""
         if self._ref is None:
             raise ValueError('the reference is closed')
         if self.depth == 'mbd':
@@ -591,7 +599,7 @@ class DepthClassifier:
     d and seed (or given), is shared by all classes (.directions), so that the DD-plot coordinates are comparable.
     depth='spatial': the same forms of data as the projection kinds, without directions.  depth='modal': the same forms;
     each class selects its own bandwidth at quantile from its own pair distances unless bandwidth is given for all
-    (.bandwidths maps each label to the bandwidth in use; None for the other kinds).
+    (.bandwidths maps each label to the bandwidth in use; None for the other kinds).  depth='kfsd': as 'modal'.
     predict(data) takes the class of largest depth, ties going to the class listed first."""
 
     def __init__(self, references: dict, J=2, deep_check=False, depth='mbd', directions=None, seed=0,
@@ -626,7 +634,7 @@ class DepthClassifier:
             self.close()
             raise
         self.bandwidths = ({label: ref.bandwidth for label, ref in zip(self.labels, self._refs)}
-                           if depth == 'modal' else None)
+                           if depth in ('modal', 'kfsd') else None)
 
     def depths(self, data: List[pd.DataFrame], deep_check=False) -> pd.DataFrame:
         """Depth of every new curve in every class: one column per class label, rows indexed as
@@ -757,6 +765,47 @@ def FunctionalModalDepthOf(data: List[pd.DataFrame], sample: List[pd.DataFrame],
     against one sample, keep a FunctionalReference(sample, depth='modal'): it keeps the sample on the GPU and selects
     the bandwidth once (.bandwidth)."""
     depth = _functional_modal_of(data, sample, quantile, bandwidth)
+    if len(sample) == 1:
+        return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+    return _FunctionalDepthSeries(df=data[0], depths=depth)
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# kernelized functional spatial depth (driver in _kfsd.py)
+# ---------------------------------------------------------------------------------------------------------------
+def FunctionalKernelSpatialDepth(data: List[pd.DataFrame], to_compute=None, quantile=DEFAULT_QUANTILE,
+                                 bandwidth=None) -> Union[_FunctionalDepthSeries, _FunctionalDepthUnivariate]:
+    """Kernelized functional spatial depth (KFSD; Sguera, Galeano & Lillo 2014): functional spatial depth after the
+    feature map phi of the Gaussian kernel k(x, y) = exp(-||x - y||^2 / sigma^2), a curve being the vector of its T d
+    values (Euclidean norm over all values, (t, c) order, no time weight, channels as given):
+    KFSD(x) = 1 - || sum_j (phi(x) - phi(x_j)) / ||phi(x) - phi(x_j)|| || / n, duplicates of x contributing nothing
+    and n counting x.  Spatial depth is global: a curve in a sparse gap between two clusters stays deep.  KFSD is
+    local: such a curve gets a low depth, which suits classification and outlier detection.
+
+    sigma is np.quantile of the n (n - 1) / 2 pair distances at quantile (0.15 by default), selected exactly as
+    FunctionalModalDepth selects its bandwidth (the same bits for the same sample); or bandwidth, used as given
+    (finite, > 0; quantile must then stay at its default).  ValueError when the selected sigma is 0 (pass
+    bandwidth=), for one curve without a bandwidth, and for more than 32 768 curves (the GPU keeps the n x n kernel
+    matrix).
+
+    `[df]` (T rows x n curve columns) is the univariate case, to_compute are column labels; a list of N DataFrames
+    (T rows x d channels, any d) the multivariate one, to_compute are list positions.  Non-finite values are
+    rejected, and so (EngineError, SD_ERR_OVERFLOW) are curves whose squared distance overflows float64."""
+    depth = _functional_kfsd(data, to_compute, quantile, bandwidth)
+    if len(data) == 1:
+        return _FunctionalDepthUnivariate(df=data[0], depths=depth)
+    return _FunctionalDepthSeries(df=data[0], depths=depth)
+
+
+def FunctionalKernelSpatialDepthOf(data: List[pd.DataFrame], sample: List[pd.DataFrame], quantile=DEFAULT_QUANTILE,
+                                   bandwidth=None) -> Union[_FunctionalDepthSeries, _FunctionalDepthUnivariate]:
+    """Out-of-sample KFSD: sigma comes from sample alone (its pair distances at quantile, or bandwidth as given) and a
+    new curve never moves it; each new curve g then gets what FunctionalKernelSpatialDepth(sample + [g],
+    bandwidth=sigma) gives it (divisor n_S + 1), bit for bit.  Univariate [df] (T x n, indexed by data[0].columns) or
+    lists of T x d DataFrames (indexed by list position); sample holds at most 32 768 curves.  To score many batches
+    against one sample, keep a FunctionalReference(sample, depth='kfsd'): it keeps the sample and its kernel matrix
+    on the GPU and selects sigma once (.bandwidth)."""
+    depth = _functional_kfsd_of(data, sample, quantile, bandwidth)
     if len(sample) == 1:
         return _FunctionalDepthUnivariate(df=data[0], depths=depth)
     return _FunctionalDepthSeries(df=data[0], depths=depth)
